@@ -81,6 +81,23 @@ def pinned(arr):
 
 _PINNED_KEEPALIVE = []
 
+DUMP_BYTES = 64 * 10 ** 6         # --dump-outputs: at most this much data in all
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: writes the per-game arrays a caller of the timed path received in its last step as <path>/<name>.npy
+    in float64 (exact for their integer values), and <path>/game_index.npy, the games (rows) written.  A result larger than
+    DUMP_BYTES is cut to a fixed, seeded sample of games, so that two builds run with the same arguments write the same rows."""
+    import numpy as np
+    games = len(next(iter(arrays.values())))
+    row_bytes = 8 * (1 + sum(a[0].size for a in arrays.values()))
+    keep = np.arange(games)
+    if games * row_bytes > DUMP_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(games, (DUMP_BYTES - 1024 * (len(arrays) + 1)) // row_bytes, replace=False))
+    os.makedirs(path, exist_ok=True)
+    for name, a in dict({k: a[keep] for k, a in arrays.items()}, game_index=keep).items():
+        np.save(os.path.join(path, name + ".npy"), a.astype(np.float64))
+
 
 def ncu_traffic(summary=None):
     """DRAM bytes (read + write) per launch of the dominant kernel, from the committed `ncu --set full` summary."""
@@ -331,6 +348,8 @@ def run_ours(args):
     wall_s = rank_max(wall_s)
     e2e_s = rank_max(e2e_s)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"actions": acts, "visit_counts": counts, "child_ids": ids, "n_children": ncs})
     h2d = G * 16
     d2h = G * (2 * 4 * S.MAX_ACTIONS + 4 + S.MAX_ACTIONS)
     assert int(counts[0].sum()) == sims - (K if K > 1 else 1)
@@ -575,6 +594,8 @@ def run_chess(args):
     dev_ms = rank_max(dev_ms)
     e2e_s = rank_max(e2e_s)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"moves": mv, "visit_counts": cnt, "child_ids": ids, "n_children": ncs})
     assert int(cnt[0].sum()) == sims - 1
     peak_tf, peak_hbm, peak_src = _peaks()
     conv_ms, conv_n, conv_flops, flops_pos = eng.time_conv(iters=20)
@@ -644,7 +665,12 @@ def main():
     ap.add_argument("--game", default="c4", choices=["c4", "ttt", "chess"], help="configs[0] is tic-tac-toe, configs[4] chess")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--full-game-moves", type=int, default=4, help="extra leg: self-play moves with subtree reuse (0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the root children of every game (rank 0's games under --gpus > 1) that the last "
+                         "step returned as DIR/<name>.npy (float64, at most 64 MB: a seeded sample of games beyond that)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU arm's results; the reference arm runs in worker processes and returns none")
     if args.games is None:
         args.games = CHESS_GAMES_PER_GPU if args.game == "chess" else GAMES_PER_GPU
     if args.sims is None:
