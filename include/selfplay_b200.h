@@ -366,6 +366,52 @@ int32_t spb_chess_time_conv(spb_chess_engine* e, uint32_t iters, float* avg_ms, 
 int32_t spb_chess_get_counters(spb_chess_engine* e, spb_counters* out);   /* reserved[0] = largest arena */
 int32_t spb_chess_reset_counters(spb_chess_engine* e);
 
+/* ---- chess self-play driver (ref: SelfPlayWorker::self_play learner_concurrent.rs:169-242, over chess::State) --------------
+ * The contract of spb_selfplay_step / spb_drain_trajectories for chess trees.  spb_config.game_id_base, game_id_stride and
+ * trajectory_capacity take effect as for the Connect4 engine (capacity 0 = 4 * num_games * SPB_CHESS_MAX_HISTORY records, at
+ * most 2^26; never less than one whole game, SPB_CHESS_MAX_HISTORY records).  The device buffers of the trajectories are
+ * allocated by the first spb_chess_selfplay_step (SPB_CHESS_MAX_HISTORY records per slot plus the output buffer, 1,624 bytes a
+ * record); an engine that never plays keeps its search footprint.  Outcomes follow the value the chess search uses (chess.rs:172:
+ * Won = +1.0 for the side to move in the terminal state, i.e. the CHECKMATED side), signed per position by
+ * learner_concurrent.rs:214-226: every position of the mated side gets +1, of the mating side -1 (DESIGN.md §7).
+ * A game whose next position would pass SPB_CHESS_MAX_HISTORY plies of history or SPB_CHESS_MAX_HISTORY records ends as a
+ * tie with SPB_CHESS_POS_ADJUDICATED set on every record (the reference has no such cap).
+ */
+#define SPB_CHESS_POS_ADJUDICATED 1u   /* spb_chess_position.flags: the game was ended as a tie at the history cap */
+
+typedef struct spb_chess_position {
+  spb_chess_state state;                            /* root the search ran from; hist_len as at that root */
+  uint32_t visit_counts[SPB_CHESS_MAX_MOVES];       /* root children in child order; 0 past n_moves */
+  uint16_t moves[SPB_CHESS_MAX_MOVES];              /* their moves; 0xFFFF past n_moves */
+  uint16_t n_moves;
+  uint16_t ply;                                     /* index of this position inside its trajectory */
+  uint8_t  repetitions;                             /* get_num_repetitions of the root (chess.rs:51-62), encoding plane 16 */
+  int8_t   outcome;                                 /* value target: +1 / 0 / -1 from this position's side to move */
+  uint8_t  flags;                                   /* SPB_CHESS_POS_* */
+  uint8_t  reserved;
+} spb_chess_position;                               /* 1,624 bytes */
+
+/*
+ * One self-play ply for every live slot on the device: pick a root child by `rule` (SPB_MOVE_*; temperature: sample
+ * ∝ N^temperature with the counter-based RNG keyed by (seed, game id, ply)), record the root, then end the game (terminal
+ * child or history cap: emit the trajectory; restart the slot from restart_roots[slot] / restart_history[slot] when
+ * restart_roots != NULL — the rules of spb_chess_reset_games, arrays of num_games entries — else leave it idle) or re-root
+ * (use_subtree, exactly as spb_chess_advance).  n_finished (nullable): games emitted by this call.  A full output buffer
+ * parks the game's slot with its history and the call returns SPB_ERR_STATE; nothing is lost: drain and call again.
+ */
+int32_t spb_chess_selfplay_step(spb_chess_engine* e, int32_t rule, float temperature, uint64_t seed, const spb_chess_state* restart_roots,
+                                const uint64_t* restart_history, uint32_t* n_finished);
+/* Copies the finished positions (ordered by game id, then ply) to buf; buf == NULL: *written = the number held. */
+int32_t spb_chess_drain_trajectories(spb_chess_engine* e, spb_chess_position* buf, size_t capacity, size_t* written,
+                                     uint64_t* game_ids /* nullable, [capacity] */);
+/*
+ * The training tensors of n records (host only, no GPU needed), each output nullable: encodings[n][19][8][8] (get_encoding of
+ * the recorded root with its recorded repetitions, chess.rs:176-249), policies[n][4672] (visit counts scattered by the policy
+ * index of each move and divided by their f32 sum: what spb_chess_root_policy returned for that root), values[n] (outcome).
+ * SPB_ERR_ARG for a malformed record (n_moves outside 1..256, side > 1, a move outside the policy).
+ */
+int32_t spb_chess_positions_to_training(const spb_chess_position* positions, size_t n, float* encodings, float* policies, float* values);
+
 /* ---- multi-GPU: trajectories to the learner rank; learner hand-off ------- */
 
 /*

@@ -20,6 +20,7 @@ pub const SPB_CHESS_MAX_HISTORY: usize = 512;
 pub const SPB_CHESS_PLANES: usize = 19;
 pub const SPB_CHESS_POLICY_SIZE: usize = 4672;
 pub const SPB_CHESS_NO_SQUARE: u8 = 64;
+pub const SPB_CHESS_POS_ADJUDICATED: u8 = 1;
 pub const SPB_COMM_ID_BYTES: usize = 128;
 pub const SPB_MAX_ACTIONS: usize = 9;
 pub const SPB_STATUS_ONGOING: u8 = 0;
@@ -104,6 +105,20 @@ pub struct spb_chess_state {
 }
 
 #[repr(C)]
+#[derive(Clone, Copy, Debug)]
+pub struct spb_chess_position {
+    pub state: spb_chess_state,
+    pub visit_counts: [u32; SPB_CHESS_MAX_MOVES],
+    pub moves: [u16; SPB_CHESS_MAX_MOVES],
+    pub n_moves: u16,
+    pub ply: u16,
+    pub repetitions: u8,
+    pub outcome: i8,
+    pub flags: u8,
+    pub reserved: u8,
+}
+
+#[repr(C)]
 pub struct spb_engine {
     _private: [u8; 0],
 }
@@ -163,6 +178,9 @@ extern "C" {
     pub fn spb_chess_time_conv(e: *mut spb_chess_engine, iters: u32, avg_ms: *mut f32, n_positions: *mut u32, flops_per_launch: *mut f64, flops_per_position: *mut f64) -> i32;
     pub fn spb_chess_get_counters(e: *mut spb_chess_engine, out: *mut spb_counters) -> i32;
     pub fn spb_chess_reset_counters(e: *mut spb_chess_engine) -> i32;
+    pub fn spb_chess_selfplay_step(e: *mut spb_chess_engine, rule: i32, temperature: f32, seed: u64, restart_roots: *const spb_chess_state, restart_history: *const u64, n_finished: *mut u32) -> i32;
+    pub fn spb_chess_drain_trajectories(e: *mut spb_chess_engine, buf: *mut spb_chess_position, capacity: usize, written: *mut usize, game_ids: *mut u64) -> i32;
+    pub fn spb_chess_positions_to_training(positions: *const spb_chess_position, n: usize, encodings: *mut f32, policies: *mut f32, values: *mut f32) -> i32;
     pub fn spb_comm_unique_id(id: *mut u8) -> i32;
     pub fn spb_comm_init(e: *mut spb_engine, id: *const u8, rank: i32, world_size: i32) -> i32;
     pub fn spb_comm_destroy(e: *mut spb_engine) -> i32;

@@ -339,6 +339,47 @@ impl ChessMcts {
         self.check(unsafe { sys::spb_chess_get_counters(self.raw, &mut c) })?;
         Ok(c)
     }
+    /// One self-play ply for every live chess game on the device (ref: learner_concurrent.rs:179-238): pick the move, record
+    /// the root, `use_subtree` or finish the game; finished slots restart from `restart_roots` (one (state, history) per slot)
+    /// or retire.  Returns the number of games that finished.  `Err` with `SPB_ERR_STATE`: the trajectory buffer is full —
+    /// drain and call again, nothing is lost.
+    pub fn self_play_step(&mut self, rule: MoveRule, restart_roots: Option<&[(ChessState, Vec<u64>)]>) -> Result<u32> {
+        let (r, t, seed) = match rule {
+            MoveRule::GreedyLastMax => (sys::SPB_MOVE_GREEDY_LAST_MAX, 0.0f32, 0u64),
+            MoveRule::Temperature { temperature, seed } => (sys::SPB_MOVE_TEMPERATURE, temperature, seed),
+        };
+        let roots: Option<Vec<ChessState>> = restart_roots.map(|v| v.iter().map(|s| s.0).collect());
+        let hist: Option<Vec<u64>> = restart_roots.map(|v| v.iter().flat_map(|s| Self::padded_history(&s.1)).collect());
+        let p = roots.as_ref().map_or(std::ptr::null(), |v| v.as_ptr());
+        let h = hist.as_ref().map_or(std::ptr::null(), |v| v.as_ptr());
+        let mut finished = 0u32;
+        self.check(unsafe { sys::spb_chess_selfplay_step(self.raw, r, t, seed, p, h, &mut finished) })?;
+        Ok(finished)
+    }
+    /// Finished games' positions ordered by (game id, ply) with their global game ids (ref: learner_concurrent.rs:202-228).
+    pub fn drain_trajectories(&mut self) -> Result<(Vec<ChessPosition>, Vec<u64>)> {
+        let mut n = 0usize;
+        self.check(unsafe { sys::spb_chess_drain_trajectories(self.raw, std::ptr::null_mut(), 0, &mut n, std::ptr::null_mut()) })?;
+        // a record is plain integers: all-zero bytes are a valid value
+        let mut pos: Vec<ChessPosition> = vec![unsafe { std::mem::zeroed() }; n];
+        let mut ids = vec![0u64; n];
+        if n > 0 {
+            self.check(unsafe { sys::spb_chess_drain_trajectories(self.raw, pos.as_mut_ptr(), n, &mut n, ids.as_mut_ptr()) })?;
+            pos.truncate(n); ids.truncate(n);
+        }
+        Ok((pos, ids))
+    }
+}
+
+pub type ChessPosition = sys::spb_chess_position;
+
+/// Chess self-play records to the training tensors `[n][19][8][8]` / `[n][4672]` / `[n]` (host only): the encoding of the
+/// recorded root, its visit counts / their sum at each move's policy index, the outcome.
+pub fn chess_positions_to_training(positions: &[ChessPosition]) -> Result<TrainingBatch> {
+    let n = positions.len();
+    let mut b = TrainingBatch { n, encodings: vec![0f32; n * sys::SPB_CHESS_PLANES * 64], policies: vec![0f32; n * sys::SPB_CHESS_POLICY_SIZE], values: vec![0f32; n] };
+    let rc = unsafe { sys::spb_chess_positions_to_training(positions.as_ptr(), n, b.encodings.as_mut_ptr(), b.policies.as_mut_ptr(), b.values.as_mut_ptr()) };
+    if rc == sys::SPB_OK { Ok(b) } else { Err(Error { code: rc, message: "spb_chess_positions_to_training: bad argument".to_string() }) }
 }
 
 /// `State::default()` chess.rs:94-102.

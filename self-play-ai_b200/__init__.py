@@ -11,4 +11,4 @@ from .engine import (  # noqa: F401
 )
 from .mcts import Args, Mcts, Tree  # noqa: F401
 from . import chess  # noqa: F401
-from .chess import ChessEngine, CHESS_STATE_DTYPE  # noqa: F401
+from .chess import ChessEngine, CHESS_STATE_DTYPE, CHESS_POSITION_DTYPE  # noqa: F401

@@ -20,6 +20,12 @@ MOVE_NONE = 0xFFFF
 CHESS_STATE_DTYPE = np.dtype([("piece", "<u8", (6,)), ("color", "<u8", (2,)), ("side", "u1"), ("castle", "u1"), ("ep", "u1"),
                               ("reserved0", "u1"), ("fifty", "<u2"), ("plies", "<u2"), ("hist_len", "<u4"), ("reserved1", "<u4")])
 assert CHESS_STATE_DTYPE.itemsize == 80
+# spb_chess_position: one searched root of a self-play trajectory (compact form of `Payload`, learner_concurrent.rs:13-18)
+CHESS_POSITION_DTYPE = np.dtype([("state", CHESS_STATE_DTYPE), ("visit_counts", "<u4", (MAX_MOVES,)), ("moves", "<u2", (MAX_MOVES,)),
+                                 ("n_moves", "<u2"), ("ply", "<u2"), ("repetitions", "u1"), ("outcome", "i1"), ("flags", "u1"),
+                                 ("reserved", "u1")])
+assert CHESS_POSITION_DTYPE.itemsize == 1624
+POS_ADJUDICATED = 1          # CHESS_POSITION_DTYPE["flags"]: the game was ended as a tie at the history cap
 
 
 def start_position() -> np.ndarray:
@@ -60,12 +66,14 @@ class ChessEngine:
     """The chess engine: `Mcts<chess Net>` + its trees on one GPU (ref: src/mcts.rs:41-44 over src/game/chess.rs and
     src/model/chess.rs) — batched `State` methods, search, re-rooting, `Model::predict`."""
 
-    def __init__(self, num_games=64, evaluator=E.EVAL_NET, c=2.0, device=0, max_nodes_per_tree=0, flags=0):
+    def __init__(self, num_games=64, evaluator=E.EVAL_NET, c=2.0, device=0, max_nodes_per_tree=0, flags=0, trajectory_capacity=0,
+                 game_id_base=0, game_id_stride=0):
         L = E.load_library()
         cfg = E.Config()
         L.spb_default_config(C.byref(cfg))
         cfg.game, cfg.num_games, cfg.evaluator, cfg.c, cfg.device = E.GAME_CHESS, num_games, evaluator, c, device
         cfg.max_nodes_per_tree, cfg.flags, cfg.leaves_per_tree = max_nodes_per_tree, flags, 1
+        cfg.trajectory_capacity, cfg.game_id_base, cfg.game_id_stride = trajectory_capacity, game_id_base, game_id_stride
         h = C.c_void_p()
         rc = L.spb_chess_create(C.byref(cfg), C.byref(h))
         if rc != 0:
@@ -200,6 +208,30 @@ class ChessEngine:
         self._chk(self._L.spb_chess_advance(self._h, None if sl is None else sl.ctypes.data, ids.ctypes.data, len(ids), out.ctypes.data))
         return out
 
+    # ---- self-play (ref: SelfPlayWorker::self_play, learner_concurrent.rs:169-242) --------------------------------------
+    def selfplay_step(self, rule=E.MOVE_GREEDY_LAST_MAX, temperature=1.25, seed=0, restart_roots=None, restart_history=None) -> int:
+        """One ply for every live slot on the device -> number of games finished (emitted) by this call.  restart_roots /
+        restart_history: num_games entries, as for reset_games.  A full trajectory buffer raises EngineError(-6): drain and
+        call again, nothing is lost."""
+        st = None if restart_roots is None else _states(restart_roots)
+        h = None if restart_history is None else _history(restart_history, self.G)
+        if st is not None:
+            assert len(st) == self.G
+        fin = C.c_uint32()
+        self._chk(self._L.spb_chess_selfplay_step(self._h, rule, temperature, seed, None if st is None else st.ctypes.data,
+                                                  None if h is None else h.ctypes.data, C.byref(fin)))
+        return fin.value
+
+    def drain_trajectories(self):
+        """-> (positions[CHESS_POSITION_DTYPE], game_ids[u64]) ordered by (game id, ply)."""
+        n = C.c_size_t()
+        self._chk(self._L.spb_chess_drain_trajectories(self._h, None, 0, C.byref(n), None))
+        pos = np.zeros(n.value, dtype=CHESS_POSITION_DTYPE)
+        ids = np.zeros(n.value, dtype=np.uint64)
+        if n.value:
+            self._chk(self._L.spb_chess_drain_trajectories(self._h, pos.ctypes.data, n.value, C.byref(n), ids.ctypes.data))
+        return pos[:n.value], ids[:n.value]
+
     def get_state(self, slot: int, node_id: int) -> np.ndarray:
         out = np.zeros(1, CHESS_STATE_DTYPE)
         self._chk(self._L.spb_chess_get_state(self._h, slot, node_id, out.ctypes.data))
@@ -235,6 +267,21 @@ class ChessEngine:
 
     def reset_counters(self):
         self._chk(self._L.spb_chess_reset_counters(self._h))
+
+
+def positions_to_training(positions):
+    """spb_chess_positions_to_training (host only): -> (encodings[n,19,8,8], policies[n,4672], values[n,1]) f32, the training
+    tensors of chess self-play records."""
+    L = E.load_library()
+    pos = np.ascontiguousarray(positions, dtype=CHESS_POSITION_DTYPE).reshape(-1)
+    n = len(pos)
+    enc = np.zeros((n, PLANES, 8, 8), np.float32)
+    pol = np.zeros((n, POLICY_SIZE), np.float32)
+    val = np.zeros((n, 1), np.float32)
+    rc = L.spb_chess_positions_to_training(pos.ctypes.data, n, enc.ctypes.data, pol.ctypes.data, val.ctypes.data)
+    if rc != 0:
+        raise E.EngineError(rc, "spb_chess_positions_to_training: bad argument")
+    return enc, pol, val
 
 
 def check_weights(blob: bytes):

@@ -141,6 +141,36 @@ uint16_t spb_chess_action(int32_t side, int32_t channel, int32_t row, int32_t co
   return ch::action(side & 1, channel, row, col);
 }
 
+// The training tensors of recorded roots (ref: learner_concurrent.rs:126-146 over chess::State; host only).  The policy is
+// computed exactly as spb_chess_root_policy computes it: f32 sum of the counts in child order, each count divided by it.
+int32_t spb_chess_positions_to_training(const spb_chess_position* positions, size_t n, float* encodings, float* policies, float* values) {
+  if (n && !positions) return SPB_ERR_ARG;
+  for (size_t i = 0; i < n; ++i) {                                     // validate everything before writing anything
+    const spb_chess_position& p = positions[i];
+    if (p.n_moves == 0 || p.n_moves > SPB_CHESS_MAX_MOVES || p.state.side > 1) return SPB_ERR_ARG;
+    for (uint32_t k = 0; k < p.n_moves; ++k) {
+      const int idx = ch::policy_index(p.state.side, p.moves[k]);
+      if (idx < 0 || idx >= SPB_CHESS_POLICY_SIZE) return SPB_ERR_ARG;
+    }
+  }
+  for (size_t i = 0; i < n; ++i) {
+    const spb_chess_position& p = positions[i];
+    if (encodings) {
+      float* o = encodings + i * (size_t)SPB_CHESS_PLANES * 64;
+      for (int t = 0; t < SPB_CHESS_PLANES * 64; ++t) o[t] = ch::encode_plane(p.state, p.repetitions, t / 64, (t / 8) % 8, t % 8);
+    }
+    if (policies) {
+      float* o = policies + i * (size_t)SPB_CHESS_POLICY_SIZE;
+      std::memset(o, 0, sizeof(float) * SPB_CHESS_POLICY_SIZE);
+      float sum = 0.0f;
+      for (uint32_t k = 0; k < p.n_moves; ++k) sum += (float)p.visit_counts[k];
+      for (uint32_t k = 0; k < p.n_moves; ++k) o[ch::policy_index(p.state.side, p.moves[k])] = (float)p.visit_counts[k] / sum;
+    }
+    if (values) values[i] = (float)p.outcome;
+  }
+  return SPB_OK;
+}
+
 int32_t spb_chess_legal_moves(spb_chess_engine* e, const spb_chess_state* states, const uint64_t* history, uint32_t n, uint16_t* moves,
                               uint32_t* counts, uint16_t* policy_index, uint8_t* status, uint32_t* repetitions) {
   CH_GUARD(e);

@@ -4,8 +4,10 @@
 //                                                   one warp) and, for the network, the lock-step pair k_chess_select ->
 //                                                   [chess_net.cu] -> k_chess_finish: exactly the reference's loop, one
 //                                                   evaluator batch per simulation step over all trees
-//   Tree::use_subtree (:161-192)                 -> k_chess_advance (breadth-first compaction into the other arena)
-//   Tree::with_root_state (:86-89)               -> k_chess_reset
+//   Tree::use_subtree (:161-192)                 -> reroot: k_chess_advance (breadth-first compaction into the other arena)
+//   Tree::with_root_state (:86-89)               -> restart_tree: k_chess_reset
+//   SelfPlayWorker::self_play
+//     (learner_concurrent.rs:169-242)            -> k_chess_selfplay_step (pick, record, end / re-root) + the drain
 #include "chess_engine.hpp"
 #include "chess_net.cuh"
 
@@ -16,17 +18,17 @@ constexpr int WARPS = 4;
 constexpr int THREADS = WARPS * 32;
 constexpr uint32_t SPLIT_MIN_TREES = 128;   // the network pipeline runs as two half-loops on two streams from 2 x this many trees on
 
-__global__ void k_chess_reset(CTrees T, const uint32_t* slots, const Pos* roots, const unsigned long long* hist, uint32_t n) {
-  const uint32_t i = blockIdx.x;
-  if (i >= n) return;
-  const uint32_t g = slots ? slots[i] : i;
-  Pos root = roots ? roots[i] : start_position();
+using ChessSelfPlay = Trajectories<spb_chess_position>;
+static_assert(sizeof(spb_chess_position) == 1624 && sizeof(spb_chess_position) % 8 == 0, "spb_chess_position layout");
+
+// Tree::with_root_state (mcts.rs:86-89) for slot g by threads t = 0..nt-1: the root, the game history that travels with it
+// (hist NULL: a game that starts at its root) and one unvisited root node.
+__device__ __forceinline__ void restart_tree(const CTrees& T, uint32_t g, Pos root, const unsigned long long* hist, uint32_t t, uint32_t nt) {
   if (!hist) root.hist_len = 0;
   if (root.hist_len > SPB_CHESS_MAX_HISTORY) root.hist_len = SPB_CHESS_MAX_HISTORY;
   if (hist)
-    for (uint32_t k = threadIdx.x; k < root.hist_len; k += blockDim.x)
-      T.root_hist[(size_t)g * SPB_CHESS_MAX_HISTORY + k] = hist[(size_t)i * SPB_CHESS_MAX_HISTORY + k];
-  if (threadIdx.x == 0) {
+    for (uint32_t k = t; k < root.hist_len; k += nt) T.root_hist[(size_t)g * SPB_CHESS_MAX_HISTORY + k] = hist[k];
+  if (t == 0) {
     T.root[g] = root;
     T.buf[g] = 0;
     T.live[g] = 1;
@@ -35,6 +37,18 @@ __global__ void k_chess_reset(CTrees T, const uint32_t* slots, const Pos* roots,
     T.rec[0][(size_t)g * T.cap] = make_uint4(0u, 0u, 0u, 0u);
     T.meta[0][(size_t)g * T.cap] = make_uint2(NO_PARENT, make_meta(MOVE_NONE, 0, ST_UNVISITED));
     T.hash[0][(size_t)g * T.cap] = 0ull;
+  }
+}
+
+// P.hist_len is null until the first self-play step; after it, a reset slot starts a new trajectory.
+__global__ void k_chess_reset(CTrees T, ChessSelfPlay P, const uint32_t* slots, const Pos* roots, const unsigned long long* hist, uint32_t n) {
+  const uint32_t i = blockIdx.x;
+  if (i >= n) return;
+  const uint32_t g = slots ? slots[i] : i;
+  restart_tree(T, g, roots ? roots[i] : start_position(), hist ? hist + (size_t)i * SPB_CHESS_MAX_HISTORY : nullptr, threadIdx.x, blockDim.x);
+  if (threadIdx.x == 0 && P.hist_len) {
+    P.hist_len[g] = 0;
+    P.parked[g] = 0;
   }
 }
 
@@ -284,13 +298,9 @@ __global__ void k_chess_root_children(CTrees T, uint16_t* moves, uint32_t* count
 // window of 32 copied nodes per round: a scan of their child counts gives each its new first_child, then the warp
 // copies the children of the 32 nodes one node after the other (lanes stride over up to 218 children).  A copied node
 // keeps its OLD first_child in rec.w until its own turn in the window.  The root position advances by the child's move
-// and the hash of the old root's move list joins the game history (chess.rs:121-122).
-__global__ void __launch_bounds__(THREADS) k_chess_advance(CTrees T, const uint32_t* slots, const uint32_t* node_ids, uint32_t n, Pos* out_states,
-                                                           int32_t* out_err) {
-  const int lane = threadIdx.x & 31;
-  const uint32_t i = blockIdx.x * WARPS + (threadIdx.x >> 5);
-  if (i >= n) return;
-  const uint32_t g = slots ? slots[i] : i;
+// and the hash of the old root's move list joins the game history (chess.rs:121-122).  The caller has checked that `id`
+// is a child of the root and that the history has room; lane 0 writes the new root to *out_state when it is not null.
+__device__ __forceinline__ void reroot(const CTrees& T, uint32_t g, uint32_t id, int lane, Pos* out_state) {
   const uint32_t b = T.buf[g], nb = b ^ 1u;
   const uint4* orec = T.rec[b] + (size_t)g * T.cap;
   const uint2* ometa = T.meta[b] + (size_t)g * T.cap;
@@ -298,24 +308,15 @@ __global__ void __launch_bounds__(THREADS) k_chess_advance(CTrees T, const uint3
   uint4* nrec = T.rec[nb] + (size_t)g * T.cap;
   uint2* nmeta = T.meta[nb] + (size_t)g * T.cap;
   unsigned long long* nhash = T.hash[nb] + (size_t)g * T.cap;
-  const uint32_t id = node_ids[i];
-  Pos root = T.root[g];
-  int32_t err = SPB_OK;
-  if (!T.live[g] || id == 0 || id >= T.n_nodes[g] || ometa[id].x != 0u) err = SPB_ERR_ARG;        // must be a child of the root
-  else if (root.hist_len >= SPB_CHESS_MAX_HISTORY) err = SPB_ERR_STATE;
-  if (err != SPB_OK) {
-    if (lane == 0) { out_err[i] = err; if (out_states) out_states[i] = root; }
-    return;
-  }
   const Move mv = (Move)meta_move(ometa[id].y);
   if (lane == 0) {
+    Pos root = T.root[g];
     T.root_hist[(size_t)g * SPB_CHESS_MAX_HISTORY + root.hist_len] = ohash[0];
     const uint32_t hl = root.hist_len + 1;
     root = apply_move(root, mv);
     root.hist_len = hl;
     T.root[g] = root;
-    if (out_states) out_states[i] = root;
-    out_err[i] = SPB_OK;
+    if (out_state) *out_state = root;
     nrec[0] = orec[id];
     nmeta[0] = make_uint2(NO_PARENT, ometa[id].y);
     nhash[0] = ohash[id];
@@ -353,6 +354,183 @@ __global__ void __launch_bounds__(THREADS) k_chess_advance(CTrees T, const uint3
     T.n_nodes[g] = n_new;
     T.buf[g] = (uint8_t)nb;
     T.leaf_depth[g] = 0;
+  }
+}
+
+__global__ void __launch_bounds__(THREADS) k_chess_advance(CTrees T, const uint32_t* slots, const uint32_t* node_ids, uint32_t n, Pos* out_states,
+                                                           int32_t* out_err) {
+  const int lane = threadIdx.x & 31;
+  const uint32_t i = blockIdx.x * WARPS + (threadIdx.x >> 5);
+  if (i >= n) return;
+  const uint32_t g = slots ? slots[i] : i;
+  const uint2* ometa = T.meta[T.buf[g]] + (size_t)g * T.cap;
+  const uint32_t id = node_ids[i];
+  int32_t err = SPB_OK;
+  if (!T.live[g] || id == 0 || id >= T.n_nodes[g] || ometa[id].x != 0u) err = SPB_ERR_ARG;        // must be a child of the root
+  else if (T.root[g].hist_len >= SPB_CHESS_MAX_HISTORY) err = SPB_ERR_STATE;
+  if (err != SPB_OK) {
+    if (lane == 0) { out_err[i] = err; if (out_states) out_states[i] = T.root[g]; }
+    return;
+  }
+  if (lane == 0) out_err[i] = SPB_OK;
+  reroot(T, g, id, lane, out_states ? out_states + i : nullptr);
+}
+
+// ---- self-play ply (ref: learner_concurrent.rs:179-238) ------------------------------------------------------------
+// Emits the finished game of slot g (learner_concurrent.rs:200-230) and restarts or retires the slot.  pk: how the game
+// ended, as stored in P.parked.  The outcome is the value of the terminal state (chess.rs:172: +1 when its side to move is
+// checkmated, 0 for a tie) for positions with that side to move, its negation for the others (:214-226).
+__device__ __forceinline__ void emit_game(const CTrees& T, const ChessSelfPlay& P, uint32_t g, uint32_t plies, uint32_t pk, unsigned long long base,
+                                          const Pos* restart_roots, const unsigned long long* restart_hist, int lane) {
+  const int value = ((pk >> 1) & 1u) ? 1 : 0;
+  const uint32_t term_side = (pk >> 2) & 1u;
+  const uint8_t flags = ((pk >> 3) & 1u) ? (uint8_t)SPB_CHESS_POS_ADJUDICATED : (uint8_t)0;
+  spb_chess_position* hist = P.hist + (size_t)g * P.max_ply;
+  SPB_ASSERT(T.error, base + plies <= P.out_cap && plies <= P.max_ply, 44);
+  for (uint32_t i = lane; i < plies; i += 32) {
+    hist[i].outcome = (int8_t)(hist[i].state.side == term_side ? value : -value);
+    hist[i].flags = flags;
+  }
+  __syncwarp();
+  constexpr uint32_t WORDS = sizeof(spb_chess_position) / 8;          // records copied as 8-byte words by the whole warp
+  const unsigned long long* src = reinterpret_cast<const unsigned long long*>(hist);
+  unsigned long long* dst = reinterpret_cast<unsigned long long*>(P.out + base);
+  for (uint32_t k = lane; k < plies * WORDS; k += 32) dst[k] = src[k];
+  const unsigned long long id = P.game_id[g];
+  for (uint32_t i = lane; i < plies; i += 32) P.out_game[base + i] = id;
+  __syncwarp();
+  if (lane == 0) finish_trajectory(P, g);
+  if (restart_roots)
+    restart_tree(T, g, restart_roots[g], restart_hist ? restart_hist + (size_t)g * SPB_CHESS_MAX_HISTORY : nullptr, (uint32_t)lane, 32u);
+  else if (lane == 0)
+    T.live[g] = 0;                                                    // trees_vec.remove(i), :230
+}
+
+// One warp per slot: pick a root child (greedy last-max or ∝ N^temperature), record the root in the slot's history, then end
+// the game (terminal child, or the history cap) or re-root at the child.
+__global__ void __launch_bounds__(THREADS) k_chess_selfplay_step(CTrees T, ChessSelfPlay P, int rule, float temperature, unsigned long long seed,
+                                                                 const Pos* restart_roots, const unsigned long long* restart_hist) {
+  __shared__ WarpScratch s_ws[WARPS];
+  const int lane = threadIdx.x & 31;
+  WarpScratch& ws = s_ws[threadIdx.x >> 5];
+  const uint32_t g = blockIdx.x * WARPS + (threadIdx.x >> 5);
+  if (g >= T.G) return;
+  const uint32_t parked = P.parked[g];
+  if (parked) {
+    // A game that ended in an earlier call while the output buffer was full: the slot has been idle since; emit now.
+    const uint32_t plies = P.hist_len[g];
+    unsigned long long base;
+    if (reserve_output(P, plies, lane, &base)) emit_game(T, P, g, plies, parked, base, restart_roots, restart_hist, lane);
+    else if (lane == 0) atomicOr(T.error, (uint32_t)ERRBIT_TRAJ_FULL);
+    return;
+  }
+  if (!T.live[g]) return;
+  const uint32_t b = T.buf[g];
+  const uint4* rec = T.rec[b] + (size_t)g * T.cap;
+  const uint2* meta = T.meta[b] + (size_t)g * T.cap;
+  const unsigned long long* hash = T.hash[b] + (size_t)g * T.cap;
+  const uint32_t y0 = meta[0].y;
+  if (meta_status(y0) != ST_EXPANDED) return;                         // nothing searched yet / terminal root
+  const uint32_t nc = meta_nc(y0), fc = rec[0].w;
+  const Pos root = T.root[g];
+  const uint32_t ply = P.hist_len[g];
+  int chosen;
+  if (rule == SPB_MOVE_TEMPERATURE) {
+    // learner_concurrent.rs:189-194: WeightedIndex over count^temperature, as k_selfplay_step draws it: an inclusive scan
+    // of the weights in child order (lanes stride over the children, 32 per round, with a carry across rounds), the ball
+    // u = U[0,1) * total, the first child whose prefix sum exceeds u.  The counter behind U is (seed, game id, ply).
+    constexpr int ROUNDS = MAX_MOVES / 32;
+    float incl[ROUNDS];
+    uint32_t positive = 0;
+    float carry = 0.0f;
+#pragma unroll
+    for (int r = 0; r < ROUNDS; ++r) {
+      incl[r] = carry;
+      if ((uint32_t)r * 32u < nc) {
+        const uint32_t i = (uint32_t)r * 32u + (uint32_t)lane;
+        const float w = i < nc ? powf((float)rec[fc + i].x, temperature) : 0.0f;
+        float x = w;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+          const float t = __shfl_up_sync(0xffffffffu, x, o);
+          if (lane >= o) x += t;
+        }
+        incl[r] = carry + x;
+        if (w > 0.0f) positive |= 1u << r;
+        carry = __shfl_sync(0xffffffffu, incl[r], 31);
+      }
+    }
+    const unsigned long long h = mix64(seed ^ mix64((P.game_id[g] << 9) + ply));   // ply < 512 = P.max_ply
+    const float u = (float)(h >> 40) * (1.0f / 16777216.0f) * carry;
+    chosen = (int)nc - 1;
+    bool found = false;
+#pragma unroll
+    for (int r = 0; r < ROUNDS; ++r) {
+      const uint32_t i = (uint32_t)r * 32u + (uint32_t)lane;
+      const unsigned ball = __ballot_sync(0xffffffffu, i < nc && u < incl[r] && ((positive >> r) & 1u));
+      if (ball && !found) { chosen = r * 32 + __ffs((int)ball) - 1; found = true; }
+    }
+  } else {
+    // main.rs:108-112: max_by(total_cmp) over visit counts -> the LAST maximal child
+    float best = -INFINITY;
+    int best_i = -1;
+    for (uint32_t i = lane; i < nc; i += 32) {
+      const float s = (float)rec[fc + i].x;
+      if (s >= best) { best = s; best_i = (int)i; }
+    }
+    chosen = warp_argmax_last32(best, best_i);
+  }
+  // learner_concurrent.rs:197-198: push the root and its visit counts (ply < P.max_ply: a game ends at P.max_ply records)
+  SPB_ASSERT(T.error, ply < P.max_ply, 45);
+  spb_chess_position* hr = P.hist + (size_t)g * P.max_ply + ply;
+  static_assert(sizeof(Pos) == 80, "spb_chess_state is copied as 10 words");
+  if (lane < 10) reinterpret_cast<unsigned long long*>(&hr->state)[lane] = reinterpret_cast<const unsigned long long*>(T.root + g)[lane];
+  for (uint32_t i = lane; i < MAX_MOVES; i += 32) {
+    const bool in = i < nc;
+    hr->visit_counts[i] = in ? rec[fc + i].x : 0u;
+    hr->moves[i] = in ? (uint16_t)meta_move(meta[fc + i].y) : MOVE_NONE;
+  }
+  const uint32_t reps = warp_repetitions(hash[0], T.root_hist + (size_t)g * SPB_CHESS_MAX_HISTORY, root.hist_len, ws, 0, lane);
+  if (lane == 0) {
+    hr->n_moves = (uint16_t)nc;
+    hr->ply = (uint16_t)ply;
+    hr->repetitions = (uint8_t)min(reps, 255u);
+    hr->outcome = 0;
+    hr->flags = 0;
+    hr->reserved = 0;
+  }
+  // the chosen child's status: cached by the search, or found now as the search would (history of the root + the root)
+  const uint32_t child = fc + (uint32_t)chosen;
+  const uint32_t cy = meta[child].y;
+  uint32_t cst = meta_status(cy);
+  if (cst == ST_UNVISITED) {
+    if (lane == 0) ws.phash[0] = hash[0];
+    __syncwarp();
+    int n;
+    unsigned long long lh;
+    uint32_t lr;
+    cst = visit_leaf(T, g, apply_move(root, (Move)meta_move(cy)), 1, lane, ws, n, lh, lr);
+  }
+  __syncwarp();                                                       // the record is complete before emit_game reads it
+  const uint32_t plies = ply + 1;
+  const bool over = cst == ST_TIED || cst == ST_WON;
+  // the device keeps SPB_CHESS_MAX_HISTORY plies of history and records per game; the reference has no cap
+  const bool capped = !over && (root.hist_len >= SPB_CHESS_MAX_HISTORY || plies >= P.max_ply);
+  if (over || capped) {
+    const uint32_t pk = 1u | ((cst == ST_WON ? 1u : 0u) << 1) | (((uint32_t)root.side ^ 1u) << 2) | ((capped ? 1u : 0u) << 3);
+    unsigned long long base;
+    if (reserve_output(P, plies, lane, &base)) {
+      emit_game(T, P, g, plies, pk, base, restart_roots, restart_hist, lane);
+    } else if (lane == 0) {
+      // parked: idle with its history until a later call emits it (the caller drains in between); nothing is lost
+      P.hist_len[g] = plies;
+      P.parked[g] = (uint8_t)pk;
+      T.live[g] = 0;
+      atomicOr(T.error, (uint32_t)ERRBIT_TRAJ_FULL);
+    }
+  } else {
+    if (lane == 0) P.hist_len[g] = plies;
+    reroot(T, g, child, lane, nullptr);                               // :233-234
   }
 }
 
@@ -406,6 +584,7 @@ int32_t spb_chess_engine::check_device_errors() {
   if (!bits) return SPB_OK;
   CH_CUDA(this, cudaMemsetAsync(T.error, 0, 4, stream));
   if (bits & ERRBIT_POOL) { set_error("a chess tree outgrew max_nodes_per_tree"); return SPB_ERR_POOL; }
+  if (bits == ERRBIT_TRAJ_FULL) { set_error("trajectory buffer full: call spb_chess_drain_trajectories"); return SPB_ERR_STATE; }
   set_error("chess kernel check failed, site " + std::to_string((bits >> 8) & 0xFF));
   return SPB_ERR_STATE;
 }
@@ -511,12 +690,8 @@ int32_t spb_chess_destroy(spb_chess_engine* e) {
 
 const char* spb_chess_last_error(const spb_chess_engine* e) { return e ? e->err.c_str() : g_create_error.c_str(); }
 
-int32_t spb_chess_reset_games(spb_chess_engine* e, const uint32_t* slots, uint32_t n, const spb_chess_state* roots, const uint64_t* history) {
-  CH_GUARD(e);
-  CH_ARG(e, n <= e->T.G, "more slots than games");
-  CH_ARG(e, !(history && !roots), "history without roots");
-  if (n == 0) return SPB_OK;
-  if (slots) for (uint32_t i = 0; i < n; ++i) CH_ARG(e, slots[i] < e->T.G, "slot out of range");
+// The roots of spb_chess_reset_games / spb_chess_selfplay_step (history: [n][SPB_CHESS_MAX_HISTORY], nullable).
+static int32_t check_roots(spb_chess_engine* e, const spb_chess_state* roots, const uint64_t* history, uint32_t n) {
   if (roots) for (uint32_t i = 0; i < n; ++i) {
     CH_ARG(e, roots[i].side <= 1 && roots[i].ep <= 64, "malformed root state");
     uint64_t kings[2] = {roots[i].piece[5] & roots[i].color[0], roots[i].piece[5] & roots[i].color[1]};
@@ -524,13 +699,24 @@ int32_t spb_chess_reset_games(spb_chess_engine* e, const uint32_t* slots, uint32
     CH_ARG(e, history || roots[i].hist_len == 0, "root with hist_len > 0 needs its history");
     CH_ARG(e, roots[i].hist_len <= SPB_CHESS_MAX_HISTORY, "hist_len > SPB_CHESS_MAX_HISTORY");
   }
+  return SPB_OK;
+}
+
+int32_t spb_chess_reset_games(spb_chess_engine* e, const uint32_t* slots, uint32_t n, const spb_chess_state* roots, const uint64_t* history) {
+  CH_GUARD(e);
+  CH_ARG(e, n <= e->T.G, "more slots than games");
+  CH_ARG(e, !(history && !roots), "history without roots");
+  if (n == 0) return SPB_OK;
+  if (slots) for (uint32_t i = 0; i < n; ++i) CH_ARG(e, slots[i] < e->T.G, "slot out of range");
+  const int32_t rc = check_roots(e, roots, history, n);
+  if (rc) return rc;
   uint32_t* d_slots = slots ? e->d_reset_slots : nullptr;
   ch::Pos* d_roots = roots ? e->d_reset_roots : nullptr;
   unsigned long long* d_hist = history ? e->d_reset_hist : nullptr;
   if (slots) CH_CUDA(e, cudaMemcpyAsync(d_slots, slots, (size_t)n * 4, cudaMemcpyHostToDevice, e->stream));
   if (roots) CH_CUDA(e, cudaMemcpyAsync(d_roots, roots, (size_t)n * sizeof(ch::Pos), cudaMemcpyHostToDevice, e->stream));
   if (history) CH_CUDA(e, cudaMemcpyAsync(d_hist, history, (size_t)n * SPB_CHESS_MAX_HISTORY * 8, cudaMemcpyHostToDevice, e->stream));
-  ch::k_chess_reset<<<n, 64, 0, e->stream>>>(e->T, d_slots, d_roots, d_hist, n);
+  ch::k_chess_reset<<<n, 64, 0, e->stream>>>(e->T, e->P, d_slots, d_roots, d_hist, n);
   CH_CUDA(e, cudaGetLastError());
   ++e->launches;
   CH_CUDA(e, cudaStreamSynchronize(e->stream));
@@ -744,6 +930,78 @@ int32_t spb_chess_node_stats(spb_chess_engine* e, uint32_t slot, uint32_t node_i
   // status in the header's terms: a node that was never reached as a leaf has not been classified yet -> reported Ongoing
   if (status) *status = h[6] == ch::ST_TIED ? SPB_STATUS_TIED : (h[6] == ch::ST_WON ? SPB_STATUS_WON : SPB_STATUS_ONGOING);
   return SPB_OK;
+}
+
+// The trajectory buffers of the self-play step, allocated by its first call (an engine that never plays does not pay for
+// them).  A failure frees what this call allocated and leaves the engine as it was.
+int32_t spb_chess_engine::ensure_selfplay() {
+  if (P.out) return SPB_OK;
+  const size_t G = T.G, max_ply = SPB_CHESS_MAX_HISTORY;
+  spb::Trajectories<spb_chess_position> Q{};
+  Q.max_ply = (uint32_t)max_ply;
+  Q.out_cap = (uint32_t)std::min<size_t>(G * max_ply * 4, (size_t)1 << 26);
+  if (cfg.trajectory_capacity) Q.out_cap = std::max<uint32_t>(cfg.trajectory_capacity, (uint32_t)max_ply);   // a whole game always fits
+  Q.id_stride = cfg.game_id_stride ? cfg.game_id_stride : (unsigned long long)G;
+  std::vector<void*> got;
+  auto alloc = [&](auto** p, size_t count) {
+    void* q = nullptr;
+    if (cudaMalloc(&q, count * sizeof(**p)) != cudaSuccess) return false;
+    got.push_back(q);
+    *p = static_cast<std::remove_reference_t<decltype(*p)>>(q);
+    return true;
+  };
+  const bool ok = alloc(&Q.hist, G * max_ply) && alloc(&Q.hist_len, G) && alloc(&Q.parked, G) && alloc(&Q.game_id, G) &&
+                  alloc(&Q.out, (size_t)Q.out_cap) && alloc(&Q.out_game, (size_t)Q.out_cap) && alloc(&Q.out_cursor, 1) && alloc(&Q.finished, 1);
+  cudaError_t ce = ok ? cudaSuccess : cudaErrorMemoryAllocation;
+  std::vector<unsigned long long> ids(G);
+  for (size_t i = 0; i < G; ++i) ids[i] = (unsigned long long)cfg.game_id_base + i;
+  if (ce == cudaSuccess) ce = cudaMemsetAsync(Q.hist_len, 0, G * 4, stream);
+  if (ce == cudaSuccess) ce = cudaMemsetAsync(Q.parked, 0, G, stream);
+  if (ce == cudaSuccess) ce = cudaMemsetAsync(Q.out_cursor, 0, 8, stream);
+  if (ce == cudaSuccess) ce = cudaMemsetAsync(Q.finished, 0, 4, stream);
+  if (ce == cudaSuccess) ce = cudaMemcpyAsync(Q.game_id, ids.data(), G * 8, cudaMemcpyHostToDevice, stream);
+  if (ce == cudaSuccess) ce = cudaStreamSynchronize(stream);
+  if (ce != cudaSuccess) {
+    for (void* q : got) cudaFree(q);
+    cudaGetLastError();                                                // an allocation failure is not sticky: clear it
+    set_error("chess self-play: cannot set up the trajectory buffers (" + std::to_string(G * max_ply) + " + " + std::to_string(Q.out_cap) +
+              " records of " + std::to_string(sizeof(spb_chess_position)) + " bytes): " + cudaGetErrorString(ce));
+    return ok ? SPB_ERR_CUDA : SPB_ERR_NOMEM;
+  }
+  allocs.insert(allocs.end(), got.begin(), got.end());
+  P = Q;
+  return SPB_OK;
+}
+
+int32_t spb_chess_selfplay_step(spb_chess_engine* e, int32_t rule, float temperature, uint64_t seed, const spb_chess_state* restart_roots,
+                                const uint64_t* restart_history, uint32_t* n_finished) {
+  CH_GUARD(e);
+  CH_ARG(e, rule == SPB_MOVE_GREEDY_LAST_MAX || rule == SPB_MOVE_TEMPERATURE, "unknown move rule");
+  CH_ARG(e, !(restart_history && !restart_roots), "history without roots");
+  const uint32_t G = e->T.G;
+  int32_t rc = check_roots(e, restart_roots, restart_history, G);
+  if (rc) return rc;
+  rc = e->ensure_selfplay();
+  if (rc) return rc;
+  // the staging of spb_chess_reset_games (every call ends with a stream synchronisation)
+  if (restart_roots) CH_CUDA(e, cudaMemcpyAsync(e->d_reset_roots, restart_roots, (size_t)G * sizeof(ch::Pos), cudaMemcpyHostToDevice, e->stream));
+  if (restart_history)
+    CH_CUDA(e, cudaMemcpyAsync(e->d_reset_hist, restart_history, (size_t)G * SPB_CHESS_MAX_HISTORY * 8, cudaMemcpyHostToDevice, e->stream));
+  CH_CUDA(e, cudaMemsetAsync(e->P.finished, 0, 4, e->stream));
+  ch::k_chess_selfplay_step<<<(G + ch::WARPS - 1) / ch::WARPS, ch::THREADS, 0, e->stream>>>(
+      e->T, e->P, rule, temperature, seed, restart_roots ? e->d_reset_roots : nullptr, restart_history ? e->d_reset_hist : nullptr);
+  CH_CUDA(e, cudaGetLastError());
+  ++e->launches;
+  uint32_t fin = 0;
+  CH_CUDA(e, cudaMemcpyAsync(&fin, e->P.finished, 4, cudaMemcpyDeviceToHost, e->stream));
+  rc = e->check_device_errors();                                       // synchronises the stream
+  if (n_finished) *n_finished = fin;
+  return rc;
+}
+
+int32_t spb_chess_drain_trajectories(spb_chess_engine* e, spb_chess_position* buf, size_t capacity, size_t* written, uint64_t* game_ids) {
+  CH_GUARD(e);
+  return drain_trajectories(e, e->P, e->stream, buf, capacity, written, game_ids);
 }
 
 int32_t spb_chess_get_counters(spb_chess_engine* e, spb_counters* out) {

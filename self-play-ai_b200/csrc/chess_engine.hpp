@@ -6,11 +6,13 @@
 #include <algorithm>
 #include <cstring>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include <cuda_runtime.h>
 
 #include "chess_tree.cuh"
+#include "trajectory.cuh"
 
 namespace spb {
 namespace chess {
@@ -34,6 +36,9 @@ struct spb_chess_engine {
   // device staging of spb_chess_reset_games (allocated once: cudaMalloc / cudaFree per call would synchronise the device)
   uint32_t* d_reset_slots = nullptr; spb::chess::Pos* d_reset_roots = nullptr; unsigned long long* d_reset_hist = nullptr;
   uint32_t* d_adv_ids = nullptr; int32_t* d_adv_err = nullptr;   // spb_chess_advance (with d_reset_slots / d_reset_roots)
+  // self-play trajectories (spb_chess_selfplay_step); all null until the first step allocates them.
+  // parked[g] = 1 | won << 1 | terminal side to move << 2 | adjudicated << 3
+  spb::Trajectories<spb_chess_position> P{};
 
   void set_error(const std::string& s) { err = s; }
   template <class T_> int32_t dalloc(T_** p, size_t count) {
@@ -45,6 +50,7 @@ struct spb_chess_engine {
     return SPB_OK;
   }
   int32_t check_device_errors();
+  int32_t ensure_selfplay();
 };
 
 extern thread_local std::string g_create_error;   // engine.cu

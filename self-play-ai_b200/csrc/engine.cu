@@ -831,35 +831,7 @@ int32_t spb_selfplay_step(spb_engine* e, int32_t rule, float temperature, uint64
 
 int32_t spb_drain_trajectories(spb_engine* e, spb_position* buf, size_t capacity, size_t* written, uint64_t* game_ids) {
   ENGINE_GUARD(e);
-  ARG_CHECK(e, written, "null written");
-  unsigned long long cur = 0;
-  cudaError_t ce = cudaMemcpyAsync(&cur, e->P.out_cursor, 8, cudaMemcpyDeviceToHost, e->stream);
-  if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
-  if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
-  size_t n = (size_t)std::min<unsigned long long>(cur, e->P.out_cap);
-  *written = n;
-  if (!buf) return SPB_OK;                        // size query
-  ARG_CHECK(e, capacity >= n, "trajectory buffer too small");
-  if (n == 0) return SPB_OK;
-  std::vector<spb_position> pos(n);
-  std::vector<unsigned long long> ids(n);
-  ce = cudaMemcpyAsync(pos.data(), e->P.out, n * sizeof(spb_position), cudaMemcpyDeviceToHost, e->stream);
-  if (ce == cudaSuccess) ce = cudaMemcpyAsync(ids.data(), e->P.out_game, n * 8, cudaMemcpyDeviceToHost, e->stream);
-  if (ce == cudaSuccess) ce = cudaMemsetAsync(e->P.out_cursor, 0, 8, e->stream);
-  if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
-  if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
-  // deterministic order: game id, then ply (games finish in a nondeterministic order on the device)
-  std::vector<size_t> order(n);
-  for (size_t i = 0; i < n; ++i) order[i] = i;
-  std::sort(order.begin(), order.end(), [&](size_t a, size_t b) {
-    if (ids[a] != ids[b]) return ids[a] < ids[b];
-    return pos[a].ply < pos[b].ply;
-  });
-  for (size_t i = 0; i < n; ++i) {
-    buf[i] = pos[order[i]];
-    if (game_ids) game_ids[i] = ids[order[i]];
-  }
-  return SPB_OK;
+  return drain_trajectories(e, e->P, e->stream, buf, capacity, written, game_ids);
 }
 
 // ---- counters -----------------------------------------------------------------------------------

@@ -13,6 +13,7 @@
 
 #include "async.cuh"
 #include "evaluator.cuh"
+#include "trajectory.cuh"
 #include "tree.cuh"
 
 namespace spb {
@@ -20,20 +21,8 @@ namespace spb {
 constexpr int CTL_WORDS = 9 * 32;   // control words of the asynchronous pipeline, one 128-byte line each
 
 // ---- self-play ply (ref: learner_concurrent.rs:179-238): device buffers of the trajectories ----------------------
-struct SelfPlay {
-  spb_position* hist;        // [G][MAX_PLY]
-  uint32_t* hist_len;        // [G]
-  uint8_t* parked;           // [G]  0, or 1 | terminal status << 1 | terminal side to move << 3: the game has ended but its trajectory
-                             //      did not fit the output buffer; the slot is idle until the next spb_selfplay_step emits it
-  unsigned long long* game_id;     // [G]
-  spb_position* out;         // [out_cap]
-  unsigned long long* out_game;    // [out_cap]
-  unsigned long long* out_cursor;  // [1]
-  uint32_t* finished;        // [1]
-  uint32_t out_cap;
-  uint32_t max_ply;
-  unsigned long long id_stride;
-};
+// parked[g] = 1 | terminal status << 1 | terminal side to move << 3
+using SelfPlay = Trajectories<spb_position>;
 
 }  // namespace spb
 

@@ -14,7 +14,6 @@
 #include <nccl.h>
 
 #include <mutex>
-#include <numeric>
 
 #include "engine.hpp"
 
@@ -73,12 +72,7 @@ NcclApi* nccl_api() {
 // Orders records by (global game id, ply): games finish in a nondeterministic order on the device and arrive rank by rank.
 void sort_records(std::vector<spb_position>& pos, std::vector<unsigned long long>& ids) {
   const size_t n = pos.size();
-  std::vector<size_t> order(n);
-  std::iota(order.begin(), order.end(), (size_t)0);
-  std::sort(order.begin(), order.end(), [&](size_t a, size_t b) {
-    if (ids[a] != ids[b]) return ids[a] < ids[b];
-    return pos[a].ply < pos[b].ply;
-  });
+  const std::vector<size_t> order = record_order(pos, ids);
   std::vector<spb_position> p2(n);
   std::vector<unsigned long long> i2(n);
   for (size_t i = 0; i < n; ++i) { p2[i] = pos[order[i]]; i2[i] = ids[order[i]]; }

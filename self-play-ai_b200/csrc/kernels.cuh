@@ -527,24 +527,6 @@ __global__ void k_mask_policies(const PState* states, uint32_t n, const float* e
 
 // ---- self-play ply (ref: learner_concurrent.rs:179-238) -------------------------------------------
 
-// Reserves `plies` records of the trajectory output buffer (lane 0; all lanes get the answer).  The cursor only moves
-// when the whole trajectory fits, so every record below the cursor is fully written: a drain never sees a hole.
-__device__ __forceinline__ bool reserve_output(const SelfPlay& P, uint32_t plies, int lane, unsigned long long* base_out) {
-  unsigned long long base = ~0ull;
-  if (lane == 0) {
-    unsigned long long cur = *reinterpret_cast<volatile unsigned long long*>(P.out_cursor);
-    for (;;) {
-      if (cur + plies > P.out_cap) { base = ~0ull; break; }
-      const unsigned long long seen = atomicCAS(P.out_cursor, cur, cur + plies);
-      if (seen == cur) { base = cur; break; }
-      cur = seen;
-    }
-  }
-  base = __shfl_sync(0xffffffffu, base, 0);
-  *base_out = base;
-  return base != ~0ull;
-}
-
 // Emits the finished game of slot g (learner_concurrent.rs:200-230) and restarts or retires the slot.
 __device__ __forceinline__ void emit_and_finish(const Trees& T, const SelfPlay& P, uint32_t g, uint32_t plies, uint32_t cstatus,
                                                 uint32_t term_player, unsigned long long base, const PState* restart_roots, int lane) {
@@ -559,10 +541,7 @@ __device__ __forceinline__ void emit_and_finish(const Trees& T, const SelfPlay& 
   }
   __syncwarp();
   if (lane == 0) {
-    atomicAdd(P.finished, 1u);
-    P.hist_len[g] = 0;
-    P.parked[g] = 0;
-    P.game_id[g] += P.id_stride;
+    finish_trajectory(P, g);
     if (restart_roots) {                                           // Tree::with_root_state for the next game
       PState nr = restart_roots[g];
       T.root_state[g] = nr;

@@ -215,6 +215,48 @@ class ChessMcts {
   }
   size_t arena_len(const ChessTree& tree) { uint32_t n = 0; check(spb_chess_arena_len(e_, tree.slot, &n)); return n; }
 
+  // ref: learner_concurrent.rs:179-238 — one self-play ply for every live game on the device (rule SPB_MOVE_*); finished
+  // slots restart from restart_roots[slot] (num_parallel_self_play_games entries) or retire.  Returns the games finished.
+  // Throws Error(SPB_ERR_STATE) when the trajectory buffer is full: drain and call again, nothing is lost.
+  uint32_t self_play_step(int rule, float temperature, uint64_t seed, const std::vector<ChessState>* restart_roots = nullptr) {
+    std::vector<spb_chess_state> roots;
+    std::vector<uint64_t> hist;
+    if (restart_roots) {
+      for (const ChessState& s : *restart_roots) {
+        spb_chess_state st = s.raw;
+        st.hist_len = (uint32_t)std::min<size_t>(s.history.size(), SPB_CHESS_MAX_HISTORY);
+        roots.push_back(st);
+        std::vector<uint64_t> h(SPB_CHESS_MAX_HISTORY, 0);
+        std::copy(s.history.begin(), s.history.begin() + st.hist_len, h.begin());
+        hist.insert(hist.end(), h.begin(), h.end());
+      }
+    }
+    uint32_t finished = 0;
+    check(spb_chess_selfplay_step(e_, rule, temperature, seed, restart_roots ? roots.data() : nullptr, restart_roots ? hist.data() : nullptr,
+                                  &finished));
+    return finished;
+  }
+  // Finished games' positions ordered by (game id, ply), with their global game ids.
+  std::pair<std::vector<spb_chess_position>, std::vector<uint64_t>> drain_trajectories() {
+    size_t n = 0;
+    check(spb_chess_drain_trajectories(e_, nullptr, 0, &n, nullptr));
+    std::vector<spb_chess_position> pos(n);
+    std::vector<uint64_t> ids(n);
+    if (n) check(spb_chess_drain_trajectories(e_, pos.data(), n, &n, ids.data()));
+    pos.resize(n);
+    ids.resize(n);
+    return {std::move(pos), std::move(ids)};
+  }
+  // The training tensors of chess records (host only): encodings [n][19][8][8], policies [n][4672], values [n].
+  struct TrainingBatch { std::vector<float> encodings, policies, values; };
+  static TrainingBatch positions_to_training(const std::vector<spb_chess_position>& positions) {
+    const size_t n = positions.size();
+    TrainingBatch b{std::vector<float>(n * SPB_CHESS_PLANES * 64), std::vector<float>(n * SPB_CHESS_POLICY_SIZE), std::vector<float>(n)};
+    const int rc = spb_chess_positions_to_training(positions.data(), n, b.encodings.data(), b.policies.data(), b.values.data());
+    if (rc != SPB_OK) throw Error(rc, "spb_chess_positions_to_training: bad argument");
+    return b;
+  }
+
  private:
   void check(int rc) { if (rc != SPB_OK) throw Error(rc, spb_chess_last_error(e_)); }
   spb_chess_engine* e_ = nullptr;
