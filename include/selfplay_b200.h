@@ -411,6 +411,19 @@ int32_t spb_chess_drain_trajectories(spb_chess_engine* e, spb_chess_position* bu
  * SPB_ERR_ARG for a malformed record (n_moves outside 1..256, side > 1, a move outside the policy).
  */
 int32_t spb_chess_positions_to_training(const spb_chess_position* positions, size_t n, float* encodings, float* policies, float* values);
+/*
+ * The same tensors built on the device, per minibatch, from records held in device memory (ref: the replay buffer the
+ * learner pops batch_size positions from, learner_concurrent.rs:87-165; the tensors of :126-146).  Output row i comes
+ * from positions[indices ? indices[i] : i]; without indices n <= n_positions.  Every pointer is device (or managed) memory
+ * of e's GPU, each output nullable: encodings[n][19][8][8], policies[n][4672], values[n].  The results are bit-identical
+ * to spb_chess_positions_to_training of the same records (a record whose counts sum to 0 gives NaN policies on both
+ * sides, with the NaN bit pattern of each processor).  Validation is that of the host function, plus indices[i] <
+ * n_positions: a malformed row gives SPB_ERR_ARG, nothing is written, and spb_chess_last_error names the first bad row.
+ * Enqueued on the engine's stream; returns once the outputs are written.
+ */
+int32_t spb_chess_positions_to_training_device(spb_chess_engine* e, const spb_chess_position* positions, size_t n_positions,
+                                               const uint64_t* indices /* nullable */, size_t n,
+                                               float* encodings, float* policies, float* values);
 
 /* ---- multi-GPU: trajectories to the learner rank; learner hand-off ------- */
 
@@ -433,6 +446,16 @@ int32_t spb_comm_destroy(spb_engine* e);
  */
 int32_t spb_gather_trajectories(spb_engine* e, int32_t learner_rank, spb_position* buf, size_t capacity, size_t* written,
                                 uint64_t* game_ids /* nullable */);
+/*
+ * The same for chess engines (ref: learner_concurrent.rs:281-288), with the contract of spb_comm_init, spb_comm_destroy and
+ * spb_gather_trajectories; the id comes from spb_comm_unique_id.  The gather hands over what spb_chess_drain_trajectories
+ * would return; an engine that never played (no trajectory buffers yet) takes part with 0 records.  spb_chess_destroy
+ * releases a live communicator.
+ */
+int32_t spb_chess_comm_init(spb_chess_engine* e, const uint8_t* id, int32_t rank, int32_t world_size);
+int32_t spb_chess_comm_destroy(spb_chess_engine* e);
+int32_t spb_chess_gather_trajectories(spb_chess_engine* e, int32_t learner_rank, spb_chess_position* buf, size_t capacity,
+                                      size_t* written, uint64_t* game_ids /* nullable */);
 /*
  * ref: learner_concurrent.rs:126-146, learner.rs:162-182 — the tensors the learners train on, from n compact records
  * (host only, no GPU needed): encodings[n][3][R][C] (get_encoding of the recorded root state, connect_four.rs:242-259),

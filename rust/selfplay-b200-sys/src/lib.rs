@@ -181,10 +181,14 @@ extern "C" {
     pub fn spb_chess_selfplay_step(e: *mut spb_chess_engine, rule: i32, temperature: f32, seed: u64, restart_roots: *const spb_chess_state, restart_history: *const u64, n_finished: *mut u32) -> i32;
     pub fn spb_chess_drain_trajectories(e: *mut spb_chess_engine, buf: *mut spb_chess_position, capacity: usize, written: *mut usize, game_ids: *mut u64) -> i32;
     pub fn spb_chess_positions_to_training(positions: *const spb_chess_position, n: usize, encodings: *mut f32, policies: *mut f32, values: *mut f32) -> i32;
+    pub fn spb_chess_positions_to_training_device(e: *mut spb_chess_engine, positions: *const spb_chess_position, n_positions: usize, indices: *const u64, n: usize, encodings: *mut f32, policies: *mut f32, values: *mut f32) -> i32;
     pub fn spb_comm_unique_id(id: *mut u8) -> i32;
     pub fn spb_comm_init(e: *mut spb_engine, id: *const u8, rank: i32, world_size: i32) -> i32;
     pub fn spb_comm_destroy(e: *mut spb_engine) -> i32;
     pub fn spb_gather_trajectories(e: *mut spb_engine, learner_rank: i32, buf: *mut spb_position, capacity: usize, written: *mut usize, game_ids: *mut u64) -> i32;
+    pub fn spb_chess_comm_init(e: *mut spb_chess_engine, id: *const u8, rank: i32, world_size: i32) -> i32;
+    pub fn spb_chess_comm_destroy(e: *mut spb_chess_engine) -> i32;
+    pub fn spb_chess_gather_trajectories(e: *mut spb_chess_engine, learner_rank: i32, buf: *mut spb_chess_position, capacity: usize, written: *mut usize, game_ids: *mut u64) -> i32;
     pub fn spb_positions_to_training(game: i32, positions: *const spb_position, n: usize, encodings: *mut f32, policies: *mut f32, values: *mut f32) -> i32;
     pub fn spb_get_counters(e: *mut spb_engine, out: *mut spb_counters) -> i32;
     pub fn spb_reset_counters(e: *mut spb_engine) -> i32;

@@ -369,6 +369,39 @@ impl ChessMcts {
         }
         Ok((pos, ids))
     }
+    /// Joins the NCCL communicator of the job (id from `comm_unique_id()` on rank 0, distributed by the host).
+    pub fn comm_init(&mut self, id: &[u8; sys::SPB_COMM_ID_BYTES], rank: i32, world_size: i32) -> Result<()> {
+        self.check(unsafe { sys::spb_chess_comm_init(self.raw, id.as_ptr(), rank, world_size) })
+    }
+    /// Leaves the communicator (dropping the engine does too).
+    pub fn comm_destroy(&mut self) -> Result<()> {
+        self.check(unsafe { sys::spb_chess_comm_destroy(self.raw) })
+    }
+    /// COLLECTIVE: every rank's finished chess trajectories to `learner_rank`, ordered by (game id, ply) — the replay-buffer
+    /// push of the reference's workers (learner_concurrent.rs:281-288).  Empty on the other ranks.
+    pub fn gather_trajectories(&mut self, learner_rank: i32) -> Result<(Vec<ChessPosition>, Vec<u64>)> {
+        let mut n = 0usize;
+        self.check(unsafe { sys::spb_chess_gather_trajectories(self.raw, learner_rank, std::ptr::null_mut(), 0, &mut n, std::ptr::null_mut()) })?;
+        let mut pos: Vec<ChessPosition> = vec![unsafe { std::mem::zeroed() }; n];
+        let mut ids = vec![0u64; n];
+        if n > 0 {
+            self.check(unsafe { sys::spb_chess_gather_trajectories(self.raw, learner_rank, pos.as_mut_ptr(), n, &mut n, ids.as_mut_ptr()) })?;
+        }
+        Ok((pos, ids))
+    }
+    /// The training tensors of `chess_positions_to_training`, built on this engine's GPU from records in its device memory
+    /// (a replay buffer of `n_positions` records; ref: learner_concurrent.rs:87-165, :126-146).  Row i comes from
+    /// `positions[indices[i]]`, or `positions[i]` when `indices` is null (then `n <= n_positions`).  Outputs (each nullable):
+    /// `encodings[n][19][8][8]`, `policies[n][4672]`, `values[n]` f32, bit-identical to the host builder.  Returns once they are
+    /// written; a malformed row is `SPB_ERR_ARG` and nothing is written.
+    ///
+    /// # Safety
+    /// Every non-null pointer is device (or managed) memory of this engine's GPU, e.g. `Tensor::data_ptr` of CUDA tensors, and
+    /// holds as many elements as stated; no other work writes the inputs or reads the outputs during the call.
+    pub unsafe fn positions_to_training_device(&mut self, positions: *const ChessPosition, n_positions: usize, indices: *const u64, n: usize,
+                                               encodings: *mut f32, policies: *mut f32, values: *mut f32) -> Result<()> {
+        self.check(sys::spb_chess_positions_to_training_device(self.raw, positions, n_positions, indices, n, encodings, policies, values))
+    }
 }
 
 pub type ChessPosition = sys::spb_chess_position;

@@ -78,7 +78,7 @@ class ChessEngine:
         rc = L.spb_chess_create(C.byref(cfg), C.byref(h))
         if rc != 0:
             raise E.EngineError(rc, L.spb_chess_last_error(None).decode())
-        self._h, self._L, self.G = h, L, num_games
+        self._h, self._L, self.G, self.device = h, L, num_games, device
 
     def close(self):
         if getattr(self, "_h", None):
@@ -232,6 +232,25 @@ class ChessEngine:
             self._chk(self._L.spb_chess_drain_trajectories(self._h, pos.ctypes.data, n.value, C.byref(n), ids.ctypes.data))
         return pos[:n.value], ids[:n.value]
 
+    # ---- multi-GPU: trajectories to the learner rank (the contract of Engine's methods) -------------------------------
+    def comm_init(self, comm_id: bytes, rank: int, world_size: int):
+        buf = (C.c_uint8 * E.COMM_ID_BYTES).from_buffer_copy(comm_id)
+        self._chk(self._L.spb_chess_comm_init(self._h, C.cast(buf, C.c_void_p), rank, world_size))
+
+    def comm_destroy(self):
+        self._chk(self._L.spb_chess_comm_destroy(self._h))
+
+    def gather_trajectories(self, learner_rank: int = 0):
+        """COLLECTIVE: -> (positions[CHESS_POSITION_DTYPE], game_ids) ordered by (game id, ply) on the learner rank, empty
+        elsewhere."""
+        n = C.c_size_t()
+        self._chk(self._L.spb_chess_gather_trajectories(self._h, learner_rank, None, 0, C.byref(n), None))
+        pos = np.zeros(n.value, dtype=CHESS_POSITION_DTYPE)
+        ids = np.zeros(n.value, dtype=np.uint64)
+        if n.value:
+            self._chk(self._L.spb_chess_gather_trajectories(self._h, learner_rank, pos.ctypes.data, n.value, C.byref(n), ids.ctypes.data))
+        return pos[:n.value], ids[:n.value]
+
     def get_state(self, slot: int, node_id: int) -> np.ndarray:
         out = np.zeros(1, CHESS_STATE_DTYPE)
         self._chk(self._L.spb_chess_get_state(self._h, slot, node_id, out.ctypes.data))
@@ -281,6 +300,41 @@ def positions_to_training(positions):
     rc = L.spb_chess_positions_to_training(pos.ctypes.data, n, enc.ctypes.data, pol.ctypes.data, val.ctypes.data)
     if rc != 0:
         raise E.EngineError(rc, "spb_chess_positions_to_training: bad argument")
+    return enc, pol, val
+
+
+def positions_to_training_device(engine: ChessEngine, positions, indices=None):
+    """spb_chess_positions_to_training_device: the tensors of positions_to_training, built on the engine's GPU ->
+    torch CUDA tensors (encodings[n,19,8,8], policies[n,4672], values[n,1]) f32, bit-identical to the host builder.
+    positions: CHESS_POSITION_DTYPE numpy array (copied to the device) or a CUDA uint8 tensor [n_positions, 1624], e.g. a
+    replay buffer kept in device memory.  indices (numpy or CUDA int64 / uint64 tensor): row i is built from
+    positions[indices[i]]; without it every record is built.  A malformed row raises EngineError(-1) and nothing is written."""
+    import torch
+    dev = torch.device("cuda", engine.device)
+    if isinstance(positions, torch.Tensor):
+        assert positions.is_cuda and positions.dtype == torch.uint8 and positions.dim() == 2 and positions.shape[1] == CHESS_POSITION_DTYPE.itemsize, \
+            (positions.device, positions.dtype, tuple(positions.shape))
+        pos = positions.contiguous()
+    else:
+        a = np.ascontiguousarray(positions, dtype=CHESS_POSITION_DTYPE).reshape(-1)
+        pos = torch.from_numpy(a.view(np.uint8).reshape(len(a), CHESS_POSITION_DTYPE.itemsize)).to(dev)
+    idx = None
+    if indices is not None:
+        if isinstance(indices, torch.Tensor):
+            assert indices.is_cuda and indices.dtype in (torch.int64, torch.uint64) and indices.dim() == 1, (indices.device, indices.dtype)
+            idx = indices.contiguous()
+        else:
+            i = np.ascontiguousarray(indices).reshape(-1)
+            assert i.dtype.kind in "iu", i.dtype
+            idx = torch.from_numpy(i.astype(np.int64)).to(dev)
+    n = len(pos) if idx is None else len(idx)
+    enc = torch.empty((n, PLANES, 8, 8), dtype=torch.float32, device=dev)
+    pol = torch.empty((n, POLICY_SIZE), dtype=torch.float32, device=dev)
+    val = torch.empty((n, 1), dtype=torch.float32, device=dev)
+    torch.cuda.current_stream(dev).synchronize()                       # the engine's stream reads the inputs
+    engine._chk(engine._L.spb_chess_positions_to_training_device(
+        engine._h, pos.data_ptr() if len(pos) else None, len(pos), None if idx is None else idx.data_ptr(), n,
+        enc.data_ptr(), pol.data_ptr(), val.data_ptr()))
     return enc, pol, val
 
 

@@ -119,6 +119,112 @@ __global__ void k_frontier_expand(const Pos* frontier, uint32_t n, const uint32_
   for (int k = 0; k < m; ++k) next[offset[i] + k] = apply_move(p, mv[k]);
 }
 
+// ---- training tensors of self-play records on the device (spb_chess_positions_to_training_device) ----------------------
+// Pass 1 validates every row as spb_chess_positions_to_training does, plus the index range; the first bad row goes to *bad
+// (atomicMin; ~0 = none).  One warp per row, grid-stride: the lanes read the row's moves coalesced.
+__global__ void __launch_bounds__(256) k_chess_training_check(const spb_chess_position* __restrict__ pos, unsigned long long n_positions,
+                                                              const unsigned long long* __restrict__ indices, unsigned long long n,
+                                                              unsigned long long* bad) {
+  const int lane = threadIdx.x & 31;
+  const unsigned long long warps = (unsigned long long)gridDim.x * (blockDim.x / 32);
+  for (unsigned long long i = blockIdx.x * (unsigned long long)(blockDim.x / 32) + threadIdx.x / 32; i < n; i += warps) {
+    const unsigned long long src = indices ? indices[i] : i;
+    bool ok = src < n_positions;
+    if (ok) {
+      const spb_chess_position& p = pos[src];
+      const uint32_t nm = p.n_moves, side = p.state.side;
+      ok = nm >= 1 && nm <= SPB_CHESS_MAX_MOVES && side <= 1;
+      if (ok)
+        for (uint32_t k = lane; k < nm; k += 32) {
+          const int idx = policy_index((int)side, p.moves[k]);
+          ok &= idx >= 0 && idx < SPB_CHESS_POLICY_SIZE;
+        }
+      ok = __all_sync(0xffffffffu, ok);
+    }
+    if (!ok && lane == 0) atomicMin(bad, i);
+  }
+}
+
+constexpr int TRAIN_THREADS = 256;                                     // one thread per child of a record
+constexpr int REC_WORDS = sizeof(spb_chess_position) / 8;
+static_assert(sizeof(spb_chess_position) % 8 == 0, "records are loaded with 8-byte words");
+static_assert(SPB_CHESS_MAX_MOVES == TRAIN_THREADS, "the scatter gives child k to thread k");
+static_assert(SPB_CHESS_POLICY_SIZE % 4 == 0 && (SPB_CHESS_PLANES * 64) % 4 == 0, "rows are whole float4s");
+
+// Pass 2 (rows validated): one CTA per row at a time.  The record is staged in shared memory, the policy row is built there
+// (zero, f32 sum of the counts in child order on one thread, count / sum scattered by policy index with the later child
+// winning a duplicated index, as on the host), then the encoding and policy rows are written once each: 16-byte streaming
+// stores when the outputs are 16-byte aligned (row strides are multiples of 16 bytes), scalar stores otherwise.  Every
+// output float is written exactly once: the kernel is bound by HBM writes (23,556 bytes out per 1,624 read).
+__global__ void __launch_bounds__(TRAIN_THREADS) k_chess_training(const spb_chess_position* __restrict__ pos,
+                                                                  const unsigned long long* __restrict__ indices, unsigned long long n,
+                                                                  float* __restrict__ encodings, float* __restrict__ policies,
+                                                                  float* __restrict__ values, bool vec_enc, bool vec_pol) {
+  __shared__ unsigned long long s_rec[REC_WORDS];
+  __shared__ __align__(16) float s_pol[SPB_CHESS_POLICY_SIZE];
+  __shared__ float s_sum;
+  const spb_chess_position& r = *reinterpret_cast<const spb_chess_position*>(s_rec);
+  const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
+  constexpr int ENC = SPB_CHESS_PLANES * 64;
+  for (unsigned long long i = blockIdx.x; i < n; i += gridDim.x) {
+    const unsigned long long src = indices ? indices[i] : i;
+    const unsigned long long* g = reinterpret_cast<const unsigned long long*>(pos + src);
+    for (int w = t; w < REC_WORDS; w += TRAIN_THREADS) s_rec[w] = __ldg(g + w);
+    if (policies) {
+      float4* z = reinterpret_cast<float4*>(s_pol);
+      for (int w = t; w < SPB_CHESS_POLICY_SIZE / 4; w += TRAIN_THREADS) z[w] = make_float4(0.f, 0.f, 0.f, 0.f);
+    }
+    __syncthreads();
+    const int nm = r.n_moves, side = r.state.side;
+    if (policies) {
+      if (t == 0) {
+        float s = 0.0f;
+        for (int k = 0; k < nm; ++k) s += (float)r.visit_counts[k];
+        s_sum = s;
+      }
+      __syncthreads();
+      const bool mine = t < nm;
+      const int idx = mine ? policy_index(side, r.moves[t]) : -1;
+      const float v = mine ? (float)r.visit_counts[t] / s_sum : 0.0f;
+      // warp w writes in round w, so a later warp overwrites an earlier one; inside a warp the highest lane of a group of
+      // equal indices writes
+      const unsigned same = __match_any_sync(0xffffffffu, idx);
+      const bool last = (31 - __clz(same)) == lane;
+      for (int round = 0; round * 32 < nm; ++round) {
+        if (warp == round && mine && last) s_pol[idx] = v;
+        __syncthreads();
+      }
+    }
+    if (encodings) {
+      float* o = encodings + i * (unsigned long long)ENC;
+      if (vec_enc) {
+        for (int w = t; w < ENC / 4; w += TRAIN_THREADS) {
+          const int e0 = w * 4;
+          float4 q;
+          q.x = encode_plane(r.state, r.repetitions, e0 / 64, (e0 / 8) % 8, e0 % 8);
+          q.y = encode_plane(r.state, r.repetitions, (e0 + 1) / 64, ((e0 + 1) / 8) % 8, (e0 + 1) % 8);
+          q.z = encode_plane(r.state, r.repetitions, (e0 + 2) / 64, ((e0 + 2) / 8) % 8, (e0 + 2) % 8);
+          q.w = encode_plane(r.state, r.repetitions, (e0 + 3) / 64, ((e0 + 3) / 8) % 8, (e0 + 3) % 8);
+          __stcs(reinterpret_cast<float4*>(o) + w, q);
+        }
+      } else {
+        for (int w = t; w < ENC; w += TRAIN_THREADS) o[w] = encode_plane(r.state, r.repetitions, w / 64, (w / 8) % 8, w % 8);
+      }
+    }
+    if (policies) {
+      float* o = policies + i * (unsigned long long)SPB_CHESS_POLICY_SIZE;
+      if (vec_pol) {
+        const float4* q = reinterpret_cast<const float4*>(s_pol);
+        for (int w = t; w < SPB_CHESS_POLICY_SIZE / 4; w += TRAIN_THREADS) __stcs(reinterpret_cast<float4*>(o) + w, q[w]);
+      } else {
+        for (int w = t; w < SPB_CHESS_POLICY_SIZE; w += TRAIN_THREADS) o[w] = s_pol[w];
+      }
+    }
+    if (values && t == 0) values[i] = (float)r.outcome;
+    __syncthreads();                                                   // s_rec / s_pol are reused by the next row
+  }
+}
+
 }  // namespace chess
 }  // namespace spb
 
@@ -168,6 +274,50 @@ int32_t spb_chess_positions_to_training(const spb_chess_position* positions, siz
     }
     if (values) values[i] = (float)p.outcome;
   }
+  return SPB_OK;
+}
+
+int32_t spb_chess_positions_to_training_device(spb_chess_engine* e, const spb_chess_position* positions, size_t n_positions,
+                                               const uint64_t* indices, size_t n, float* encodings, float* policies, float* values) {
+  CH_GUARD(e);
+  CH_ARG(e, indices || n <= n_positions, "n > n_positions without indices");
+  if (n == 0) return SPB_OK;
+  CH_ARG(e, positions, "null positions");
+  const void* ptrs[5] = {positions, indices, encodings, policies, values};
+  const char* names[5] = {"positions", "indices", "encodings", "policies", "values"};
+  for (int k = 0; k < 5; ++k) {
+    if (!ptrs[k]) continue;
+    cudaPointerAttributes a{};
+    const cudaError_t ce = cudaPointerGetAttributes(&a, ptrs[k]);
+    if (ce != cudaSuccess) cudaGetLastError();
+    const bool ok = ce == cudaSuccess && (a.type == cudaMemoryTypeManaged || (a.type == cudaMemoryTypeDevice && a.device == e->cfg.device));
+    CH_ARG(e, ok, std::string(names[k]) + " is not device memory of the engine's GPU");
+  }
+  const unsigned long long none = ~0ull;
+  unsigned long long* d_bad = e->d_misc;                               // the engine's scratch word; every call ends synchronised
+  const auto* idx = reinterpret_cast<const unsigned long long*>(indices);
+  int sms = 0;
+  CH_CUDA(e, cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, e->cfg.device));
+  CH_CUDA(e, cudaMemsetAsync(d_bad, 0xFF, 8, e->stream));
+  const unsigned long long check_blocks = std::min<unsigned long long>((n + 7) / 8, (unsigned long long)sms * 8);
+  ch::k_chess_training_check<<<(unsigned)check_blocks, 256, 0, e->stream>>>(positions, n_positions, idx, n, d_bad);
+  CH_CUDA(e, cudaGetLastError());
+  ++e->launches;
+  unsigned long long bad = none;
+  CH_CUDA(e, cudaMemcpyAsync(&bad, d_bad, 8, cudaMemcpyDeviceToHost, e->stream));
+  CH_CUDA(e, cudaStreamSynchronize(e->stream));
+  if (bad != none) {
+    e->set_error("malformed training row " + std::to_string(bad) +
+                 (indices ? " (index out of range, or n_moves outside 1..256, side > 1 or a move outside the policy)"
+                          : " (n_moves outside 1..256, side > 1 or a move outside the policy)"));
+    return SPB_ERR_ARG;
+  }
+  const bool vec_enc = (reinterpret_cast<uintptr_t>(encodings) & 15) == 0, vec_pol = (reinterpret_cast<uintptr_t>(policies) & 15) == 0;
+  const unsigned long long blocks = std::min<unsigned long long>(n, (unsigned long long)sms * 8);
+  ch::k_chess_training<<<(unsigned)blocks, ch::TRAIN_THREADS, 0, e->stream>>>(positions, idx, n, encodings, policies, values, vec_enc, vec_pol);
+  CH_CUDA(e, cudaGetLastError());
+  ++e->launches;
+  CH_CUDA(e, cudaStreamSynchronize(e->stream));
   return SPB_OK;
 }
 

@@ -676,6 +676,7 @@ int32_t spb_chess_destroy(spb_chess_engine* e) {
   if (!e) return SPB_ERR_ARG;
   cudaSetDevice(e->cfg.device);
   if (e->stream) cudaStreamSynchronize(e->stream);
+  spb_chess_comm_destroy(e);
   ch::net_destroy(e->net);
   for (void* p : e->allocs) cudaFree(p);
   if (e->ev0) cudaEventDestroy(e->ev0);

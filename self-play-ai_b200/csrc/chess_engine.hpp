@@ -39,6 +39,12 @@ struct spb_chess_engine {
   // self-play trajectories (spb_chess_selfplay_step); all null until the first step allocates them.
   // parked[g] = 1 | won << 1 | terminal side to move << 2 | adjudicated << 3
   spb::Trajectories<spb_chess_position> P{};
+  // multi-GPU trajectory gather (gather.cu): NCCL communicator of this engine's rank, records staged on the learner rank
+  void* nccl_comm = nullptr;
+  int comm_rank = -1, comm_world = 0;
+  bool gather_pending = false;
+  std::vector<spb_chess_position> gather_pos;
+  std::vector<unsigned long long> gather_ids;
 
   void set_error(const std::string& s) { err = s; }
   template <class T_> int32_t dalloc(T_** p, size_t count) {

@@ -4,7 +4,8 @@
 // the finished trajectories go to the learner rank: the role of the replay-buffer push of the reference's workers
 // (ref: src/learner_concurrent.rs:281-288).  NCCL has no gatherv: all-gather of the per-rank record counts, then grouped
 // ncclSend / ncclRecv of the records into one device buffer on the learner rank; the learner orders them by
-// (global game id, ply), so an R-rank generation is byte-identical to the same games played on one rank.
+// (global game id, ply), so an R-rank generation is byte-identical to the same games played on one rank.  The Connect4 /
+// tic-tac-toe engine (spb_position records) and the chess engine (spb_chess_position) run the same code.
 // spb_positions_to_training builds the tensors the learners train on (ref: src/learner_concurrent.rs:126-146,
 // src/learner.rs:162-182) from the compact records.
 //
@@ -14,7 +15,9 @@
 #include <nccl.h>
 
 #include <mutex>
+#include <type_traits>
 
+#include "chess_engine.hpp"
 #include "engine.hpp"
 
 using namespace spb;
@@ -70,14 +73,145 @@ NcclApi* nccl_api() {
   } while (0)
 
 // Orders records by (global game id, ply): games finish in a nondeterministic order on the device and arrive rank by rank.
-void sort_records(std::vector<spb_position>& pos, std::vector<unsigned long long>& ids) {
+template <class Rec>
+void sort_records(std::vector<Rec>& pos, std::vector<unsigned long long>& ids) {
   const size_t n = pos.size();
   const std::vector<size_t> order = record_order(pos, ids);
-  std::vector<spb_position> p2(n);
+  std::vector<Rec> p2(n);
   std::vector<unsigned long long> i2(n);
   for (size_t i = 0; i < n; ++i) { p2[i] = pos[order[i]]; i2[i] = ids[order[i]]; }
   pos.swap(p2);
   ids.swap(i2);
+}
+
+// The engine types name their entry points in error texts.
+template <class Eng> const char* api_prefix() { return std::is_same<Eng, spb_chess_engine>::value ? "spb_chess_" : "spb_"; }
+
+// spb_comm_init / spb_chess_comm_init
+template <class Eng>
+int32_t comm_init(Eng* e, const uint8_t* id, int32_t rank, int32_t world_size) {
+  if (!e || !id) return SPB_ERR_ARG;
+  if (cudaSetDevice(e->cfg.device) != cudaSuccess) { e->set_error("cudaSetDevice failed"); return SPB_ERR_CUDA; }
+  if (world_size < 1 || rank < 0 || rank >= world_size) { e->set_error("rank / world_size out of range"); return SPB_ERR_ARG; }
+  if (e->nccl_comm) { e->set_error(std::string("communicator already initialised (") + api_prefix<Eng>() + "comm_destroy first)"); return SPB_ERR_STATE; }
+  NcclApi* N = nccl_api();
+  if (!N->error.empty()) { e->set_error(N->error); return SPB_ERR_STATE; }
+  ncclUniqueId u;
+  std::memcpy(&u, id, sizeof u);
+  ncclComm_t comm = nullptr;
+  SPB_NCCL(e, N->CommInitRank(&comm, world_size, u, rank));
+  e->nccl_comm = comm;
+  e->comm_rank = rank;
+  e->comm_world = world_size;
+  return SPB_OK;
+}
+
+// spb_comm_destroy / spb_chess_comm_destroy (also called by the engines' destroy)
+template <class Eng>
+int32_t comm_destroy(Eng* e) {
+  if (!e) return SPB_ERR_ARG;
+  if (e->nccl_comm) {
+    cudaSetDevice(e->cfg.device);
+    cudaStreamSynchronize(e->stream);
+    NcclApi* N = nccl_api();
+    if (N->CommDestroy) N->CommDestroy(static_cast<ncclComm_t>(e->nccl_comm));
+    e->nccl_comm = nullptr;
+    e->comm_rank = -1;
+    e->comm_world = 0;
+  }
+  return SPB_OK;
+}
+
+// spb_gather_trajectories / spb_chess_gather_trajectories over the engine's trajectory buffers P (record type Rec).  Everything
+// runs on e->stream: the self-play steps that filled P ran there, and the chess search's second stream rejoins it before
+// spb_chess_search returns.  Buffers not allocated yet (a chess engine that never played, P.out == NULL) take part with 0
+// records and stay unallocated.
+template <class Eng, class Rec>
+int32_t gather_trajectories(Eng* e, int32_t learner_rank, Rec* buf, size_t capacity, size_t* written, uint64_t* game_ids) {
+  if (!e || !written) return SPB_ERR_ARG;
+  if (cudaSetDevice(e->cfg.device) != cudaSuccess) { e->set_error("cudaSetDevice failed"); return SPB_ERR_CUDA; }
+  if (!e->nccl_comm) { e->set_error(std::string("no communicator: call ") + api_prefix<Eng>() + "comm_init first"); return SPB_ERR_STATE; }
+  if (learner_rank < 0 || learner_rank >= e->comm_world) { e->set_error("learner rank out of range"); return SPB_ERR_ARG; }
+  NcclApi* N = nccl_api();
+  ncclComm_t comm = static_cast<ncclComm_t>(e->nccl_comm);
+  const int rank = e->comm_rank, world = e->comm_world;
+  const bool learner = rank == learner_rank;
+  const auto& P = e->P;
+
+  if (!e->gather_pending) {
+    // ---- the collective: counts, then the records -----------------------------------------------------------------
+    unsigned long long n_local = 0;
+    if (P.out) {
+      SPB_CUDA_E(e, cudaMemcpyAsync(&n_local, P.out_cursor, 8, cudaMemcpyDeviceToHost, e->stream));
+      SPB_CUDA_E(e, cudaStreamSynchronize(e->stream));
+      n_local = std::min<unsigned long long>(n_local, P.out_cap);
+    }
+    unsigned long long* d_counts = nullptr;
+    SPB_CUDA_E(e, cudaMalloc((void**)&d_counts, (size_t)world * 8));
+    std::vector<unsigned long long> counts((size_t)world, 0);
+    cudaError_t ce = cudaMemcpyAsync(d_counts + rank, &n_local, 8, cudaMemcpyHostToDevice, e->stream);
+    ncclResult_t nr = ce == cudaSuccess ? N->AllGather(d_counts + rank, d_counts, 1, ncclUint64, comm, e->stream) : ncclSuccess;
+    if (ce == cudaSuccess && nr == ncclSuccess) ce = cudaMemcpyAsync(counts.data(), d_counts, (size_t)world * 8, cudaMemcpyDeviceToHost, e->stream);
+    if (ce == cudaSuccess && nr == ncclSuccess) ce = cudaStreamSynchronize(e->stream);
+    cudaFree(d_counts);
+    if (nr != ncclSuccess) { e->set_error(std::string("ncclAllGather: ") + N->GetErrorString(nr)); return SPB_ERR_CUDA; }
+    if (ce != cudaSuccess) { e->set_error(std::string("gather counts: ") + cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
+    size_t total = 0;
+    std::vector<size_t> off((size_t)world, 0);
+    for (int r = 0; r < world; ++r) { off[r] = total; total += (size_t)counts[r]; }
+
+    Rec* d_pos = nullptr;
+    unsigned long long* d_ids = nullptr;
+    if (learner && total) {
+      ce = cudaMalloc((void**)&d_pos, total * sizeof(Rec));
+      if (ce == cudaSuccess) ce = cudaMalloc((void**)&d_ids, total * 8);
+      if (ce != cudaSuccess) { if (d_pos) cudaFree(d_pos); e->set_error("gather: out of device memory"); return SPB_ERR_NOMEM; }
+    }
+    nr = N->GroupStart();
+    if (learner) {
+      for (int r = 0; r < world && nr == ncclSuccess; ++r) {
+        if (r == rank || counts[r] == 0) continue;
+        nr = N->Recv(d_pos + off[r], (size_t)counts[r] * sizeof(Rec), ncclUint8, r, comm, e->stream);
+        if (nr == ncclSuccess) nr = N->Recv(d_ids + off[r], (size_t)counts[r] * 8, ncclUint8, r, comm, e->stream);
+      }
+    } else if (n_local) {
+      nr = N->Send(P.out, (size_t)n_local * sizeof(Rec), ncclUint8, learner_rank, comm, e->stream);
+      if (nr == ncclSuccess) nr = N->Send(P.out_game, (size_t)n_local * 8, ncclUint8, learner_rank, comm, e->stream);
+    }
+    ncclResult_t nr2 = N->GroupEnd();
+    if (nr == ncclSuccess) nr = nr2;
+    ce = cudaSuccess;
+    if (learner && n_local) {
+      ce = cudaMemcpyAsync(d_pos + off[rank], P.out, (size_t)n_local * sizeof(Rec), cudaMemcpyDeviceToDevice, e->stream);
+      if (ce == cudaSuccess) ce = cudaMemcpyAsync(d_ids + off[rank], P.out_game, (size_t)n_local * 8, cudaMemcpyDeviceToDevice, e->stream);
+    }
+    if (ce == cudaSuccess && P.out) ce = cudaMemsetAsync(P.out_cursor, 0, 8, e->stream);   // the local buffer has been handed over
+    e->gather_pos.assign(learner ? total : 0, Rec{});
+    e->gather_ids.assign(learner ? total : 0, 0ull);
+    if (ce == cudaSuccess && learner && total) {
+      ce = cudaMemcpyAsync(e->gather_pos.data(), d_pos, total * sizeof(Rec), cudaMemcpyDeviceToHost, e->stream);
+      if (ce == cudaSuccess) ce = cudaMemcpyAsync(e->gather_ids.data(), d_ids, total * 8, cudaMemcpyDeviceToHost, e->stream);
+    }
+    if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
+    if (d_pos) cudaFree(d_pos);
+    if (d_ids) cudaFree(d_ids);
+    if (nr != ncclSuccess) { e->set_error(std::string("gather send/recv: ") + N->GetErrorString(nr)); return SPB_ERR_CUDA; }
+    if (ce != cudaSuccess) { e->set_error(std::string("gather: ") + cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
+    if (learner) sort_records(e->gather_pos, e->gather_ids);
+    e->gather_pending = true;
+  }
+  // ---- hand the gathered records to the caller (learner rank; the others hold none) ---------------------------------
+  const size_t n = e->gather_pos.size();
+  *written = n;
+  if (learner && n && (!buf || capacity < n)) return SPB_OK;       // size query: the records stay staged for the next call
+  if (n) {
+    std::memcpy(buf, e->gather_pos.data(), n * sizeof(Rec));
+    if (game_ids) std::memcpy(game_ids, e->gather_ids.data(), n * 8);
+  }
+  e->gather_pos.clear();
+  e->gather_ids.clear();
+  e->gather_pending = false;
+  return SPB_OK;
 }
 
 }  // namespace
@@ -95,120 +229,18 @@ int32_t spb_comm_unique_id(uint8_t* id) {
   return SPB_OK;
 }
 
-int32_t spb_comm_init(spb_engine* e, const uint8_t* id, int32_t rank, int32_t world_size) {
-  if (!e || !id) return SPB_ERR_ARG;
-  if (cudaSetDevice(e->cfg.device) != cudaSuccess) { e->set_error("cudaSetDevice failed"); return SPB_ERR_CUDA; }
-  if (world_size < 1 || rank < 0 || rank >= world_size) { e->set_error("rank / world_size out of range"); return SPB_ERR_ARG; }
-  if (e->nccl_comm) { e->set_error("communicator already initialised (spb_comm_destroy first)"); return SPB_ERR_STATE; }
-  NcclApi* N = nccl_api();
-  if (!N->error.empty()) { e->set_error(N->error); return SPB_ERR_STATE; }
-  ncclUniqueId u;
-  std::memcpy(&u, id, sizeof u);
-  ncclComm_t comm = nullptr;
-  SPB_NCCL(e, N->CommInitRank(&comm, world_size, u, rank));
-  e->nccl_comm = comm;
-  e->comm_rank = rank;
-  e->comm_world = world_size;
-  return SPB_OK;
-}
-
-int32_t spb_comm_destroy(spb_engine* e) {
-  if (!e) return SPB_ERR_ARG;
-  if (e->nccl_comm) {
-    cudaSetDevice(e->cfg.device);
-    cudaStreamSynchronize(e->stream);
-    NcclApi* N = nccl_api();
-    if (N->CommDestroy) N->CommDestroy(static_cast<ncclComm_t>(e->nccl_comm));
-    e->nccl_comm = nullptr;
-    e->comm_rank = -1;
-    e->comm_world = 0;
-  }
-  return SPB_OK;
-}
-
+int32_t spb_comm_init(spb_engine* e, const uint8_t* id, int32_t rank, int32_t world_size) { return comm_init(e, id, rank, world_size); }
+int32_t spb_comm_destroy(spb_engine* e) { return comm_destroy(e); }
 int32_t spb_gather_trajectories(spb_engine* e, int32_t learner_rank, spb_position* buf, size_t capacity, size_t* written,
                                 uint64_t* game_ids) {
-  if (!e || !written) return SPB_ERR_ARG;
-  if (cudaSetDevice(e->cfg.device) != cudaSuccess) { e->set_error("cudaSetDevice failed"); return SPB_ERR_CUDA; }
-  if (!e->nccl_comm) { e->set_error("no communicator: call spb_comm_init first"); return SPB_ERR_STATE; }
-  if (learner_rank < 0 || learner_rank >= e->comm_world) { e->set_error("learner rank out of range"); return SPB_ERR_ARG; }
-  NcclApi* N = nccl_api();
-  ncclComm_t comm = static_cast<ncclComm_t>(e->nccl_comm);
-  const int rank = e->comm_rank, world = e->comm_world;
-  const bool learner = rank == learner_rank;
+  return gather_trajectories(e, learner_rank, buf, capacity, written, game_ids);
+}
 
-  if (!e->gather_pending) {
-    // ---- the collective: counts, then the records -----------------------------------------------------------------
-    unsigned long long n_local = 0;
-    SPB_CUDA_E(e, cudaMemcpyAsync(&n_local, e->P.out_cursor, 8, cudaMemcpyDeviceToHost, e->stream));
-    SPB_CUDA_E(e, cudaStreamSynchronize(e->stream));
-    n_local = std::min<unsigned long long>(n_local, e->P.out_cap);
-    unsigned long long* d_counts = nullptr;
-    SPB_CUDA_E(e, cudaMalloc((void**)&d_counts, (size_t)world * 8));
-    std::vector<unsigned long long> counts((size_t)world, 0);
-    cudaError_t ce = cudaMemcpyAsync(d_counts + rank, &n_local, 8, cudaMemcpyHostToDevice, e->stream);
-    ncclResult_t nr = ce == cudaSuccess ? N->AllGather(d_counts + rank, d_counts, 1, ncclUint64, comm, e->stream) : ncclSuccess;
-    if (ce == cudaSuccess && nr == ncclSuccess) ce = cudaMemcpyAsync(counts.data(), d_counts, (size_t)world * 8, cudaMemcpyDeviceToHost, e->stream);
-    if (ce == cudaSuccess && nr == ncclSuccess) ce = cudaStreamSynchronize(e->stream);
-    cudaFree(d_counts);
-    if (nr != ncclSuccess) { e->set_error(std::string("ncclAllGather: ") + N->GetErrorString(nr)); return SPB_ERR_CUDA; }
-    if (ce != cudaSuccess) { e->set_error(std::string("gather counts: ") + cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
-    size_t total = 0;
-    std::vector<size_t> off((size_t)world, 0);
-    for (int r = 0; r < world; ++r) { off[r] = total; total += (size_t)counts[r]; }
-
-    spb_position* d_pos = nullptr;
-    unsigned long long* d_ids = nullptr;
-    if (learner && total) {
-      ce = cudaMalloc((void**)&d_pos, total * sizeof(spb_position));
-      if (ce == cudaSuccess) ce = cudaMalloc((void**)&d_ids, total * 8);
-      if (ce != cudaSuccess) { if (d_pos) cudaFree(d_pos); e->set_error("gather: out of device memory"); return SPB_ERR_NOMEM; }
-    }
-    nr = N->GroupStart();
-    if (learner) {
-      for (int r = 0; r < world && nr == ncclSuccess; ++r) {
-        if (r == rank || counts[r] == 0) continue;
-        nr = N->Recv(d_pos + off[r], (size_t)counts[r] * sizeof(spb_position), ncclUint8, r, comm, e->stream);
-        if (nr == ncclSuccess) nr = N->Recv(d_ids + off[r], (size_t)counts[r] * 8, ncclUint8, r, comm, e->stream);
-      }
-    } else if (n_local) {
-      nr = N->Send(e->P.out, (size_t)n_local * sizeof(spb_position), ncclUint8, learner_rank, comm, e->stream);
-      if (nr == ncclSuccess) nr = N->Send(e->P.out_game, (size_t)n_local * 8, ncclUint8, learner_rank, comm, e->stream);
-    }
-    ncclResult_t nr2 = N->GroupEnd();
-    if (nr == ncclSuccess) nr = nr2;
-    ce = cudaSuccess;
-    if (learner && n_local) {
-      ce = cudaMemcpyAsync(d_pos + off[rank], e->P.out, (size_t)n_local * sizeof(spb_position), cudaMemcpyDeviceToDevice, e->stream);
-      if (ce == cudaSuccess) ce = cudaMemcpyAsync(d_ids + off[rank], e->P.out_game, (size_t)n_local * 8, cudaMemcpyDeviceToDevice, e->stream);
-    }
-    if (ce == cudaSuccess) ce = cudaMemsetAsync(e->P.out_cursor, 0, 8, e->stream);   // the local buffer has been handed over
-    e->gather_pos.assign(learner ? total : 0, spb_position{});
-    e->gather_ids.assign(learner ? total : 0, 0ull);
-    if (ce == cudaSuccess && learner && total) {
-      ce = cudaMemcpyAsync(e->gather_pos.data(), d_pos, total * sizeof(spb_position), cudaMemcpyDeviceToHost, e->stream);
-      if (ce == cudaSuccess) ce = cudaMemcpyAsync(e->gather_ids.data(), d_ids, total * 8, cudaMemcpyDeviceToHost, e->stream);
-    }
-    if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
-    if (d_pos) cudaFree(d_pos);
-    if (d_ids) cudaFree(d_ids);
-    if (nr != ncclSuccess) { e->set_error(std::string("gather send/recv: ") + N->GetErrorString(nr)); return SPB_ERR_CUDA; }
-    if (ce != cudaSuccess) { e->set_error(std::string("gather: ") + cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
-    if (learner) sort_records(e->gather_pos, e->gather_ids);
-    e->gather_pending = true;
-  }
-  // ---- hand the gathered records to the caller (learner rank; the others hold none) ---------------------------------
-  const size_t n = e->gather_pos.size();
-  *written = n;
-  if (learner && n && (!buf || capacity < n)) return SPB_OK;       // size query: the records stay staged for the next call
-  if (n) {
-    std::memcpy(buf, e->gather_pos.data(), n * sizeof(spb_position));
-    if (game_ids) std::memcpy(game_ids, e->gather_ids.data(), n * 8);
-  }
-  e->gather_pos.clear();
-  e->gather_ids.clear();
-  e->gather_pending = false;
-  return SPB_OK;
+int32_t spb_chess_comm_init(spb_chess_engine* e, const uint8_t* id, int32_t rank, int32_t world_size) { return comm_init(e, id, rank, world_size); }
+int32_t spb_chess_comm_destroy(spb_chess_engine* e) { return comm_destroy(e); }
+int32_t spb_chess_gather_trajectories(spb_chess_engine* e, int32_t learner_rank, spb_chess_position* buf, size_t capacity, size_t* written,
+                                      uint64_t* game_ids) {
+  return gather_trajectories(e, learner_rank, buf, capacity, written, game_ids);
 }
 
 // ref: learner_concurrent.rs:126-146 / learner.rs:162-182 — the (N,3,R,C) / (N,A) / (N,1) training tensors.

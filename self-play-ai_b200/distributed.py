@@ -21,20 +21,22 @@ def shard_range(num_games_total: int, rank: int, world: int):
     return lo, lo + per + (1 if rank < extra else 0)
 
 
-def merge_trajectories(parts):
-    """parts: list of (positions[POSITION_DTYPE], game_ids[u64]) from every rank -> one (positions, ids)
-    ordered by (game id, ply)."""
-    pos = np.concatenate([p for p, _ in parts]) if parts else np.zeros(0, POSITION_DTYPE)
+def merge_trajectories(parts, dtype=POSITION_DTYPE):
+    """parts: list of (positions, game_ids[u64]) from every rank -> one (positions, ids) ordered by (game id, ply).  The
+    record type is that of the parts (POSITION_DTYPE, chess.CHESS_POSITION_DTYPE); `dtype` types an empty result."""
+    pos = np.concatenate([p for p, _ in parts]) if parts else np.zeros(0, dtype)
     ids = np.concatenate([g for _, g in parts]) if parts else np.zeros(0, np.uint64)
     order = np.lexsort((pos["ply"], ids))
     return pos[order], ids[order]
 
 
-def gather_records(pos: np.ndarray, ids: np.ndarray, dst: int = 0, device=None):
-    """Variable-length gather of (positions, game ids) to rank `dst` over the default process group."""
+def gather_records(pos: np.ndarray, ids: np.ndarray, dst: int = 0, device=None, dtype=None):
+    """Variable-length gather of (positions, game ids) to rank `dst` over the default process group.  The record type is
+    that of `pos` (POSITION_DTYPE or chess.CHESS_POSITION_DTYPE), or `dtype` when given; every rank passes the same."""
     import torch
     import torch.distributed as dist
 
+    dtype = np.dtype(dtype) if dtype is not None else (pos.dtype if pos.dtype.names else POSITION_DTYPE)
     world, rank = dist.get_world_size(), dist.get_rank()
     dev = device if device is not None else (torch.device("cuda", torch.cuda.current_device()) if dist.get_backend() == "nccl" else torch.device("cpu"))
     n = torch.tensor([len(pos)], dtype=torch.int64, device=dev)
@@ -42,23 +44,23 @@ def gather_records(pos: np.ndarray, ids: np.ndarray, dst: int = 0, device=None):
     dist.all_gather(counts, n)
     counts = [int(c.item()) for c in counts]
     cap = max(1, max(counts))
-    rec = POSITION_DTYPE.itemsize + 8
-    buf = np.zeros((cap, rec), np.uint8)
+    size = dtype.itemsize
+    buf = np.zeros((cap, size + 8), np.uint8)
     if len(pos):
-        buf[:len(pos), :POSITION_DTYPE.itemsize] = pos.view(np.uint8).reshape(len(pos), -1)
-        buf[:len(pos), POSITION_DTYPE.itemsize:] = np.ascontiguousarray(ids, dtype=np.uint64).view(np.uint8).reshape(len(pos), 8)
+        buf[:len(pos), :size] = np.ascontiguousarray(pos, dtype=dtype).view(np.uint8).reshape(len(pos), -1)
+        buf[:len(pos), size:] = np.ascontiguousarray(ids, dtype=np.uint64).view(np.uint8).reshape(len(pos), 8)
     mine = torch.from_numpy(buf).to(dev)
     out = [torch.zeros_like(mine) for _ in range(world)] if rank == dst else None
     dist.gather(mine, out, dst=dst)
     if rank != dst:
-        return np.zeros(0, POSITION_DTYPE), np.zeros(0, np.uint64)
+        return np.zeros(0, dtype), np.zeros(0, np.uint64)
     parts = []
     for r in range(world):
         a = out[r].cpu().numpy()[:counts[r]]
-        p = np.ascontiguousarray(a[:, :POSITION_DTYPE.itemsize]).view(POSITION_DTYPE).reshape(-1)
-        g = np.ascontiguousarray(a[:, POSITION_DTYPE.itemsize:]).view(np.uint64).reshape(-1)
+        p = np.ascontiguousarray(a[:, :size]).view(dtype).reshape(-1)
+        g = np.ascontiguousarray(a[:, size:]).view(np.uint64).reshape(-1)
         parts.append((p, g))
-    return merge_trajectories(parts)
+    return merge_trajectories(parts, dtype)
 
 
 def gather_trajectories(engine, dst: int = 0):

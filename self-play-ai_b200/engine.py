@@ -130,6 +130,10 @@ ABI = {
     "spb_chess_selfplay_step": (C.c_int32, [_vp, C.c_int32, C.c_float, C.c_uint64, _vp, _vp, _u32p]),
     "spb_chess_drain_trajectories": (C.c_int32, [_vp, _vp, C.c_size_t, C.POINTER(C.c_size_t), _vp]),
     "spb_chess_positions_to_training": (C.c_int32, [_vp, C.c_size_t, _vp, _vp, _vp]),
+    "spb_chess_positions_to_training_device": (C.c_int32, [_vp, _vp, C.c_size_t, _vp, C.c_size_t, _vp, _vp, _vp]),
+    "spb_chess_comm_init": (C.c_int32, [_vp, _vp, C.c_int32, C.c_int32]),
+    "spb_chess_comm_destroy": (C.c_int32, [_vp]),
+    "spb_chess_gather_trajectories": (C.c_int32, [_vp, C.c_int32, _vp, C.c_size_t, C.POINTER(C.c_size_t), _vp]),
     "spb_get_counters": (C.c_int32, [_vp, C.POINTER(Counters)]),
     "spb_reset_counters": (C.c_int32, [_vp]),
     "spb_last_search_timing": (C.c_int32, [_vp, _f32p, _f32p, _u32p]),
