@@ -203,6 +203,15 @@ int32_t spb_arena_len(spb_engine* e, uint32_t slot, uint32_t* out);
 int32_t spb_node_stats(spb_engine* e, uint32_t slot, uint32_t node_id, uint32_t* visit_count,
                        float* value_sum, float* prior, uint32_t* first_child, uint32_t* n_children);
 
+/* EXTENSION (not in the reference, mcts.rs:204-207 is a TODO): Dirichlet noise on the root priors; DESIGN.md §4.6.
+ * epsilon = 0 disables it (the default); otherwise 0 < epsilon <= 1 and alpha finite > 0, else SPB_ERR_ARG.
+ * Only the PUCT score of the root's children sees P' = (1 - epsilon) * P + epsilon * eta; stored priors never change.
+ * eta is a pure function of (seed, game id, root ply, number of root children). */
+int32_t spb_set_root_noise(spb_engine* e, float alpha, float epsilon, uint64_t seed);
+/* The eta the next search of `slot`'s current root uses (drawn if needed): eta[SPB_MAX_ACTIONS] in child order,
+ * *n = number of root children.  SPB_ERR_STATE while noise is off. */
+int32_t spb_root_noise(spb_engine* e, uint32_t slot, float* eta, uint32_t* n);
+
 /* ---- evaluator at the predict boundary (ref: Model::predict model/mod.rs:36-98) ---- */
 
 /*
@@ -351,6 +360,11 @@ int32_t spb_chess_arena_len(spb_chess_engine* e, uint32_t slot, uint32_t* out);
 /* Node fields (mcts.rs:20-30); status = SPB_STATUS_* (Ongoing until the node has been reached as a leaf). */
 int32_t spb_chess_node_stats(spb_chess_engine* e, uint32_t slot, uint32_t node_id, uint32_t* visit_count, float* value_sum, float* prior,
                              uint32_t* first_child, uint32_t* n_children, uint16_t* move, uint8_t* status);
+/* EXTENSION: spb_set_root_noise / spb_root_noise for chess trees (DESIGN.md §4.6).  The eta buffer (SPB_CHESS_MAX_MOVES floats
+ * per game) is allocated by the first call with epsilon > 0.  The game id is spb_config.game_id_base + slot until the first
+ * self-play step, then the slot's current game id; the root ply is spb_chess_state.plies. */
+int32_t spb_chess_set_root_noise(spb_chess_engine* e, float alpha, float epsilon, uint64_t seed);
+int32_t spb_chess_root_noise(spb_chess_engine* e, uint32_t slot, float* eta /* [SPB_CHESS_MAX_MOVES] */, uint32_t* n);
 /* Model::predict (model/mod.rs:36-98): policies[n][4672] = softmax masked to the legal moves and renormalised
  * (chess.rs:251-271), values[n], raw_logits[n][4672] (each nullable).  n <= num_games. */
 int32_t spb_chess_predict(spb_chess_engine* e, const spb_chess_state* states, const uint64_t* history, uint32_t n, float* policies, float* values,

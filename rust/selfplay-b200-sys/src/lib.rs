@@ -145,6 +145,10 @@ extern "C" {
     pub fn spb_get_state(e: *mut spb_engine, slot: u32, node_id: u32, out: *mut spb_state) -> i32;
     pub fn spb_arena_len(e: *mut spb_engine, slot: u32, out: *mut u32) -> i32;
     pub fn spb_node_stats(e: *mut spb_engine, slot: u32, node_id: u32, visit_count: *mut u32, value_sum: *mut f32, prior: *mut f32, first_child: *mut u32, n_children: *mut u32) -> i32;
+    /// EXTENSION (DESIGN.md §4.6): Dirichlet noise on the root priors; epsilon = 0 turns it off.
+    pub fn spb_set_root_noise(e: *mut spb_engine, alpha: f32, epsilon: f32, seed: u64) -> i32;
+    /// eta[SPB_MAX_ACTIONS] of the slot's current root (child order), *n = number of root children.
+    pub fn spb_root_noise(e: *mut spb_engine, slot: u32, eta: *mut f32, n: *mut u32) -> i32;
     pub fn spb_predict(e: *mut spb_engine, states: *const spb_state, n: u32, policies: *mut f32, values: *mut f32, raw_logits: *mut f32) -> i32;
     pub fn spb_game_next_states(e: *mut spb_engine, states: *const spb_state, actions: *const u8, n: u32, out_states: *mut spb_state, err: *mut i32) -> i32;
     pub fn spb_game_valid_actions(e: *mut spb_engine, states: *const spb_state, n: u32, masks: *mut u32) -> i32;
@@ -174,6 +178,9 @@ extern "C" {
     pub fn spb_chess_get_state(e: *mut spb_chess_engine, slot: u32, node_id: u32, out: *mut spb_chess_state) -> i32;
     pub fn spb_chess_arena_len(e: *mut spb_chess_engine, slot: u32, out: *mut u32) -> i32;
     pub fn spb_chess_node_stats(e: *mut spb_chess_engine, slot: u32, node_id: u32, visit_count: *mut u32, value_sum: *mut f32, prior: *mut f32, first_child: *mut u32, n_children: *mut u32, mv: *mut u16, status: *mut u8) -> i32;
+    pub fn spb_chess_set_root_noise(e: *mut spb_chess_engine, alpha: f32, epsilon: f32, seed: u64) -> i32;
+    /// eta[SPB_CHESS_MAX_MOVES] of the slot's current root (child order), *n = number of legal moves of the root.
+    pub fn spb_chess_root_noise(e: *mut spb_chess_engine, slot: u32, eta: *mut f32, n: *mut u32) -> i32;
     pub fn spb_chess_predict(e: *mut spb_chess_engine, states: *const spb_chess_state, history: *const u64, n: u32, policies: *mut f32, values: *mut f32, raw_logits: *mut f32) -> i32;
     pub fn spb_chess_time_conv(e: *mut spb_chess_engine, iters: u32, avg_ms: *mut f32, n_positions: *mut u32, flops_per_launch: *mut f64, flops_per_position: *mut f64) -> i32;
     pub fn spb_chess_get_counters(e: *mut spb_chess_engine, out: *mut spb_counters) -> i32;

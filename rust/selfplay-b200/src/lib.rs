@@ -70,6 +70,17 @@ impl<S: AbiState> Mcts<S> {
     pub fn load_weights(&mut self, safetensors: &[u8]) -> Result<()> {
         self.check(unsafe { sys::spb_load_weights(self.raw, safetensors.as_ptr() as *const _, safetensors.len()) })
     }
+    /// EXTENSION (not in the reference, mcts.rs:204-207 is a TODO; DESIGN.md §4.6): Dirichlet noise on the root priors of
+    /// every search, P' = (1 - epsilon) P + epsilon eta with eta ~ Dir(alpha).  epsilon = 0 turns it off (the default).
+    pub fn set_root_noise(&mut self, alpha: f32, epsilon: f32, seed: u64) -> Result<()> {
+        self.check(unsafe { sys::spb_set_root_noise(self.raw, alpha, epsilon, seed) })
+    }
+    /// The eta the next search of `tree`'s root uses, one entry per root child (child order).
+    pub fn root_noise(&mut self, tree: &Tree<S>) -> Result<Vec<f32>> {
+        let (mut eta, mut n) = ([0f32; sys::SPB_MAX_ACTIONS], 0u32);
+        self.check(unsafe { sys::spb_root_noise(self.raw, tree.slot, eta.as_mut_ptr(), &mut n) })?;
+        Ok(eta[..n as usize].to_vec())
+    }
     /// ref: `Tree::with_root_state` mcts.rs:86 / `Tree::default` mcts.rs:67.
     pub fn new_tree(&mut self, slot: u32, root: Option<&S>) -> Result<Tree<S>> {
         let abi = root.map(|s| s.to_abi());
@@ -249,6 +260,17 @@ impl ChessMcts {
         let n = history.len().min(sys::SPB_CHESS_MAX_HISTORY);
         h[..n].copy_from_slice(&history[..n]);
         h
+    }
+    /// EXTENSION (DESIGN.md §4.6): Dirichlet noise on the root priors, as `Mcts::set_root_noise`.
+    pub fn set_root_noise(&mut self, alpha: f32, epsilon: f32, seed: u64) -> Result<()> {
+        self.check(unsafe { sys::spb_chess_set_root_noise(self.raw, alpha, epsilon, seed) })
+    }
+    /// The eta the next search of `tree`'s root uses, one entry per legal move of the root (child order).
+    pub fn root_noise(&mut self, tree: &ChessTree) -> Result<Vec<f32>> {
+        let (mut eta, mut n) = (vec![0f32; sys::SPB_CHESS_MAX_MOVES], 0u32);
+        self.check(unsafe { sys::spb_chess_root_noise(self.raw, tree.slot, eta.as_mut_ptr(), &mut n) })?;
+        eta.truncate(n as usize);
+        Ok(eta)
     }
     /// ref: `Tree::with_root_state` mcts.rs:86.  `root = None`: the start position.
     pub fn new_tree(&mut self, slot: u32, root: Option<(&ChessState, &[u64])>) -> Result<ChessTree> {

@@ -201,6 +201,18 @@ class ChessEngine:
         self._chk(self._L.spb_chess_root_policy(self._h, slot, p.ctypes.data))
         return p
 
+    # ---- EXTENSION: Dirichlet noise at the root (DESIGN.md §4.6) ------------------------------
+    def set_root_noise(self, alpha: float, epsilon: float, seed: int = 0):
+        """P' = (1 - epsilon) P + epsilon eta, eta ~ Dir(alpha), at the root of every search; epsilon = 0 turns it off."""
+        self._chk(self._L.spb_chess_set_root_noise(self._h, alpha, epsilon, seed))
+
+    def root_noise(self, slot: int) -> np.ndarray:
+        """The eta the next search of `slot`'s root uses, one entry per legal move of the root (child order)."""
+        eta = np.zeros(MAX_MOVES, np.float32)
+        n = C.c_uint32()
+        self._chk(self._L.spb_chess_root_noise(self._h, slot, eta.ctypes.data_as(C.POINTER(C.c_float)), C.byref(n)))
+        return eta[:n.value].copy()
+
     def advance(self, child_ids, slots=None) -> np.ndarray:
         ids = np.ascontiguousarray(child_ids, dtype=np.uint32)
         sl = None if slots is None else np.ascontiguousarray(slots, dtype=np.uint32)

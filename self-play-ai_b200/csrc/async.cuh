@@ -266,7 +266,7 @@ __device__ __forceinline__ void tree_phase(const Trees& T, const AsyncCtl& C, ui
     uint32_t leaf, linfo;
     int depth;
     PState st;
-    descend<G, true>(rec, root, T.c, lane, path, leaf, depth, st, linfo, T.error, n_nodes);
+    descend<G, true>(rec, root, T.c, root_noise_of(T, g), lane, path, leaf, depth, st, linfo, T.error, n_nodes);
     SPB_ASSERT(T.error, leaf < n_nodes && depth < G::MAX_DEPTH, 3);
     ctr[CTR_SIMS] += 1;
     ctr[CTR_PATHSUM] += (unsigned)depth;

@@ -8,8 +8,11 @@
 //   Tree::with_root_state (:86-89)               -> restart_tree: k_chess_reset
 //   SelfPlayWorker::self_play
 //     (learner_concurrent.rs:169-242)            -> k_chess_selfplay_step (pick, record, end / re-root) + the drain
+#include <cfloat>
+
 #include "chess_engine.hpp"
 #include "chess_net.cuh"
+#include "root_noise.cuh"
 
 namespace spb {
 namespace chess {
@@ -89,7 +92,7 @@ __global__ void __launch_bounds__(THREADS) k_chess_search_fused(CTrees T, uint32
     Pos pos = root;
     uint32_t node, lmeta;
     int depth;
-    if (!descend(rec, meta, hash, T.c, lane, ws, pos, node, depth, lmeta, T.error)) break;
+    if (!descend(rec, meta, hash, T.c, root_noise_of(T, g), lane, ws, pos, node, depth, lmeta, T.error)) break;
     ctr[CTR_SIMS] += 1;
     ctr[CTR_PATHSUM] += (unsigned)depth;
     uint32_t st = meta_status(lmeta);
@@ -140,6 +143,28 @@ __global__ void __launch_bounds__(THREADS) k_chess_search_fused(CTrees T, uint32
   flush_counters(T, ctr, lane);
 }
 
+// EXTENSION (DESIGN.md §4.6): eta of every live root, one warp per slot, launched at the head of spb_chess_search (and by
+// spb_chess_root_noise).  n = the root's legal-move count; the game id is P.game_id[g], or game_id_base + g (the value that
+// array will hold) while the self-play buffers do not exist yet; the ply is the root's plies.
+__global__ void __launch_bounds__(THREADS) k_chess_root_noise(CTrees T, const unsigned long long* game_id, unsigned long long game_id_base, float alpha,
+                                                              unsigned long long seed) {
+  __shared__ WarpScratch s_ws[WARPS];
+  const int lane = threadIdx.x & 31;
+  WarpScratch& ws = s_ws[threadIdx.x >> 5];
+  const uint32_t g = blockIdx.x * WARPS + (threadIdx.x >> 5);
+  if (g >= T.G) return;
+  if (!T.live[g]) {
+    if (lane == 0) T.noise_n[g] = 0;
+    return;
+  }
+  const Pos root = T.root[g];
+  const uint32_t n = (uint32_t)warp_legal_moves(root, lane, ws, T.error);
+  const unsigned long long id = game_id ? game_id[g] : game_id_base + g;
+  warp_dirichlet<(MAX_MOVES + 31) / 32>(noise_key(seed, id, root.plies, n), n, alpha, lane, T.root_noise + (size_t)g * SPB_CHESS_MAX_MOVES,
+                                        SPB_CHESS_MAX_MOVES);
+  if (lane == 0) T.noise_n[g] = n;
+}
+
 // ---- lock-step pipeline for the network --------------------------------------------------------------------------
 // k_chess_select: the select of one simulation per tree; terminal leaves are backed up at once, the others are stored
 // with their legal moves as the tree's pending leaf and appended to the evaluator's work list (mcts.rs:236-252).
@@ -157,7 +182,7 @@ __global__ void __launch_bounds__(THREADS) k_chess_select(CTrees T, TreeRange R)
   Pos pos = T.root[g];
   uint32_t node, lmeta;
   int depth;
-  if (!descend(rec, meta, hash, T.c, lane, ws, pos, node, depth, lmeta, T.error)) return;
+  if (!descend(rec, meta, hash, T.c, root_noise_of(T, g), lane, ws, pos, node, depth, lmeta, T.error)) return;
   ctr[CTR_SIMS] += 1;
   ctr[CTR_PATHSUM] += (unsigned)depth;
   uint32_t st = meta_status(lmeta);
@@ -724,11 +749,56 @@ int32_t spb_chess_reset_games(spb_chess_engine* e, const uint32_t* slots, uint32
   return SPB_OK;
 }
 
+// EXTENSION (DESIGN.md §4.6): eta of every live root into T.root_noise (k_chess_root_noise).
+static int32_t launch_chess_root_noise(spb_chess_engine* e) {
+  ch::k_chess_root_noise<<<(e->T.G + ch::WARPS - 1) / ch::WARPS, ch::THREADS, 0, e->stream>>>(e->T, e->P.game_id, (unsigned long long)e->cfg.game_id_base,
+                                                                                             e->noise_alpha, e->noise_seed);
+  CH_CUDA(e, cudaGetLastError());
+  ++e->launches;
+  return SPB_OK;
+}
+
+int32_t spb_chess_set_root_noise(spb_chess_engine* e, float alpha, float epsilon, uint64_t seed) {
+  CH_GUARD(e);
+  CH_ARG(e, epsilon >= 0.0f && epsilon <= 1.0f, "root noise: epsilon must be in [0, 1]");
+  CH_ARG(e, epsilon == 0.0f || (alpha > 0.0f && alpha <= FLT_MAX), "root noise: alpha must be finite and > 0");
+  if (epsilon > 0.0f && !e->d_noise_eta) {                             // first use: an engine that never enables noise keeps its footprint
+    int32_t rc = e->dalloc(&e->d_noise_eta, (size_t)e->T.G * SPB_CHESS_MAX_MOVES);
+    if (!rc) rc = e->dalloc(&e->d_noise_n, (size_t)e->T.G);
+    if (rc) return rc;
+  }
+  CH_CUDA(e, cudaStreamSynchronize(e->stream));
+  e->noise_alpha = alpha;
+  e->noise_seed = seed;
+  e->T.noise_n = e->d_noise_n;
+  e->T.noise_eps = epsilon;
+  e->T.noise_omeps = 1.0f - epsilon;                                   // rounded to f32 once, here
+  e->T.root_noise = epsilon > 0.0f ? e->d_noise_eta : nullptr;
+  return SPB_OK;
+}
+
+int32_t spb_chess_root_noise(spb_chess_engine* e, uint32_t slot, float* eta, uint32_t* n) {
+  CH_GUARD(e);
+  CH_ARG(e, slot < e->T.G && eta && n, "bad argument");
+  if (!e->T.root_noise) { e->set_error("root noise is off (spb_chess_set_root_noise)"); return SPB_ERR_STATE; }
+  int32_t rc = launch_chess_root_noise(e);
+  if (rc) return rc;
+  uint32_t hn = 0;
+  CH_CUDA(e, cudaMemcpyAsync(eta, e->T.root_noise + (size_t)slot * SPB_CHESS_MAX_MOVES, SPB_CHESS_MAX_MOVES * 4, cudaMemcpyDeviceToHost, e->stream));
+  CH_CUDA(e, cudaMemcpyAsync(&hn, e->T.noise_n + slot, 4, cudaMemcpyDeviceToHost, e->stream));
+  rc = e->check_device_errors();                                       // synchronises the stream
+  if (rc) return rc;
+  for (uint32_t i = hn; i < SPB_CHESS_MAX_MOVES; ++i) eta[i] = 0.0f;
+  *n = hn;
+  return SPB_OK;
+}
+
 int32_t spb_chess_search(spb_chess_engine* e, uint32_t num_searches) {
   CH_GUARD(e);
   if (num_searches == 0) return SPB_OK;
   const uint32_t blocks = (e->T.G + ch::WARPS - 1) / ch::WARPS;
   CH_CUDA(e, cudaEventRecord(e->ev0, e->stream));
+  if (e->T.root_noise) { const int32_t rc = launch_chess_root_noise(e); if (rc) return rc; }   // eta of every root, before any descent
   const ch::TreeRange all{0u, e->T.G, e->T.eval_list, e->T.eval_count};
   if (e->cfg.evaluator == SPB_EVAL_NET) {
     CH_ARG(e, e->net && ch::net_loaded(e->net), "no weights loaded (spb_chess_load_weights)");

@@ -45,6 +45,12 @@ struct spb_chess_engine {
   bool gather_pending = false;
   std::vector<spb_chess_position> gather_pos;
   std::vector<unsigned long long> gather_ids;
+  // EXTENSION: Dirichlet noise at the root (spb_chess_set_root_noise).  [G][SPB_CHESS_MAX_MOVES] of eta, allocated by the first
+  // call that turns the noise on; T.root_noise points at it while it is on.
+  float* d_noise_eta = nullptr;
+  uint32_t* d_noise_n = nullptr;
+  float noise_alpha = 0.0f;
+  unsigned long long noise_seed = 0;
 
   void set_error(const std::string& s) { err = s; }
   template <class T_> int32_t dalloc(T_** p, size_t count) {

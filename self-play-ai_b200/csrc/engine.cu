@@ -1,5 +1,7 @@
 // engine.cu — the host engine and the C entry points that launch kernels (include/selfplay_b200.h).
 // Device code: kernels.cuh (tree / game / self-play kernels), async.cuh (asynchronous pipeline), evaluator_umma.cu.
+#include <cfloat>
+
 #include "kernels.cuh"
 
 
@@ -228,6 +230,7 @@ int32_t spb_engine::search_t(uint32_t num_searches) {
   const bool async = split && T.K == 1 && !(cfg.flags & SPB_FLAG_LOCKSTEP);
   SPB_CUDA(cudaEventRecord(ev0, stream));
   last_eval_launches = 0;
+  if (T.root_noise) { int32_t rc = launch_root_noise(); if (rc != SPB_OK) return rc; }   // eta of every root, before any descent
   if (async) {
     int32_t rc = search_async<G>(num_searches);
     if (rc != SPB_OK) return rc;
@@ -318,6 +321,16 @@ int32_t spb_engine::search_t(uint32_t num_searches) {
     return SPB_ERR_STATE;
   }
   return rc;
+}
+
+// EXTENSION (DESIGN.md §4.6): eta of every live root into T.root_noise (k_root_noise).
+int32_t spb_engine::launch_root_noise() {
+  const uint32_t blocks = (T.G + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK;
+  if (cfg.game == SPB_GAME_CONNECT4) k_root_noise<Connect4><<<blocks, THREADS, 0, stream>>>(T, P.game_id, noise_alpha, noise_seed);
+  else k_root_noise<TicTacToe><<<blocks, THREADS, 0, stream>>>(T, P.game_id, noise_alpha, noise_seed);
+  SPB_CHECK_LAUNCH();
+  ++launches;
+  return SPB_OK;
 }
 
 // One search through the asynchronous pipeline: rings reset, every live tree queued, ONE resident kernel until all trees
@@ -626,6 +639,44 @@ int32_t spb_get_state(spb_engine* e, uint32_t slot, uint32_t node_id, spb_state*
   if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
   if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
   *out = ps_to_abi(ps);
+  return SPB_OK;
+}
+
+int32_t spb_set_root_noise(spb_engine* e, float alpha, float epsilon, uint64_t seed) {
+  ENGINE_GUARD(e);
+  ARG_CHECK(e, epsilon >= 0.0f && epsilon <= 1.0f, "root noise: epsilon must be in [0, 1]");
+  ARG_CHECK(e, epsilon == 0.0f || (alpha > 0.0f && alpha <= FLT_MAX), "root noise: alpha must be finite and > 0");
+  if (epsilon > 0.0f && !e->d_noise_eta) {
+    int32_t rc = e->dalloc(&e->d_noise_eta, (size_t)e->T.G * SPB_MAX_ACTIONS);
+    if (!rc) rc = e->dalloc(&e->d_noise_n, (size_t)e->T.G);
+    if (rc) return rc;
+  }
+  cudaStreamSynchronize(e->stream);
+  e->noise_alpha = alpha;
+  e->noise_seed = seed;
+  e->T.noise_n = e->d_noise_n;
+  e->T.noise_eps = epsilon;
+  e->T.noise_omeps = 1.0f - epsilon;   // rounded to f32 once, here
+  e->T.root_noise = epsilon > 0.0f ? e->d_noise_eta : nullptr;
+  // the captured step graph holds the previous Trees (and with it the noise settings): the next search captures anew
+  if (e->step_graph) { cudaGraphExecDestroy(e->step_graph); e->step_graph = nullptr; }
+  return SPB_OK;
+}
+
+int32_t spb_root_noise(spb_engine* e, uint32_t slot, float* eta, uint32_t* n) {
+  ENGINE_GUARD(e);
+  ARG_CHECK(e, slot < e->T.G && eta && n, "bad argument");
+  if (!e->T.root_noise) { e->set_error("root noise is off (spb_set_root_noise)"); return SPB_ERR_STATE; }
+  int32_t rc = e->launch_root_noise();
+  if (rc) return rc;
+  float h[SPB_MAX_ACTIONS];
+  uint32_t hn = 0;
+  cudaError_t ce = cudaMemcpyAsync(h, e->T.root_noise + (size_t)slot * SPB_MAX_ACTIONS, sizeof h, cudaMemcpyDeviceToHost, e->stream);
+  if (ce == cudaSuccess) ce = cudaMemcpyAsync(&hn, e->T.noise_n + slot, 4, cudaMemcpyDeviceToHost, e->stream);
+  if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
+  if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
+  for (uint32_t i = 0; i < SPB_MAX_ACTIONS; ++i) eta[i] = i < hn ? h[i] : 0.0f;
+  *n = hn;
   return SPB_OK;
 }
 

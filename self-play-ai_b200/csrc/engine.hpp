@@ -81,6 +81,12 @@ struct spb_engine {
   std::vector<spb_position> gather_pos;
   std::vector<unsigned long long> gather_ids;
   int A = 0, max_depth = 0, eval_stride = 0, max_ply = 0;
+  // EXTENSION: Dirichlet noise at the root (spb_set_root_noise).  The buffers are allocated by the first call that turns
+  // the noise on; T.root_noise points at them while it is on.
+  float* d_noise_eta = nullptr;
+  uint32_t* d_noise_n = nullptr;
+  float noise_alpha = 0.0f;
+  unsigned long long noise_seed = 0;
 
   void set_error(const std::string& s) { err = s; }
 
@@ -116,6 +122,7 @@ struct spb_engine {
   template <class G> int32_t search_t(uint32_t num_searches);
   template <class G> int32_t launch_eval_step(uint32_t parity);
   template <class G> int32_t search_async(uint32_t num_searches);
+  int32_t launch_root_noise();
 };
 
 #define SPB_CHECK_LAUNCH() SPB_CUDA(cudaGetLastError())

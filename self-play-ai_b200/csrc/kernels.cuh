@@ -9,6 +9,7 @@
 //   * asynchronous (default for the network): async.cuh — tree warps inside the resident evaluator kernel.
 #pragma once
 #include "engine.hpp"
+#include "root_noise.cuh"
 
 namespace spb {
 
@@ -56,7 +57,7 @@ __global__ void __launch_bounds__(THREADS) k_search_fused(Trees T, uint32_t num_
     uint32_t leaf, linfo;
     int depth;
     PState st;
-    descend<G>(rec, root, T.c, lane, path, leaf, depth, st, linfo, T.error, n_nodes);
+    descend<G>(rec, root, T.c, root_noise_of(T, g), lane, path, leaf, depth, st, linfo, T.error, n_nodes);
     SPB_ASSERT(T.error, leaf < n_nodes && depth < G::MAX_DEPTH, 6);
     ctr[CTR_SIMS] += 1;
     ctr[CTR_PATHSUM] += (unsigned)depth;
@@ -81,6 +82,25 @@ __global__ void __launch_bounds__(THREADS) k_search_fused(Trees T, uint32_t num_
   }
   if (lane == 0) T.n_nodes[g] = n_nodes;
   flush_counters(T, ctr, lane);
+}
+
+// EXTENSION (DESIGN.md §4.6): eta of every live root, one warp per slot, launched at the head of spb_search (and by
+// spb_root_noise).  The draw depends on (seed, game id, root ply, number of legal moves) only, so repeated searches of one
+// root see the same eta and a new root (advance, self-play step, restart) gets a fresh one.  A terminal root has no children.
+template <class G>
+__global__ void __launch_bounds__(THREADS) k_root_noise(Trees T, const unsigned long long* game_id, float alpha, unsigned long long seed) {
+  const int lane = threadIdx.x & 31;
+  const uint32_t g = blockIdx.x * WARPS_PER_BLOCK + (threadIdx.x >> 5);
+  if (g >= T.G) return;
+  if (!T.live[g]) {
+    if (lane == 0) T.noise_n[g] = 0;
+    return;
+  }
+  const PState root = T.root_state[g];
+  const uint32_t n = ps_status(root) == SPB_STATUS_ONGOING ? (uint32_t)__popc(G::valid_mask(root)) : 0u;
+  const unsigned long long key = noise_key(seed, game_id[g], ps_num_actions(root), n);
+  warp_dirichlet<1>(key, n, alpha, lane, T.root_noise + (size_t)g * SPB_MAX_ACTIONS, SPB_MAX_ACTIONS);
+  if (lane == 0) T.noise_n[g] = n;
 }
 
 // Split pipeline.  do_finish: expand + backup the leaf whose evaluation is in eval_out.
@@ -186,7 +206,7 @@ __global__ void __launch_bounds__(THREADS) k_tree_step(Trees T, int do_finish, i
     uint32_t leaf, linfo;
     int depth;
     PState st;
-    descend<G>(rec, T.root_state[g], T.c, lane, path, leaf, depth, st, linfo, T.error, n_nodes);
+    descend<G>(rec, T.root_state[g], T.c, root_noise_of(T, g), lane, path, leaf, depth, st, linfo, T.error, n_nodes);
     SPB_ASSERT(T.error, leaf < n_nodes && depth < G::MAX_DEPTH, 7);
     WTRACE(3);
     ctr[CTR_SIMS] += 1;
@@ -287,7 +307,7 @@ __global__ void __launch_bounds__(THREADS) k_tree_step_multi(Trees T, int do_fin
       uint32_t leaf, linfo;
       int depth;
       PState st;
-      descend<G>(rec, root, T.c, lane, path, leaf, depth, st, linfo, T.error);
+      descend<G>(rec, root, T.c, root_noise_of(T, g), lane, path, leaf, depth, st, linfo, T.error);
       ctr[CTR_SIMS] += 1;
       ctr[CTR_PATHSUM] += (unsigned)depth;
       const uint32_t status = info_status(linfo);

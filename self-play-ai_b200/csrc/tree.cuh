@@ -74,7 +74,26 @@ struct Trees {
   float* eval_out;       // [G*K][EVAL_STRIDE]  probs (softmax, unmasked) + value
   unsigned long long* counters;  // [CTR_COUNT]
   uint32_t* error;       // [1]
+  // EXTENSION: Dirichlet noise at the root (root_noise.cuh, DESIGN.md §4.6).  root_noise is nullptr while the noise is off.
+  float* root_noise;     // [G][SPB_MAX_ACTIONS]  eta of the current root, child order (k_root_noise)
+  uint32_t* noise_n;     // [G]  number of root children eta was drawn for
+  float noise_eps, noise_omeps;   // epsilon and 1 - epsilon (rounded to f32 once, on the host)
 };
+
+// The root's noise as a descent sees it: the engine's eta array (nullptr -> the stored priors everywhere), the tree's row
+// of it and the two mixing weights.  The row's address is formed only at depth 0.
+struct RootNoise {
+  const float* eta;      // [G][stride]
+  uint32_t row;          // g * stride
+  float eps, omeps;
+};
+__device__ __forceinline__ RootNoise root_noise_of(const Trees& T, uint32_t g) {
+  return RootNoise{T.root_noise, g * (uint32_t)SPB_MAX_ACTIONS, T.noise_eps, T.noise_omeps};
+}
+// P' = (1 - eps) * P + eps * eta, each operation rounded (no FMA contraction); the stored prior is never modified.
+__device__ __forceinline__ float noisy_prior(float prior, float eta, float eps, float omeps) {
+  return __fadd_rn(__fmul_rn(omeps, prior), __fmul_rn(eps, eta));
+}
 
 // get_ucb, mcts.rs:91-100 — every operation individually rounded (no FMA contraction), evaluated in
 // the reference's order: q + ((c * prior) * sqrt(N_parent)) / (1 + N_child).
@@ -122,9 +141,10 @@ __device__ __forceinline__ NodeRec ld_rec(const NodeRec* p) {
 }
 
 // Descend from the root to a leaf (mcts.rs:237-241), replaying the moves on the bitboards.
-// All lanes return the same (leaf, depth, st, leaf_info).
+// All lanes return the same (leaf, depth, st, leaf_info).  With noise.eta set, the root's children (depth 0 only) are
+// scored with the noisy prior.
 template <class G, bool COHERENT = false>
-__device__ __forceinline__ void descend(const NodeRec* rec, const PState& root, float c, int lane,
+__device__ __forceinline__ void descend(const NodeRec* rec, const PState& root, float c, const RootNoise& noise, int lane,
                                         WarpPath& path, uint32_t& leaf, int& depth, PState& st, uint32_t& leaf_info,
                                         uint32_t* err, uint32_t n_nodes = 0xFFFFFFFFu) {
   NodeRec r0 = ld_rec<COHERENT>(rec);
@@ -142,7 +162,9 @@ __device__ __forceinline__ void descend(const NodeRec* rec, const PState& root, 
     SPB_ASSERT(err, fc + (uint32_t)nc <= n_nodes && nc <= G::A && depth + 1 < G::MAX_DEPTH, 1);
     if (lane < nc) {
       ch = ld_rec<COHERENT>(rec + fc + lane);                // 16-B vector load, children contiguous
-      score = puct_score(c, Np, ch.N, ch.W, ch.P);
+      float p = ch.P;
+      if (noise.eta != nullptr && depth == 0) p = noisy_prior(p, noise.eta[noise.row + lane], noise.eps, noise.omeps);
+      score = puct_score(c, Np, ch.N, ch.W, p);
       idx = lane;
       if (score != score) atomicOr(err, ERRBIT_NAN);         // the reference would panic (partial_cmp().unwrap())
     }

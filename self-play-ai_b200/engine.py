@@ -88,6 +88,8 @@ ABI = {
     "spb_get_state": (C.c_int32, [_vp, C.c_uint32, C.c_uint32, C.POINTER(State)]),
     "spb_arena_len": (C.c_int32, [_vp, C.c_uint32, _u32p]),
     "spb_node_stats": (C.c_int32, [_vp, C.c_uint32, C.c_uint32, _u32p, _f32p, _f32p, _u32p, _u32p]),
+    "spb_set_root_noise": (C.c_int32, [_vp, C.c_float, C.c_float, C.c_uint64]),
+    "spb_root_noise": (C.c_int32, [_vp, C.c_uint32, _f32p, _u32p]),
     "spb_predict": (C.c_int32, [_vp, _vp, C.c_uint32, _vp, _vp, _vp]),
     "spb_game_next_states": (C.c_int32, [_vp, _vp, _vp, C.c_uint32, _vp, _vp]),
     "spb_game_valid_actions": (C.c_int32, [_vp, _vp, C.c_uint32, _vp]),
@@ -123,6 +125,8 @@ ABI = {
     "spb_chess_get_state": (C.c_int32, [_vp, C.c_uint32, C.c_uint32, _vp]),
     "spb_chess_arena_len": (C.c_int32, [_vp, C.c_uint32, _u32p]),
     "spb_chess_node_stats": (C.c_int32, [_vp, C.c_uint32, C.c_uint32, _u32p, _f32p, _f32p, _u32p, _u32p, C.POINTER(C.c_uint16), _u8p]),
+    "spb_chess_set_root_noise": (C.c_int32, [_vp, C.c_float, C.c_float, C.c_uint64]),
+    "spb_chess_root_noise": (C.c_int32, [_vp, C.c_uint32, _f32p, _u32p]),
     "spb_chess_predict": (C.c_int32, [_vp, _vp, _vp, C.c_uint32, _vp, _vp, _vp]),
     "spb_chess_time_conv": (C.c_int32, [_vp, C.c_uint32, _f32p, _u32p, C.POINTER(C.c_double), C.POINTER(C.c_double)]),
     "spb_chess_get_counters": (C.c_int32, [_vp, C.POINTER(Counters)]),
@@ -330,6 +334,18 @@ class Engine:
         w, p = C.c_float(), C.c_float()
         self._chk(self._L.spb_node_stats(self._h, slot, node_id, C.byref(n), C.byref(w), C.byref(p), C.byref(fc), C.byref(nc)))
         return dict(visit_count=n.value, value_sum=w.value, prior=p.value, first_child=fc.value, n_children=nc.value)
+
+    # ---- EXTENSION: Dirichlet noise at the root (DESIGN.md §4.6) ------------------------------
+    def set_root_noise(self, alpha: float, epsilon: float, seed: int = 0):
+        """P' = (1 - epsilon) P + epsilon eta, eta ~ Dir(alpha), at the root of every search; epsilon = 0 turns it off."""
+        self._chk(self._L.spb_set_root_noise(self._h, alpha, epsilon, seed))
+
+    def root_noise(self, slot: int) -> np.ndarray:
+        """The eta the next search of `slot`'s root uses, one entry per root child (child order)."""
+        eta = np.zeros(MAX_ACTIONS, np.float32)
+        n = C.c_uint32()
+        self._chk(self._L.spb_root_noise(self._h, slot, eta.ctypes.data_as(_f32p), C.byref(n)))
+        return eta[:n.value].copy()
 
     # ---- evaluator / game rules --------------------------------------------------------------
     def predict(self, states, want_logits=False):

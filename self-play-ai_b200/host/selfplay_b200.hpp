@@ -117,6 +117,14 @@ class Mcts {
   // ref: tree.arena[id].state (learner_concurrent.rs:184,195; main.rs:92) and tree.arena.len()
   State node_state(const Tree& tree, size_t id) { State s; check(spb_get_state(e_, tree.slot, (uint32_t)id, &s.raw)); return s; }
   size_t arena_len(const Tree& tree) { uint32_t n = 0; check(spb_arena_len(e_, tree.slot, &n)); return n; }
+  // EXTENSION (DESIGN.md §4.6): Dirichlet noise on the root priors; epsilon = 0 turns it off.
+  void set_root_noise(float alpha, float epsilon, uint64_t seed) { check(spb_set_root_noise(e_, alpha, epsilon, seed)); }
+  std::vector<float> root_noise(const Tree& tree) {
+    float eta[SPB_MAX_ACTIONS];
+    uint32_t n = 0;
+    check(spb_root_noise(e_, tree.slot, eta, &n));
+    return std::vector<float>(eta, eta + n);
+  }
   uint8_t action_taken(const Tree& tree, size_t child_index) {     // node.action_taken of the root's child_index-th child (mcts.rs:25)
     uint8_t a[SPB_MAX_ACTIONS]; uint32_t n = 0;
     check(spb_root_children(e_, tree.slot, a, nullptr, nullptr, &n));
@@ -189,6 +197,15 @@ class ChessMcts {
     return mv;
   }
   uint64_t perft(const ChessState& s, uint32_t depth) { uint64_t n = 0; check(spb_chess_perft(e_, &s.raw, depth, &n)); return n; }
+  // EXTENSION (DESIGN.md §4.6): Dirichlet noise on the root priors, as Mcts::set_root_noise.
+  void set_root_noise(float alpha, float epsilon, uint64_t seed) { check(spb_chess_set_root_noise(e_, alpha, epsilon, seed)); }
+  std::vector<float> root_noise(const ChessTree& tree) {
+    std::vector<float> eta(SPB_CHESS_MAX_MOVES);
+    uint32_t n = 0;
+    check(spb_chess_root_noise(e_, tree.slot, eta.data(), &n));
+    eta.resize(n);
+    return eta;
+  }
   // ref: Mcts::search, mcts.rs:196-332: per tree [(child arena id, visit count)] with the children's moves.
   struct Result { std::vector<uint16_t> moves; std::vector<std::pair<size_t, float>> child_id_to_probs; };
   std::vector<Result> search(std::vector<ChessTree*>& trees) {
