@@ -279,10 +279,10 @@ int32_t spb_chess_positions_to_training(const spb_chess_position* positions, siz
 
 int32_t spb_chess_positions_to_training_device(spb_chess_engine* e, const spb_chess_position* positions, size_t n_positions,
                                                const uint64_t* indices, size_t n, float* encodings, float* policies, float* values) {
-  CH_GUARD(e);
-  CH_ARG(e, indices || n <= n_positions, "n > n_positions without indices");
+  SPB_GUARD(e);
+  SPB_ARG(e, indices || n <= n_positions, "n > n_positions without indices");
   if (n == 0) return SPB_OK;
-  CH_ARG(e, positions, "null positions");
+  SPB_ARG(e, positions, "null positions");
   const void* ptrs[5] = {positions, indices, encodings, policies, values};
   const char* names[5] = {"positions", "indices", "encodings", "policies", "values"};
   for (int k = 0; k < 5; ++k) {
@@ -291,21 +291,21 @@ int32_t spb_chess_positions_to_training_device(spb_chess_engine* e, const spb_ch
     const cudaError_t ce = cudaPointerGetAttributes(&a, ptrs[k]);
     if (ce != cudaSuccess) cudaGetLastError();
     const bool ok = ce == cudaSuccess && (a.type == cudaMemoryTypeManaged || (a.type == cudaMemoryTypeDevice && a.device == e->cfg.device));
-    CH_ARG(e, ok, std::string(names[k]) + " is not device memory of the engine's GPU");
+    SPB_ARG(e, ok, std::string(names[k]) + " is not device memory of the engine's GPU");
   }
   const unsigned long long none = ~0ull;
   unsigned long long* d_bad = e->d_misc;                               // the engine's scratch word; every call ends synchronised
   const auto* idx = reinterpret_cast<const unsigned long long*>(indices);
   int sms = 0;
-  CH_CUDA(e, cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, e->cfg.device));
-  CH_CUDA(e, cudaMemsetAsync(d_bad, 0xFF, 8, e->stream));
+  SPB_CUDA(e, cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, e->cfg.device));
+  SPB_CUDA(e, cudaMemsetAsync(d_bad, 0xFF, 8, e->stream));
   const unsigned long long check_blocks = std::min<unsigned long long>((n + 7) / 8, (unsigned long long)sms * 8);
   ch::k_chess_training_check<<<(unsigned)check_blocks, 256, 0, e->stream>>>(positions, n_positions, idx, n, d_bad);
-  CH_CUDA(e, cudaGetLastError());
+  SPB_CUDA(e, cudaGetLastError());
   ++e->launches;
   unsigned long long bad = none;
-  CH_CUDA(e, cudaMemcpyAsync(&bad, d_bad, 8, cudaMemcpyDeviceToHost, e->stream));
-  CH_CUDA(e, cudaStreamSynchronize(e->stream));
+  SPB_CUDA(e, cudaMemcpyAsync(&bad, d_bad, 8, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   if (bad != none) {
     e->set_error("malformed training row " + std::to_string(bad) +
                  (indices ? " (index out of range, or n_moves outside 1..256, side > 1 or a move outside the policy)"
@@ -315,17 +315,17 @@ int32_t spb_chess_positions_to_training_device(spb_chess_engine* e, const spb_ch
   const bool vec_enc = (reinterpret_cast<uintptr_t>(encodings) & 15) == 0, vec_pol = (reinterpret_cast<uintptr_t>(policies) & 15) == 0;
   const unsigned long long blocks = std::min<unsigned long long>(n, (unsigned long long)sms * 8);
   ch::k_chess_training<<<(unsigned)blocks, ch::TRAIN_THREADS, 0, e->stream>>>(positions, idx, n, encodings, policies, values, vec_enc, vec_pol);
-  CH_CUDA(e, cudaGetLastError());
+  SPB_CUDA(e, cudaGetLastError());
   ++e->launches;
-  CH_CUDA(e, cudaStreamSynchronize(e->stream));
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   return SPB_OK;
 }
 
 int32_t spb_chess_legal_moves(spb_chess_engine* e, const spb_chess_state* states, const uint64_t* history, uint32_t n, uint16_t* moves,
                               uint32_t* counts, uint16_t* policy_index, uint8_t* status, uint32_t* repetitions) {
-  CH_GUARD(e);
+  SPB_GUARD(e);
   if (n == 0) return SPB_OK;
-  if (!states) { e->set_error("null states"); return SPB_ERR_ARG; }
+  SPB_ARG(e, states, "null states");
   Scratch sc;
   auto* d_states = sc.alloc<ch::Pos>(n);
   auto* d_hist = history ? sc.alloc<uint64_t>((size_t)n * SPB_CHESS_MAX_HISTORY) : nullptr;
@@ -338,27 +338,27 @@ int32_t spb_chess_legal_moves(spb_chess_engine* e, const spb_chess_state* states
     e->set_error("chess: out of device memory");
     return SPB_ERR_NOMEM;
   }
-  CH_CUDA(e, cudaMemcpyAsync(d_states, states, (size_t)n * sizeof(ch::Pos), cudaMemcpyHostToDevice, e->stream));
-  if (history) CH_CUDA(e, cudaMemcpyAsync(d_hist, history, (size_t)n * SPB_CHESS_MAX_HISTORY * 8, cudaMemcpyHostToDevice, e->stream));
-  if (d_moves) CH_CUDA(e, cudaMemsetAsync(d_moves, 0xFF, (size_t)n * SPB_CHESS_MAX_MOVES * 2, e->stream));
-  if (d_pidx) CH_CUDA(e, cudaMemsetAsync(d_pidx, 0xFF, (size_t)n * SPB_CHESS_MAX_MOVES * 2, e->stream));
+  SPB_CUDA(e, cudaMemcpyAsync(d_states, states, (size_t)n * sizeof(ch::Pos), cudaMemcpyHostToDevice, e->stream));
+  if (history) SPB_CUDA(e, cudaMemcpyAsync(d_hist, history, (size_t)n * SPB_CHESS_MAX_HISTORY * 8, cudaMemcpyHostToDevice, e->stream));
+  if (d_moves) SPB_CUDA(e, cudaMemsetAsync(d_moves, 0xFF, (size_t)n * SPB_CHESS_MAX_MOVES * 2, e->stream));
+  if (d_pidx) SPB_CUDA(e, cudaMemsetAsync(d_pidx, 0xFF, (size_t)n * SPB_CHESS_MAX_MOVES * 2, e->stream));
   ch::k_legal<<<(n + 63) / 64, 64, 0, e->stream>>>(d_states, d_hist, n, d_moves, d_counts, d_pidx, d_status, d_reps);
-  CH_CUDA(e, cudaGetLastError());
+  SPB_CUDA(e, cudaGetLastError());
   ++e->launches;
-  if (moves) CH_CUDA(e, cudaMemcpyAsync(moves, d_moves, (size_t)n * SPB_CHESS_MAX_MOVES * 2, cudaMemcpyDeviceToHost, e->stream));
-  if (policy_index) CH_CUDA(e, cudaMemcpyAsync(policy_index, d_pidx, (size_t)n * SPB_CHESS_MAX_MOVES * 2, cudaMemcpyDeviceToHost, e->stream));
-  if (counts) CH_CUDA(e, cudaMemcpyAsync(counts, d_counts, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
-  if (repetitions) CH_CUDA(e, cudaMemcpyAsync(repetitions, d_reps, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
-  if (status) CH_CUDA(e, cudaMemcpyAsync(status, d_status, (size_t)n, cudaMemcpyDeviceToHost, e->stream));
-  CH_CUDA(e, cudaStreamSynchronize(e->stream));
+  if (moves) SPB_CUDA(e, cudaMemcpyAsync(moves, d_moves, (size_t)n * SPB_CHESS_MAX_MOVES * 2, cudaMemcpyDeviceToHost, e->stream));
+  if (policy_index) SPB_CUDA(e, cudaMemcpyAsync(policy_index, d_pidx, (size_t)n * SPB_CHESS_MAX_MOVES * 2, cudaMemcpyDeviceToHost, e->stream));
+  if (counts) SPB_CUDA(e, cudaMemcpyAsync(counts, d_counts, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
+  if (repetitions) SPB_CUDA(e, cudaMemcpyAsync(repetitions, d_reps, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
+  if (status) SPB_CUDA(e, cudaMemcpyAsync(status, d_status, (size_t)n, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   return SPB_OK;
 }
 
 int32_t spb_chess_next_states(spb_chess_engine* e, const spb_chess_state* states, uint64_t* history, const uint16_t* moves, uint32_t n,
                               spb_chess_state* out_states, int32_t* err) {
-  CH_GUARD(e);
+  SPB_GUARD(e);
   if (n == 0) return SPB_OK;
-  if (!states || !moves || !out_states || !err) { e->set_error("null argument"); return SPB_ERR_ARG; }
+  SPB_ARG(e, states && moves && out_states && err, "null argument");
   Scratch sc;
   auto* d_states = sc.alloc<ch::Pos>(n);
   auto* d_out = sc.alloc<ch::Pos>(n);
@@ -366,42 +366,42 @@ int32_t spb_chess_next_states(spb_chess_engine* e, const spb_chess_state* states
   auto* d_moves = sc.alloc<uint16_t>(n);
   auto* d_err = sc.alloc<int32_t>(n);
   if (!d_states || !d_out || (history && !d_hist) || !d_moves || !d_err) { e->set_error("chess: out of device memory"); return SPB_ERR_NOMEM; }
-  CH_CUDA(e, cudaMemcpyAsync(d_states, states, (size_t)n * sizeof(ch::Pos), cudaMemcpyHostToDevice, e->stream));
-  CH_CUDA(e, cudaMemcpyAsync(d_moves, moves, (size_t)n * 2, cudaMemcpyHostToDevice, e->stream));
-  if (history) CH_CUDA(e, cudaMemcpyAsync(d_hist, history, (size_t)n * SPB_CHESS_MAX_HISTORY * 8, cudaMemcpyHostToDevice, e->stream));
+  SPB_CUDA(e, cudaMemcpyAsync(d_states, states, (size_t)n * sizeof(ch::Pos), cudaMemcpyHostToDevice, e->stream));
+  SPB_CUDA(e, cudaMemcpyAsync(d_moves, moves, (size_t)n * 2, cudaMemcpyHostToDevice, e->stream));
+  if (history) SPB_CUDA(e, cudaMemcpyAsync(d_hist, history, (size_t)n * SPB_CHESS_MAX_HISTORY * 8, cudaMemcpyHostToDevice, e->stream));
   ch::k_next<<<(n + 63) / 64, 64, 0, e->stream>>>(d_states, d_hist, d_moves, n, d_out, d_err);
-  CH_CUDA(e, cudaGetLastError());
+  SPB_CUDA(e, cudaGetLastError());
   ++e->launches;
-  CH_CUDA(e, cudaMemcpyAsync(out_states, d_out, (size_t)n * sizeof(ch::Pos), cudaMemcpyDeviceToHost, e->stream));
-  CH_CUDA(e, cudaMemcpyAsync(err, d_err, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
-  if (history) CH_CUDA(e, cudaMemcpyAsync(history, d_hist, (size_t)n * SPB_CHESS_MAX_HISTORY * 8, cudaMemcpyDeviceToHost, e->stream));
-  CH_CUDA(e, cudaStreamSynchronize(e->stream));
+  SPB_CUDA(e, cudaMemcpyAsync(out_states, d_out, (size_t)n * sizeof(ch::Pos), cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaMemcpyAsync(err, d_err, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
+  if (history) SPB_CUDA(e, cudaMemcpyAsync(history, d_hist, (size_t)n * SPB_CHESS_MAX_HISTORY * 8, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   return SPB_OK;
 }
 
 int32_t spb_chess_encode(spb_chess_engine* e, const spb_chess_state* states, const uint64_t* history, uint32_t n, float* out) {
-  CH_GUARD(e);
+  SPB_GUARD(e);
   if (n == 0) return SPB_OK;
-  if (!states || !out) { e->set_error("null argument"); return SPB_ERR_ARG; }
+  SPB_ARG(e, states && out, "null argument");
   Scratch sc;
   auto* d_states = sc.alloc<ch::Pos>(n);
   auto* d_hist = history ? sc.alloc<uint64_t>((size_t)n * SPB_CHESS_MAX_HISTORY) : nullptr;
   auto* d_out = sc.alloc<float>((size_t)n * SPB_CHESS_PLANES * 64);
   if (!d_states || (history && !d_hist) || !d_out) { e->set_error("chess: out of device memory"); return SPB_ERR_NOMEM; }
-  CH_CUDA(e, cudaMemcpyAsync(d_states, states, (size_t)n * sizeof(ch::Pos), cudaMemcpyHostToDevice, e->stream));
-  if (history) CH_CUDA(e, cudaMemcpyAsync(d_hist, history, (size_t)n * SPB_CHESS_MAX_HISTORY * 8, cudaMemcpyHostToDevice, e->stream));
+  SPB_CUDA(e, cudaMemcpyAsync(d_states, states, (size_t)n * sizeof(ch::Pos), cudaMemcpyHostToDevice, e->stream));
+  if (history) SPB_CUDA(e, cudaMemcpyAsync(d_hist, history, (size_t)n * SPB_CHESS_MAX_HISTORY * 8, cudaMemcpyHostToDevice, e->stream));
   ch::k_encode<<<n, 128, 0, e->stream>>>(d_states, d_hist, n, d_out);
-  CH_CUDA(e, cudaGetLastError());
+  SPB_CUDA(e, cudaGetLastError());
   ++e->launches;
-  CH_CUDA(e, cudaMemcpyAsync(out, d_out, (size_t)n * SPB_CHESS_PLANES * 64 * 4, cudaMemcpyDeviceToHost, e->stream));
-  CH_CUDA(e, cudaStreamSynchronize(e->stream));
+  SPB_CUDA(e, cudaMemcpyAsync(out, d_out, (size_t)n * SPB_CHESS_PLANES * 64 * 4, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   return SPB_OK;
 }
 
 int32_t spb_chess_perft(spb_chess_engine* e, const spb_chess_state* state, uint32_t depth, uint64_t* nodes) {
-  CH_GUARD(e);
-  if (!state || !nodes) { e->set_error("null argument"); return SPB_ERR_ARG; }
-  if (depth > 8) { e->set_error("perft depth > 8"); return SPB_ERR_ARG; }
+  SPB_GUARD(e);
+  SPB_ARG(e, state && nodes, "null argument");
+  SPB_ARG(e, depth <= 8, "perft depth > 8");
   // Breadth first on the device while the frontier is too narrow to fill the GPU (or the rest too deep for one thread):
   // k_frontier_count gives every position its output offset, k_frontier_expand writes its children there.  Every
   // frontier position is then searched to the remaining depth by one device thread (k_perft).
@@ -410,21 +410,21 @@ int32_t spb_chess_perft(spb_chess_engine* e, const spb_chess_state* state, uint3
   ch::Pos* d_f = nullptr;
   if (cudaMalloc(&d_f, sizeof(ch::Pos)) != cudaSuccess || !d_total) { e->set_error("chess: out of device memory"); return SPB_ERR_NOMEM; }
   struct Free { ch::Pos*& p; ~Free() { cudaFree(p); } } free_f{d_f};
-  CH_CUDA(e, cudaMemcpyAsync(d_f, state, sizeof(ch::Pos), cudaMemcpyHostToDevice, e->stream));
+  SPB_CUDA(e, cudaMemcpyAsync(d_f, state, sizeof(ch::Pos), cudaMemcpyHostToDevice, e->stream));
   uint32_t n = 1, remaining = depth;
   while (remaining > 0 && (n < 4096 || remaining > (uint32_t)ch::PERFT_DEV_DEPTH)) {
     uint32_t* d_off = nullptr;
     if (cudaMalloc(&d_off, (size_t)n * 4) != cudaSuccess) { e->set_error("chess: out of device memory"); return SPB_ERR_NOMEM; }
     struct FreeOff { uint32_t* p; ~FreeOff() { cudaFree(p); } } free_off{d_off};
-    CH_CUDA(e, cudaMemsetAsync(d_total, 0, 8, e->stream));
+    SPB_CUDA(e, cudaMemsetAsync(d_total, 0, 8, e->stream));
     ch::k_frontier_count<<<(n + 63) / 64, 64, 0, e->stream>>>(d_f, n, d_off, d_total);
-    CH_CUDA(e, cudaGetLastError());
+    SPB_CUDA(e, cudaGetLastError());
     unsigned long long m = 0;
-    CH_CUDA(e, cudaMemcpyAsync(&m, d_total, 8, cudaMemcpyDeviceToHost, e->stream));
-    CH_CUDA(e, cudaStreamSynchronize(e->stream));
+    SPB_CUDA(e, cudaMemcpyAsync(&m, d_total, 8, cudaMemcpyDeviceToHost, e->stream));
+    SPB_CUDA(e, cudaStreamSynchronize(e->stream));
     e->launches += 1;
     if (m == 0) { *nodes = 0; return SPB_OK; }
-    if (m > (1ull << 23)) { e->set_error("perft frontier too large"); return SPB_ERR_ARG; }
+    SPB_ARG(e, m <= (1ull << 23), "perft frontier too large");
     ch::Pos* d_next = nullptr;
     if (cudaMalloc(&d_next, (size_t)m * sizeof(ch::Pos)) != cudaSuccess) { e->set_error("chess: out of device memory"); return SPB_ERR_NOMEM; }
     ch::k_frontier_expand<<<(n + 63) / 64, 64, 0, e->stream>>>(d_f, n, d_off, d_next);
@@ -432,18 +432,18 @@ int32_t spb_chess_perft(spb_chess_engine* e, const spb_chess_state* state, uint3
     cudaStreamSynchronize(e->stream);
     cudaFree(d_f);
     d_f = d_next;
-    CH_CUDA(e, err);
+    SPB_CUDA(e, err);
     e->launches += 1;
     n = (uint32_t)m;
     --remaining;
   }
-  CH_CUDA(e, cudaMemsetAsync(d_total, 0, 8, e->stream));
+  SPB_CUDA(e, cudaMemsetAsync(d_total, 0, 8, e->stream));
   ch::k_perft<<<(n + 63) / 64, 64, 0, e->stream>>>(d_f, n, (int)remaining, d_total);
-  CH_CUDA(e, cudaGetLastError());
+  SPB_CUDA(e, cudaGetLastError());
   ++e->launches;
   unsigned long long total = 0;
-  CH_CUDA(e, cudaMemcpyAsync(&total, d_total, 8, cudaMemcpyDeviceToHost, e->stream));
-  CH_CUDA(e, cudaStreamSynchronize(e->stream));
+  SPB_CUDA(e, cudaMemcpyAsync(&total, d_total, 8, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   *nodes = total;
   return SPB_OK;
 }

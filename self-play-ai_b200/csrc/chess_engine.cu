@@ -8,8 +8,6 @@
 //   Tree::with_root_state (:86-89)               -> restart_tree: k_chess_reset
 //   SelfPlayWorker::self_play
 //     (learner_concurrent.rs:169-242)            -> k_chess_selfplay_step (pick, record, end / re-root) + the drain
-#include <cfloat>
-
 #include "chess_engine.hpp"
 #include "chess_net.cuh"
 #include "root_noise.cuh"
@@ -602,150 +600,131 @@ __global__ void k_chess_nodes_live(CTrees T, unsigned long long* out) {
 using namespace spb;
 namespace ch = spb::chess;
 
-int32_t spb_chess_engine::check_device_errors() {
-  uint32_t bits = 0;
-  CH_CUDA(this, cudaMemcpyAsync(&bits, T.error, 4, cudaMemcpyDeviceToHost, stream));
-  CH_CUDA(this, cudaStreamSynchronize(stream));
-  if (!bits) return SPB_OK;
-  CH_CUDA(this, cudaMemsetAsync(T.error, 0, 4, stream));
-  if (bits & ERRBIT_POOL) { set_error("a chess tree outgrew max_nodes_per_tree"); return SPB_ERR_POOL; }
-  if (bits == ERRBIT_TRAJ_FULL) { set_error("trajectory buffer full: call spb_chess_drain_trajectories"); return SPB_ERR_STATE; }
-  set_error("chess kernel check failed, site " + std::to_string((bits >> 8) & 0xFF));
-  return SPB_ERR_STATE;
+// Everything but the self-play trajectories, which the first spb_chess_selfplay_step allocates.
+int32_t spb_chess_engine::init() {
+  int32_t rc = open_device();
+  if (rc) return rc;
+  SPB_CUDA(this, cudaStreamCreateWithFlags(&stream2, cudaStreamNonBlocking));
+  SPB_CUDA(this, cudaEventCreateWithFlags(&ev_fork, cudaEventDisableTiming));
+  SPB_CUDA(this, cudaEventCreateWithFlags(&ev_join, cudaEventDisableTiming));
+  T.G = cfg.num_games; T.cap = cfg.max_nodes_per_tree; T.c = cfg.c;
+  const size_t G = T.G, pool = G * (size_t)T.cap;
+  for (int b = 0; b < 2 && !rc; ++b) {
+    if (!rc) rc = dalloc(&T.rec[b], pool);
+    if (!rc) rc = dalloc(&T.meta[b], pool);
+    if (!rc) rc = dalloc(&T.hash[b], pool);
+  }
+  if (!rc) rc = dalloc(&T.root, G);
+  if (!rc) rc = dalloc(&T.root_hist, G * SPB_CHESS_MAX_HISTORY);
+  if (!rc) rc = dalloc(&T.n_nodes, G);
+  if (!rc) rc = dalloc(&T.buf, G);
+  if (!rc) rc = dalloc(&T.live, G);
+  if (!rc) rc = dalloc(&T.counters, (size_t)CTR_COUNT);
+  if (!rc) rc = dalloc(&T.error, 1);
+  if (!rc) rc = dalloc(&T.leaf_node, G);
+  if (!rc) rc = dalloc(&T.leaf_depth, G);
+  if (!rc) rc = dalloc(&T.path, G * ch::MAX_DEPTH);
+  if (!rc) rc = dalloc(&T.leaf_pos, G);
+  if (!rc) rc = dalloc(&T.leaf_moves, G * ch::MAX_MOVES);
+  if (!rc) rc = dalloc(&T.leaf_nmoves, G);
+  if (!rc) rc = dalloc(&T.leaf_reps, G);
+  if (!rc) rc = dalloc(&T.leaf_hash, G);
+  if (!rc) rc = dalloc(&T.eval_list, G);
+  if (!rc) rc = dalloc(&T.eval_count, 2);
+  if (!rc) rc = dalloc(&T.eval_value, G);
+  if (!rc && (cfg.evaluator == SPB_EVAL_NET || (cfg.flags & SPB_FLAG_FORCE_SPLIT))) rc = dalloc(&T.eval_logits, G * (size_t)ch::LOGIT_STRIDE);
+  if (!rc) rc = dalloc(&d_rc_moves, G * ch::MAX_MOVES);
+  if (!rc) rc = dalloc(&d_rc_counts, G * ch::MAX_MOVES);
+  if (!rc) rc = dalloc(&d_rc_ids, G * ch::MAX_MOVES);
+  if (!rc) rc = dalloc(&d_rc_n, G);
+  if (!rc) rc = dalloc(&d_misc, 4);
+  if (!rc) rc = dalloc(&d_reset_slots, G);
+  if (!rc) rc = dalloc(&d_reset_roots, G);
+  if (!rc) rc = dalloc(&d_reset_hist, G * SPB_CHESS_MAX_HISTORY);
+  if (!rc) rc = dalloc(&d_adv_ids, G);
+  if (!rc) rc = dalloc(&d_adv_err, G);
+  if (rc) return rc;
+  SPB_CUDA(this, cudaMemsetAsync(T.live, 0, G, stream));
+  SPB_CUDA(this, cudaMemsetAsync(T.buf, 0, G, stream));
+  SPB_CUDA(this, cudaMemsetAsync(T.n_nodes, 0, G * 4, stream));
+  SPB_CUDA(this, cudaMemsetAsync(T.leaf_depth, 0, G * 4, stream));
+  SPB_CUDA(this, cudaMemsetAsync(T.counters, 0, CTR_COUNT * 8, stream));
+  SPB_CUDA(this, cudaMemsetAsync(T.error, 0, 4, stream));
+  SPB_CUDA(this, cudaMemsetAsync(T.eval_count, 0, 8, stream));
+  SPB_CUDA(this, cudaStreamSynchronize(stream));
+  return SPB_OK;
+}
+
+// The second stream rejoins the first before every spb_chess_search returns, so the wait in HostEngine::release covers it.
+void spb_chess_engine::release() {
+  HostEngine::release();
+  ch::net_destroy(net);
+  if (stream2) cudaStreamDestroy(stream2);
+  if (ev_fork) cudaEventDestroy(ev_fork);
+  if (ev_join) cudaEventDestroy(ev_join);
 }
 
 extern "C" {
 
+// The checks of spb_chess_create beyond HostEngine::config_error (max_nodes_per_tree 0 already replaced by its default).
+static const char* config_error(const spb_config& c) {
+  if (const char* m = spb_chess_engine::config_error(c)) return m;
+  if (c.game != SPB_GAME_CHESS) return "spb_chess_create needs game = SPB_GAME_CHESS";
+  if (c.num_games == 0 || c.num_games > (1u << 20)) return "num_games out of range";
+  if (c.leaves_per_tree != 1) return "chess search runs one leaf per tree per step";
+  if (c.max_nodes_per_tree < 512 || c.max_nodes_per_tree > (1u << 24)) return "max_nodes_per_tree out of range";
+  return nullptr;
+}
+
 int32_t spb_chess_create(const spb_config* cfg, spb_chess_engine** out) {
   if (!cfg || !out) { g_create_error = "null argument"; return SPB_ERR_ARG; }
   *out = nullptr;
-  if (cfg->abi_version != SPB_ABI_VERSION) { g_create_error = "abi_version mismatch"; return SPB_ERR_ARG; }
-  if (cfg->game != SPB_GAME_CHESS) { g_create_error = "spb_chess_create needs game = SPB_GAME_CHESS"; return SPB_ERR_ARG; }
-  if (cfg->num_games == 0 || cfg->num_games > (1u << 20)) { g_create_error = "num_games out of range"; return SPB_ERR_ARG; }
-  if (cfg->leaves_per_tree != 1) { g_create_error = "chess search runs one leaf per tree per step"; return SPB_ERR_ARG; }
-  if (cfg->evaluator < SPB_EVAL_NET || cfg->evaluator > SPB_EVAL_UNIFORM) { g_create_error = "unknown evaluator"; return SPB_ERR_ARG; }
-  if (!(cfg->c == cfg->c)) { g_create_error = "c is NaN"; return SPB_ERR_ARG; }
-  spb_chess_engine* e = new (std::nothrow) spb_chess_engine();
-  if (!e) { g_create_error = "out of host memory"; return SPB_ERR_NOMEM; }
-  e->cfg = *cfg;
-  if (e->cfg.max_nodes_per_tree == 0) e->cfg.max_nodes_per_tree = 32768;
-  auto fail = [&](int32_t rc, const std::string& msg) {
-    g_create_error = msg;
-    spb_chess_destroy(e);
-    return rc;
-  };
-  if (e->cfg.max_nodes_per_tree < 512 || e->cfg.max_nodes_per_tree > (1u << 24)) return fail(SPB_ERR_ARG, "max_nodes_per_tree out of range");
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail(SPB_ERR_CUDA, "no CUDA device (this library has no CPU fallback)");
-  if (cfg->device < 0 || cfg->device >= ndev) return fail(SPB_ERR_ARG, "device ordinal out of range");
-  cudaDeviceProp prop;
-  if (cudaSetDevice(cfg->device) != cudaSuccess || cudaGetDeviceProperties(&prop, cfg->device) != cudaSuccess) return fail(SPB_ERR_CUDA, "cudaSetDevice failed");
-  if (prop.major != 10) return fail(SPB_ERR_CUDA, "device is not sm_100 (B200); this library is built for sm_100a only");
-  if (cudaStreamCreateWithFlags(&e->stream, cudaStreamNonBlocking) != cudaSuccess || cudaStreamCreateWithFlags(&e->stream2, cudaStreamNonBlocking) != cudaSuccess ||
-      cudaEventCreateWithFlags(&e->ev_fork, cudaEventDisableTiming) != cudaSuccess || cudaEventCreateWithFlags(&e->ev_join, cudaEventDisableTiming) != cudaSuccess ||
-      cudaEventCreate(&e->ev0) != cudaSuccess ||
-      cudaEventCreate(&e->ev1) != cudaSuccess)
-    return fail(SPB_ERR_CUDA, "stream / event creation failed");
-  ch::CTrees& T = e->T;
-  T.G = cfg->num_games; T.cap = e->cfg.max_nodes_per_tree; T.c = cfg->c;
-  const size_t G = T.G, pool = G * (size_t)T.cap;
-  int32_t rc = SPB_OK;
-  for (int b = 0; b < 2 && !rc; ++b) {
-    if (!rc) rc = e->dalloc(&T.rec[b], pool);
-    if (!rc) rc = e->dalloc(&T.meta[b], pool);
-    if (!rc) rc = e->dalloc(&T.hash[b], pool);
-  }
-  if (!rc) rc = e->dalloc(&T.root, G);
-  if (!rc) rc = e->dalloc(&T.root_hist, G * SPB_CHESS_MAX_HISTORY);
-  if (!rc) rc = e->dalloc(&T.n_nodes, G);
-  if (!rc) rc = e->dalloc(&T.buf, G);
-  if (!rc) rc = e->dalloc(&T.live, G);
-  if (!rc) rc = e->dalloc(&T.counters, (size_t)CTR_COUNT);
-  if (!rc) rc = e->dalloc(&T.error, 1);
-  if (!rc) rc = e->dalloc(&T.leaf_node, G);
-  if (!rc) rc = e->dalloc(&T.leaf_depth, G);
-  if (!rc) rc = e->dalloc(&T.path, G * ch::MAX_DEPTH);
-  if (!rc) rc = e->dalloc(&T.leaf_pos, G);
-  if (!rc) rc = e->dalloc(&T.leaf_moves, G * ch::MAX_MOVES);
-  if (!rc) rc = e->dalloc(&T.leaf_nmoves, G);
-  if (!rc) rc = e->dalloc(&T.leaf_reps, G);
-  if (!rc) rc = e->dalloc(&T.leaf_hash, G);
-  if (!rc) rc = e->dalloc(&T.eval_list, G);
-  if (!rc) rc = e->dalloc(&T.eval_count, 2);
-  if (!rc) rc = e->dalloc(&T.eval_value, G);
-  if (!rc && (cfg->evaluator == SPB_EVAL_NET || (cfg->flags & SPB_FLAG_FORCE_SPLIT))) rc = e->dalloc(&T.eval_logits, G * (size_t)ch::LOGIT_STRIDE);
-  if (!rc) rc = e->dalloc(&e->d_rc_moves, G * ch::MAX_MOVES);
-  if (!rc) rc = e->dalloc(&e->d_rc_counts, G * ch::MAX_MOVES);
-  if (!rc) rc = e->dalloc(&e->d_rc_ids, G * ch::MAX_MOVES);
-  if (!rc) rc = e->dalloc(&e->d_rc_n, G);
-  if (!rc) rc = e->dalloc(&e->d_misc, 4);
-  if (!rc) rc = e->dalloc(&e->d_reset_slots, G);
-  if (!rc) rc = e->dalloc(&e->d_reset_roots, G);
-  if (!rc) rc = e->dalloc(&e->d_reset_hist, G * SPB_CHESS_MAX_HISTORY);
-  if (!rc) rc = e->dalloc(&e->d_adv_ids, G);
-  if (!rc) rc = e->dalloc(&e->d_adv_err, G);
-  if (rc) return fail(rc, e->err);
-  cudaMemsetAsync(T.live, 0, G, e->stream);
-  cudaMemsetAsync(T.buf, 0, G, e->stream);
-  cudaMemsetAsync(T.n_nodes, 0, G * 4, e->stream);
-  cudaMemsetAsync(T.leaf_depth, 0, G * 4, e->stream);
-  cudaMemsetAsync(T.counters, 0, CTR_COUNT * 8, e->stream);
-  cudaMemsetAsync(T.error, 0, 4, e->stream);
-  cudaMemsetAsync(T.eval_count, 0, 8, e->stream);
-  if (cudaStreamSynchronize(e->stream) != cudaSuccess) return fail(SPB_ERR_CUDA, "device initialisation failed");
-  *out = e;
-  return SPB_OK;
+  spb_config c = *cfg;
+  if (c.max_nodes_per_tree == 0) c.max_nodes_per_tree = 32768;
+  if (const char* m = config_error(c)) { g_create_error = m; return SPB_ERR_ARG; }
+  return spb_chess_engine::create(c, out);
 }
 
 int32_t spb_chess_destroy(spb_chess_engine* e) {
   if (!e) return SPB_ERR_ARG;
-  cudaSetDevice(e->cfg.device);
-  if (e->stream) cudaStreamSynchronize(e->stream);
   spb_chess_comm_destroy(e);
-  ch::net_destroy(e->net);
-  for (void* p : e->allocs) cudaFree(p);
-  if (e->ev0) cudaEventDestroy(e->ev0);
-  if (e->ev1) cudaEventDestroy(e->ev1);
-  if (e->stream2) cudaStreamDestroy(e->stream2);
-  if (e->ev_fork) cudaEventDestroy(e->ev_fork);
-  if (e->ev_join) cudaEventDestroy(e->ev_join);
-  if (e->stream) cudaStreamDestroy(e->stream);
+  e->release();
   delete e;
   return SPB_OK;
 }
 
-const char* spb_chess_last_error(const spb_chess_engine* e) { return e ? e->err.c_str() : g_create_error.c_str(); }
+const char* spb_chess_last_error(const spb_chess_engine* e) { return spb_chess_engine::last_error(e); }
 
 // The roots of spb_chess_reset_games / spb_chess_selfplay_step (history: [n][SPB_CHESS_MAX_HISTORY], nullable).
 static int32_t check_roots(spb_chess_engine* e, const spb_chess_state* roots, const uint64_t* history, uint32_t n) {
   if (roots) for (uint32_t i = 0; i < n; ++i) {
-    CH_ARG(e, roots[i].side <= 1 && roots[i].ep <= 64, "malformed root state");
+    SPB_ARG(e, roots[i].side <= 1 && roots[i].ep <= 64, "malformed root state");
     uint64_t kings[2] = {roots[i].piece[5] & roots[i].color[0], roots[i].piece[5] & roots[i].color[1]};
-    CH_ARG(e, kings[0] && !(kings[0] & (kings[0] - 1)) && kings[1] && !(kings[1] & (kings[1] - 1)), "root state needs one king per side");
-    CH_ARG(e, history || roots[i].hist_len == 0, "root with hist_len > 0 needs its history");
-    CH_ARG(e, roots[i].hist_len <= SPB_CHESS_MAX_HISTORY, "hist_len > SPB_CHESS_MAX_HISTORY");
+    SPB_ARG(e, kings[0] && !(kings[0] & (kings[0] - 1)) && kings[1] && !(kings[1] & (kings[1] - 1)), "root state needs one king per side");
+    SPB_ARG(e, history || roots[i].hist_len == 0, "root with hist_len > 0 needs its history");
+    SPB_ARG(e, roots[i].hist_len <= SPB_CHESS_MAX_HISTORY, "hist_len > SPB_CHESS_MAX_HISTORY");
   }
   return SPB_OK;
 }
 
 int32_t spb_chess_reset_games(spb_chess_engine* e, const uint32_t* slots, uint32_t n, const spb_chess_state* roots, const uint64_t* history) {
-  CH_GUARD(e);
-  CH_ARG(e, n <= e->T.G, "more slots than games");
-  CH_ARG(e, !(history && !roots), "history without roots");
+  SPB_GUARD(e);
+  SPB_ARG(e, n <= e->T.G, "more slots than games");
+  SPB_ARG(e, !(history && !roots), "history without roots");
   if (n == 0) return SPB_OK;
-  if (slots) for (uint32_t i = 0; i < n; ++i) CH_ARG(e, slots[i] < e->T.G, "slot out of range");
+  if (slots) for (uint32_t i = 0; i < n; ++i) SPB_ARG(e, slots[i] < e->T.G, "slot out of range");
   const int32_t rc = check_roots(e, roots, history, n);
   if (rc) return rc;
   uint32_t* d_slots = slots ? e->d_reset_slots : nullptr;
   ch::Pos* d_roots = roots ? e->d_reset_roots : nullptr;
   unsigned long long* d_hist = history ? e->d_reset_hist : nullptr;
-  if (slots) CH_CUDA(e, cudaMemcpyAsync(d_slots, slots, (size_t)n * 4, cudaMemcpyHostToDevice, e->stream));
-  if (roots) CH_CUDA(e, cudaMemcpyAsync(d_roots, roots, (size_t)n * sizeof(ch::Pos), cudaMemcpyHostToDevice, e->stream));
-  if (history) CH_CUDA(e, cudaMemcpyAsync(d_hist, history, (size_t)n * SPB_CHESS_MAX_HISTORY * 8, cudaMemcpyHostToDevice, e->stream));
+  if (slots) SPB_CUDA(e, cudaMemcpyAsync(d_slots, slots, (size_t)n * 4, cudaMemcpyHostToDevice, e->stream));
+  if (roots) SPB_CUDA(e, cudaMemcpyAsync(d_roots, roots, (size_t)n * sizeof(ch::Pos), cudaMemcpyHostToDevice, e->stream));
+  if (history) SPB_CUDA(e, cudaMemcpyAsync(d_hist, history, (size_t)n * SPB_CHESS_MAX_HISTORY * 8, cudaMemcpyHostToDevice, e->stream));
   ch::k_chess_reset<<<n, 64, 0, e->stream>>>(e->T, e->P, d_slots, d_roots, d_hist, n);
-  CH_CUDA(e, cudaGetLastError());
+  SPB_CUDA(e, cudaGetLastError());
   ++e->launches;
-  CH_CUDA(e, cudaStreamSynchronize(e->stream));
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   return SPB_OK;
 }
 
@@ -753,55 +732,30 @@ int32_t spb_chess_reset_games(spb_chess_engine* e, const uint32_t* slots, uint32
 static int32_t launch_chess_root_noise(spb_chess_engine* e) {
   ch::k_chess_root_noise<<<(e->T.G + ch::WARPS - 1) / ch::WARPS, ch::THREADS, 0, e->stream>>>(e->T, e->P.game_id, (unsigned long long)e->cfg.game_id_base,
                                                                                              e->noise_alpha, e->noise_seed);
-  CH_CUDA(e, cudaGetLastError());
+  SPB_CUDA(e, cudaGetLastError());
   ++e->launches;
   return SPB_OK;
 }
 
 int32_t spb_chess_set_root_noise(spb_chess_engine* e, float alpha, float epsilon, uint64_t seed) {
-  CH_GUARD(e);
-  CH_ARG(e, epsilon >= 0.0f && epsilon <= 1.0f, "root noise: epsilon must be in [0, 1]");
-  CH_ARG(e, epsilon == 0.0f || (alpha > 0.0f && alpha <= FLT_MAX), "root noise: alpha must be finite and > 0");
-  if (epsilon > 0.0f && !e->d_noise_eta) {                             // first use: an engine that never enables noise keeps its footprint
-    int32_t rc = e->dalloc(&e->d_noise_eta, (size_t)e->T.G * SPB_CHESS_MAX_MOVES);
-    if (!rc) rc = e->dalloc(&e->d_noise_n, (size_t)e->T.G);
-    if (rc) return rc;
-  }
-  CH_CUDA(e, cudaStreamSynchronize(e->stream));
-  e->noise_alpha = alpha;
-  e->noise_seed = seed;
-  e->T.noise_n = e->d_noise_n;
-  e->T.noise_eps = epsilon;
-  e->T.noise_omeps = 1.0f - epsilon;                                   // rounded to f32 once, here
-  e->T.root_noise = epsilon > 0.0f ? e->d_noise_eta : nullptr;
-  return SPB_OK;
+  SPB_GUARD(e);
+  return e->set_root_noise(alpha, epsilon, seed, SPB_CHESS_MAX_MOVES);
 }
 
 int32_t spb_chess_root_noise(spb_chess_engine* e, uint32_t slot, float* eta, uint32_t* n) {
-  CH_GUARD(e);
-  CH_ARG(e, slot < e->T.G && eta && n, "bad argument");
-  if (!e->T.root_noise) { e->set_error("root noise is off (spb_chess_set_root_noise)"); return SPB_ERR_STATE; }
-  int32_t rc = launch_chess_root_noise(e);
-  if (rc) return rc;
-  uint32_t hn = 0;
-  CH_CUDA(e, cudaMemcpyAsync(eta, e->T.root_noise + (size_t)slot * SPB_CHESS_MAX_MOVES, SPB_CHESS_MAX_MOVES * 4, cudaMemcpyDeviceToHost, e->stream));
-  CH_CUDA(e, cudaMemcpyAsync(&hn, e->T.noise_n + slot, 4, cudaMemcpyDeviceToHost, e->stream));
-  rc = e->check_device_errors();                                       // synchronises the stream
-  if (rc) return rc;
-  for (uint32_t i = hn; i < SPB_CHESS_MAX_MOVES; ++i) eta[i] = 0.0f;
-  *n = hn;
-  return SPB_OK;
+  SPB_GUARD(e);
+  return e->root_noise(slot, eta, n, SPB_CHESS_MAX_MOVES, [e] { return launch_chess_root_noise(e); });
 }
 
 int32_t spb_chess_search(spb_chess_engine* e, uint32_t num_searches) {
-  CH_GUARD(e);
+  SPB_GUARD(e);
   if (num_searches == 0) return SPB_OK;
   const uint32_t blocks = (e->T.G + ch::WARPS - 1) / ch::WARPS;
-  CH_CUDA(e, cudaEventRecord(e->ev0, e->stream));
+  SPB_CUDA(e, cudaEventRecord(e->ev0, e->stream));
   if (e->T.root_noise) { const int32_t rc = launch_chess_root_noise(e); if (rc) return rc; }   // eta of every root, before any descent
   const ch::TreeRange all{0u, e->T.G, e->T.eval_list, e->T.eval_count};
   if (e->cfg.evaluator == SPB_EVAL_NET) {
-    CH_ARG(e, e->net && ch::net_loaded(e->net), "no weights loaded (spb_chess_load_weights)");
+    SPB_ARG(e, e->net && ch::net_loaded(e->net), "no weights loaded (spb_chess_load_weights)");
     // mcts.rs:214: one evaluator batch per simulation step.  Trees never interact, so the lock-step loop runs separately
     // over the two halves of the trees, on two streams: while the convolutions of one half hold the tensor pipes, the
     // select / expand + backup kernels of the other half run in the SMs' spare issue slots and shared memory (a k_conv CTA
@@ -812,22 +766,22 @@ int32_t spb_chess_search(spb_chess_engine* e, uint32_t num_searches) {
     const int nh = split ? 2 : 1;
     cudaStream_t st[2] = {e->stream, e->stream2};
     if (split) {
-      CH_CUDA(e, cudaEventRecord(e->ev_fork, e->stream));
-      CH_CUDA(e, cudaStreamWaitEvent(e->stream2, e->ev_fork, 0));
+      SPB_CUDA(e, cudaEventRecord(e->ev_fork, e->stream));
+      SPB_CUDA(e, cudaStreamWaitEvent(e->stream2, e->ev_fork, 0));
     }
     auto enqueue = [&]() -> int32_t {
       for (uint32_t s = 0; s < num_searches; ++s) {
         for (int h = 0; h < nh; ++h) {
           const ch::TreeRange& R = half[h];
           const uint32_t hb = (R.g1 - R.g0 + ch::WARPS - 1) / ch::WARPS;
-          CH_CUDA(e, cudaMemsetAsync(R.count, 0, 4, st[h]));
+          SPB_CUDA(e, cudaMemsetAsync(R.count, 0, 4, st[h]));
           ch::k_chess_select<<<hb, ch::THREADS, 0, st[h]>>>(e->T, R);
-          CH_CUDA(e, cudaGetLastError());
+          SPB_CUDA(e, cudaGetLastError());
           uint32_t launched = 0;
           const int32_t rc = ch::net_forward_leaves(e, h, R.list, R.count, st[h], &launched);
           if (rc) return rc;
           ch::k_chess_finish<false><<<hb, ch::THREADS, 0, st[h]>>>(e->T, R);
-          CH_CUDA(e, cudaGetLastError());
+          SPB_CUDA(e, cudaGetLastError());
           e->launches += 2 + launched;
         }
       }
@@ -843,81 +797,81 @@ int32_t spb_chess_search(spb_chess_engine* e, uint32_t num_searches) {
   } else if (e->cfg.flags & SPB_FLAG_FORCE_SPLIT) {
     // parity harness: the built-in evaluators through the kernels of the network pipeline (select -> evaluate -> finish)
     for (uint32_t s = 0; s < num_searches; ++s) {
-      CH_CUDA(e, cudaMemsetAsync(e->T.eval_count, 0, 4, e->stream));
+      SPB_CUDA(e, cudaMemsetAsync(e->T.eval_count, 0, 4, e->stream));
       ch::k_chess_select<<<blocks, ch::THREADS, 0, e->stream>>>(e->T, all);
       if (e->cfg.evaluator == SPB_EVAL_DET) ch::k_chess_builtin_eval<SPB_EVAL_DET><<<blocks, ch::THREADS, 0, e->stream>>>(e->T, all);
       else ch::k_chess_builtin_eval<SPB_EVAL_UNIFORM><<<blocks, ch::THREADS, 0, e->stream>>>(e->T, all);
       ch::k_chess_finish<true><<<blocks, ch::THREADS, 0, e->stream>>>(e->T, all);
-      CH_CUDA(e, cudaGetLastError());
+      SPB_CUDA(e, cudaGetLastError());
       e->launches += 3;
     }
   } else {
     if (e->cfg.evaluator == SPB_EVAL_DET) ch::k_chess_search_fused<SPB_EVAL_DET><<<blocks, ch::THREADS, 0, e->stream>>>(e->T, num_searches);
     else ch::k_chess_search_fused<SPB_EVAL_UNIFORM><<<blocks, ch::THREADS, 0, e->stream>>>(e->T, num_searches);
-    CH_CUDA(e, cudaGetLastError());
+    SPB_CUDA(e, cudaGetLastError());
     ++e->launches;
   }
-  CH_CUDA(e, cudaEventRecord(e->ev1, e->stream));
+  SPB_CUDA(e, cudaEventRecord(e->ev1, e->stream));
   const int32_t rc = e->check_device_errors();
   if (rc) return rc;
-  CH_CUDA(e, cudaEventElapsedTime(&e->last_search_ms, e->ev0, e->ev1));
+  SPB_CUDA(e, cudaEventElapsedTime(&e->last_search_ms, e->ev0, e->ev1));
   return SPB_OK;
 }
 
 int32_t spb_chess_last_search_ms(spb_chess_engine* e, float* ms) {
-  CH_GUARD(e);
-  CH_ARG(e, ms, "null argument");
+  SPB_GUARD(e);
+  SPB_ARG(e, ms, "null argument");
   *ms = e->last_search_ms;
   return SPB_OK;
 }
 
 static int32_t fetch_root_children(spb_chess_engine* e) {
   ch::k_chess_root_children<<<e->T.G, 64, 0, e->stream>>>(e->T, e->d_rc_moves, e->d_rc_counts, e->d_rc_ids, e->d_rc_n);
-  CH_CUDA(e, cudaGetLastError());
+  SPB_CUDA(e, cudaGetLastError());
   ++e->launches;
   return SPB_OK;
 }
 
 int32_t spb_chess_root_children_all(spb_chess_engine* e, uint16_t* moves, uint32_t* visit_counts, uint32_t* child_ids, uint32_t* n_children) {
-  CH_GUARD(e);
+  SPB_GUARD(e);
   int32_t rc = fetch_root_children(e);
   if (rc) return rc;
   const size_t G = e->T.G, M = ch::MAX_MOVES;
-  if (moves) CH_CUDA(e, cudaMemcpyAsync(moves, e->d_rc_moves, G * M * 2, cudaMemcpyDeviceToHost, e->stream));
-  if (visit_counts) CH_CUDA(e, cudaMemcpyAsync(visit_counts, e->d_rc_counts, G * M * 4, cudaMemcpyDeviceToHost, e->stream));
-  if (child_ids) CH_CUDA(e, cudaMemcpyAsync(child_ids, e->d_rc_ids, G * M * 4, cudaMemcpyDeviceToHost, e->stream));
-  if (n_children) CH_CUDA(e, cudaMemcpyAsync(n_children, e->d_rc_n, G * 4, cudaMemcpyDeviceToHost, e->stream));
-  CH_CUDA(e, cudaStreamSynchronize(e->stream));
+  if (moves) SPB_CUDA(e, cudaMemcpyAsync(moves, e->d_rc_moves, G * M * 2, cudaMemcpyDeviceToHost, e->stream));
+  if (visit_counts) SPB_CUDA(e, cudaMemcpyAsync(visit_counts, e->d_rc_counts, G * M * 4, cudaMemcpyDeviceToHost, e->stream));
+  if (child_ids) SPB_CUDA(e, cudaMemcpyAsync(child_ids, e->d_rc_ids, G * M * 4, cudaMemcpyDeviceToHost, e->stream));
+  if (n_children) SPB_CUDA(e, cudaMemcpyAsync(n_children, e->d_rc_n, G * 4, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   return SPB_OK;
 }
 
 int32_t spb_chess_root_children(spb_chess_engine* e, uint32_t slot, uint16_t* moves, uint32_t* visit_counts, uint32_t* child_ids, uint32_t* n_children) {
-  CH_GUARD(e);
-  CH_ARG(e, slot < e->T.G, "slot out of range");
-  CH_ARG(e, n_children, "null argument");
+  SPB_GUARD(e);
+  SPB_ARG(e, slot < e->T.G, "slot out of range");
+  SPB_ARG(e, n_children, "null argument");
   int32_t rc = fetch_root_children(e);
   if (rc) return rc;
   const size_t M = ch::MAX_MOVES;
-  if (moves) CH_CUDA(e, cudaMemcpyAsync(moves, e->d_rc_moves + slot * M, M * 2, cudaMemcpyDeviceToHost, e->stream));
-  if (visit_counts) CH_CUDA(e, cudaMemcpyAsync(visit_counts, e->d_rc_counts + slot * M, M * 4, cudaMemcpyDeviceToHost, e->stream));
-  if (child_ids) CH_CUDA(e, cudaMemcpyAsync(child_ids, e->d_rc_ids + slot * M, M * 4, cudaMemcpyDeviceToHost, e->stream));
-  CH_CUDA(e, cudaMemcpyAsync(n_children, e->d_rc_n + slot, 4, cudaMemcpyDeviceToHost, e->stream));
-  CH_CUDA(e, cudaStreamSynchronize(e->stream));
+  if (moves) SPB_CUDA(e, cudaMemcpyAsync(moves, e->d_rc_moves + slot * M, M * 2, cudaMemcpyDeviceToHost, e->stream));
+  if (visit_counts) SPB_CUDA(e, cudaMemcpyAsync(visit_counts, e->d_rc_counts + slot * M, M * 4, cudaMemcpyDeviceToHost, e->stream));
+  if (child_ids) SPB_CUDA(e, cudaMemcpyAsync(child_ids, e->d_rc_ids + slot * M, M * 4, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaMemcpyAsync(n_children, e->d_rc_n + slot, 4, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   return SPB_OK;
 }
 
 // Policy of Mcts::search's result (mcts.rs:315-328): the root children's visit counts scattered into the 73x8x8 table by
 // set_prob (chess.rs:505-514), then normalize (divide by the sum, chess.rs:516-518).
 int32_t spb_chess_root_policy(spb_chess_engine* e, uint32_t slot, float* out) {
-  CH_GUARD(e);
-  CH_ARG(e, out, "null argument");
+  SPB_GUARD(e);
+  SPB_ARG(e, out, "null argument");
   uint16_t mv[ch::MAX_MOVES];
   uint32_t cnt[ch::MAX_MOVES], n = 0;
   int32_t rc = spb_chess_root_children(e, slot, mv, cnt, nullptr, &n);
   if (rc) return rc;
   ch::Pos root;
-  CH_CUDA(e, cudaMemcpyAsync(&root, e->T.root + slot, sizeof root, cudaMemcpyDeviceToHost, e->stream));
-  CH_CUDA(e, cudaStreamSynchronize(e->stream));
+  SPB_CUDA(e, cudaMemcpyAsync(&root, e->T.root + slot, sizeof root, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   std::memset(out, 0, sizeof(float) * SPB_CHESS_POLICY_SIZE);
   float sum = 0.0f;
   for (uint32_t i = 0; i < n; ++i) sum += (float)cnt[i];               // integers: exact in any order
@@ -926,24 +880,24 @@ int32_t spb_chess_root_policy(spb_chess_engine* e, uint32_t slot, float* out) {
 }
 
 int32_t spb_chess_advance(spb_chess_engine* e, const uint32_t* slots, const uint32_t* child_ids, uint32_t n, spb_chess_state* out_states) {
-  CH_GUARD(e);
-  CH_ARG(e, child_ids && n <= e->T.G, "bad argument");
+  SPB_GUARD(e);
+  SPB_ARG(e, child_ids && n <= e->T.G, "bad argument");
   if (n == 0) return SPB_OK;
-  if (slots) for (uint32_t i = 0; i < n; ++i) CH_ARG(e, slots[i] < e->T.G, "slot out of range");
+  if (slots) for (uint32_t i = 0; i < n; ++i) SPB_ARG(e, slots[i] < e->T.G, "slot out of range");
   // persistent device staging (every call ends with a stream synchronisation): the per-move call of the self-play loop
   uint32_t* d_slots = slots ? e->d_reset_slots : nullptr;
   uint32_t* d_ids = e->d_adv_ids;
   ch::Pos* d_out = e->d_reset_roots;
   int32_t* d_err = e->d_adv_err;
-  if (slots) CH_CUDA(e, cudaMemcpyAsync(d_slots, slots, (size_t)n * 4, cudaMemcpyHostToDevice, e->stream));
-  CH_CUDA(e, cudaMemcpyAsync(d_ids, child_ids, (size_t)n * 4, cudaMemcpyHostToDevice, e->stream));
+  if (slots) SPB_CUDA(e, cudaMemcpyAsync(d_slots, slots, (size_t)n * 4, cudaMemcpyHostToDevice, e->stream));
+  SPB_CUDA(e, cudaMemcpyAsync(d_ids, child_ids, (size_t)n * 4, cudaMemcpyHostToDevice, e->stream));
   ch::k_chess_advance<<<(n + ch::WARPS - 1) / ch::WARPS, ch::THREADS, 0, e->stream>>>(e->T, d_slots, d_ids, n, d_out, d_err);
-  CH_CUDA(e, cudaGetLastError());
+  SPB_CUDA(e, cudaGetLastError());
   ++e->launches;
   std::vector<int32_t> err(n);
-  CH_CUDA(e, cudaMemcpyAsync(err.data(), d_err, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
-  if (out_states) CH_CUDA(e, cudaMemcpyAsync(out_states, d_out, (size_t)n * sizeof(ch::Pos), cudaMemcpyDeviceToHost, e->stream));
-  CH_CUDA(e, cudaStreamSynchronize(e->stream));
+  SPB_CUDA(e, cudaMemcpyAsync(err.data(), d_err, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
+  if (out_states) SPB_CUDA(e, cudaMemcpyAsync(out_states, d_out, (size_t)n * sizeof(ch::Pos), cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   for (uint32_t i = 0; i < n; ++i)
     if (err[i] != SPB_OK) {
       e->set_error(err[i] == SPB_ERR_STATE ? "game history full (SPB_CHESS_MAX_HISTORY plies)" : "spb_chess_advance: not a child of the root");
@@ -953,45 +907,42 @@ int32_t spb_chess_advance(spb_chess_engine* e, const uint32_t* slots, const uint
 }
 
 int32_t spb_chess_get_state(spb_chess_engine* e, uint32_t slot, uint32_t node_id, spb_chess_state* out) {
-  CH_GUARD(e);
-  CH_ARG(e, out && slot < e->T.G, "bad argument");
+  SPB_GUARD(e);
+  SPB_ARG(e, out && slot < e->T.G, "bad argument");
   ch::Scratch sc;
   ch::Pos* d_out = sc.alloc<ch::Pos>(1);
   int32_t* d_err = sc.alloc<int32_t>(1);
   if (!d_out || !d_err) { e->set_error("chess: out of device memory"); return SPB_ERR_NOMEM; }
   ch::k_chess_get_state<<<1, 1, 0, e->stream>>>(e->T, slot, node_id, d_out, d_err);
-  CH_CUDA(e, cudaGetLastError());
+  SPB_CUDA(e, cudaGetLastError());
   ++e->launches;
   int32_t err = 0;
-  CH_CUDA(e, cudaMemcpyAsync(&err, d_err, 4, cudaMemcpyDeviceToHost, e->stream));
-  CH_CUDA(e, cudaMemcpyAsync(out, d_out, sizeof(ch::Pos), cudaMemcpyDeviceToHost, e->stream));
-  CH_CUDA(e, cudaStreamSynchronize(e->stream));
+  SPB_CUDA(e, cudaMemcpyAsync(&err, d_err, 4, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaMemcpyAsync(out, d_out, sizeof(ch::Pos), cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   if (err) { e->set_error("spb_chess_get_state: node out of range"); return err; }
   return SPB_OK;
 }
 
 int32_t spb_chess_arena_len(spb_chess_engine* e, uint32_t slot, uint32_t* out) {
-  CH_GUARD(e);
-  CH_ARG(e, out && slot < e->T.G, "bad argument");
-  CH_CUDA(e, cudaMemcpyAsync(out, e->T.n_nodes + slot, 4, cudaMemcpyDeviceToHost, e->stream));
-  CH_CUDA(e, cudaStreamSynchronize(e->stream));
-  return SPB_OK;
+  SPB_GUARD(e);
+  return e->arena_len(slot, out);
 }
 
 int32_t spb_chess_node_stats(spb_chess_engine* e, uint32_t slot, uint32_t node_id, uint32_t* visit_count, float* value_sum, float* prior,
                              uint32_t* first_child, uint32_t* n_children, uint16_t* move, uint8_t* status) {
-  CH_GUARD(e);
-  CH_ARG(e, slot < e->T.G, "slot out of range");
+  SPB_GUARD(e);
+  SPB_ARG(e, slot < e->T.G, "slot out of range");
   ch::Scratch sc;
   uint32_t* d = sc.alloc<uint32_t>(8);
   if (!d) { e->set_error("chess: out of device memory"); return SPB_ERR_NOMEM; }
   ch::k_chess_node_stats<<<1, 1, 0, e->stream>>>(e->T, slot, node_id, d);
-  CH_CUDA(e, cudaGetLastError());
+  SPB_CUDA(e, cudaGetLastError());
   ++e->launches;
   uint32_t h[8];
-  CH_CUDA(e, cudaMemcpyAsync(h, d, 32, cudaMemcpyDeviceToHost, e->stream));
-  CH_CUDA(e, cudaStreamSynchronize(e->stream));
-  CH_ARG(e, h[7] == 0, "node out of range");
+  SPB_CUDA(e, cudaMemcpyAsync(h, d, 32, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
+  SPB_ARG(e, h[7] == 0, "node out of range");
   if (visit_count) *visit_count = h[0];
   if (value_sum) std::memcpy(value_sum, &h[1], 4);
   if (prior) std::memcpy(prior, &h[2], 4);
@@ -1003,102 +954,47 @@ int32_t spb_chess_node_stats(spb_chess_engine* e, uint32_t slot, uint32_t node_i
   return SPB_OK;
 }
 
-// The trajectory buffers of the self-play step, allocated by its first call (an engine that never plays does not pay for
-// them).  A failure frees what this call allocated and leaves the engine as it was.
-int32_t spb_chess_engine::ensure_selfplay() {
-  if (P.out) return SPB_OK;
-  const size_t G = T.G, max_ply = SPB_CHESS_MAX_HISTORY;
-  spb::Trajectories<spb_chess_position> Q{};
-  Q.max_ply = (uint32_t)max_ply;
-  Q.out_cap = (uint32_t)std::min<size_t>(G * max_ply * 4, (size_t)1 << 26);
-  if (cfg.trajectory_capacity) Q.out_cap = std::max<uint32_t>(cfg.trajectory_capacity, (uint32_t)max_ply);   // a whole game always fits
-  Q.id_stride = cfg.game_id_stride ? cfg.game_id_stride : (unsigned long long)G;
-  std::vector<void*> got;
-  auto alloc = [&](auto** p, size_t count) {
-    void* q = nullptr;
-    if (cudaMalloc(&q, count * sizeof(**p)) != cudaSuccess) return false;
-    got.push_back(q);
-    *p = static_cast<std::remove_reference_t<decltype(*p)>>(q);
-    return true;
-  };
-  const bool ok = alloc(&Q.hist, G * max_ply) && alloc(&Q.hist_len, G) && alloc(&Q.parked, G) && alloc(&Q.game_id, G) &&
-                  alloc(&Q.out, (size_t)Q.out_cap) && alloc(&Q.out_game, (size_t)Q.out_cap) && alloc(&Q.out_cursor, 1) && alloc(&Q.finished, 1);
-  cudaError_t ce = ok ? cudaSuccess : cudaErrorMemoryAllocation;
-  std::vector<unsigned long long> ids(G);
-  for (size_t i = 0; i < G; ++i) ids[i] = (unsigned long long)cfg.game_id_base + i;
-  if (ce == cudaSuccess) ce = cudaMemsetAsync(Q.hist_len, 0, G * 4, stream);
-  if (ce == cudaSuccess) ce = cudaMemsetAsync(Q.parked, 0, G, stream);
-  if (ce == cudaSuccess) ce = cudaMemsetAsync(Q.out_cursor, 0, 8, stream);
-  if (ce == cudaSuccess) ce = cudaMemsetAsync(Q.finished, 0, 4, stream);
-  if (ce == cudaSuccess) ce = cudaMemcpyAsync(Q.game_id, ids.data(), G * 8, cudaMemcpyHostToDevice, stream);
-  if (ce == cudaSuccess) ce = cudaStreamSynchronize(stream);
-  if (ce != cudaSuccess) {
-    for (void* q : got) cudaFree(q);
-    cudaGetLastError();                                                // an allocation failure is not sticky: clear it
-    set_error("chess self-play: cannot set up the trajectory buffers (" + std::to_string(G * max_ply) + " + " + std::to_string(Q.out_cap) +
-              " records of " + std::to_string(sizeof(spb_chess_position)) + " bytes): " + cudaGetErrorString(ce));
-    return ok ? SPB_ERR_CUDA : SPB_ERR_NOMEM;
-  }
-  allocs.insert(allocs.end(), got.begin(), got.end());
-  P = Q;
-  return SPB_OK;
-}
-
 int32_t spb_chess_selfplay_step(spb_chess_engine* e, int32_t rule, float temperature, uint64_t seed, const spb_chess_state* restart_roots,
                                 const uint64_t* restart_history, uint32_t* n_finished) {
-  CH_GUARD(e);
-  CH_ARG(e, rule == SPB_MOVE_GREEDY_LAST_MAX || rule == SPB_MOVE_TEMPERATURE, "unknown move rule");
-  CH_ARG(e, !(restart_history && !restart_roots), "history without roots");
+  SPB_GUARD(e);
+  SPB_ARG(e, rule == SPB_MOVE_GREEDY_LAST_MAX || rule == SPB_MOVE_TEMPERATURE, "unknown move rule");
+  SPB_ARG(e, !(restart_history && !restart_roots), "history without roots");
   const uint32_t G = e->T.G;
   int32_t rc = check_roots(e, restart_roots, restart_history, G);
   if (rc) return rc;
-  rc = e->ensure_selfplay();
-  if (rc) return rc;
+  if (!e->P.out) {                                                     // the first step allocates the trajectory buffers
+    rc = e->alloc_trajectories(SPB_CHESS_MAX_HISTORY);
+    if (rc) return rc;
+  }
   // the staging of spb_chess_reset_games (every call ends with a stream synchronisation)
-  if (restart_roots) CH_CUDA(e, cudaMemcpyAsync(e->d_reset_roots, restart_roots, (size_t)G * sizeof(ch::Pos), cudaMemcpyHostToDevice, e->stream));
+  if (restart_roots) SPB_CUDA(e, cudaMemcpyAsync(e->d_reset_roots, restart_roots, (size_t)G * sizeof(ch::Pos), cudaMemcpyHostToDevice, e->stream));
   if (restart_history)
-    CH_CUDA(e, cudaMemcpyAsync(e->d_reset_hist, restart_history, (size_t)G * SPB_CHESS_MAX_HISTORY * 8, cudaMemcpyHostToDevice, e->stream));
-  CH_CUDA(e, cudaMemsetAsync(e->P.finished, 0, 4, e->stream));
+    SPB_CUDA(e, cudaMemcpyAsync(e->d_reset_hist, restart_history, (size_t)G * SPB_CHESS_MAX_HISTORY * 8, cudaMemcpyHostToDevice, e->stream));
+  SPB_CUDA(e, cudaMemsetAsync(e->P.finished, 0, 4, e->stream));
   ch::k_chess_selfplay_step<<<(G + ch::WARPS - 1) / ch::WARPS, ch::THREADS, 0, e->stream>>>(
       e->T, e->P, rule, temperature, seed, restart_roots ? e->d_reset_roots : nullptr, restart_history ? e->d_reset_hist : nullptr);
-  CH_CUDA(e, cudaGetLastError());
+  SPB_CUDA(e, cudaGetLastError());
   ++e->launches;
   uint32_t fin = 0;
-  CH_CUDA(e, cudaMemcpyAsync(&fin, e->P.finished, 4, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaMemcpyAsync(&fin, e->P.finished, 4, cudaMemcpyDeviceToHost, e->stream));
   rc = e->check_device_errors();                                       // synchronises the stream
   if (n_finished) *n_finished = fin;
   return rc;
 }
 
 int32_t spb_chess_drain_trajectories(spb_chess_engine* e, spb_chess_position* buf, size_t capacity, size_t* written, uint64_t* game_ids) {
-  CH_GUARD(e);
-  return drain_trajectories(e, e->P, e->stream, buf, capacity, written, game_ids);
+  SPB_GUARD(e);
+  return e->drain_trajectories(buf, capacity, written, game_ids);
 }
 
 int32_t spb_chess_get_counters(spb_chess_engine* e, spb_counters* out) {
-  CH_GUARD(e);
-  CH_ARG(e, out, "null argument");
-  unsigned long long c[CTR_COUNT], live[2] = {0, 0};
-  CH_CUDA(e, cudaMemsetAsync(e->d_misc, 0, 16, e->stream));
-  ch::k_chess_nodes_live<<<(e->T.G + 127) / 128, 128, 0, e->stream>>>(e->T, e->d_misc);
-  CH_CUDA(e, cudaGetLastError());
-  ++e->launches;
-  CH_CUDA(e, cudaMemcpyAsync(c, e->T.counters, sizeof c, cudaMemcpyDeviceToHost, e->stream));
-  CH_CUDA(e, cudaMemcpyAsync(live, e->d_misc, 16, cudaMemcpyDeviceToHost, e->stream));
-  CH_CUDA(e, cudaStreamSynchronize(e->stream));
-  std::memset(out, 0, sizeof *out);
-  out->simulations = c[CTR_SIMS]; out->evaluations = c[CTR_EVALS]; out->terminal_leaves = c[CTR_TERMINAL];
-  out->path_length_sum = c[CTR_PATHSUM]; out->children_created = c[CTR_CHILDREN];
-  out->nodes_live = live[0]; out->kernel_launches = e->launches;
-  out->reserved[0] = live[1];   // largest arena
-  return SPB_OK;
+  SPB_GUARD(e);
+  return e->get_counters(out, true, [e] { ch::k_chess_nodes_live<<<(e->T.G + 127) / 128, 128, 0, e->stream>>>(e->T, e->d_misc); });
 }
 
 int32_t spb_chess_reset_counters(spb_chess_engine* e) {
-  CH_GUARD(e);
-  CH_CUDA(e, cudaMemsetAsync(e->T.counters, 0, CTR_COUNT * 8, e->stream));
-  e->launches = 0;
-  return SPB_OK;
+  SPB_GUARD(e);
+  return e->reset_counters();
 }
 
 }  // extern "C"

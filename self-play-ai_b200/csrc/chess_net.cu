@@ -651,8 +651,7 @@ cudaError_t net_time_conv(Net* net, const uint32_t* count_dev, uint32_t iters, c
 }
 
 int32_t net_forward_leaves(spb_chess_engine* e, int set, const uint32_t* list, const uint32_t* count_dev, cudaStream_t stream, uint32_t* launched) {
-  const cudaError_t ce = net_forward(e->net, set, e->T.leaf_pos, e->T.leaf_reps, list, count_dev, e->T.eval_logits, e->T.eval_value, stream, launched);
-  if (ce != cudaSuccess) { e->set_error(std::string("chess network launch: ") + cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
+  SPB_CUDA(e, net_forward(e->net, set, e->T.leaf_pos, e->T.leaf_reps, list, count_dev, e->T.eval_logits, e->T.eval_value, stream, launched));
   return SPB_OK;
 }
 
@@ -721,12 +720,12 @@ namespace ch = spb::chess;
 extern "C" {
 
 int32_t spb_chess_load_weights(spb_chess_engine* e, const void* blob, size_t n) {
-  CH_GUARD(e);
-  CH_ARG(e, blob && n > 8, "null / empty weight blob");
+  SPB_GUARD(e);
+  SPB_ARG(e, blob && n > 8, "null / empty weight blob");
   ch::HostNet host;
   std::string err;
   if (!ch::parse_safetensors_chess(blob, n, &host, &err)) { e->set_error("spb_chess_load_weights: " + err); return SPB_ERR_WEIGHTS; }
-  cudaStreamSynchronize(e->stream);
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   if (!e->net) {
     e->net = ch::net_create(e->T.G, &err);
     if (!e->net) { e->set_error("spb_chess_load_weights: " + err); return SPB_ERR_NOMEM; }
@@ -749,15 +748,14 @@ int32_t spb_chess_check_weights(const void* blob, size_t n, char* err, size_t er
 
 int32_t spb_chess_time_conv(spb_chess_engine* e, uint32_t iters, float* avg_ms, uint32_t* n_positions, double* flops_per_launch,
                             double* flops_per_position) {
-  CH_GUARD(e);
-  CH_ARG(e, avg_ms && n_positions && flops_per_launch && flops_per_position && iters > 0, "bad argument");
-  CH_ARG(e, e->net && ch::net_loaded(e->net), "no weights loaded (spb_chess_load_weights)");
+  SPB_GUARD(e);
+  SPB_ARG(e, avg_ms && n_positions && flops_per_launch && flops_per_position && iters > 0, "bad argument");
+  SPB_ARG(e, e->net && ch::net_loaded(e->net), "no weights loaded (spb_chess_load_weights)");
   uint32_t n = 0;
-  CH_CUDA(e, cudaMemcpyAsync(&n, e->T.eval_count, 4, cudaMemcpyDeviceToHost, e->stream));
-  CH_CUDA(e, cudaStreamSynchronize(e->stream));
-  CH_ARG(e, n > 0, "no evaluator batch resident (run spb_chess_search first)");
-  const cudaError_t ce = ch::net_time_conv(e->net, e->T.eval_count, iters, e->stream, e->ev0, e->ev1, avg_ms);
-  if (ce != cudaSuccess) { e->set_error(std::string("chess conv timing: ") + cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
+  SPB_CUDA(e, cudaMemcpyAsync(&n, e->T.eval_count, 4, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
+  SPB_ARG(e, n > 0, "no evaluator batch resident (run spb_chess_search first)");
+  SPB_CUDA(e, ch::net_time_conv(e->net, e->T.eval_count, iters, e->stream, e->ev0, e->ev1, avg_ms));
   e->launches += iters + 1;
   *n_positions = n;
   *flops_per_launch = (double)n * 2.0 * 64 * 256 * 9 * 256;           // algorithmic: the 64 real cells of a position
@@ -767,11 +765,11 @@ int32_t spb_chess_time_conv(spb_chess_engine* e, uint32_t iters, float* avg_ms, 
 
 int32_t spb_chess_predict(spb_chess_engine* e, const spb_chess_state* states, const uint64_t* history, uint32_t n, float* policies, float* values,
                           float* raw_logits) {
-  CH_GUARD(e);
+  SPB_GUARD(e);
   if (n == 0) return SPB_OK;
-  CH_ARG(e, states, "null states");
-  CH_ARG(e, e->net && ch::net_loaded(e->net), "no weights loaded (spb_chess_load_weights)");
-  CH_ARG(e, n <= e->T.G, "more states than the engine's num_games (the network's batch capacity)");
+  SPB_ARG(e, states, "null states");
+  SPB_ARG(e, e->net && ch::net_loaded(e->net), "no weights loaded (spb_chess_load_weights)");
+  SPB_ARG(e, n <= e->T.G, "more states than the engine's num_games (the network's batch capacity)");
   ch::Scratch sc;
   auto* d_states = sc.alloc<ch::Pos>(n);
   auto* d_hist = history ? sc.alloc<unsigned long long>((size_t)n * SPB_CHESS_MAX_HISTORY) : nullptr;
@@ -786,24 +784,23 @@ int32_t spb_chess_predict(spb_chess_engine* e, const spb_chess_state* states, co
     e->set_error("chess: out of device memory");
     return SPB_ERR_NOMEM;
   }
-  CH_CUDA(e, cudaMemcpyAsync(d_states, states, (size_t)n * sizeof(ch::Pos), cudaMemcpyHostToDevice, e->stream));
-  if (history) CH_CUDA(e, cudaMemcpyAsync(d_hist, history, (size_t)n * SPB_CHESS_MAX_HISTORY * 8, cudaMemcpyHostToDevice, e->stream));
-  CH_CUDA(e, cudaMemcpyAsync(d_count, &n, 4, cudaMemcpyHostToDevice, e->stream));
+  SPB_CUDA(e, cudaMemcpyAsync(d_states, states, (size_t)n * sizeof(ch::Pos), cudaMemcpyHostToDevice, e->stream));
+  if (history) SPB_CUDA(e, cudaMemcpyAsync(d_hist, history, (size_t)n * SPB_CHESS_MAX_HISTORY * 8, cudaMemcpyHostToDevice, e->stream));
+  SPB_CUDA(e, cudaMemcpyAsync(d_count, &n, 4, cudaMemcpyHostToDevice, e->stream));
   ch::k_predict_prepare<<<(n + 3) / 4, 128, 0, e->stream>>>(d_states, d_hist, n, d_moves, d_nmoves, d_reps, e->T.error);
-  CH_CUDA(e, cudaGetLastError());
+  SPB_CUDA(e, cudaGetLastError());
   uint32_t launched = 0;
-  const cudaError_t ce = ch::net_forward(e->net, 0, d_states, d_reps, nullptr, d_count, d_logits, d_values, e->stream, &launched);
-  if (ce != cudaSuccess) { e->set_error(std::string("chess network launch: ") + cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
+  SPB_CUDA(e, ch::net_forward(e->net, 0, d_states, d_reps, nullptr, d_count, d_logits, d_values, e->stream, &launched));
   e->launches += 1 + launched;
   if (policies) {
     ch::k_predict_mask<<<n, 256, 0, e->stream>>>(d_logits, d_states, d_moves, d_nmoves, n, d_pol);
-    CH_CUDA(e, cudaGetLastError());
+    SPB_CUDA(e, cudaGetLastError());
     ++e->launches;
-    CH_CUDA(e, cudaMemcpyAsync(policies, d_pol, (size_t)n * SPB_CHESS_POLICY_SIZE * 4, cudaMemcpyDeviceToHost, e->stream));
+    SPB_CUDA(e, cudaMemcpyAsync(policies, d_pol, (size_t)n * SPB_CHESS_POLICY_SIZE * 4, cudaMemcpyDeviceToHost, e->stream));
   }
-  if (values) CH_CUDA(e, cudaMemcpyAsync(values, d_values, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
-  if (raw_logits) CH_CUDA(e, cudaMemcpyAsync(raw_logits, d_logits, (size_t)n * SPB_CHESS_POLICY_SIZE * 4, cudaMemcpyDeviceToHost, e->stream));
-  CH_CUDA(e, cudaStreamSynchronize(e->stream));
+  if (values) SPB_CUDA(e, cudaMemcpyAsync(values, d_values, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
+  if (raw_logits) SPB_CUDA(e, cudaMemcpyAsync(raw_logits, d_logits, (size_t)n * SPB_CHESS_POLICY_SIZE * 4, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   return e->check_device_errors();
 }
 

@@ -1,7 +1,6 @@
-// engine.cu — the host engine and the C entry points that launch kernels (include/selfplay_b200.h).
+// engine.cu — the Connect4 / tic-tac-toe host engine (spb_engine, engine.hpp) and the C entry points that launch kernels
+// (include/selfplay_b200.h).  What it shares with the chess engine is in host_engine.hpp.
 // Device code: kernels.cuh (tree / game / self-play kernels), async.cuh (asynchronous pipeline), evaluator_umma.cu.
-#include <cfloat>
-
 #include "kernels.cuh"
 
 
@@ -14,16 +13,8 @@ thread_local std::string g_create_error;
 
 
 int32_t spb_engine::init() {
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) { set_error("no CUDA device (this library has no CPU fallback)"); return SPB_ERR_CUDA; }
-  if (cfg.device < 0 || cfg.device >= ndev) { set_error("device ordinal out of range"); return SPB_ERR_ARG; }
-  SPB_CUDA(cudaSetDevice(cfg.device));
-  cudaDeviceProp prop;
-  SPB_CUDA(cudaGetDeviceProperties(&prop, cfg.device));
-  if (prop.major != 10) { set_error("device is not sm_100 (B200); this library is built for sm_100a only"); return SPB_ERR_CUDA; }
-  SPB_CUDA(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
-  SPB_CUDA(cudaEventCreate(&ev0));
-  SPB_CUDA(cudaEventCreate(&ev1));
+  int32_t rc = open_device();
+  if (rc) return rc;
   const bool c4 = cfg.game == SPB_GAME_CONNECT4;
   A = c4 ? Connect4::A : TicTacToe::A;
   max_depth = c4 ? Connect4::MAX_DEPTH : TicTacToe::MAX_DEPTH;
@@ -31,7 +22,6 @@ int32_t spb_engine::init() {
   max_ply = c4 ? 42 : 9;
   T.G = cfg.num_games; T.K = cfg.leaves_per_tree; T.cap = cfg.max_nodes_per_tree; T.c = cfg.c;
   const size_t G = T.G, slots = G * T.K, pool = G * (size_t)T.cap;
-  int32_t rc;
   for (int b = 0; b < 2; ++b) {
     if ((rc = dalloc(&T.rec[b], pool))) return rc;
     if ((rc = dalloc(&T.par[b], pool))) return rc;
@@ -48,7 +38,7 @@ int32_t spb_engine::init() {
   if ((rc = dalloc(&T.eval_out, slots * eval_stride))) return rc;
   if ((rc = dalloc(&T.counters, (size_t)CTR_COUNT))) return rc;
   if ((rc = dalloc(&T.error, 1))) return rc;
-  if ((rc = dalloc(&d_rc_actions, G * SPB_MAX_ACTIONS))) return rc;
+  if ((rc = dalloc(&d_rc_moves, G * SPB_MAX_ACTIONS))) return rc;
   if ((rc = dalloc(&d_rc_counts, G * SPB_MAX_ACTIONS))) return rc;
   if ((rc = dalloc(&d_rc_ids, G * SPB_MAX_ACTIONS))) return rc;
   if ((rc = dalloc(&d_rc_n, G))) return rc;
@@ -68,53 +58,25 @@ int32_t spb_engine::init() {
     ctl.abort = d_ctl_words + 6 * 32;
     ctl.stats = reinterpret_cast<unsigned long long*>(d_ctl_words + 7 * 32);   // 2 lines: ASTAT_COUNT u64
     ctl.stall_ns = 2000000000ull;             // 2 s without a single hand-off anywhere: a bug, reported as SPB_ERR_STATE
-    SPB_CUDA(cudaMemsetAsync(ctl.sims_left, 0, G * 4, stream));
+    SPB_CUDA(this, cudaMemsetAsync(ctl.sims_left, 0, G * 4, stream));
   }
-  // self-play buffers
-  P.max_ply = (uint32_t)max_ply;
-  P.out_cap = (uint32_t)std::min<size_t>(G * max_ply * 4, (size_t)1 << 26);
-  if (cfg.trajectory_capacity) P.out_cap = std::max<uint32_t>(cfg.trajectory_capacity, (uint32_t)max_ply);   // a whole game always fits
-  P.id_stride = cfg.game_id_stride ? cfg.game_id_stride : (unsigned long long)G;
-  if ((rc = dalloc(&P.hist, G * max_ply))) return rc;
-  if ((rc = dalloc(&P.hist_len, G))) return rc;
-  if ((rc = dalloc(&P.parked, G))) return rc;
-  if ((rc = dalloc(&P.game_id, G))) return rc;
-  if ((rc = dalloc(&P.out, (size_t)P.out_cap))) return rc;
-  if ((rc = dalloc(&P.out_game, (size_t)P.out_cap))) return rc;
-  if ((rc = dalloc(&P.out_cursor, 1))) return rc;
-  if ((rc = dalloc(&P.finished, 1))) return rc;
-  SPB_CUDA(cudaMemsetAsync(T.live, 0, G, stream));
-  SPB_CUDA(cudaMemsetAsync(T.buf, 0, G, stream));
-  SPB_CUDA(cudaMemsetAsync(T.n_nodes, 0, G * 4, stream));
-  SPB_CUDA(cudaMemsetAsync(T.leaf_info, 0, slots * 4, stream));
-  SPB_CUDA(cudaMemsetAsync(T.leaf_state, 0, slots * sizeof(PState), stream));
-  SPB_CUDA(cudaMemsetAsync(T.eval_count, 0, 16, stream));
-  SPB_CUDA(cudaMemsetAsync(T.eval_out, 0, slots * eval_stride * 4, stream));
-  SPB_CUDA(cudaMemsetAsync(T.counters, 0, CTR_COUNT * 8, stream));
-  SPB_CUDA(cudaMemsetAsync(T.error, 0, 4, stream));
-  SPB_CUDA(cudaMemsetAsync(P.hist_len, 0, G * 4, stream));
-  SPB_CUDA(cudaMemsetAsync(P.parked, 0, G, stream));
-  SPB_CUDA(cudaMemsetAsync(P.out_cursor, 0, 8, stream));
-  SPB_CUDA(cudaMemsetAsync(P.finished, 0, 4, stream));
-  {
-    std::vector<unsigned long long> ids(G);
-    unsigned long long base = cfg.game_id_base;
-    for (size_t i = 0; i < G; ++i) ids[i] = base + i;
-    SPB_CUDA(cudaMemcpyAsync(P.game_id, ids.data(), G * 8, cudaMemcpyHostToDevice, stream));
-    SPB_CUDA(cudaStreamSynchronize(stream));
-  }
-  return SPB_OK;
+  SPB_CUDA(this, cudaMemsetAsync(T.live, 0, G, stream));
+  SPB_CUDA(this, cudaMemsetAsync(T.buf, 0, G, stream));
+  SPB_CUDA(this, cudaMemsetAsync(T.n_nodes, 0, G * 4, stream));
+  SPB_CUDA(this, cudaMemsetAsync(T.leaf_info, 0, slots * 4, stream));
+  SPB_CUDA(this, cudaMemsetAsync(T.leaf_state, 0, slots * sizeof(PState), stream));
+  SPB_CUDA(this, cudaMemsetAsync(T.eval_count, 0, 16, stream));
+  SPB_CUDA(this, cudaMemsetAsync(T.eval_out, 0, slots * eval_stride * 4, stream));
+  SPB_CUDA(this, cudaMemsetAsync(T.counters, 0, CTR_COUNT * 8, stream));
+  SPB_CUDA(this, cudaMemsetAsync(T.error, 0, 4, stream));
+  return alloc_trajectories((uint32_t)max_ply);   // self-play buffers, allocated with the engine
 }
 
-void spb_engine::destroy() {
-  if (step_graph) cudaGraphExecDestroy(step_graph);
-  for (void* p : allocs) cudaFree(p);
-  allocs.clear();
+void spb_engine::release() {
+  HostEngine::release();
+  drop_step_graph();
   if (h_stage) cudaFreeHost(h_stage);
   if (d_stage) cudaFree(d_stage);
-  if (ev0) cudaEventDestroy(ev0);
-  if (ev1) cudaEventDestroy(ev1);
-  if (stream) cudaStreamDestroy(stream);
 }
 
 // The reference's arena is a Vec that grows without bound (mcts.rs:19,151-157).  Here every tree owns a fixed
@@ -123,12 +85,12 @@ void spb_engine::destroy() {
 // before any tree is touched, so a failure leaves the engine as it was.
 int32_t spb_engine::ensure_capacity(uint32_t num_searches) {
   unsigned long long mx = 0;
-  SPB_CUDA(cudaMemsetAsync(d_misc, 0, 8, stream));
+  SPB_CUDA(this, cudaMemsetAsync(d_misc, 0, 8, stream));
   k_max_nodes<<<(T.G + 127) / 128, 128, 0, stream>>>(T, d_misc);
-  SPB_CHECK_LAUNCH();
+  SPB_CUDA(this, cudaGetLastError());
   ++launches;
-  SPB_CUDA(cudaMemcpyAsync(&mx, d_misc, 8, cudaMemcpyDeviceToHost, stream));
-  SPB_CUDA(cudaStreamSynchronize(stream));
+  SPB_CUDA(this, cudaMemcpyAsync(&mx, d_misc, 8, cudaMemcpyDeviceToHost, stream));
+  SPB_CUDA(this, cudaStreamSynchronize(stream));
   const unsigned long long need = mx + (unsigned long long)num_searches * (unsigned long long)A;
   if (need <= T.cap || (cfg.flags & SPB_FLAG_FIXED_POOL)) return SPB_OK;   // fixed pool: the device flag reports exhaustion
   unsigned long long ncap = std::max<unsigned long long>(need, 2ull * T.cap);
@@ -167,21 +129,7 @@ int32_t spb_engine::ensure_capacity(uint32_t num_searches) {
   }
   T.cap = (uint32_t)ncap;
   cfg.max_nodes_per_tree = T.cap;
-  if (step_graph) { cudaGraphExecDestroy(step_graph); step_graph = nullptr; }   // the graph captured the old pointers
-  return SPB_OK;
-}
-
-int32_t spb_engine::check_device_errors() {
-  uint32_t e = 0;
-  SPB_CUDA(cudaMemcpyAsync(&e, T.error, 4, cudaMemcpyDeviceToHost, stream));
-  SPB_CUDA(cudaStreamSynchronize(stream));
-  if (e) {
-    SPB_CUDA(cudaMemsetAsync(T.error, 0, 4, stream));
-    if (e & ERRBIT_POOL) { set_error("node pool exhausted: raise spb_config.max_nodes_per_tree"); return SPB_ERR_POOL; }
-    if (e & ERRBIT_TRAJ_FULL) { set_error("trajectory buffer full: call spb_drain_trajectories"); return SPB_ERR_STATE; }
-    if (e & ERRBIT_BOUNDS) { set_error("bounds check failed at site " + std::to_string((e >> 8) & 0xFFu) + " (checked build, see SPB_ASSERT in csrc/)"); return SPB_ERR_STATE; }
-    if (e & ERRBIT_NAN) { set_error("NaN PUCT score (the reference panics here, mcts.rs:109)"); return SPB_ERR_STATE; }
-  }
+  drop_step_graph();   // the graph captured the old pointers
   return SPB_OK;
 }
 
@@ -189,9 +137,8 @@ template <class G>
 int32_t spb_engine::launch_eval_step(uint32_t parity) {
   const uint32_t slots = T.G * T.K;
   if (cfg.evaluator == SPB_EVAL_NET) {
-    cudaError_t e = evaluator.launch(T.leaf_state, T.eval_list, &T.eval_count[parity & 1], slots, T.eval_out, G::EVAL_STRIDE,
-                                     nullptr, (cfg.flags & SPB_FLAG_EVAL_SIMT) != 0, stream);
-    if (e != cudaSuccess) { set_error(std::string("evaluator launch: ") + cudaGetErrorString(e)); return SPB_ERR_CUDA; }
+    SPB_CUDA(this, evaluator.launch(T.leaf_state, T.eval_list, &T.eval_count[parity & 1], slots, T.eval_out, G::EVAL_STRIDE, nullptr,
+                                    (cfg.flags & SPB_FLAG_EVAL_SIMT) != 0, stream));
   } else if (cfg.evaluator == SPB_EVAL_DET) {
     k_eval_builtin<G, SPB_EVAL_DET><<<(slots + 255) / 256, 256, 0, stream>>>(T.leaf_state, T.eval_list, &T.eval_count[parity & 1], T.eval_out);
   } else {
@@ -228,7 +175,7 @@ int32_t spb_engine::search_t(uint32_t num_searches) {
   // The network evaluator (and the built-in evaluators under SPB_FLAG_FORCE_SPLIT) run through the asynchronous
   // pipeline unless the lock-step pipeline is asked for; K > 1 leaves per tree is a lock-step extension.
   const bool async = split && T.K == 1 && !(cfg.flags & SPB_FLAG_LOCKSTEP);
-  SPB_CUDA(cudaEventRecord(ev0, stream));
+  SPB_CUDA(this, cudaEventRecord(ev0, stream));
   last_eval_launches = 0;
   if (T.root_noise) { int32_t rc = launch_root_noise(); if (rc != SPB_OK) return rc; }   // eta of every root, before any descent
   if (async) {
@@ -237,35 +184,35 @@ int32_t spb_engine::search_t(uint32_t num_searches) {
   } else if (!split) {
     if (cfg.evaluator == SPB_EVAL_DET) k_search_fused<G, SPB_EVAL_DET><<<blocks, THREADS, 0, stream>>>(T, num_searches);
     else k_search_fused<G, SPB_EVAL_UNIFORM><<<blocks, THREADS, 0, stream>>>(T, num_searches);
-    SPB_CHECK_LAUNCH();
+    SPB_CUDA(this, cudaGetLastError());
     ++launches;
   } else if (T.K > 1) {
     // EXTENSION: K leaves per tree per step with virtual loss (see k_tree_step_multi).
     const uint32_t K = T.K, steps = (num_searches + K - 1) / K;
-    SPB_CUDA(cudaMemsetAsync(T.eval_count, 0, 8, stream));
+    SPB_CUDA(this, cudaMemsetAsync(T.eval_count, 0, 8, stream));
     k_tree_step_multi<G><<<blocks, THREADS, 0, stream>>>(T, 0, std::min(K, num_searches), 0u);
-    SPB_CHECK_LAUNCH();
+    SPB_CUDA(this, cudaGetLastError());
     ++launches;
     for (uint32_t j = 0; j < steps; ++j) {
       const bool last = (j == steps - 1);
       if (last) {
-        SPB_CUDA(cudaMemcpyAsync(&T.eval_count[2], &T.eval_count[j & 1u], 4, cudaMemcpyDeviceToDevice, stream));
+        SPB_CUDA(this, cudaMemcpyAsync(&T.eval_count[2], &T.eval_count[j & 1u], 4, cudaMemcpyDeviceToDevice, stream));
         last_eval_parity = 2;
       }
       int32_t rc = launch_eval_step<G>(j);
       if (rc != SPB_OK) return rc;
-      SPB_CHECK_LAUNCH();
+      SPB_CUDA(this, cudaGetLastError());
       ++last_eval_launches;
       const uint32_t done_after = std::min(num_searches, (j + 1) * K);
       const uint32_t k_next = last ? 0u : std::min(K, num_searches - done_after);
       k_tree_step_multi<G><<<blocks, THREADS, 0, stream>>>(T, 1, k_next, j + 1);
-      SPB_CHECK_LAUNCH();
+      SPB_CUDA(this, cudaGetLastError());
       ++launches;
     }
   } else {
     // step j: select writes eval_count[j&1]; the kernel also zeroes eval_count[(j+1)&1].
-    SPB_CUDA(cudaMemsetAsync(T.eval_count, 0, 8, stream));
-    SPB_CUDA(launch_pdl(k_tree_step<G>, blocks, THREADS, stream, T, 0, 1, 0u));
+    SPB_CUDA(this, cudaMemsetAsync(T.eval_count, 0, 8, stream));
+    SPB_CUDA(this, launch_pdl(k_tree_step<G>, blocks, THREADS, stream, T, 0, 1, 0u));
     ++launches;
     uint32_t j = 0;
     const bool use_graph = !(cfg.flags & SPB_FLAG_NO_GRAPH) && num_searches > 2;
@@ -273,7 +220,7 @@ int32_t spb_engine::search_t(uint32_t num_searches) {
       // One graph = two steps (parities 0,1): eval(0) step(1) eval(1) step(0).
       if (!step_graph) {
         cudaGraph_t graph;
-        SPB_CUDA(cudaStreamBeginCapture(stream, cudaStreamCaptureModeThreadLocal));
+        SPB_CUDA(this, cudaStreamBeginCapture(stream, cudaStreamCaptureModeThreadLocal));
         int32_t rc = launch_eval_step<G>(0u);
         cudaError_t pe = launch_pdl(k_tree_step<G>, blocks, THREADS, stream, T, 1, 1, 1u);
         if (rc == SPB_OK) rc = launch_eval_step<G>(1u);
@@ -283,11 +230,11 @@ int32_t spb_engine::search_t(uint32_t num_searches) {
         if (rc != SPB_OK) return rc;
         if (ce == cudaSuccess) ce = pe;
         if (ce != cudaSuccess) { set_error(std::string("graph capture: ") + cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
-        SPB_CUDA(cudaGraphInstantiate(&step_graph, graph, 0));
+        SPB_CUDA(this, cudaGraphInstantiate(&step_graph, graph, 0));
         cudaGraphDestroy(graph);
       }
       while (j + 2 <= num_searches - 1) {
-        SPB_CUDA(cudaGraphLaunch(step_graph, stream));
+        SPB_CUDA(this, cudaGraphLaunch(step_graph, stream));
         launches += 4;
         last_eval_launches += 2;
         j += 2;
@@ -296,22 +243,22 @@ int32_t spb_engine::search_t(uint32_t num_searches) {
     for (; j < num_searches; ++j) {
       int32_t rc = launch_eval_step<G>(j);
       if (rc != SPB_OK) return rc;
-      SPB_CHECK_LAUNCH();
+      SPB_CUDA(this, cudaGetLastError());
       ++last_eval_launches;
       const int last = (j == num_searches - 1);
       if (last) {   // keep the size of the last work list: the final tree step clears the ping-pong counter
-        SPB_CUDA(cudaMemcpyAsync(&T.eval_count[2], &T.eval_count[j & 1u], 4, cudaMemcpyDeviceToDevice, stream));
+        SPB_CUDA(this, cudaMemcpyAsync(&T.eval_count[2], &T.eval_count[j & 1u], 4, cudaMemcpyDeviceToDevice, stream));
         last_eval_parity = 2;
       }
-      SPB_CUDA(launch_pdl(k_tree_step<G>, blocks, THREADS, stream, T, 1, last ? 0 : 1, j + 1));
+      SPB_CUDA(this, launch_pdl(k_tree_step<G>, blocks, THREADS, stream, T, 1, last ? 0 : 1, j + 1));
       ++launches;
     }
   }
-  SPB_CUDA(cudaEventRecord(ev1, stream));
+  SPB_CUDA(this, cudaEventRecord(ev1, stream));
   uint32_t ctl_host[CTL_WORDS];
-  if (async) SPB_CUDA(cudaMemcpyAsync(ctl_host, d_ctl_words, sizeof ctl_host, cudaMemcpyDeviceToHost, stream));
+  if (async) SPB_CUDA(this, cudaMemcpyAsync(ctl_host, d_ctl_words, sizeof ctl_host, cudaMemcpyDeviceToHost, stream));
   int32_t rc = check_device_errors();   // synchronises the stream
-  SPB_CUDA(cudaEventElapsedTime(&last_search_ms, ev0, ev1));
+  SPB_CUDA(this, cudaEventElapsedTime(&last_search_ms, ev0, ev1));
   if (async) std::memcpy(last_async_stats, &ctl_host[7 * 32], sizeof(uint64_t) * ASTAT_COUNT);
   if (rc == SPB_OK && async && (ctl_host[6 * 32] != 0u || ctl_host[5 * 32] != ctl_host[4 * 32])) {
     char msg[256];
@@ -328,7 +275,7 @@ int32_t spb_engine::launch_root_noise() {
   const uint32_t blocks = (T.G + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK;
   if (cfg.game == SPB_GAME_CONNECT4) k_root_noise<Connect4><<<blocks, THREADS, 0, stream>>>(T, P.game_id, noise_alpha, noise_seed);
   else k_root_noise<TicTacToe><<<blocks, THREADS, 0, stream>>>(T, P.game_id, noise_alpha, noise_seed);
-  SPB_CHECK_LAUNCH();
+  SPB_CUDA(this, cudaGetLastError());
   ++launches;
   return SPB_OK;
 }
@@ -337,20 +284,19 @@ int32_t spb_engine::launch_root_noise() {
 // have completed their simulations (network: evaluator CTAs + tree warps; built-in evaluators: evaluator warps + tree warps).
 template <class G>
 int32_t spb_engine::search_async(uint32_t num_searches) {
-  SPB_CUDA(cudaMemsetAsync(d_ctl_words, 0, (size_t)CTL_WORDS * 4, stream));
-  SPB_CUDA(cudaMemsetAsync(d_ring_slots, 0, 2 * (size_t)ring_size * 8, stream));
+  SPB_CUDA(this, cudaMemsetAsync(d_ctl_words, 0, (size_t)CTL_WORDS * 4, stream));
+  SPB_CUDA(this, cudaMemsetAsync(d_ring_slots, 0, 2 * (size_t)ring_size * 8, stream));
   k_async_init<<<(T.G + 127) / 128, 128, 0, stream>>>(T, ctl, num_searches);
-  SPB_CHECK_LAUNCH();
+  SPB_CUDA(this, cudaGetLastError());
   ++launches;
   if (cfg.evaluator == SPB_EVAL_NET) {
-    cudaError_t e = evaluator.launch_ring(T, ctl, stream);
-    if (e != cudaSuccess) { set_error(std::string("evaluator launch: ") + cudaGetErrorString(e)); return SPB_ERR_CUDA; }
+    SPB_CUDA(this, evaluator.launch_ring(T, ctl, stream));
     ++last_eval_launches;
   } else {
     const uint32_t grid = std::max(1u, std::min(592u, (T.G + 3u) / 4u));
     if (cfg.evaluator == SPB_EVAL_DET) k_async_builtin<G, SPB_EVAL_DET><<<grid, THREADS, 0, stream>>>(T, ctl);
     else k_async_builtin<G, SPB_EVAL_UNIFORM><<<grid, THREADS, 0, stream>>>(T, ctl);
-    SPB_CHECK_LAUNCH();
+    SPB_CUDA(this, cudaGetLastError());
   }
   ++launches;
   last_eval_parity = -1;
@@ -360,17 +306,6 @@ int32_t spb_engine::search_async(uint32_t num_searches) {
 // ------------------------------------------------------------------------------------------------
 // C ABI
 // ------------------------------------------------------------------------------------------------
-#define ENGINE_GUARD(e)                                   \
-  if (!(e)) return SPB_ERR_ARG;                           \
-  if (cudaSetDevice((e)->cfg.device) != cudaSuccess) {    \
-    (e)->set_error("cudaSetDevice failed");               \
-    return SPB_ERR_CUDA;                                  \
-  }
-#define ARG_CHECK(e, cond, msg)        \
-  if (!(cond)) {                       \
-    (e)->set_error(msg);               \
-    return SPB_ERR_ARG;                \
-  }
 #define DISPATCH_GAME(e, CALL_C4, CALL_TTT) ((e)->cfg.game == SPB_GAME_CONNECT4 ? (CALL_C4) : (CALL_TTT))
 
 extern "C" {
@@ -391,54 +326,46 @@ int32_t spb_default_config(spb_config* cfg) {
   return SPB_OK;
 }
 
+// The checks of spb_create beyond HostEngine::config_error (max_nodes_per_tree 0 already replaced by its default).
+static const char* config_error(const spb_config& c) {
+  if (const char* m = spb_engine::config_error(c)) return m;
+  if (c.game != SPB_GAME_CONNECT4 && c.game != SPB_GAME_TICTACTOE) return "unknown game";
+  if (c.num_games == 0 || c.num_games > (1u << 22)) return "num_games out of range";
+  if (c.leaves_per_tree < 1 || c.leaves_per_tree > 16) return "leaves_per_tree must be in 1..16";
+  if (c.max_nodes_per_tree < 16 || c.max_nodes_per_tree > MAX_CAP) return "max_nodes_per_tree out of range";
+  return nullptr;
+}
+
 int32_t spb_create(const spb_config* cfg, spb_engine** out) {
   if (!cfg || !out) { g_create_error = "null argument"; return SPB_ERR_ARG; }
   *out = nullptr;
-  if (cfg->abi_version != SPB_ABI_VERSION) { g_create_error = "abi_version mismatch"; return SPB_ERR_ARG; }
-  if (cfg->game != SPB_GAME_CONNECT4 && cfg->game != SPB_GAME_TICTACTOE) { g_create_error = "unknown game"; return SPB_ERR_ARG; }
-  if (cfg->num_games == 0 || cfg->num_games > (1u << 22)) { g_create_error = "num_games out of range"; return SPB_ERR_ARG; }
-  if (cfg->leaves_per_tree < 1 || cfg->leaves_per_tree > 16) { g_create_error = "leaves_per_tree must be in 1..16"; return SPB_ERR_ARG; }
-  if (cfg->evaluator < SPB_EVAL_NET || cfg->evaluator > SPB_EVAL_UNIFORM) { g_create_error = "unknown evaluator"; return SPB_ERR_ARG; }
-  if (!(cfg->c == cfg->c)) { g_create_error = "c is NaN"; return SPB_ERR_ARG; }
-  spb_engine* e = new (std::nothrow) spb_engine();
-  if (!e) { g_create_error = "out of host memory"; return SPB_ERR_NOMEM; }
-  e->cfg = *cfg;
-  if (e->cfg.max_nodes_per_tree == 0) e->cfg.max_nodes_per_tree = 16384;
-  if (e->cfg.max_nodes_per_tree < 16 || e->cfg.max_nodes_per_tree > MAX_CAP) { g_create_error = "max_nodes_per_tree out of range"; delete e; return SPB_ERR_ARG; }
-  int32_t rc = e->init();
-  if (rc != SPB_OK) {
-    g_create_error = e->err;
-    e->destroy();
-    delete e;
-    return rc;
-  }
-  *out = e;
-  return SPB_OK;
+  spb_config c = *cfg;
+  if (c.max_nodes_per_tree == 0) c.max_nodes_per_tree = 16384;
+  if (const char* m = config_error(c)) { g_create_error = m; return SPB_ERR_ARG; }
+  return spb_engine::create(c, out);
 }
 
 int32_t spb_destroy(spb_engine* e) {
   if (!e) return SPB_ERR_ARG;
-  cudaSetDevice(e->cfg.device);
-  cudaStreamSynchronize(e->stream);
   spb_comm_destroy(e);
-  e->destroy();
+  e->release();
   delete e;
   return SPB_OK;
 }
 
-const char* spb_last_error(const spb_engine* e) { return e ? e->err.c_str() : g_create_error.c_str(); }
+const char* spb_last_error(const spb_engine* e) { return spb_engine::last_error(e); }
 
 int32_t spb_load_weights(spb_engine* e, const void* blob, size_t n) {
-  ENGINE_GUARD(e);
-  ARG_CHECK(e, blob && n > 8, "null / empty weight blob");
+  SPB_GUARD(e);
+  SPB_ARG(e, blob && n > 8, "null / empty weight blob");
   HostNet net;
   std::string err;
   if (!parse_safetensors_net(blob, n, e->cfg.game, &net, &err)) { e->set_error("spb_load_weights: " + err); return SPB_ERR_WEIGHTS; }
-  cudaStreamSynchronize(e->stream);
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   if (!e->evaluator.upload(net, &err)) { e->set_error("spb_load_weights: " + err); return SPB_ERR_CUDA; }
   // The captured step graph holds the address of the previous weight image in its kernel nodes (hot swap between
   // generations, learner_concurrent.rs:158-159): drop it, the next search captures the new one.
-  if (e->step_graph) { cudaGraphExecDestroy(e->step_graph); e->step_graph = nullptr; }
+  e->drop_step_graph();
   e->last_eval_parity = -1;
   return SPB_OK;
 }
@@ -457,51 +384,44 @@ int32_t spb_check_weights(int32_t game, const void* blob, size_t n, char* err, s
 }
 
 int32_t spb_reset_games(spb_engine* e, const uint32_t* slots, uint32_t n, const spb_state* roots) {
-  ENGINE_GUARD(e);
-  ARG_CHECK(e, n <= e->T.G, "more slots than games");
+  SPB_GUARD(e);
+  SPB_ARG(e, n <= e->T.G, "more slots than games");
   if (n == 0) return SPB_OK;
-  if (slots) for (uint32_t i = 0; i < n; ++i) ARG_CHECK(e, slots[i] < e->T.G, "slot out of range");
+  if (slots) for (uint32_t i = 0; i < n; ++i) SPB_ARG(e, slots[i] < e->T.G, "slot out of range");
   size_t off_roots = ((size_t)n * 4 + 15) & ~(size_t)15;
   size_t bytes = off_roots + (size_t)n * sizeof(PState);
   int32_t rc = e->ensure_stage(bytes);
   if (rc) return rc;
-  {
-    auto* hs = static_cast<uint8_t*>(e->h_stage);
-    if (slots) std::memcpy(hs, slots, (size_t)n * 4);
-    if (roots) {
-      PState* hp = reinterpret_cast<PState*>(hs + off_roots);
-      for (uint32_t i = 0; i < n; ++i) hp[i] = ps_from_abi(roots[i]);
-    }
+  auto* hs = static_cast<uint8_t*>(e->h_stage);
+  if (slots) std::memcpy(hs, slots, (size_t)n * 4);
+  if (roots) {
+    PState* hp = reinterpret_cast<PState*>(hs + off_roots);
+    for (uint32_t i = 0; i < n; ++i) hp[i] = ps_from_abi(roots[i]);
   }
-  {
-    cudaError_t ce = cudaMemcpyAsync(e->d_stage, e->h_stage, bytes, cudaMemcpyHostToDevice, e->stream);
-    if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
-    auto* ds = static_cast<uint8_t*>(e->d_stage);
-    k_reset<<<(n + 127) / 128, 128, 0, e->stream>>>(e->T, e->P.hist_len, e->P.parked, slots ? reinterpret_cast<uint32_t*>(ds) : nullptr,
-                                                    roots ? reinterpret_cast<PState*>(ds + off_roots) : nullptr, n);
-    ++e->launches;
-    ce = cudaGetLastError();
-    if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);   // staging buffer is reused by the next call
-    if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
-  }
+  SPB_CUDA(e, cudaMemcpyAsync(e->d_stage, e->h_stage, bytes, cudaMemcpyHostToDevice, e->stream));
+  auto* ds = static_cast<uint8_t*>(e->d_stage);
+  k_reset<<<(n + 127) / 128, 128, 0, e->stream>>>(e->T, e->P.hist_len, e->P.parked, slots ? reinterpret_cast<uint32_t*>(ds) : nullptr,
+                                                  roots ? reinterpret_cast<PState*>(ds + off_roots) : nullptr, n);
+  ++e->launches;
+  SPB_CUDA(e, cudaGetLastError());
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));   // staging buffer is reused by the next call
   return SPB_OK;
 }
 
 int32_t spb_search(spb_engine* e, uint32_t num_searches) {
-  ENGINE_GUARD(e);
+  SPB_GUARD(e);
   return DISPATCH_GAME(e, e->search_t<Connect4>(num_searches), e->search_t<TicTacToe>(num_searches));
 }
 
 static int32_t fetch_root_children(spb_engine* e) {
-  k_root_children<<<(e->T.G + 127) / 128, 128, 0, e->stream>>>(e->T, e->d_rc_actions, e->d_rc_counts, e->d_rc_ids, e->d_rc_n);
+  k_root_children<<<(e->T.G + 127) / 128, 128, 0, e->stream>>>(e->T, e->d_rc_moves, e->d_rc_counts, e->d_rc_ids, e->d_rc_n);
   ++e->launches;
-  cudaError_t ce = cudaGetLastError();
-  if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
+  SPB_CUDA(e, cudaGetLastError());
   return SPB_OK;
 }
 
 int32_t spb_root_children_all(spb_engine* e, uint8_t* actions, uint32_t* visit_counts, uint32_t* child_ids, uint32_t* n_children) {
-  ENGINE_GUARD(e);
+  SPB_GUARD(e);
   int32_t rc = fetch_root_children(e);
   if (rc) return rc;
   const size_t G = e->T.G;
@@ -511,13 +431,11 @@ int32_t spb_root_children_all(spb_engine* e, uint8_t* actions, uint32_t* visit_c
   rc = e->ensure_stage(bytes);
   if (rc) return rc;
   auto* hs = static_cast<uint8_t*>(e->h_stage);
-  cudaError_t ce = cudaSuccess;
-  if (visit_counts) ce = cudaMemcpyAsync(hs + o_counts, e->d_rc_counts, G * SPB_MAX_ACTIONS * 4, cudaMemcpyDeviceToHost, e->stream);
-  if (ce == cudaSuccess && child_ids) ce = cudaMemcpyAsync(hs + o_ids, e->d_rc_ids, G * SPB_MAX_ACTIONS * 4, cudaMemcpyDeviceToHost, e->stream);
-  if (ce == cudaSuccess && n_children) ce = cudaMemcpyAsync(hs + o_n, e->d_rc_n, G * 4, cudaMemcpyDeviceToHost, e->stream);
-  if (ce == cudaSuccess && actions) ce = cudaMemcpyAsync(hs + o_act, e->d_rc_actions, G * SPB_MAX_ACTIONS, cudaMemcpyDeviceToHost, e->stream);
-  if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
-  if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
+  if (visit_counts) SPB_CUDA(e, cudaMemcpyAsync(hs + o_counts, e->d_rc_counts, G * SPB_MAX_ACTIONS * 4, cudaMemcpyDeviceToHost, e->stream));
+  if (child_ids) SPB_CUDA(e, cudaMemcpyAsync(hs + o_ids, e->d_rc_ids, G * SPB_MAX_ACTIONS * 4, cudaMemcpyDeviceToHost, e->stream));
+  if (n_children) SPB_CUDA(e, cudaMemcpyAsync(hs + o_n, e->d_rc_n, G * 4, cudaMemcpyDeviceToHost, e->stream));
+  if (actions) SPB_CUDA(e, cudaMemcpyAsync(hs + o_act, e->d_rc_moves, G * SPB_MAX_ACTIONS, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   if (visit_counts) std::memcpy(visit_counts, hs + o_counts, G * SPB_MAX_ACTIONS * 4);
   if (child_ids) std::memcpy(child_ids, hs + o_ids, G * SPB_MAX_ACTIONS * 4);
   if (n_children) std::memcpy(n_children, hs + o_n, G * 4);
@@ -526,19 +444,16 @@ int32_t spb_root_children_all(spb_engine* e, uint8_t* actions, uint32_t* visit_c
 }
 
 int32_t spb_root_children(spb_engine* e, uint32_t slot, uint8_t* actions, uint32_t* visit_counts, uint32_t* child_ids, uint32_t* n_children) {
-  ENGINE_GUARD(e);
-  ARG_CHECK(e, slot < e->T.G, "slot out of range");
+  SPB_GUARD(e);
+  SPB_ARG(e, slot < e->T.G, "slot out of range");
   int32_t rc = fetch_root_children(e);
   if (rc) return rc;
   uint8_t a[SPB_MAX_ACTIONS]; uint32_t c[SPB_MAX_ACTIONS], ids[SPB_MAX_ACTIONS], n = 0;
-  {
-    cudaError_t ce = cudaMemcpyAsync(a, e->d_rc_actions + (size_t)slot * SPB_MAX_ACTIONS, SPB_MAX_ACTIONS, cudaMemcpyDeviceToHost, e->stream);
-    if (ce == cudaSuccess) ce = cudaMemcpyAsync(c, e->d_rc_counts + (size_t)slot * SPB_MAX_ACTIONS, SPB_MAX_ACTIONS * 4, cudaMemcpyDeviceToHost, e->stream);
-    if (ce == cudaSuccess) ce = cudaMemcpyAsync(ids, e->d_rc_ids + (size_t)slot * SPB_MAX_ACTIONS, SPB_MAX_ACTIONS * 4, cudaMemcpyDeviceToHost, e->stream);
-    if (ce == cudaSuccess) ce = cudaMemcpyAsync(&n, e->d_rc_n + slot, 4, cudaMemcpyDeviceToHost, e->stream);
-    if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
-    if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
-  }
+  SPB_CUDA(e, cudaMemcpyAsync(a, e->d_rc_moves + (size_t)slot * SPB_MAX_ACTIONS, SPB_MAX_ACTIONS, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaMemcpyAsync(c, e->d_rc_counts + (size_t)slot * SPB_MAX_ACTIONS, SPB_MAX_ACTIONS * 4, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaMemcpyAsync(ids, e->d_rc_ids + (size_t)slot * SPB_MAX_ACTIONS, SPB_MAX_ACTIONS * 4, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaMemcpyAsync(&n, e->d_rc_n + slot, 4, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   for (uint32_t i = 0; i < n; ++i) {
     if (actions) actions[i] = a[i];
     if (visit_counts) visit_counts[i] = c[i];
@@ -549,8 +464,8 @@ int32_t spb_root_children(spb_engine* e, uint32_t slot, uint8_t* actions, uint32
 }
 
 int32_t spb_root_policy(spb_engine* e, uint32_t slot, float* policy) {
-  ENGINE_GUARD(e);
-  ARG_CHECK(e, policy, "null policy");
+  SPB_GUARD(e);
+  SPB_ARG(e, policy, "null policy");
   uint8_t a[SPB_MAX_ACTIONS]; uint32_t c[SPB_MAX_ACTIONS], n = 0;
   int32_t rc = spb_root_children(e, slot, a, c, nullptr, &n);
   if (rc) return rc;
@@ -565,24 +480,21 @@ int32_t spb_root_policy(spb_engine* e, uint32_t slot, float* policy) {
 }
 
 int32_t spb_advance(spb_engine* e, const uint32_t* slots, const uint32_t* node_ids, uint32_t n, spb_state* out_states) {
-  ENGINE_GUARD(e);
-  ARG_CHECK(e, node_ids, "null node_ids");
-  ARG_CHECK(e, n <= e->T.G, "more slots than games");
+  SPB_GUARD(e);
+  SPB_ARG(e, node_ids, "null node_ids");
+  SPB_ARG(e, n <= e->T.G, "more slots than games");
   if (n == 0) return SPB_OK;
   // validate against arena lengths (one D2H of n_nodes)
   std::vector<uint32_t> nn(e->T.G);
-  {
-    cudaError_t ce = cudaMemcpyAsync(nn.data(), e->T.n_nodes, (size_t)e->T.G * 4, cudaMemcpyDeviceToHost, e->stream);
-    if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
-    if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
-  }
+  SPB_CUDA(e, cudaMemcpyAsync(nn.data(), e->T.n_nodes, (size_t)e->T.G * 4, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   std::vector<uint8_t> seen(e->T.G, 0);
   for (uint32_t i = 0; i < n; ++i) {
     uint32_t g = slots ? slots[i] : i;
-    ARG_CHECK(e, g < e->T.G, "slot out of range");
-    ARG_CHECK(e, !seen[g], "slot listed twice");
+    SPB_ARG(e, g < e->T.G, "slot out of range");
+    SPB_ARG(e, !seen[g], "slot listed twice");
     seen[g] = 1;
-    ARG_CHECK(e, node_ids[i] < nn[g], "node id out of range");
+    SPB_ARG(e, node_ids[i] < nn[g], "node id out of range");
   }
   size_t o_ids = ((size_t)n * 4 + 15) & ~(size_t)15, o_out = o_ids * 2;
   size_t bytes = o_out + (size_t)n * sizeof(PState);
@@ -592,8 +504,7 @@ int32_t spb_advance(spb_engine* e, const uint32_t* slots, const uint32_t* node_i
   auto* ds = static_cast<uint8_t*>(e->d_stage);
   if (slots) std::memcpy(hs, slots, (size_t)n * 4);
   std::memcpy(hs + o_ids, node_ids, (size_t)n * 4);
-  cudaError_t ce = cudaMemcpyAsync(ds, hs, o_out, cudaMemcpyHostToDevice, e->stream);
-  if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
+  SPB_CUDA(e, cudaMemcpyAsync(ds, hs, o_out, cudaMemcpyHostToDevice, e->stream));
   const uint32_t blocks = (n + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK;
   const uint32_t* dsl = slots ? reinterpret_cast<uint32_t*>(ds) : nullptr;
   const uint32_t* dn = reinterpret_cast<uint32_t*>(ds + o_ids);
@@ -601,10 +512,9 @@ int32_t spb_advance(spb_engine* e, const uint32_t* slots, const uint32_t* node_i
   if (e->cfg.game == SPB_GAME_CONNECT4) k_advance<Connect4><<<blocks, THREADS, 0, e->stream>>>(e->T, dsl, dn, n, dout);
   else k_advance<TicTacToe><<<blocks, THREADS, 0, e->stream>>>(e->T, dsl, dn, n, dout);
   ++e->launches;
-  ce = cudaGetLastError();
-  if (ce == cudaSuccess) ce = cudaMemcpyAsync(hs + o_out, dout, (size_t)n * sizeof(PState), cudaMemcpyDeviceToHost, e->stream);
-  if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
-  if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
+  SPB_CUDA(e, cudaGetLastError());
+  SPB_CUDA(e, cudaMemcpyAsync(hs + o_out, dout, (size_t)n * sizeof(PState), cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   if (out_states) {
     const PState* hp = reinterpret_cast<const PState*>(hs + o_out);
     for (uint32_t i = 0; i < n; ++i) out_states[i] = ps_to_abi(hp[i]);
@@ -613,90 +523,59 @@ int32_t spb_advance(spb_engine* e, const uint32_t* slots, const uint32_t* node_i
 }
 
 int32_t spb_arena_len(spb_engine* e, uint32_t slot, uint32_t* out) {
-  ENGINE_GUARD(e);
-  ARG_CHECK(e, slot < e->T.G && out, "bad argument");
-  cudaError_t ce = cudaMemcpyAsync(out, e->T.n_nodes + slot, 4, cudaMemcpyDeviceToHost, e->stream);
-  if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
-  if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
-  return SPB_OK;
+  SPB_GUARD(e);
+  return e->arena_len(slot, out);
 }
 
 int32_t spb_get_state(spb_engine* e, uint32_t slot, uint32_t node_id, spb_state* out) {
-  ENGINE_GUARD(e);
-  ARG_CHECK(e, slot < e->T.G && out, "bad argument");
+  SPB_GUARD(e);
+  SPB_ARG(e, slot < e->T.G && out, "bad argument");
   uint32_t len = 0;
   int32_t rc = spb_arena_len(e, slot, &len);
   if (rc) return rc;
-  ARG_CHECK(e, node_id < len, "node id out of range");
+  SPB_ARG(e, node_id < len, "node id out of range");
   rc = e->ensure_stage(sizeof(PState));
   if (rc) return rc;
   if (e->cfg.game == SPB_GAME_CONNECT4) k_get_state<Connect4><<<1, 1, 0, e->stream>>>(e->T, slot, node_id, static_cast<PState*>(e->d_stage));
   else k_get_state<TicTacToe><<<1, 1, 0, e->stream>>>(e->T, slot, node_id, static_cast<PState*>(e->d_stage));
   ++e->launches;
   PState ps;
-  cudaError_t ce = cudaGetLastError();
-  if (ce == cudaSuccess) ce = cudaMemcpyAsync(&ps, e->d_stage, sizeof ps, cudaMemcpyDeviceToHost, e->stream);
-  if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
-  if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
+  SPB_CUDA(e, cudaGetLastError());
+  SPB_CUDA(e, cudaMemcpyAsync(&ps, e->d_stage, sizeof ps, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   *out = ps_to_abi(ps);
   return SPB_OK;
 }
 
 int32_t spb_set_root_noise(spb_engine* e, float alpha, float epsilon, uint64_t seed) {
-  ENGINE_GUARD(e);
-  ARG_CHECK(e, epsilon >= 0.0f && epsilon <= 1.0f, "root noise: epsilon must be in [0, 1]");
-  ARG_CHECK(e, epsilon == 0.0f || (alpha > 0.0f && alpha <= FLT_MAX), "root noise: alpha must be finite and > 0");
-  if (epsilon > 0.0f && !e->d_noise_eta) {
-    int32_t rc = e->dalloc(&e->d_noise_eta, (size_t)e->T.G * SPB_MAX_ACTIONS);
-    if (!rc) rc = e->dalloc(&e->d_noise_n, (size_t)e->T.G);
-    if (rc) return rc;
-  }
-  cudaStreamSynchronize(e->stream);
-  e->noise_alpha = alpha;
-  e->noise_seed = seed;
-  e->T.noise_n = e->d_noise_n;
-  e->T.noise_eps = epsilon;
-  e->T.noise_omeps = 1.0f - epsilon;   // rounded to f32 once, here
-  e->T.root_noise = epsilon > 0.0f ? e->d_noise_eta : nullptr;
+  SPB_GUARD(e);
+  const int32_t rc = e->set_root_noise(alpha, epsilon, seed, SPB_MAX_ACTIONS);
   // the captured step graph holds the previous Trees (and with it the noise settings): the next search captures anew
-  if (e->step_graph) { cudaGraphExecDestroy(e->step_graph); e->step_graph = nullptr; }
-  return SPB_OK;
+  if (rc == SPB_OK) e->drop_step_graph();
+  return rc;
 }
 
 int32_t spb_root_noise(spb_engine* e, uint32_t slot, float* eta, uint32_t* n) {
-  ENGINE_GUARD(e);
-  ARG_CHECK(e, slot < e->T.G && eta && n, "bad argument");
-  if (!e->T.root_noise) { e->set_error("root noise is off (spb_set_root_noise)"); return SPB_ERR_STATE; }
-  int32_t rc = e->launch_root_noise();
-  if (rc) return rc;
-  float h[SPB_MAX_ACTIONS];
-  uint32_t hn = 0;
-  cudaError_t ce = cudaMemcpyAsync(h, e->T.root_noise + (size_t)slot * SPB_MAX_ACTIONS, sizeof h, cudaMemcpyDeviceToHost, e->stream);
-  if (ce == cudaSuccess) ce = cudaMemcpyAsync(&hn, e->T.noise_n + slot, 4, cudaMemcpyDeviceToHost, e->stream);
-  if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
-  if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
-  for (uint32_t i = 0; i < SPB_MAX_ACTIONS; ++i) eta[i] = i < hn ? h[i] : 0.0f;
-  *n = hn;
-  return SPB_OK;
+  SPB_GUARD(e);
+  return e->root_noise(slot, eta, n, SPB_MAX_ACTIONS, [e] { return e->launch_root_noise(); });
 }
 
 int32_t spb_node_stats(spb_engine* e, uint32_t slot, uint32_t node_id, uint32_t* visit_count, float* value_sum, float* prior,
                        uint32_t* first_child, uint32_t* n_children) {
-  ENGINE_GUARD(e);
-  ARG_CHECK(e, slot < e->T.G, "slot out of range");
+  SPB_GUARD(e);
+  SPB_ARG(e, slot < e->T.G, "slot out of range");
   uint32_t len = 0;
   int32_t rc = spb_arena_len(e, slot, &len);
   if (rc) return rc;
-  ARG_CHECK(e, node_id < len, "node id out of range");
+  SPB_ARG(e, node_id < len, "node id out of range");
   rc = e->ensure_stage(sizeof(NodeRec));
   if (rc) return rc;
   k_node_stats<<<1, 1, 0, e->stream>>>(e->T, slot, node_id, static_cast<NodeRec*>(e->d_stage));
   ++e->launches;
   NodeRec r;
-  cudaError_t ce = cudaGetLastError();
-  if (ce == cudaSuccess) ce = cudaMemcpyAsync(&r, e->d_stage, sizeof r, cudaMemcpyDeviceToHost, e->stream);
-  if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
-  if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
+  SPB_CUDA(e, cudaGetLastError());
+  SPB_CUDA(e, cudaMemcpyAsync(&r, e->d_stage, sizeof r, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   if (visit_count) *visit_count = r.N;
   if (value_sum) *value_sum = r.W;
   if (prior) *prior = r.P;
@@ -721,40 +600,34 @@ static int32_t predict_t(spb_engine* e, const spb_state* states, uint32_t n, flo
   PState* hp = reinterpret_cast<PState*>(hs + o_states);
   for (uint32_t i = 0; i < n; ++i) hp[i] = ps_from_abi(states[i]);
   *reinterpret_cast<uint32_t*>(hs + o_cnt) = n;
-  cudaError_t ce = cudaMemcpyAsync(ds, hs, o_cnt + 4, cudaMemcpyHostToDevice, e->stream);
-  if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
+  SPB_CUDA(e, cudaMemcpyAsync(ds, hs, o_cnt + 4, cudaMemcpyHostToDevice, e->stream));
   PState* dstates = reinterpret_cast<PState*>(ds + o_states);
   uint32_t* dcnt = reinterpret_cast<uint32_t*>(ds + o_cnt);
   float* dout = reinterpret_cast<float*>(ds + o_out);
   float* dlog = reinterpret_cast<float*>(ds + o_log);
   if (e->cfg.evaluator == SPB_EVAL_NET) {
     if (!e->evaluator.loaded()) { e->set_error("no weights loaded: call spb_load_weights first"); return SPB_ERR_STATE; }
-    ce = cudaMemsetAsync(dlog, 0, (size_t)n * G::A * 4, e->stream);
-    if (ce == cudaSuccess)
-      ce = e->evaluator.launch(dstates, nullptr, dcnt, n, dout, G::EVAL_STRIDE, raw_logits ? dlog : nullptr,
-                               (e->cfg.flags & SPB_FLAG_EVAL_SIMT) != 0, e->stream);
+    SPB_CUDA(e, cudaMemsetAsync(dlog, 0, (size_t)n * G::A * 4, e->stream));
+    SPB_CUDA(e, e->evaluator.launch(dstates, nullptr, dcnt, n, dout, G::EVAL_STRIDE, raw_logits ? dlog : nullptr,
+                                    (e->cfg.flags & SPB_FLAG_EVAL_SIMT) != 0, e->stream));
   } else {
     // identity work list: k_eval_builtin indexes states by list entry, so build 0..n-1 in the logits area
     std::vector<uint32_t> idl(n);
     for (uint32_t i = 0; i < n; ++i) idl[i] = i;
-    ce = cudaMemcpyAsync(dlog, idl.data(), (size_t)n * 4, cudaMemcpyHostToDevice, e->stream);
-    if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
-    if (ce == cudaSuccess) {
-      if (e->cfg.evaluator == SPB_EVAL_DET)
-        k_eval_builtin<G, SPB_EVAL_DET><<<(n + 255) / 256, 256, 0, e->stream>>>(dstates, reinterpret_cast<uint32_t*>(dlog), dcnt, dout);
-      else
-        k_eval_builtin<G, SPB_EVAL_UNIFORM><<<(n + 255) / 256, 256, 0, e->stream>>>(dstates, reinterpret_cast<uint32_t*>(dlog), dcnt, dout);
-      ce = cudaGetLastError();
-    }
+    SPB_CUDA(e, cudaMemcpyAsync(dlog, idl.data(), (size_t)n * 4, cudaMemcpyHostToDevice, e->stream));
+    SPB_CUDA(e, cudaStreamSynchronize(e->stream));
+    if (e->cfg.evaluator == SPB_EVAL_DET)
+      k_eval_builtin<G, SPB_EVAL_DET><<<(n + 255) / 256, 256, 0, e->stream>>>(dstates, reinterpret_cast<uint32_t*>(dlog), dcnt, dout);
+    else
+      k_eval_builtin<G, SPB_EVAL_UNIFORM><<<(n + 255) / 256, 256, 0, e->stream>>>(dstates, reinterpret_cast<uint32_t*>(dlog), dcnt, dout);
+    SPB_CUDA(e, cudaGetLastError());
   }
   ++e->launches;
-  if (ce != cudaSuccess) { e->set_error(std::string("evaluator: ") + cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
   k_mask_policies<G><<<(n + 127) / 128, 128, 0, e->stream>>>(dstates, n, dout, reinterpret_cast<float*>(ds + o_pol), reinterpret_cast<float*>(ds + o_val));
   ++e->launches;
-  ce = cudaGetLastError();
-  if (ce == cudaSuccess) ce = cudaMemcpyAsync(hs + o_pol, ds + o_pol, bytes - o_pol, cudaMemcpyDeviceToHost, e->stream);
-  if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
-  if (ce != cudaSuccess) { e->set_error(std::string("predict: ") + cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
+  SPB_CUDA(e, cudaGetLastError());
+  SPB_CUDA(e, cudaMemcpyAsync(hs + o_pol, ds + o_pol, bytes - o_pol, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   if (policies) std::memcpy(policies, hs + o_pol, (size_t)n * G::A * 4);
   if (values) std::memcpy(values, hs + o_val, (size_t)n * 4);
   if (raw_logits && e->cfg.evaluator == SPB_EVAL_NET) std::memcpy(raw_logits, hs + o_log, (size_t)n * G::A * 4);
@@ -764,8 +637,8 @@ static int32_t predict_t(spb_engine* e, const spb_state* states, uint32_t n, flo
 extern "C" {
 
 int32_t spb_predict(spb_engine* e, const spb_state* states, uint32_t n, float* policies, float* values, float* raw_logits) {
-  ENGINE_GUARD(e);
-  ARG_CHECK(e, states || n == 0, "null states");
+  SPB_GUARD(e);
+  SPB_ARG(e, states || n == 0, "null states");
   if (n == 0) return SPB_OK;
   return DISPATCH_GAME(e, predict_t<Connect4>(e, states, n, policies, values, raw_logits),
                        predict_t<TicTacToe>(e, states, n, policies, values, raw_logits));
@@ -781,8 +654,8 @@ static int32_t upload_states(spb_engine* e, const spb_state* states, uint32_t n,
 }
 
 int32_t spb_game_next_states(spb_engine* e, const spb_state* states, const uint8_t* actions, uint32_t n, spb_state* out_states, int32_t* err) {
-  ENGINE_GUARD(e);
-  ARG_CHECK(e, states && actions && out_states && err, "null argument");
+  SPB_GUARD(e);
+  SPB_ARG(e, states && actions && out_states && err, "null argument");
   if (n == 0) return SPB_OK;
   const size_t o_act = (size_t)n * sizeof(PState), o_out = (o_act + n + 15) & ~(size_t)15, o_err = o_out + (size_t)n * sizeof(PState);
   int32_t rc = upload_states(e, states, n, o_err + (size_t)n * 4);
@@ -790,17 +663,15 @@ int32_t spb_game_next_states(spb_engine* e, const spb_state* states, const uint8
   auto* hs = static_cast<uint8_t*>(e->h_stage);
   auto* ds = static_cast<uint8_t*>(e->d_stage);
   std::memcpy(hs + o_act, actions, n);
-  cudaError_t ce = cudaMemcpyAsync(ds, hs, o_out, cudaMemcpyHostToDevice, e->stream);
-  if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
+  SPB_CUDA(e, cudaMemcpyAsync(ds, hs, o_out, cudaMemcpyHostToDevice, e->stream));
   if (e->cfg.game == SPB_GAME_CONNECT4)
     k_game_next<Connect4><<<(n + 127) / 128, 128, 0, e->stream>>>((PState*)ds, ds + o_act, n, (PState*)(ds + o_out), (int32_t*)(ds + o_err));
   else
     k_game_next<TicTacToe><<<(n + 127) / 128, 128, 0, e->stream>>>((PState*)ds, ds + o_act, n, (PState*)(ds + o_out), (int32_t*)(ds + o_err));
   ++e->launches;
-  ce = cudaGetLastError();
-  if (ce == cudaSuccess) ce = cudaMemcpyAsync(hs + o_out, ds + o_out, (size_t)n * (sizeof(PState) + 4), cudaMemcpyDeviceToHost, e->stream);
-  if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
-  if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
+  SPB_CUDA(e, cudaGetLastError());
+  SPB_CUDA(e, cudaMemcpyAsync(hs + o_out, ds + o_out, (size_t)n * (sizeof(PState) + 4), cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   const PState* hp = reinterpret_cast<const PState*>(hs + o_out);
   const int32_t* he = reinterpret_cast<const int32_t*>(hs + o_err);
   for (uint32_t i = 0; i < n; ++i) { out_states[i] = ps_to_abi(hp[i]); err[i] = he[i]; }
@@ -808,29 +679,27 @@ int32_t spb_game_next_states(spb_engine* e, const spb_state* states, const uint8
 }
 
 int32_t spb_game_valid_actions(spb_engine* e, const spb_state* states, uint32_t n, uint32_t* masks) {
-  ENGINE_GUARD(e);
-  ARG_CHECK(e, states && masks, "null argument");
+  SPB_GUARD(e);
+  SPB_ARG(e, states && masks, "null argument");
   if (n == 0) return SPB_OK;
   const size_t o_out = (size_t)n * sizeof(PState);
   int32_t rc = upload_states(e, states, n, o_out + (size_t)n * 4);
   if (rc) return rc;
   auto* hs = static_cast<uint8_t*>(e->h_stage);
   auto* ds = static_cast<uint8_t*>(e->d_stage);
-  cudaError_t ce = cudaMemcpyAsync(ds, hs, o_out, cudaMemcpyHostToDevice, e->stream);
-  if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
+  SPB_CUDA(e, cudaMemcpyAsync(ds, hs, o_out, cudaMemcpyHostToDevice, e->stream));
   if (e->cfg.game == SPB_GAME_CONNECT4) k_game_valid<Connect4><<<(n + 127) / 128, 128, 0, e->stream>>>((PState*)ds, n, (uint32_t*)(ds + o_out));
   else k_game_valid<TicTacToe><<<(n + 127) / 128, 128, 0, e->stream>>>((PState*)ds, n, (uint32_t*)(ds + o_out));
   ++e->launches;
-  ce = cudaGetLastError();
-  if (ce == cudaSuccess) ce = cudaMemcpyAsync(masks, ds + o_out, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream);
-  if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
-  if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
+  SPB_CUDA(e, cudaGetLastError());
+  SPB_CUDA(e, cudaMemcpyAsync(masks, ds + o_out, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   return SPB_OK;
 }
 
 int32_t spb_game_encode(spb_engine* e, const spb_state* states, uint32_t n, float* out) {
-  ENGINE_GUARD(e);
-  ARG_CHECK(e, states && out, "null argument");
+  SPB_GUARD(e);
+  SPB_ARG(e, states && out, "null argument");
   if (n == 0) return SPB_OK;
   const bool c4 = e->cfg.game == SPB_GAME_CONNECT4;
   const size_t E = c4 ? 3 * 6 * 7 : 27;
@@ -839,85 +708,56 @@ int32_t spb_game_encode(spb_engine* e, const spb_state* states, uint32_t n, floa
   if (rc) return rc;
   auto* hs = static_cast<uint8_t*>(e->h_stage);
   auto* ds = static_cast<uint8_t*>(e->d_stage);
-  cudaError_t ce = cudaMemcpyAsync(ds, hs, o_out, cudaMemcpyHostToDevice, e->stream);
-  if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
+  SPB_CUDA(e, cudaMemcpyAsync(ds, hs, o_out, cudaMemcpyHostToDevice, e->stream));
   const size_t total = (size_t)n * E;
   if (c4) k_game_encode<Connect4><<<(unsigned)((total + 255) / 256), 256, 0, e->stream>>>((PState*)ds, n, (float*)(ds + o_out));
   else k_game_encode<TicTacToe><<<(unsigned)((total + 255) / 256), 256, 0, e->stream>>>((PState*)ds, n, (float*)(ds + o_out));
   ++e->launches;
-  ce = cudaGetLastError();
-  if (ce == cudaSuccess) ce = cudaMemcpyAsync(out, ds + o_out, total * 4, cudaMemcpyDeviceToHost, e->stream);
-  if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
-  if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
+  SPB_CUDA(e, cudaGetLastError());
+  SPB_CUDA(e, cudaMemcpyAsync(out, ds + o_out, total * 4, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   return SPB_OK;
 }
 
 // ---- self-play ----------------------------------------------------------------------------------
 int32_t spb_selfplay_step(spb_engine* e, int32_t rule, float temperature, uint64_t seed, const spb_state* restart_roots, uint32_t* n_finished) {
-  ENGINE_GUARD(e);
-  ARG_CHECK(e, rule == SPB_MOVE_GREEDY_LAST_MAX || rule == SPB_MOVE_TEMPERATURE, "unknown move rule");
+  SPB_GUARD(e);
+  SPB_ARG(e, rule == SPB_MOVE_GREEDY_LAST_MAX || rule == SPB_MOVE_TEMPERATURE, "unknown move rule");
   const uint32_t G = e->T.G;
   PState* droots = nullptr;
   if (restart_roots) {
     int32_t rc = upload_states(e, restart_roots, G, 0);
     if (rc) return rc;
-    cudaError_t ce = cudaMemcpyAsync(e->d_stage, e->h_stage, (size_t)G * sizeof(PState), cudaMemcpyHostToDevice, e->stream);
-    if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
+    SPB_CUDA(e, cudaMemcpyAsync(e->d_stage, e->h_stage, (size_t)G * sizeof(PState), cudaMemcpyHostToDevice, e->stream));
     droots = static_cast<PState*>(e->d_stage);
   }
-  cudaError_t ce = cudaMemsetAsync(e->P.finished, 0, 4, e->stream);
-  if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
+  SPB_CUDA(e, cudaMemsetAsync(e->P.finished, 0, 4, e->stream));
   const uint32_t blocks = (G + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK;
   if (e->cfg.game == SPB_GAME_CONNECT4) k_selfplay_step<Connect4><<<blocks, THREADS, 0, e->stream>>>(e->T, e->P, rule, temperature, seed, droots);
   else k_selfplay_step<TicTacToe><<<blocks, THREADS, 0, e->stream>>>(e->T, e->P, rule, temperature, seed, droots);
   ++e->launches;
   uint32_t fin = 0;
-  ce = cudaGetLastError();
-  if (ce == cudaSuccess) ce = cudaMemcpyAsync(&fin, e->P.finished, 4, cudaMemcpyDeviceToHost, e->stream);
-  if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
+  SPB_CUDA(e, cudaGetLastError());
+  SPB_CUDA(e, cudaMemcpyAsync(&fin, e->P.finished, 4, cudaMemcpyDeviceToHost, e->stream));
   int32_t rc = e->check_device_errors();
   if (n_finished) *n_finished = fin;
   return rc;
 }
 
 int32_t spb_drain_trajectories(spb_engine* e, spb_position* buf, size_t capacity, size_t* written, uint64_t* game_ids) {
-  ENGINE_GUARD(e);
-  return drain_trajectories(e, e->P, e->stream, buf, capacity, written, game_ids);
+  SPB_GUARD(e);
+  return e->drain_trajectories(buf, capacity, written, game_ids);
 }
 
 // ---- counters -----------------------------------------------------------------------------------
 int32_t spb_get_counters(spb_engine* e, spb_counters* out) {
-  ENGINE_GUARD(e);
-  ARG_CHECK(e, out, "null out");
-  std::memset(out, 0, sizeof *out);
-  unsigned long long c[CTR_COUNT], live = 0;
-  cudaError_t ce = cudaMemsetAsync(e->d_misc, 0, 8, e->stream);
-  if (ce == cudaSuccess) {
-    k_nodes_live<<<(e->T.G + 127) / 128, 128, 0, e->stream>>>(e->T, e->d_misc);
-    ++e->launches;
-    ce = cudaGetLastError();
-  }
-  if (ce == cudaSuccess) ce = cudaMemcpyAsync(c, e->T.counters, sizeof c, cudaMemcpyDeviceToHost, e->stream);
-  if (ce == cudaSuccess) ce = cudaMemcpyAsync(&live, e->d_misc, 8, cudaMemcpyDeviceToHost, e->stream);
-  if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
-  if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
-  out->simulations = c[CTR_SIMS];
-  out->evaluations = c[CTR_EVALS];
-  out->terminal_leaves = c[CTR_TERMINAL];
-  out->path_length_sum = c[CTR_PATHSUM];
-  out->children_created = c[CTR_CHILDREN];
-  out->nodes_live = live;
-  out->kernel_launches = e->launches;
-  return SPB_OK;
+  SPB_GUARD(e);
+  return e->get_counters(out, false, [e] { k_nodes_live<<<(e->T.G + 127) / 128, 128, 0, e->stream>>>(e->T, e->d_misc); });
 }
 
 int32_t spb_reset_counters(spb_engine* e) {
-  ENGINE_GUARD(e);
-  cudaError_t ce = cudaMemsetAsync(e->T.counters, 0, CTR_COUNT * 8, e->stream);
-  if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
-  if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
-  e->launches = 0;
-  return SPB_OK;
+  SPB_GUARD(e);
+  return e->reset_counters();
 }
 
 int32_t spb_last_search_timing(spb_engine* e, float* search_ms, float* evaluator_ms, uint32_t* evaluator_launches) {
@@ -929,33 +769,31 @@ int32_t spb_last_search_timing(spb_engine* e, float* search_ms, float* evaluator
 }
 
 int32_t spb_time_evaluator(spb_engine* e, uint32_t iters, float* avg_ms, uint32_t* n_positions, double* flops_per_position) {
-  ENGINE_GUARD(e);
-  ARG_CHECK(e, iters > 0 && avg_ms, "bad argument");
+  SPB_GUARD(e);
+  SPB_ARG(e, iters > 0 && avg_ms, "bad argument");
   if (e->cfg.evaluator != SPB_EVAL_NET || !e->evaluator.loaded()) { e->set_error("needs the network evaluator with weights loaded"); return SPB_ERR_STATE; }
   const uint32_t slots = e->T.G * e->T.K;
   const uint32_t* cnt = &e->T.eval_count[2];
   const bool simt = (e->cfg.flags & SPB_FLAG_EVAL_SIMT) != 0;
-  cudaError_t ce = cudaSuccess;
   // Lock-step pipeline: the work list of the last simulation step.  Asynchronous pipeline (no step lists): the latest
   // evaluated leaf of every slot, as one static list of G positions.
   const uint32_t* list = e->T.eval_list;
   if (e->last_eval_parity < 0) {
     list = nullptr;
-    ce = cudaMemcpyAsync(&e->T.eval_count[2], &slots, 4, cudaMemcpyHostToDevice, e->stream);
-    if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
+    SPB_CUDA(e, cudaMemcpyAsync(&e->T.eval_count[2], &slots, 4, cudaMemcpyHostToDevice, e->stream));
+    SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   }
-  for (int w = 0; w < 2 && ce == cudaSuccess; ++w)    // warm-up
-    ce = e->evaluator.launch(e->T.leaf_state, list, cnt, slots, e->T.eval_out, e->eval_stride, nullptr, simt, e->stream, /*overlap=*/false);
-  if (ce == cudaSuccess) ce = cudaEventRecord(e->ev0, e->stream);
-  for (uint32_t i = 0; i < iters && ce == cudaSuccess; ++i)
-    ce = e->evaluator.launch(e->T.leaf_state, list, cnt, slots, e->T.eval_out, e->eval_stride, nullptr, simt, e->stream, /*overlap=*/false);
-  if (ce == cudaSuccess) ce = cudaEventRecord(e->ev1, e->stream);
+  for (int w = 0; w < 2; ++w)    // warm-up
+    SPB_CUDA(e, e->evaluator.launch(e->T.leaf_state, list, cnt, slots, e->T.eval_out, e->eval_stride, nullptr, simt, e->stream, /*overlap=*/false));
+  SPB_CUDA(e, cudaEventRecord(e->ev0, e->stream));
+  for (uint32_t i = 0; i < iters; ++i)
+    SPB_CUDA(e, e->evaluator.launch(e->T.leaf_state, list, cnt, slots, e->T.eval_out, e->eval_stride, nullptr, simt, e->stream, /*overlap=*/false));
+  SPB_CUDA(e, cudaEventRecord(e->ev1, e->stream));
   uint32_t n = 0;
-  if (ce == cudaSuccess) ce = cudaMemcpyAsync(&n, cnt, 4, cudaMemcpyDeviceToHost, e->stream);
-  if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
+  SPB_CUDA(e, cudaMemcpyAsync(&n, cnt, 4, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   float ms = 0.f;
-  if (ce == cudaSuccess) ce = cudaEventElapsedTime(&ms, e->ev0, e->ev1);
-  if (ce != cudaSuccess) { e->set_error(std::string("spb_time_evaluator: ") + cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
+  SPB_CUDA(e, cudaEventElapsedTime(&ms, e->ev0, e->ev1));
   e->launches += iters + 2;
   *avg_ms = ms / (float)iters;
   if (n_positions) *n_positions = n;
@@ -970,9 +808,8 @@ int32_t spb_last_async_stats(spb_engine* e, uint64_t* out, uint32_t n) {
 }
 
 int32_t spb_synchronize(spb_engine* e) {
-  ENGINE_GUARD(e);
-  cudaError_t ce = cudaStreamSynchronize(e->stream);
-  if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
+  SPB_GUARD(e);
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   return SPB_OK;
 }
 

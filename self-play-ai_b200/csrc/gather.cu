@@ -5,7 +5,8 @@
 // (ref: src/learner_concurrent.rs:281-288).  NCCL has no gatherv: all-gather of the per-rank record counts, then grouped
 // ncclSend / ncclRecv of the records into one device buffer on the learner rank; the learner orders them by
 // (global game id, ply), so an R-rank generation is byte-identical to the same games played on one rank.  The Connect4 /
-// tic-tac-toe engine (spb_position records) and the chess engine (spb_chess_position) run the same code.
+// tic-tac-toe engine (spb_position records) and the chess engine (spb_chess_position) run the same code, over the state
+// the two share (HostEngine, host_engine.hpp).
 // spb_positions_to_training builds the tensors the learners train on (ref: src/learner_concurrent.rs:126-146,
 // src/learner.rs:162-182) from the compact records.
 //
@@ -15,7 +16,6 @@
 #include <nccl.h>
 
 #include <mutex>
-#include <type_traits>
 
 #include "chess_engine.hpp"
 #include "engine.hpp"
@@ -84,16 +84,13 @@ void sort_records(std::vector<Rec>& pos, std::vector<unsigned long long>& ids) {
   ids.swap(i2);
 }
 
-// The engine types name their entry points in error texts.
-template <class Eng> const char* api_prefix() { return std::is_same<Eng, spb_chess_engine>::value ? "spb_chess_" : "spb_"; }
-
 // spb_comm_init / spb_chess_comm_init
-template <class Eng>
-int32_t comm_init(Eng* e, const uint8_t* id, int32_t rank, int32_t world_size) {
-  if (!e || !id) return SPB_ERR_ARG;
-  if (cudaSetDevice(e->cfg.device) != cudaSuccess) { e->set_error("cudaSetDevice failed"); return SPB_ERR_CUDA; }
-  if (world_size < 1 || rank < 0 || rank >= world_size) { e->set_error("rank / world_size out of range"); return SPB_ERR_ARG; }
-  if (e->nccl_comm) { e->set_error(std::string("communicator already initialised (") + api_prefix<Eng>() + "comm_destroy first)"); return SPB_ERR_STATE; }
+template <class Trees, class Rec, class Move>
+int32_t comm_init(HostEngine<Trees, Rec, Move>* e, const uint8_t* id, int32_t rank, int32_t world_size) {
+  if (!id) return SPB_ERR_ARG;
+  SPB_GUARD(e);
+  SPB_ARG(e, world_size >= 1 && rank >= 0 && rank < world_size, "rank / world_size out of range");
+  if (e->nccl_comm) { e->set_error(std::string("communicator already initialised (") + e->api + "comm_destroy first)"); return SPB_ERR_STATE; }
   NcclApi* N = nccl_api();
   if (!N->error.empty()) { e->set_error(N->error); return SPB_ERR_STATE; }
   ncclUniqueId u;
@@ -107,8 +104,8 @@ int32_t comm_init(Eng* e, const uint8_t* id, int32_t rank, int32_t world_size) {
 }
 
 // spb_comm_destroy / spb_chess_comm_destroy (also called by the engines' destroy)
-template <class Eng>
-int32_t comm_destroy(Eng* e) {
+template <class Trees, class Rec, class Move>
+int32_t comm_destroy(HostEngine<Trees, Rec, Move>* e) {
   if (!e) return SPB_ERR_ARG;
   if (e->nccl_comm) {
     cudaSetDevice(e->cfg.device);
@@ -126,12 +123,13 @@ int32_t comm_destroy(Eng* e) {
 // runs on e->stream: the self-play steps that filled P ran there, and the chess search's second stream rejoins it before
 // spb_chess_search returns.  Buffers not allocated yet (a chess engine that never played, P.out == NULL) take part with 0
 // records and stay unallocated.
-template <class Eng, class Rec>
-int32_t gather_trajectories(Eng* e, int32_t learner_rank, Rec* buf, size_t capacity, size_t* written, uint64_t* game_ids) {
-  if (!e || !written) return SPB_ERR_ARG;
-  if (cudaSetDevice(e->cfg.device) != cudaSuccess) { e->set_error("cudaSetDevice failed"); return SPB_ERR_CUDA; }
-  if (!e->nccl_comm) { e->set_error(std::string("no communicator: call ") + api_prefix<Eng>() + "comm_init first"); return SPB_ERR_STATE; }
-  if (learner_rank < 0 || learner_rank >= e->comm_world) { e->set_error("learner rank out of range"); return SPB_ERR_ARG; }
+template <class Trees, class Rec, class Move>
+int32_t gather_trajectories(HostEngine<Trees, Rec, Move>* e, int32_t learner_rank, Rec* buf, size_t capacity, size_t* written,
+                            uint64_t* game_ids) {
+  if (!written) return SPB_ERR_ARG;
+  SPB_GUARD(e);
+  if (!e->nccl_comm) { e->set_error(std::string("no communicator: call ") + e->api + "comm_init first"); return SPB_ERR_STATE; }
+  SPB_ARG(e, learner_rank >= 0 && learner_rank < e->comm_world, "learner rank out of range");
   NcclApi* N = nccl_api();
   ncclComm_t comm = static_cast<ncclComm_t>(e->nccl_comm);
   const int rank = e->comm_rank, world = e->comm_world;
@@ -142,12 +140,12 @@ int32_t gather_trajectories(Eng* e, int32_t learner_rank, Rec* buf, size_t capac
     // ---- the collective: counts, then the records -----------------------------------------------------------------
     unsigned long long n_local = 0;
     if (P.out) {
-      SPB_CUDA_E(e, cudaMemcpyAsync(&n_local, P.out_cursor, 8, cudaMemcpyDeviceToHost, e->stream));
-      SPB_CUDA_E(e, cudaStreamSynchronize(e->stream));
+      SPB_CUDA(e, cudaMemcpyAsync(&n_local, P.out_cursor, 8, cudaMemcpyDeviceToHost, e->stream));
+      SPB_CUDA(e, cudaStreamSynchronize(e->stream));
       n_local = std::min<unsigned long long>(n_local, P.out_cap);
     }
     unsigned long long* d_counts = nullptr;
-    SPB_CUDA_E(e, cudaMalloc((void**)&d_counts, (size_t)world * 8));
+    SPB_CUDA(e, cudaMalloc((void**)&d_counts, (size_t)world * 8));
     std::vector<unsigned long long> counts((size_t)world, 0);
     cudaError_t ce = cudaMemcpyAsync(d_counts + rank, &n_local, 8, cudaMemcpyHostToDevice, e->stream);
     ncclResult_t nr = ce == cudaSuccess ? N->AllGather(d_counts + rank, d_counts, 1, ncclUint64, comm, e->stream) : ncclSuccess;

@@ -1,7 +1,7 @@
 // trajectory.cuh — the trajectory buffers of the self-play ply (ref: learner_concurrent.rs:179-238), shared by the
 // Connect4 / tic-tac-toe engine (kernels.cuh, record spb_position) and the chess engine (chess_engine.cu, record
-// spb_chess_position): per-slot in-progress histories on the device, one output buffer of finished games, and the
-// drain that hands them to the host ordered by (game id, ply).
+// spb_chess_position): per-slot in-progress histories on the device, one output buffer of finished games, and the order
+// in which the drain (HostEngine::drain_trajectories, host_engine.hpp) and the gather hand them over: (game id, ply).
 #pragma once
 #include <algorithm>
 #include <numeric>
@@ -69,39 +69,6 @@ std::vector<size_t> record_order(const std::vector<Rec>& pos, const std::vector<
     return pos[a].ply < pos[b].ply;
   });
   return order;
-}
-
-// spb_drain_trajectories / spb_chess_drain_trajectories: copies the finished records out (buf == NULL: size query) and
-// empties the output buffer.  Buffers not allocated yet (P.out == NULL) hold no record.
-template <class Eng, class Rec>
-int32_t drain_trajectories(Eng* e, const Trajectories<Rec>& P, cudaStream_t stream, Rec* buf, size_t capacity, size_t* written,
-                           uint64_t* game_ids) {
-  if (!written) { e->set_error("null written"); return SPB_ERR_ARG; }
-  unsigned long long cur = 0;
-  cudaError_t ce = cudaSuccess;
-  if (P.out) {
-    ce = cudaMemcpyAsync(&cur, P.out_cursor, 8, cudaMemcpyDeviceToHost, stream);
-    if (ce == cudaSuccess) ce = cudaStreamSynchronize(stream);
-    if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
-  }
-  const size_t n = (size_t)std::min<unsigned long long>(cur, P.out_cap);
-  *written = n;
-  if (!buf) return SPB_OK;                        // size query
-  if (capacity < n) { e->set_error("trajectory buffer too small"); return SPB_ERR_ARG; }
-  if (n == 0) return SPB_OK;
-  std::vector<Rec> pos(n);
-  std::vector<unsigned long long> ids(n);
-  ce = cudaMemcpyAsync(pos.data(), P.out, n * sizeof(Rec), cudaMemcpyDeviceToHost, stream);
-  if (ce == cudaSuccess) ce = cudaMemcpyAsync(ids.data(), P.out_game, n * 8, cudaMemcpyDeviceToHost, stream);
-  if (ce == cudaSuccess) ce = cudaMemsetAsync(P.out_cursor, 0, 8, stream);
-  if (ce == cudaSuccess) ce = cudaStreamSynchronize(stream);
-  if (ce != cudaSuccess) { e->set_error(cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
-  const std::vector<size_t> order = record_order(pos, ids);
-  for (size_t i = 0; i < n; ++i) {
-    buf[i] = pos[order[i]];
-    if (game_ids) game_ids[i] = ids[order[i]];
-  }
-  return SPB_OK;
 }
 
 }  // namespace spb

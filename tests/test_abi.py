@@ -51,13 +51,56 @@ def test_create_rejects_bad_config():
     cfg = S.Config()
     L.spb_default_config(C.byref(cfg))
     h = C.c_void_p()
-    for field, val in [("abi_version", 99), ("game", 7), ("num_games", 0), ("leaves_per_tree", 0), ("evaluator", 9)]:
+    for field, val in [("abi_version", 99), ("game", 7), ("num_games", 0), ("leaves_per_tree", 0), ("evaluator", 9),
+                       ("c", float("nan")), ("max_nodes_per_tree", 8), ("num_games", 2**22 + 1), ("leaves_per_tree", 17)]:
         bad = S.Config.from_buffer_copy(cfg)
         setattr(bad, field, val)
         assert L.spb_create(C.byref(bad), C.byref(h)) == -1, field
         assert L.spb_last_error(None)
     assert L.spb_create(None, C.byref(h)) == -1
     assert L.spb_destroy(None) == -1 and L.spb_search(None, 1) == -1
+
+
+def chess_config():
+    cfg = S.Config()
+    S.load_library().spb_default_config(C.byref(cfg))
+    cfg.game, cfg.num_games, cfg.evaluator = S.GAME_CHESS, 4, S.EVAL_DET
+    return cfg
+
+
+def test_chess_create_rejects_bad_config():
+    L = S.load_library()
+    h = C.c_void_p()
+    for field, val in [("abi_version", 99), ("game", S.GAME_C4), ("num_games", 0), ("num_games", 2**20 + 1),
+                       ("leaves_per_tree", 2), ("evaluator", 9), ("c", float("nan")), ("max_nodes_per_tree", 100)]:
+        bad = chess_config()
+        setattr(bad, field, val)
+        assert L.spb_chess_create(C.byref(bad), C.byref(h)) == -1, field
+        assert L.spb_chess_last_error(None), field
+    assert L.spb_chess_create(None, C.byref(h)) == -1
+
+
+def test_chess_create_fails_loudly_without_a_gpu():
+    import torch
+    if torch.cuda.is_available():
+        pytest.skip("GPU present")
+    L = S.load_library()
+    h = C.c_void_p()
+    assert L.spb_chess_create(C.byref(chess_config()), C.byref(h)) == -2
+    assert b"no CPU fallback" in L.spb_chess_last_error(None)
+
+
+def test_every_entry_point_rejects_a_null_engine():
+    # every function of the header whose first parameter is an engine handle, called with NULL, NULL pointers and zeros
+    L = S.load_library()
+    names = re.findall(r"\b(spb_[a-z_0-9]+)\s*\(\s*(?:const\s+)?(?:spb_engine|spb_chess_engine)\s*\*", HEADER)
+    names = sorted(set(n for n in names if not n.endswith("last_error")))
+    assert any(n.startswith("spb_chess_") for n in names) and len(names) > 50
+    for name in names:
+        f = getattr(L, name)
+        assert f.argtypes is not None, name
+        args = [None if t in (C.c_void_p, C.c_char_p) or issubclass(t, C._Pointer) else 0 for t in f.argtypes]
+        assert f(*args) == -1, name
 
 
 @pytest.mark.parametrize("game", [S.GAME_TTT, S.GAME_C4])
