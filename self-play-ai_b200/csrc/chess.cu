@@ -231,7 +231,19 @@ __global__ void __launch_bounds__(TRAIN_THREADS) k_chess_training(const spb_ches
 using namespace spb;
 namespace ch = spb::chess;
 
-using spb::chess::Scratch;
+// The device buffers of one spb_chess_perft, freed when it returns: the frontier of every level (up to 2^23 positions of
+// 80 bytes, its size known only once the level before it is counted, and read while the next level is written) and the
+// output offsets of every level expanded.  They do not go in the engine's grow-only stage, which would keep them.
+struct PerftBuffers {
+  std::vector<void*> ptrs;
+  ~PerftBuffers() { for (void* p : ptrs) cudaFree(p); }
+  template <class T> T* alloc(size_t count) {
+    void* p = nullptr;
+    if (cudaMalloc(&p, count * sizeof(T)) != cudaSuccess) { cudaGetLastError(); return nullptr; }
+    ptrs.push_back(p);
+    return static_cast<T*>(p);
+  }
+};
 
 extern "C" {
 
@@ -326,27 +338,28 @@ int32_t spb_chess_legal_moves(spb_chess_engine* e, const spb_chess_state* states
   SPB_GUARD(e);
   if (n == 0) return SPB_OK;
   SPB_ARG(e, states, "null states");
-  Scratch sc;
-  auto* d_states = sc.alloc<ch::Pos>(n);
-  auto* d_hist = history ? sc.alloc<uint64_t>((size_t)n * SPB_CHESS_MAX_HISTORY) : nullptr;
-  auto* d_moves = moves ? sc.alloc<uint16_t>((size_t)n * SPB_CHESS_MAX_MOVES) : nullptr;
-  auto* d_pidx = policy_index ? sc.alloc<uint16_t>((size_t)n * SPB_CHESS_MAX_MOVES) : nullptr;
-  auto* d_counts = sc.alloc<uint32_t>(n);
-  auto* d_reps = sc.alloc<uint32_t>(n);
-  auto* d_status = sc.alloc<uint8_t>(n);
-  if (!d_states || (history && !d_hist) || (moves && !d_moves) || (policy_index && !d_pidx) || !d_counts || !d_reps || !d_status) {
-    e->set_error("chess: out of device memory");
-    return SPB_ERR_NOMEM;
-  }
+  const size_t hist_bytes = (size_t)n * SPB_CHESS_MAX_HISTORY * 8, row_bytes = (size_t)n * SPB_CHESS_MAX_MOVES * 2;
+  StageLayout L;
+  const size_t o_states = L.take((size_t)n * sizeof(ch::Pos)), o_hist = L.take(history ? hist_bytes : 0);
+  const size_t o_moves = L.take(moves ? row_bytes : 0), o_pidx = L.take(policy_index ? row_bytes : 0);
+  const size_t o_counts = L.take((size_t)n * 4), o_reps = L.take((size_t)n * 4), o_status = L.take(n);
+  if (int32_t rc = e->ensure_stage(L.bytes, 0)) return rc;
+  auto* d_states = e->d_at<ch::Pos>(o_states);
+  auto* d_hist = history ? e->d_at<uint64_t>(o_hist) : nullptr;
+  auto* d_moves = moves ? e->d_at<uint16_t>(o_moves) : nullptr;
+  auto* d_pidx = policy_index ? e->d_at<uint16_t>(o_pidx) : nullptr;
+  auto* d_counts = e->d_at<uint32_t>(o_counts);
+  auto* d_reps = e->d_at<uint32_t>(o_reps);
+  auto* d_status = e->d_at<uint8_t>(o_status);
   SPB_CUDA(e, cudaMemcpyAsync(d_states, states, (size_t)n * sizeof(ch::Pos), cudaMemcpyHostToDevice, e->stream));
-  if (history) SPB_CUDA(e, cudaMemcpyAsync(d_hist, history, (size_t)n * SPB_CHESS_MAX_HISTORY * 8, cudaMemcpyHostToDevice, e->stream));
-  if (d_moves) SPB_CUDA(e, cudaMemsetAsync(d_moves, 0xFF, (size_t)n * SPB_CHESS_MAX_MOVES * 2, e->stream));
-  if (d_pidx) SPB_CUDA(e, cudaMemsetAsync(d_pidx, 0xFF, (size_t)n * SPB_CHESS_MAX_MOVES * 2, e->stream));
+  if (history) SPB_CUDA(e, cudaMemcpyAsync(d_hist, history, hist_bytes, cudaMemcpyHostToDevice, e->stream));
+  if (moves) SPB_CUDA(e, cudaMemsetAsync(d_moves, 0xFF, row_bytes, e->stream));
+  if (policy_index) SPB_CUDA(e, cudaMemsetAsync(d_pidx, 0xFF, row_bytes, e->stream));
   ch::k_legal<<<(n + 63) / 64, 64, 0, e->stream>>>(d_states, d_hist, n, d_moves, d_counts, d_pidx, d_status, d_reps);
   SPB_CUDA(e, cudaGetLastError());
   ++e->launches;
-  if (moves) SPB_CUDA(e, cudaMemcpyAsync(moves, d_moves, (size_t)n * SPB_CHESS_MAX_MOVES * 2, cudaMemcpyDeviceToHost, e->stream));
-  if (policy_index) SPB_CUDA(e, cudaMemcpyAsync(policy_index, d_pidx, (size_t)n * SPB_CHESS_MAX_MOVES * 2, cudaMemcpyDeviceToHost, e->stream));
+  if (moves) SPB_CUDA(e, cudaMemcpyAsync(moves, d_moves, row_bytes, cudaMemcpyDeviceToHost, e->stream));
+  if (policy_index) SPB_CUDA(e, cudaMemcpyAsync(policy_index, d_pidx, row_bytes, cudaMemcpyDeviceToHost, e->stream));
   if (counts) SPB_CUDA(e, cudaMemcpyAsync(counts, d_counts, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
   if (repetitions) SPB_CUDA(e, cudaMemcpyAsync(repetitions, d_reps, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
   if (status) SPB_CUDA(e, cudaMemcpyAsync(status, d_status, (size_t)n, cudaMemcpyDeviceToHost, e->stream));
@@ -359,22 +372,25 @@ int32_t spb_chess_next_states(spb_chess_engine* e, const spb_chess_state* states
   SPB_GUARD(e);
   if (n == 0) return SPB_OK;
   SPB_ARG(e, states && moves && out_states && err, "null argument");
-  Scratch sc;
-  auto* d_states = sc.alloc<ch::Pos>(n);
-  auto* d_out = sc.alloc<ch::Pos>(n);
-  auto* d_hist = history ? sc.alloc<uint64_t>((size_t)n * SPB_CHESS_MAX_HISTORY) : nullptr;
-  auto* d_moves = sc.alloc<uint16_t>(n);
-  auto* d_err = sc.alloc<int32_t>(n);
-  if (!d_states || !d_out || (history && !d_hist) || !d_moves || !d_err) { e->set_error("chess: out of device memory"); return SPB_ERR_NOMEM; }
+  const size_t hist_bytes = (size_t)n * SPB_CHESS_MAX_HISTORY * 8;
+  StageLayout L;
+  const size_t o_states = L.take((size_t)n * sizeof(ch::Pos)), o_out = L.take((size_t)n * sizeof(ch::Pos)), o_hist = L.take(history ? hist_bytes : 0);
+  const size_t o_moves = L.take((size_t)n * 2), o_err = L.take((size_t)n * 4);
+  if (int32_t rc = e->ensure_stage(L.bytes, 0)) return rc;
+  auto* d_states = e->d_at<ch::Pos>(o_states);
+  auto* d_out = e->d_at<ch::Pos>(o_out);
+  auto* d_hist = history ? e->d_at<uint64_t>(o_hist) : nullptr;
+  auto* d_moves = e->d_at<uint16_t>(o_moves);
+  auto* d_err = e->d_at<int32_t>(o_err);
   SPB_CUDA(e, cudaMemcpyAsync(d_states, states, (size_t)n * sizeof(ch::Pos), cudaMemcpyHostToDevice, e->stream));
   SPB_CUDA(e, cudaMemcpyAsync(d_moves, moves, (size_t)n * 2, cudaMemcpyHostToDevice, e->stream));
-  if (history) SPB_CUDA(e, cudaMemcpyAsync(d_hist, history, (size_t)n * SPB_CHESS_MAX_HISTORY * 8, cudaMemcpyHostToDevice, e->stream));
+  if (history) SPB_CUDA(e, cudaMemcpyAsync(d_hist, history, hist_bytes, cudaMemcpyHostToDevice, e->stream));
   ch::k_next<<<(n + 63) / 64, 64, 0, e->stream>>>(d_states, d_hist, d_moves, n, d_out, d_err);
   SPB_CUDA(e, cudaGetLastError());
   ++e->launches;
   SPB_CUDA(e, cudaMemcpyAsync(out_states, d_out, (size_t)n * sizeof(ch::Pos), cudaMemcpyDeviceToHost, e->stream));
   SPB_CUDA(e, cudaMemcpyAsync(err, d_err, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
-  if (history) SPB_CUDA(e, cudaMemcpyAsync(history, d_hist, (size_t)n * SPB_CHESS_MAX_HISTORY * 8, cudaMemcpyDeviceToHost, e->stream));
+  if (history) SPB_CUDA(e, cudaMemcpyAsync(history, d_hist, hist_bytes, cudaMemcpyDeviceToHost, e->stream));
   SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   return SPB_OK;
 }
@@ -383,17 +399,19 @@ int32_t spb_chess_encode(spb_chess_engine* e, const spb_chess_state* states, con
   SPB_GUARD(e);
   if (n == 0) return SPB_OK;
   SPB_ARG(e, states && out, "null argument");
-  Scratch sc;
-  auto* d_states = sc.alloc<ch::Pos>(n);
-  auto* d_hist = history ? sc.alloc<uint64_t>((size_t)n * SPB_CHESS_MAX_HISTORY) : nullptr;
-  auto* d_out = sc.alloc<float>((size_t)n * SPB_CHESS_PLANES * 64);
-  if (!d_states || (history && !d_hist) || !d_out) { e->set_error("chess: out of device memory"); return SPB_ERR_NOMEM; }
+  const size_t hist_bytes = (size_t)n * SPB_CHESS_MAX_HISTORY * 8, out_bytes = (size_t)n * SPB_CHESS_PLANES * 64 * 4;
+  StageLayout L;
+  const size_t o_states = L.take((size_t)n * sizeof(ch::Pos)), o_hist = L.take(history ? hist_bytes : 0), o_out = L.take(out_bytes);
+  if (int32_t rc = e->ensure_stage(L.bytes, 0)) return rc;
+  auto* d_states = e->d_at<ch::Pos>(o_states);
+  auto* d_hist = history ? e->d_at<uint64_t>(o_hist) : nullptr;
+  auto* d_out = e->d_at<float>(o_out);
   SPB_CUDA(e, cudaMemcpyAsync(d_states, states, (size_t)n * sizeof(ch::Pos), cudaMemcpyHostToDevice, e->stream));
-  if (history) SPB_CUDA(e, cudaMemcpyAsync(d_hist, history, (size_t)n * SPB_CHESS_MAX_HISTORY * 8, cudaMemcpyHostToDevice, e->stream));
+  if (history) SPB_CUDA(e, cudaMemcpyAsync(d_hist, history, hist_bytes, cudaMemcpyHostToDevice, e->stream));
   ch::k_encode<<<n, 128, 0, e->stream>>>(d_states, d_hist, n, d_out);
   SPB_CUDA(e, cudaGetLastError());
   ++e->launches;
-  SPB_CUDA(e, cudaMemcpyAsync(out, d_out, (size_t)n * SPB_CHESS_PLANES * 64 * 4, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaMemcpyAsync(out, d_out, out_bytes, cudaMemcpyDeviceToHost, e->stream));
   SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   return SPB_OK;
 }
@@ -405,17 +423,15 @@ int32_t spb_chess_perft(spb_chess_engine* e, const spb_chess_state* state, uint3
   // Breadth first on the device while the frontier is too narrow to fill the GPU (or the rest too deep for one thread):
   // k_frontier_count gives every position its output offset, k_frontier_expand writes its children there.  Every
   // frontier position is then searched to the remaining depth by one device thread (k_perft).
-  Scratch sc;
-  auto* d_total = sc.alloc<unsigned long long>(1);
-  ch::Pos* d_f = nullptr;
-  if (cudaMalloc(&d_f, sizeof(ch::Pos)) != cudaSuccess || !d_total) { e->set_error("chess: out of device memory"); return SPB_ERR_NOMEM; }
-  struct Free { ch::Pos*& p; ~Free() { cudaFree(p); } } free_f{d_f};
+  unsigned long long* d_total = e->d_misc;                             // the engine's scratch word; every call ends synchronised
+  PerftBuffers buf;
+  ch::Pos* d_f = buf.alloc<ch::Pos>(1);
+  if (!d_f) { e->set_error("chess: out of device memory"); return SPB_ERR_NOMEM; }
   SPB_CUDA(e, cudaMemcpyAsync(d_f, state, sizeof(ch::Pos), cudaMemcpyHostToDevice, e->stream));
   uint32_t n = 1, remaining = depth;
   while (remaining > 0 && (n < 4096 || remaining > (uint32_t)ch::PERFT_DEV_DEPTH)) {
-    uint32_t* d_off = nullptr;
-    if (cudaMalloc(&d_off, (size_t)n * 4) != cudaSuccess) { e->set_error("chess: out of device memory"); return SPB_ERR_NOMEM; }
-    struct FreeOff { uint32_t* p; ~FreeOff() { cudaFree(p); } } free_off{d_off};
+    uint32_t* d_off = buf.alloc<uint32_t>(n);
+    if (!d_off) { e->set_error("chess: out of device memory"); return SPB_ERR_NOMEM; }
     SPB_CUDA(e, cudaMemsetAsync(d_total, 0, 8, e->stream));
     ch::k_frontier_count<<<(n + 63) / 64, 64, 0, e->stream>>>(d_f, n, d_off, d_total);
     SPB_CUDA(e, cudaGetLastError());
@@ -425,15 +441,12 @@ int32_t spb_chess_perft(spb_chess_engine* e, const spb_chess_state* state, uint3
     e->launches += 1;
     if (m == 0) { *nodes = 0; return SPB_OK; }
     SPB_ARG(e, m <= (1ull << 23), "perft frontier too large");
-    ch::Pos* d_next = nullptr;
-    if (cudaMalloc(&d_next, (size_t)m * sizeof(ch::Pos)) != cudaSuccess) { e->set_error("chess: out of device memory"); return SPB_ERR_NOMEM; }
+    ch::Pos* d_next = buf.alloc<ch::Pos>(m);
+    if (!d_next) { e->set_error("chess: out of device memory"); return SPB_ERR_NOMEM; }
     ch::k_frontier_expand<<<(n + 63) / 64, 64, 0, e->stream>>>(d_f, n, d_off, d_next);
-    const cudaError_t err = cudaGetLastError();
-    cudaStreamSynchronize(e->stream);
-    cudaFree(d_f);
-    d_f = d_next;
-    SPB_CUDA(e, err);
+    SPB_CUDA(e, cudaGetLastError());
     e->launches += 1;
+    d_f = d_next;
     n = (uint32_t)m;
     --remaining;
   }

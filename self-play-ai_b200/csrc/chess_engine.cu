@@ -638,11 +638,6 @@ int32_t spb_chess_engine::init() {
   if (!rc) rc = dalloc(&d_rc_ids, G * ch::MAX_MOVES);
   if (!rc) rc = dalloc(&d_rc_n, G);
   if (!rc) rc = dalloc(&d_misc, 4);
-  if (!rc) rc = dalloc(&d_reset_slots, G);
-  if (!rc) rc = dalloc(&d_reset_roots, G);
-  if (!rc) rc = dalloc(&d_reset_hist, G * SPB_CHESS_MAX_HISTORY);
-  if (!rc) rc = dalloc(&d_adv_ids, G);
-  if (!rc) rc = dalloc(&d_adv_err, G);
   if (rc) return rc;
   SPB_CUDA(this, cudaMemsetAsync(T.live, 0, G, stream));
   SPB_CUDA(this, cudaMemsetAsync(T.buf, 0, G, stream));
@@ -695,8 +690,10 @@ int32_t spb_chess_destroy(spb_chess_engine* e) {
 
 const char* spb_chess_last_error(const spb_chess_engine* e) { return spb_chess_engine::last_error(e); }
 
-// The roots of spb_chess_reset_games / spb_chess_selfplay_step (history: [n][SPB_CHESS_MAX_HISTORY], nullable).
-static int32_t check_roots(spb_chess_engine* e, const spb_chess_state* roots, const uint64_t* history, uint32_t n) {
+// The roots of spb_chess_reset_games / spb_chess_selfplay_step (history: [n][SPB_CHESS_MAX_HISTORY], nullable): checked, then
+// copied with the slots to the stage.  Each device pointer is set when its host array is given.
+static int32_t stage_roots(spb_chess_engine* e, const uint32_t* slots, const spb_chess_state* roots, const uint64_t* history, uint32_t n,
+                           uint32_t** d_slots, ch::Pos** d_roots, unsigned long long** d_hist) {
   if (roots) for (uint32_t i = 0; i < n; ++i) {
     SPB_ARG(e, roots[i].side <= 1 && roots[i].ep <= 64, "malformed root state");
     uint64_t kings[2] = {roots[i].piece[5] & roots[i].color[0], roots[i].piece[5] & roots[i].color[1]};
@@ -704,6 +701,13 @@ static int32_t check_roots(spb_chess_engine* e, const spb_chess_state* roots, co
     SPB_ARG(e, history || roots[i].hist_len == 0, "root with hist_len > 0 needs its history");
     SPB_ARG(e, roots[i].hist_len <= SPB_CHESS_MAX_HISTORY, "hist_len > SPB_CHESS_MAX_HISTORY");
   }
+  const size_t hist_bytes = (size_t)n * SPB_CHESS_MAX_HISTORY * 8;
+  StageLayout L;
+  const size_t o_slots = L.take(slots ? (size_t)n * 4 : 0), o_roots = L.take(roots ? (size_t)n * sizeof(ch::Pos) : 0), o_hist = L.take(history ? hist_bytes : 0);
+  if (int32_t rc = e->ensure_stage(L.bytes, 0)) return rc;
+  if (slots) SPB_CUDA(e, cudaMemcpyAsync(*d_slots = e->d_at<uint32_t>(o_slots), slots, (size_t)n * 4, cudaMemcpyHostToDevice, e->stream));
+  if (roots) SPB_CUDA(e, cudaMemcpyAsync(*d_roots = e->d_at<ch::Pos>(o_roots), roots, (size_t)n * sizeof(ch::Pos), cudaMemcpyHostToDevice, e->stream));
+  if (history) SPB_CUDA(e, cudaMemcpyAsync(*d_hist = e->d_at<unsigned long long>(o_hist), history, hist_bytes, cudaMemcpyHostToDevice, e->stream));
   return SPB_OK;
 }
 
@@ -713,14 +717,8 @@ int32_t spb_chess_reset_games(spb_chess_engine* e, const uint32_t* slots, uint32
   SPB_ARG(e, !(history && !roots), "history without roots");
   if (n == 0) return SPB_OK;
   if (slots) for (uint32_t i = 0; i < n; ++i) SPB_ARG(e, slots[i] < e->T.G, "slot out of range");
-  const int32_t rc = check_roots(e, roots, history, n);
-  if (rc) return rc;
-  uint32_t* d_slots = slots ? e->d_reset_slots : nullptr;
-  ch::Pos* d_roots = roots ? e->d_reset_roots : nullptr;
-  unsigned long long* d_hist = history ? e->d_reset_hist : nullptr;
-  if (slots) SPB_CUDA(e, cudaMemcpyAsync(d_slots, slots, (size_t)n * 4, cudaMemcpyHostToDevice, e->stream));
-  if (roots) SPB_CUDA(e, cudaMemcpyAsync(d_roots, roots, (size_t)n * sizeof(ch::Pos), cudaMemcpyHostToDevice, e->stream));
-  if (history) SPB_CUDA(e, cudaMemcpyAsync(d_hist, history, (size_t)n * SPB_CHESS_MAX_HISTORY * 8, cudaMemcpyHostToDevice, e->stream));
+  uint32_t* d_slots = nullptr; ch::Pos* d_roots = nullptr; unsigned long long* d_hist = nullptr;
+  if (int32_t rc = stage_roots(e, slots, roots, history, n, &d_slots, &d_roots, &d_hist)) return rc;
   ch::k_chess_reset<<<n, 64, 0, e->stream>>>(e->T, e->P, d_slots, d_roots, d_hist, n);
   SPB_CUDA(e, cudaGetLastError());
   ++e->launches;
@@ -884,11 +882,13 @@ int32_t spb_chess_advance(spb_chess_engine* e, const uint32_t* slots, const uint
   SPB_ARG(e, child_ids && n <= e->T.G, "bad argument");
   if (n == 0) return SPB_OK;
   if (slots) for (uint32_t i = 0; i < n; ++i) SPB_ARG(e, slots[i] < e->T.G, "slot out of range");
-  // persistent device staging (every call ends with a stream synchronisation): the per-move call of the self-play loop
-  uint32_t* d_slots = slots ? e->d_reset_slots : nullptr;
-  uint32_t* d_ids = e->d_adv_ids;
-  ch::Pos* d_out = e->d_reset_roots;
-  int32_t* d_err = e->d_adv_err;
+  StageLayout L;
+  const size_t o_slots = L.take(slots ? (size_t)n * 4 : 0), o_ids = L.take((size_t)n * 4), o_out = L.take((size_t)n * sizeof(ch::Pos)), o_err = L.take((size_t)n * 4);
+  if (int32_t rc = e->ensure_stage(L.bytes, 0)) return rc;
+  uint32_t* d_slots = slots ? e->d_at<uint32_t>(o_slots) : nullptr;
+  uint32_t* d_ids = e->d_at<uint32_t>(o_ids);
+  ch::Pos* d_out = e->d_at<ch::Pos>(o_out);
+  int32_t* d_err = e->d_at<int32_t>(o_err);
   if (slots) SPB_CUDA(e, cudaMemcpyAsync(d_slots, slots, (size_t)n * 4, cudaMemcpyHostToDevice, e->stream));
   SPB_CUDA(e, cudaMemcpyAsync(d_ids, child_ids, (size_t)n * 4, cudaMemcpyHostToDevice, e->stream));
   ch::k_chess_advance<<<(n + ch::WARPS - 1) / ch::WARPS, ch::THREADS, 0, e->stream>>>(e->T, d_slots, d_ids, n, d_out, d_err);
@@ -909,10 +909,11 @@ int32_t spb_chess_advance(spb_chess_engine* e, const uint32_t* slots, const uint
 int32_t spb_chess_get_state(spb_chess_engine* e, uint32_t slot, uint32_t node_id, spb_chess_state* out) {
   SPB_GUARD(e);
   SPB_ARG(e, out && slot < e->T.G, "bad argument");
-  ch::Scratch sc;
-  ch::Pos* d_out = sc.alloc<ch::Pos>(1);
-  int32_t* d_err = sc.alloc<int32_t>(1);
-  if (!d_out || !d_err) { e->set_error("chess: out of device memory"); return SPB_ERR_NOMEM; }
+  StageLayout L;
+  const size_t o_out = L.take(sizeof(ch::Pos)), o_err = L.take(4);
+  if (int32_t rc = e->ensure_stage(L.bytes, 0)) return rc;
+  ch::Pos* d_out = e->d_at<ch::Pos>(o_out);
+  int32_t* d_err = e->d_at<int32_t>(o_err);
   ch::k_chess_get_state<<<1, 1, 0, e->stream>>>(e->T, slot, node_id, d_out, d_err);
   SPB_CUDA(e, cudaGetLastError());
   ++e->launches;
@@ -933,9 +934,8 @@ int32_t spb_chess_node_stats(spb_chess_engine* e, uint32_t slot, uint32_t node_i
                              uint32_t* first_child, uint32_t* n_children, uint16_t* move, uint8_t* status) {
   SPB_GUARD(e);
   SPB_ARG(e, slot < e->T.G, "slot out of range");
-  ch::Scratch sc;
-  uint32_t* d = sc.alloc<uint32_t>(8);
-  if (!d) { e->set_error("chess: out of device memory"); return SPB_ERR_NOMEM; }
+  if (int32_t rc = e->ensure_stage(32, 0)) return rc;
+  uint32_t* d = e->d_at<uint32_t>(0);
   ch::k_chess_node_stats<<<1, 1, 0, e->stream>>>(e->T, slot, node_id, d);
   SPB_CUDA(e, cudaGetLastError());
   ++e->launches;
@@ -960,19 +960,15 @@ int32_t spb_chess_selfplay_step(spb_chess_engine* e, int32_t rule, float tempera
   SPB_ARG(e, rule == SPB_MOVE_GREEDY_LAST_MAX || rule == SPB_MOVE_TEMPERATURE, "unknown move rule");
   SPB_ARG(e, !(restart_history && !restart_roots), "history without roots");
   const uint32_t G = e->T.G;
-  int32_t rc = check_roots(e, restart_roots, restart_history, G);
+  ch::Pos* d_roots = nullptr; unsigned long long* d_hist = nullptr;
+  int32_t rc = stage_roots(e, nullptr, restart_roots, restart_history, G, nullptr, &d_roots, &d_hist);
   if (rc) return rc;
   if (!e->P.out) {                                                     // the first step allocates the trajectory buffers
     rc = e->alloc_trajectories(SPB_CHESS_MAX_HISTORY);
     if (rc) return rc;
   }
-  // the staging of spb_chess_reset_games (every call ends with a stream synchronisation)
-  if (restart_roots) SPB_CUDA(e, cudaMemcpyAsync(e->d_reset_roots, restart_roots, (size_t)G * sizeof(ch::Pos), cudaMemcpyHostToDevice, e->stream));
-  if (restart_history)
-    SPB_CUDA(e, cudaMemcpyAsync(e->d_reset_hist, restart_history, (size_t)G * SPB_CHESS_MAX_HISTORY * 8, cudaMemcpyHostToDevice, e->stream));
   SPB_CUDA(e, cudaMemsetAsync(e->P.finished, 0, 4, e->stream));
-  ch::k_chess_selfplay_step<<<(G + ch::WARPS - 1) / ch::WARPS, ch::THREADS, 0, e->stream>>>(
-      e->T, e->P, rule, temperature, seed, restart_roots ? e->d_reset_roots : nullptr, restart_history ? e->d_reset_hist : nullptr);
+  ch::k_chess_selfplay_step<<<(G + ch::WARPS - 1) / ch::WARPS, ch::THREADS, 0, e->stream>>>(e->T, e->P, rule, temperature, seed, d_roots, d_hist);
   SPB_CUDA(e, cudaGetLastError());
   ++e->launches;
   uint32_t fin = 0;

@@ -26,26 +26,7 @@ struct spb_chess_engine : spb::HostEngine<spb::chess::CTrees, spb_chess_position
   cudaStream_t stream2 = nullptr;   // the second half of the trees in the network pipeline
   cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
   spb::chess::Net* net = nullptr;
-  // device staging of spb_chess_reset_games (allocated once: cudaMalloc / cudaFree per call would synchronise the device)
-  uint32_t* d_reset_slots = nullptr; spb::chess::Pos* d_reset_roots = nullptr; unsigned long long* d_reset_hist = nullptr;
-  uint32_t* d_adv_ids = nullptr; int32_t* d_adv_err = nullptr;   // spb_chess_advance (with d_reset_slots / d_reset_roots)
 
   int32_t init();
   void release();
 };
-
-namespace spb {
-namespace chess {
-// device scratch for one call of a test / tooling entry point: a few plain allocations, freed on return
-struct Scratch {
-  std::vector<void*> ptrs;
-  ~Scratch() { for (void* p : ptrs) cudaFree(p); }
-  template <class T> T* alloc(size_t count) {
-    void* p = nullptr;
-    if (cudaMalloc(&p, std::max<size_t>(count, 1) * sizeof(T)) != cudaSuccess) return nullptr;
-    ptrs.push_back(p);
-    return static_cast<T*>(p);
-  }
-};
-}  // namespace chess
-}  // namespace spb

@@ -770,22 +770,23 @@ int32_t spb_chess_predict(spb_chess_engine* e, const spb_chess_state* states, co
   SPB_ARG(e, states, "null states");
   SPB_ARG(e, e->net && ch::net_loaded(e->net), "no weights loaded (spb_chess_load_weights)");
   SPB_ARG(e, n <= e->T.G, "more states than the engine's num_games (the network's batch capacity)");
-  ch::Scratch sc;
-  auto* d_states = sc.alloc<ch::Pos>(n);
-  auto* d_hist = history ? sc.alloc<unsigned long long>((size_t)n * SPB_CHESS_MAX_HISTORY) : nullptr;
-  auto* d_moves = sc.alloc<ch::Move>((size_t)n * ch::MAX_MOVES);
-  auto* d_nmoves = sc.alloc<uint32_t>(n);
-  auto* d_reps = sc.alloc<uint32_t>(n);
-  auto* d_count = sc.alloc<uint32_t>(1);
-  auto* d_logits = sc.alloc<float>((size_t)n * SPB_CHESS_POLICY_SIZE);
-  auto* d_values = sc.alloc<float>(n);
-  auto* d_pol = policies ? sc.alloc<float>((size_t)n * SPB_CHESS_POLICY_SIZE) : nullptr;
-  if (!d_states || (history && !d_hist) || !d_moves || !d_nmoves || !d_reps || !d_count || !d_logits || !d_values || (policies && !d_pol)) {
-    e->set_error("chess: out of device memory");
-    return SPB_ERR_NOMEM;
-  }
+  const size_t hist_bytes = (size_t)n * SPB_CHESS_MAX_HISTORY * 8, row_bytes = (size_t)n * SPB_CHESS_POLICY_SIZE * 4;
+  spb::StageLayout L;
+  const size_t o_states = L.take((size_t)n * sizeof(ch::Pos)), o_hist = L.take(history ? hist_bytes : 0), o_moves = L.take((size_t)n * ch::MAX_MOVES * sizeof(ch::Move));
+  const size_t o_nmoves = L.take((size_t)n * 4), o_reps = L.take((size_t)n * 4), o_count = L.take(4), o_logits = L.take(row_bytes), o_values = L.take((size_t)n * 4);
+  const size_t o_pol = L.take(policies ? row_bytes : 0);
+  if (int32_t rc = e->ensure_stage(L.bytes, 0)) return rc;
+  auto* d_states = e->d_at<ch::Pos>(o_states);
+  auto* d_hist = history ? e->d_at<unsigned long long>(o_hist) : nullptr;
+  auto* d_moves = e->d_at<ch::Move>(o_moves);
+  auto* d_nmoves = e->d_at<uint32_t>(o_nmoves);
+  auto* d_reps = e->d_at<uint32_t>(o_reps);
+  auto* d_count = e->d_at<uint32_t>(o_count);
+  auto* d_logits = e->d_at<float>(o_logits);
+  auto* d_values = e->d_at<float>(o_values);
+  auto* d_pol = policies ? e->d_at<float>(o_pol) : nullptr;
   SPB_CUDA(e, cudaMemcpyAsync(d_states, states, (size_t)n * sizeof(ch::Pos), cudaMemcpyHostToDevice, e->stream));
-  if (history) SPB_CUDA(e, cudaMemcpyAsync(d_hist, history, (size_t)n * SPB_CHESS_MAX_HISTORY * 8, cudaMemcpyHostToDevice, e->stream));
+  if (history) SPB_CUDA(e, cudaMemcpyAsync(d_hist, history, hist_bytes, cudaMemcpyHostToDevice, e->stream));
   SPB_CUDA(e, cudaMemcpyAsync(d_count, &n, 4, cudaMemcpyHostToDevice, e->stream));
   ch::k_predict_prepare<<<(n + 3) / 4, 128, 0, e->stream>>>(d_states, d_hist, n, d_moves, d_nmoves, d_reps, e->T.error);
   SPB_CUDA(e, cudaGetLastError());
@@ -796,10 +797,10 @@ int32_t spb_chess_predict(spb_chess_engine* e, const spb_chess_state* states, co
     ch::k_predict_mask<<<n, 256, 0, e->stream>>>(d_logits, d_states, d_moves, d_nmoves, n, d_pol);
     SPB_CUDA(e, cudaGetLastError());
     ++e->launches;
-    SPB_CUDA(e, cudaMemcpyAsync(policies, d_pol, (size_t)n * SPB_CHESS_POLICY_SIZE * 4, cudaMemcpyDeviceToHost, e->stream));
+    SPB_CUDA(e, cudaMemcpyAsync(policies, d_pol, row_bytes, cudaMemcpyDeviceToHost, e->stream));
   }
   if (values) SPB_CUDA(e, cudaMemcpyAsync(values, d_values, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
-  if (raw_logits) SPB_CUDA(e, cudaMemcpyAsync(raw_logits, d_logits, (size_t)n * SPB_CHESS_POLICY_SIZE * 4, cudaMemcpyDeviceToHost, e->stream));
+  if (raw_logits) SPB_CUDA(e, cudaMemcpyAsync(raw_logits, d_logits, row_bytes, cudaMemcpyDeviceToHost, e->stream));
   SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   return e->check_device_errors();
 }

@@ -75,8 +75,6 @@ int32_t spb_engine::init() {
 void spb_engine::release() {
   HostEngine::release();
   drop_step_graph();
-  if (h_stage) cudaFreeHost(h_stage);
-  if (d_stage) cudaFree(d_stage);
 }
 
 // The reference's arena is a Vec that grows without bound (mcts.rs:19,151-157).  Here every tree owns a fixed
@@ -388,20 +386,17 @@ int32_t spb_reset_games(spb_engine* e, const uint32_t* slots, uint32_t n, const 
   SPB_ARG(e, n <= e->T.G, "more slots than games");
   if (n == 0) return SPB_OK;
   if (slots) for (uint32_t i = 0; i < n; ++i) SPB_ARG(e, slots[i] < e->T.G, "slot out of range");
-  size_t off_roots = ((size_t)n * 4 + 15) & ~(size_t)15;
-  size_t bytes = off_roots + (size_t)n * sizeof(PState);
-  int32_t rc = e->ensure_stage(bytes);
-  if (rc) return rc;
-  auto* hs = static_cast<uint8_t*>(e->h_stage);
-  if (slots) std::memcpy(hs, slots, (size_t)n * 4);
+  StageLayout L;
+  const size_t o_slots = L.take(slots ? (size_t)n * 4 : 0), o_roots = L.take(roots ? (size_t)n * sizeof(PState) : 0);
+  if (int32_t rc = e->ensure_stage(L.bytes, L.bytes)) return rc;
+  if (slots) std::memcpy(e->h_at<uint32_t>(o_slots), slots, (size_t)n * 4);
   if (roots) {
-    PState* hp = reinterpret_cast<PState*>(hs + off_roots);
+    PState* hp = e->h_at<PState>(o_roots);
     for (uint32_t i = 0; i < n; ++i) hp[i] = ps_from_abi(roots[i]);
   }
-  SPB_CUDA(e, cudaMemcpyAsync(e->d_stage, e->h_stage, bytes, cudaMemcpyHostToDevice, e->stream));
-  auto* ds = static_cast<uint8_t*>(e->d_stage);
-  k_reset<<<(n + 127) / 128, 128, 0, e->stream>>>(e->T, e->P.hist_len, e->P.parked, slots ? reinterpret_cast<uint32_t*>(ds) : nullptr,
-                                                  roots ? reinterpret_cast<PState*>(ds + off_roots) : nullptr, n);
+  if (L.bytes) SPB_CUDA(e, cudaMemcpyAsync(e->d_stage, e->h_stage, L.bytes, cudaMemcpyHostToDevice, e->stream));
+  k_reset<<<(n + 127) / 128, 128, 0, e->stream>>>(e->T, e->P.hist_len, e->P.parked, slots ? e->d_at<uint32_t>(o_slots) : nullptr,
+                                                  roots ? e->d_at<PState>(o_roots) : nullptr, n);
   ++e->launches;
   SPB_CUDA(e, cudaGetLastError());
   SPB_CUDA(e, cudaStreamSynchronize(e->stream));   // staging buffer is reused by the next call
@@ -426,11 +421,11 @@ int32_t spb_root_children_all(spb_engine* e, uint8_t* actions, uint32_t* visit_c
   if (rc) return rc;
   const size_t G = e->T.G;
   // one pinned staging area, one sync
-  size_t o_counts = 0, o_ids = G * SPB_MAX_ACTIONS * 4, o_n = o_ids + G * SPB_MAX_ACTIONS * 4, o_act = o_n + G * 4;
-  size_t bytes = o_act + G * SPB_MAX_ACTIONS;
-  rc = e->ensure_stage(bytes);
+  StageLayout L;
+  const size_t o_counts = L.take(G * SPB_MAX_ACTIONS * 4), o_ids = L.take(G * SPB_MAX_ACTIONS * 4), o_n = L.take(G * 4), o_act = L.take(G * SPB_MAX_ACTIONS);
+  rc = e->ensure_stage(0, L.bytes);
   if (rc) return rc;
-  auto* hs = static_cast<uint8_t*>(e->h_stage);
+  auto* hs = e->h_at<uint8_t>(0);
   if (visit_counts) SPB_CUDA(e, cudaMemcpyAsync(hs + o_counts, e->d_rc_counts, G * SPB_MAX_ACTIONS * 4, cudaMemcpyDeviceToHost, e->stream));
   if (child_ids) SPB_CUDA(e, cudaMemcpyAsync(hs + o_ids, e->d_rc_ids, G * SPB_MAX_ACTIONS * 4, cudaMemcpyDeviceToHost, e->stream));
   if (n_children) SPB_CUDA(e, cudaMemcpyAsync(hs + o_n, e->d_rc_n, G * 4, cudaMemcpyDeviceToHost, e->stream));
@@ -496,27 +491,24 @@ int32_t spb_advance(spb_engine* e, const uint32_t* slots, const uint32_t* node_i
     seen[g] = 1;
     SPB_ARG(e, node_ids[i] < nn[g], "node id out of range");
   }
-  size_t o_ids = ((size_t)n * 4 + 15) & ~(size_t)15, o_out = o_ids * 2;
-  size_t bytes = o_out + (size_t)n * sizeof(PState);
-  int32_t rc = e->ensure_stage(bytes);
-  if (rc) return rc;
-  auto* hs = static_cast<uint8_t*>(e->h_stage);
-  auto* ds = static_cast<uint8_t*>(e->d_stage);
-  if (slots) std::memcpy(hs, slots, (size_t)n * 4);
-  std::memcpy(hs + o_ids, node_ids, (size_t)n * 4);
-  SPB_CUDA(e, cudaMemcpyAsync(ds, hs, o_out, cudaMemcpyHostToDevice, e->stream));
+  StageLayout L;
+  const size_t o_slots = L.take(slots ? (size_t)n * 4 : 0), o_ids = L.take((size_t)n * 4), o_out = L.take((size_t)n * sizeof(PState));
+  if (int32_t rc = e->ensure_stage(L.bytes, L.bytes)) return rc;
+  if (slots) std::memcpy(e->h_at<uint32_t>(o_slots), slots, (size_t)n * 4);
+  std::memcpy(e->h_at<uint32_t>(o_ids), node_ids, (size_t)n * 4);
+  SPB_CUDA(e, cudaMemcpyAsync(e->d_stage, e->h_stage, o_out, cudaMemcpyHostToDevice, e->stream));   // the inputs: everything before o_out
   const uint32_t blocks = (n + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK;
-  const uint32_t* dsl = slots ? reinterpret_cast<uint32_t*>(ds) : nullptr;
-  const uint32_t* dn = reinterpret_cast<uint32_t*>(ds + o_ids);
-  PState* dout = reinterpret_cast<PState*>(ds + o_out);
+  const uint32_t* dsl = slots ? e->d_at<uint32_t>(o_slots) : nullptr;
+  const uint32_t* dn = e->d_at<uint32_t>(o_ids);
+  PState* dout = e->d_at<PState>(o_out);
   if (e->cfg.game == SPB_GAME_CONNECT4) k_advance<Connect4><<<blocks, THREADS, 0, e->stream>>>(e->T, dsl, dn, n, dout);
   else k_advance<TicTacToe><<<blocks, THREADS, 0, e->stream>>>(e->T, dsl, dn, n, dout);
   ++e->launches;
   SPB_CUDA(e, cudaGetLastError());
-  SPB_CUDA(e, cudaMemcpyAsync(hs + o_out, dout, (size_t)n * sizeof(PState), cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaMemcpyAsync(e->h_at<PState>(o_out), dout, (size_t)n * sizeof(PState), cudaMemcpyDeviceToHost, e->stream));
   SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   if (out_states) {
-    const PState* hp = reinterpret_cast<const PState*>(hs + o_out);
+    const PState* hp = e->h_at<PState>(o_out);
     for (uint32_t i = 0; i < n; ++i) out_states[i] = ps_to_abi(hp[i]);
   }
   return SPB_OK;
@@ -534,10 +526,10 @@ int32_t spb_get_state(spb_engine* e, uint32_t slot, uint32_t node_id, spb_state*
   int32_t rc = spb_arena_len(e, slot, &len);
   if (rc) return rc;
   SPB_ARG(e, node_id < len, "node id out of range");
-  rc = e->ensure_stage(sizeof(PState));
+  rc = e->ensure_stage(sizeof(PState), 0);
   if (rc) return rc;
-  if (e->cfg.game == SPB_GAME_CONNECT4) k_get_state<Connect4><<<1, 1, 0, e->stream>>>(e->T, slot, node_id, static_cast<PState*>(e->d_stage));
-  else k_get_state<TicTacToe><<<1, 1, 0, e->stream>>>(e->T, slot, node_id, static_cast<PState*>(e->d_stage));
+  if (e->cfg.game == SPB_GAME_CONNECT4) k_get_state<Connect4><<<1, 1, 0, e->stream>>>(e->T, slot, node_id, e->d_at<PState>(0));
+  else k_get_state<TicTacToe><<<1, 1, 0, e->stream>>>(e->T, slot, node_id, e->d_at<PState>(0));
   ++e->launches;
   PState ps;
   SPB_CUDA(e, cudaGetLastError());
@@ -568,9 +560,9 @@ int32_t spb_node_stats(spb_engine* e, uint32_t slot, uint32_t node_id, uint32_t*
   int32_t rc = spb_arena_len(e, slot, &len);
   if (rc) return rc;
   SPB_ARG(e, node_id < len, "node id out of range");
-  rc = e->ensure_stage(sizeof(NodeRec));
+  rc = e->ensure_stage(sizeof(NodeRec), 0);
   if (rc) return rc;
-  k_node_stats<<<1, 1, 0, e->stream>>>(e->T, slot, node_id, static_cast<NodeRec*>(e->d_stage));
+  k_node_stats<<<1, 1, 0, e->stream>>>(e->T, slot, node_id, e->d_at<NodeRec>(0));
   ++e->launches;
   NodeRec r;
   SPB_CUDA(e, cudaGetLastError());
@@ -589,22 +581,19 @@ int32_t spb_node_stats(spb_engine* e, uint32_t slot, uint32_t node_id, uint32_t*
 // ---- predict ------------------------------------------------------------------------------------
 template <class G>
 static int32_t predict_t(spb_engine* e, const spb_state* states, uint32_t n, float* policies, float* values, float* raw_logits) {
-  const size_t o_states = 0, o_cnt = (size_t)n * sizeof(PState), o_out = (o_cnt + 16 + 15) & ~(size_t)15;
-  const size_t o_pol = o_out + (size_t)n * G::EVAL_STRIDE * 4, o_val = o_pol + (size_t)n * G::A * 4;
-  const size_t o_log = (o_val + (size_t)n * 4 + 15) & ~(size_t)15;
-  const size_t bytes = o_log + (size_t)n * G::A * 4;
-  int32_t rc = e->ensure_stage(bytes);
-  if (rc) return rc;
-  auto* hs = static_cast<uint8_t*>(e->h_stage);
-  auto* ds = static_cast<uint8_t*>(e->d_stage);
-  PState* hp = reinterpret_cast<PState*>(hs + o_states);
+  StageLayout L;
+  const size_t o_states = L.take((size_t)n * sizeof(PState)), o_cnt = L.take(4), o_out = L.take((size_t)n * G::EVAL_STRIDE * 4);
+  const size_t o_pol = L.take((size_t)n * G::A * 4), o_val = L.take((size_t)n * 4), o_log = L.take((size_t)n * G::A * 4);
+  if (int32_t rc = e->ensure_stage(L.bytes, L.bytes)) return rc;
+  auto* hs = e->h_at<uint8_t>(0);
+  PState* hp = e->h_at<PState>(o_states);
   for (uint32_t i = 0; i < n; ++i) hp[i] = ps_from_abi(states[i]);
-  *reinterpret_cast<uint32_t*>(hs + o_cnt) = n;
-  SPB_CUDA(e, cudaMemcpyAsync(ds, hs, o_cnt + 4, cudaMemcpyHostToDevice, e->stream));
-  PState* dstates = reinterpret_cast<PState*>(ds + o_states);
-  uint32_t* dcnt = reinterpret_cast<uint32_t*>(ds + o_cnt);
-  float* dout = reinterpret_cast<float*>(ds + o_out);
-  float* dlog = reinterpret_cast<float*>(ds + o_log);
+  *e->h_at<uint32_t>(o_cnt) = n;
+  SPB_CUDA(e, cudaMemcpyAsync(e->d_stage, hs, o_cnt + 4, cudaMemcpyHostToDevice, e->stream));
+  PState* dstates = e->d_at<PState>(o_states);
+  uint32_t* dcnt = e->d_at<uint32_t>(o_cnt);
+  float* dout = e->d_at<float>(o_out);
+  float* dlog = e->d_at<float>(o_log);
   if (e->cfg.evaluator == SPB_EVAL_NET) {
     if (!e->evaluator.loaded()) { e->set_error("no weights loaded: call spb_load_weights first"); return SPB_ERR_STATE; }
     SPB_CUDA(e, cudaMemsetAsync(dlog, 0, (size_t)n * G::A * 4, e->stream));
@@ -623,10 +612,10 @@ static int32_t predict_t(spb_engine* e, const spb_state* states, uint32_t n, flo
     SPB_CUDA(e, cudaGetLastError());
   }
   ++e->launches;
-  k_mask_policies<G><<<(n + 127) / 128, 128, 0, e->stream>>>(dstates, n, dout, reinterpret_cast<float*>(ds + o_pol), reinterpret_cast<float*>(ds + o_val));
+  k_mask_policies<G><<<(n + 127) / 128, 128, 0, e->stream>>>(dstates, n, dout, e->d_at<float>(o_pol), e->d_at<float>(o_val));
   ++e->launches;
   SPB_CUDA(e, cudaGetLastError());
-  SPB_CUDA(e, cudaMemcpyAsync(hs + o_pol, ds + o_pol, bytes - o_pol, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaMemcpyAsync(hs + o_pol, e->d_at<uint8_t>(o_pol), L.bytes - o_pol, cudaMemcpyDeviceToHost, e->stream));   // policies, values, logits
   SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   if (policies) std::memcpy(policies, hs + o_pol, (size_t)n * G::A * 4);
   if (values) std::memcpy(values, hs + o_val, (size_t)n * 4);
@@ -645,10 +634,11 @@ int32_t spb_predict(spb_engine* e, const spb_state* states, uint32_t n, float* p
 }
 
 // ---- game rules ---------------------------------------------------------------------------------
-static int32_t upload_states(spb_engine* e, const spb_state* states, uint32_t n, size_t extra_bytes) {
-  int32_t rc = e->ensure_stage((size_t)n * sizeof(PState) + extra_bytes + 64);
+// Grows the stage and converts the n states into the pinned stage at offset 0: the states come first in every layout below.
+static int32_t upload_states(spb_engine* e, const spb_state* states, uint32_t n, size_t d_bytes, size_t h_bytes) {
+  const int32_t rc = e->ensure_stage(d_bytes, h_bytes);
   if (rc) return rc;
-  PState* hp = static_cast<PState*>(e->h_stage);
+  PState* hp = e->h_at<PState>(0);
   for (uint32_t i = 0; i < n; ++i) hp[i] = ps_from_abi(states[i]);
   return SPB_OK;
 }
@@ -657,23 +647,21 @@ int32_t spb_game_next_states(spb_engine* e, const spb_state* states, const uint8
   SPB_GUARD(e);
   SPB_ARG(e, states && actions && out_states && err, "null argument");
   if (n == 0) return SPB_OK;
-  const size_t o_act = (size_t)n * sizeof(PState), o_out = (o_act + n + 15) & ~(size_t)15, o_err = o_out + (size_t)n * sizeof(PState);
-  int32_t rc = upload_states(e, states, n, o_err + (size_t)n * 4);
-  if (rc) return rc;
-  auto* hs = static_cast<uint8_t*>(e->h_stage);
-  auto* ds = static_cast<uint8_t*>(e->d_stage);
-  std::memcpy(hs + o_act, actions, n);
-  SPB_CUDA(e, cudaMemcpyAsync(ds, hs, o_out, cudaMemcpyHostToDevice, e->stream));
+  StageLayout L;
+  const size_t o_states = L.take((size_t)n * sizeof(PState)), o_act = L.take(n), o_out = L.take((size_t)n * sizeof(PState)), o_err = L.take((size_t)n * 4);
+  if (int32_t rc = upload_states(e, states, n, L.bytes, L.bytes)) return rc;
+  std::memcpy(e->h_at<uint8_t>(o_act), actions, n);
+  SPB_CUDA(e, cudaMemcpyAsync(e->d_stage, e->h_stage, o_out, cudaMemcpyHostToDevice, e->stream));   // the inputs: everything before o_out
   if (e->cfg.game == SPB_GAME_CONNECT4)
-    k_game_next<Connect4><<<(n + 127) / 128, 128, 0, e->stream>>>((PState*)ds, ds + o_act, n, (PState*)(ds + o_out), (int32_t*)(ds + o_err));
+    k_game_next<Connect4><<<(n + 127) / 128, 128, 0, e->stream>>>(e->d_at<PState>(o_states), e->d_at<uint8_t>(o_act), n, e->d_at<PState>(o_out), e->d_at<int32_t>(o_err));
   else
-    k_game_next<TicTacToe><<<(n + 127) / 128, 128, 0, e->stream>>>((PState*)ds, ds + o_act, n, (PState*)(ds + o_out), (int32_t*)(ds + o_err));
+    k_game_next<TicTacToe><<<(n + 127) / 128, 128, 0, e->stream>>>(e->d_at<PState>(o_states), e->d_at<uint8_t>(o_act), n, e->d_at<PState>(o_out), e->d_at<int32_t>(o_err));
   ++e->launches;
   SPB_CUDA(e, cudaGetLastError());
-  SPB_CUDA(e, cudaMemcpyAsync(hs + o_out, ds + o_out, (size_t)n * (sizeof(PState) + 4), cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaMemcpyAsync(e->h_at<uint8_t>(o_out), e->d_at<uint8_t>(o_out), L.bytes - o_out, cudaMemcpyDeviceToHost, e->stream));   // states, errors
   SPB_CUDA(e, cudaStreamSynchronize(e->stream));
-  const PState* hp = reinterpret_cast<const PState*>(hs + o_out);
-  const int32_t* he = reinterpret_cast<const int32_t*>(hs + o_err);
+  const PState* hp = e->h_at<PState>(o_out);
+  const int32_t* he = e->h_at<int32_t>(o_err);
   for (uint32_t i = 0; i < n; ++i) { out_states[i] = ps_to_abi(hp[i]); err[i] = he[i]; }
   return SPB_OK;
 }
@@ -682,17 +670,15 @@ int32_t spb_game_valid_actions(spb_engine* e, const spb_state* states, uint32_t 
   SPB_GUARD(e);
   SPB_ARG(e, states && masks, "null argument");
   if (n == 0) return SPB_OK;
-  const size_t o_out = (size_t)n * sizeof(PState);
-  int32_t rc = upload_states(e, states, n, o_out + (size_t)n * 4);
-  if (rc) return rc;
-  auto* hs = static_cast<uint8_t*>(e->h_stage);
-  auto* ds = static_cast<uint8_t*>(e->d_stage);
-  SPB_CUDA(e, cudaMemcpyAsync(ds, hs, o_out, cudaMemcpyHostToDevice, e->stream));
-  if (e->cfg.game == SPB_GAME_CONNECT4) k_game_valid<Connect4><<<(n + 127) / 128, 128, 0, e->stream>>>((PState*)ds, n, (uint32_t*)(ds + o_out));
-  else k_game_valid<TicTacToe><<<(n + 127) / 128, 128, 0, e->stream>>>((PState*)ds, n, (uint32_t*)(ds + o_out));
+  StageLayout L;
+  const size_t o_states = L.take((size_t)n * sizeof(PState)), o_out = L.take((size_t)n * 4);
+  if (int32_t rc = upload_states(e, states, n, L.bytes, o_out)) return rc;
+  SPB_CUDA(e, cudaMemcpyAsync(e->d_stage, e->h_stage, o_out, cudaMemcpyHostToDevice, e->stream));
+  if (e->cfg.game == SPB_GAME_CONNECT4) k_game_valid<Connect4><<<(n + 127) / 128, 128, 0, e->stream>>>(e->d_at<PState>(o_states), n, e->d_at<uint32_t>(o_out));
+  else k_game_valid<TicTacToe><<<(n + 127) / 128, 128, 0, e->stream>>>(e->d_at<PState>(o_states), n, e->d_at<uint32_t>(o_out));
   ++e->launches;
   SPB_CUDA(e, cudaGetLastError());
-  SPB_CUDA(e, cudaMemcpyAsync(masks, ds + o_out, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaMemcpyAsync(masks, e->d_at<uint32_t>(o_out), (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
   SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   return SPB_OK;
 }
@@ -702,19 +688,16 @@ int32_t spb_game_encode(spb_engine* e, const spb_state* states, uint32_t n, floa
   SPB_ARG(e, states && out, "null argument");
   if (n == 0) return SPB_OK;
   const bool c4 = e->cfg.game == SPB_GAME_CONNECT4;
-  const size_t E = c4 ? 3 * 6 * 7 : 27;
-  const size_t o_out = (size_t)n * sizeof(PState);
-  int32_t rc = upload_states(e, states, n, o_out + (size_t)n * E * 4);
-  if (rc) return rc;
-  auto* hs = static_cast<uint8_t*>(e->h_stage);
-  auto* ds = static_cast<uint8_t*>(e->d_stage);
-  SPB_CUDA(e, cudaMemcpyAsync(ds, hs, o_out, cudaMemcpyHostToDevice, e->stream));
-  const size_t total = (size_t)n * E;
-  if (c4) k_game_encode<Connect4><<<(unsigned)((total + 255) / 256), 256, 0, e->stream>>>((PState*)ds, n, (float*)(ds + o_out));
-  else k_game_encode<TicTacToe><<<(unsigned)((total + 255) / 256), 256, 0, e->stream>>>((PState*)ds, n, (float*)(ds + o_out));
+  const size_t total = (size_t)n * (c4 ? 3 * 6 * 7 : 27);
+  StageLayout L;
+  const size_t o_states = L.take((size_t)n * sizeof(PState)), o_out = L.take(total * 4);
+  if (int32_t rc = upload_states(e, states, n, L.bytes, o_out)) return rc;
+  SPB_CUDA(e, cudaMemcpyAsync(e->d_stage, e->h_stage, o_out, cudaMemcpyHostToDevice, e->stream));
+  if (c4) k_game_encode<Connect4><<<(unsigned)((total + 255) / 256), 256, 0, e->stream>>>(e->d_at<PState>(o_states), n, e->d_at<float>(o_out));
+  else k_game_encode<TicTacToe><<<(unsigned)((total + 255) / 256), 256, 0, e->stream>>>(e->d_at<PState>(o_states), n, e->d_at<float>(o_out));
   ++e->launches;
   SPB_CUDA(e, cudaGetLastError());
-  SPB_CUDA(e, cudaMemcpyAsync(out, ds + o_out, total * 4, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaMemcpyAsync(out, e->d_at<float>(o_out), total * 4, cudaMemcpyDeviceToHost, e->stream));
   SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   return SPB_OK;
 }
@@ -726,10 +709,10 @@ int32_t spb_selfplay_step(spb_engine* e, int32_t rule, float temperature, uint64
   const uint32_t G = e->T.G;
   PState* droots = nullptr;
   if (restart_roots) {
-    int32_t rc = upload_states(e, restart_roots, G, 0);
-    if (rc) return rc;
-    SPB_CUDA(e, cudaMemcpyAsync(e->d_stage, e->h_stage, (size_t)G * sizeof(PState), cudaMemcpyHostToDevice, e->stream));
-    droots = static_cast<PState*>(e->d_stage);
+    const size_t bytes = (size_t)G * sizeof(PState);
+    if (int32_t rc = upload_states(e, restart_roots, G, bytes, bytes)) return rc;
+    SPB_CUDA(e, cudaMemcpyAsync(e->d_stage, e->h_stage, bytes, cudaMemcpyHostToDevice, e->stream));
+    droots = e->d_at<PState>(0);
   }
   SPB_CUDA(e, cudaMemsetAsync(e->P.finished, 0, 4, e->stream));
   const uint32_t blocks = (G + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK;

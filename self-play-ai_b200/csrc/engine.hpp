@@ -29,9 +29,6 @@ struct spb_engine : spb::HostEngine<spb::Trees, spb_position, uint8_t> {
   using Evaluator = spb::Evaluator; using AsyncCtl = spb::AsyncCtl;
   spb_engine() : HostEngine("spb_") {}
   Evaluator evaluator;
-  // staging
-  void* h_stage = nullptr; size_t h_stage_bytes = 0;   // pinned
-  void* d_stage = nullptr; size_t d_stage_bytes = 0;
   float last_eval_ms = 0.f;
   uint32_t last_eval_launches = 0;
   int last_eval_parity = -1;   // parity of the work list the last evaluator launch of spb_search consumed
@@ -46,23 +43,6 @@ struct spb_engine : spb::HostEngine<spb::Trees, spb_position, uint8_t> {
   int A = 0, max_depth = 0, eval_stride = 0, max_ply = 0;
 
   int32_t ensure_capacity(uint32_t num_searches);
-  int32_t ensure_stage(size_t bytes) {
-    if (bytes > h_stage_bytes) {
-      if (h_stage) cudaFreeHost(h_stage);
-      h_stage = nullptr; h_stage_bytes = 0;
-      size_t nb = std::max(bytes, (size_t)1 << 20);
-      SPB_CUDA(this, cudaMallocHost(&h_stage, nb));
-      h_stage_bytes = nb;
-    }
-    if (bytes > d_stage_bytes) {
-      if (d_stage) cudaFree(d_stage);
-      d_stage = nullptr; d_stage_bytes = 0;
-      size_t nb = std::max(bytes, (size_t)1 << 20);
-      SPB_CUDA(this, cudaMalloc(&d_stage, nb));
-      d_stage_bytes = nb;
-    }
-    return SPB_OK;
-  }
   void drop_step_graph() {
     if (step_graph) { cudaGraphExecDestroy(step_graph); step_graph = nullptr; }
   }

@@ -35,6 +35,13 @@ extern thread_local std::string g_create_error;   // text of the last failure th
 
 namespace spb {
 
+// Byte offsets of an entry point's arrays in the engine's stage: take(n) reserves the next n bytes, 16-byte aligned, and
+// returns their offset; `bytes` is what the stage must hold.
+struct StageLayout {
+  size_t bytes = 0;
+  size_t take(size_t n) { const size_t off = bytes; bytes = (bytes + n + 15) & ~(size_t)15; return off; }
+};
+
 // Trees: the device trees (Trees / chess::CTrees); Rec: the trajectory record; Move: the move of a root child as the
 // whole-batch root query reports it (action index / chess move).
 template <class Trees, class Rec, class Move>
@@ -67,8 +74,35 @@ struct HostEngine {
   uint32_t* d_noise_n = nullptr;
   float noise_alpha = 0.0f;
   unsigned long long noise_seed = 0;
+  // Staging of the inputs and outputs of an entry point, grow-only: device bytes and pinned host bytes.  Every entry point
+  // that uses them synchronises its stream before it returns: the next call reuses them, and a grow frees the old buffer.
+  void* d_stage = nullptr; size_t d_stage_bytes = 0;
+  void* h_stage = nullptr; size_t h_stage_bytes = 0;
 
   void set_error(const std::string& s) { err = s; }
+
+  // At least d_bytes of device and h_bytes of pinned host stage (0: a call that copies straight between the caller's
+  // memory and the device needs no pinned bytes).
+  int32_t ensure_stage(size_t d_bytes, size_t h_bytes) {
+    const auto grow = [this](void** p, size_t* have, size_t want, bool pinned) -> int32_t {
+      if (want <= *have) return SPB_OK;
+      if (*p) pinned ? cudaFreeHost(*p) : cudaFree(*p);
+      *p = nullptr; *have = 0;
+      const size_t nb = std::max(want, (size_t)1 << 20);
+      const cudaError_t ce = pinned ? cudaMallocHost(p, nb) : cudaMalloc(p, nb);
+      if (ce != cudaSuccess) {
+        cudaGetLastError();                                              // an allocation failure is not sticky: clear it
+        set_error(std::string("cannot grow the ") + (pinned ? "pinned" : "device") + " stage to " + std::to_string(nb) + " bytes: " + cudaGetErrorString(ce));
+        return SPB_ERR_NOMEM;
+      }
+      *have = nb;
+      return SPB_OK;
+    };
+    const int32_t rc = grow(&d_stage, &d_stage_bytes, d_bytes, false);
+    return rc ? rc : grow(&h_stage, &h_stage_bytes, h_bytes, true);
+  }
+  template <class T_> T_* d_at(size_t off) const { return reinterpret_cast<T_*>(static_cast<char*>(d_stage) + off); }
+  template <class T_> T_* h_at(size_t off) const { return reinterpret_cast<T_*>(static_cast<char*>(h_stage) + off); }
 
   template <class T_> int32_t dalloc(T_** p, size_t count) {
     void* q = nullptr;
@@ -119,12 +153,15 @@ struct HostEngine {
     return SPB_OK;
   }
 
-  // Waits for the stream, then frees what open_device() and dalloc() made (also of an engine whose creation failed).
+  // Waits for the stream, then frees what open_device(), dalloc() and ensure_stage() made (also of an engine whose creation
+  // failed).
   void release() {
     cudaSetDevice(cfg.device);
     if (stream) cudaStreamSynchronize(stream);
     for (void* p : allocs) cudaFree(p);
     allocs.clear();
+    if (d_stage) cudaFree(d_stage);
+    if (h_stage) cudaFreeHost(h_stage);
     if (ev0) cudaEventDestroy(ev0);
     if (ev1) cudaEventDestroy(ev1);
     if (stream) cudaStreamDestroy(stream);
