@@ -265,6 +265,17 @@ int32_t spb_selfplay_step(spb_engine* e, int32_t rule, float temperature, uint64
 /* Copies finished positions (ordered by game sequence number, then ply) to `buf`. */
 int32_t spb_drain_trajectories(spb_engine* e, spb_position* buf, size_t capacity, size_t* written,
                                uint64_t* game_ids /* nullable, [capacity] global game id per position */);
+/*
+ * The learner hand-off in device memory: the records spb_drain_trajectories returns, byte for byte and in the same order,
+ * written to buf_dev (e.g. a slice of a replay buffer on the GPU) and game_ids_dev (nullable).  buf_dev == NULL: size
+ * query, *written = the number held.  capacity < *written is SPB_ERR_ARG and nothing is drained.  When there are records
+ * to write, buf_dev and game_ids_dev must be device (or managed) memory of e's GPU, 8-byte aligned, else SPB_ERR_ARG naming
+ * the argument and nothing is drained.  The records are ordered on the device
+ * (whole trajectories are moved as runs); scratch comes from the engine's grow-only staging.  Enqueued on the engine's
+ * stream; returns once the outputs are written.
+ */
+int32_t spb_drain_trajectories_device(spb_engine* e, spb_position* buf_dev, size_t capacity, size_t* written,
+                                      uint64_t* game_ids_dev /* nullable */);
 
 /* ---- chess (ref: src/game/chess.rs, src/model/chess.rs; BASELINE config 5) ------------------------------------------ */
 /*
@@ -418,6 +429,9 @@ int32_t spb_chess_selfplay_step(spb_chess_engine* e, int32_t rule, float tempera
 /* Copies the finished positions (ordered by game id, then ply) to buf; buf == NULL: *written = the number held. */
 int32_t spb_chess_drain_trajectories(spb_chess_engine* e, spb_chess_position* buf, size_t capacity, size_t* written,
                                      uint64_t* game_ids /* nullable, [capacity] */);
+/* spb_drain_trajectories_device for chess records; an engine that never played holds 0 records and allocates nothing. */
+int32_t spb_chess_drain_trajectories_device(spb_chess_engine* e, spb_chess_position* buf_dev, size_t capacity, size_t* written,
+                                            uint64_t* game_ids_dev /* nullable */);
 /*
  * The training tensors of n records (host only, no GPU needed), each output nullable: encodings[n][19][8][8] (get_encoding of
  * the recorded root with its recorded repetitions, chess.rs:176-249), policies[n][4672] (visit counts scattered by the policy
@@ -429,7 +443,7 @@ int32_t spb_chess_positions_to_training(const spb_chess_position* positions, siz
  * The same tensors built on the device, per minibatch, from records held in device memory (ref: the replay buffer the
  * learner pops batch_size positions from, learner_concurrent.rs:87-165; the tensors of :126-146).  Output row i comes
  * from positions[indices ? indices[i] : i]; without indices n <= n_positions.  Every pointer is device (or managed) memory
- * of e's GPU, each output nullable: encodings[n][19][8][8], policies[n][4672], values[n].  The results are bit-identical
+ * of e's GPU (records and indices 8-byte aligned, outputs 4-byte aligned), each output nullable: encodings[n][19][8][8], policies[n][4672], values[n].  The results are bit-identical
  * to spb_chess_positions_to_training of the same records (a record whose counts sum to 0 gives NaN policies on both
  * sides, with the NaN bit pattern of each processor).  Validation is that of the host function, plus indices[i] <
  * n_positions: a malformed row gives SPB_ERR_ARG, nothing is written, and spb_chess_last_error names the first bad row.
@@ -461,6 +475,17 @@ int32_t spb_comm_destroy(spb_engine* e);
 int32_t spb_gather_trajectories(spb_engine* e, int32_t learner_rank, spb_position* buf, size_t capacity, size_t* written,
                                 uint64_t* game_ids /* nullable */);
 /*
+ * The device form of the gather, with its contract (COLLECTIVE; *written = 0 on the other ranks): on the learner rank the
+ * ordered records go to buf_dev / game_ids_dev (nullable), with the pointer rules of spb_drain_trajectories_device.  If
+ * buf_dev is NULL or capacity < *written the gathered records stay staged in device memory and the next call (no
+ * collective) delivers them; the pointers are checked at that delivery, after the collective, and a bad one returns
+ * SPB_ERR_ARG with the records still staged.  *written == 0 stages nothing: the next call is a new collective, so a
+ * learner makes its delivering call only when *written > 0.  A gather staged by one form cannot be claimed by the
+ * other: that call returns SPB_ERR_STATE, naming the call to make, and the records stay staged.
+ */
+int32_t spb_gather_trajectories_device(spb_engine* e, int32_t learner_rank, spb_position* buf_dev, size_t capacity,
+                                       size_t* written, uint64_t* game_ids_dev /* nullable */);
+/*
  * The same for chess engines (ref: learner_concurrent.rs:281-288), with the contract of spb_comm_init, spb_comm_destroy and
  * spb_gather_trajectories; the id comes from spb_comm_unique_id.  The gather hands over what spb_chess_drain_trajectories
  * would return; an engine that never played (no trajectory buffers yet) takes part with 0 records.  spb_chess_destroy
@@ -470,6 +495,8 @@ int32_t spb_chess_comm_init(spb_chess_engine* e, const uint8_t* id, int32_t rank
 int32_t spb_chess_comm_destroy(spb_chess_engine* e);
 int32_t spb_chess_gather_trajectories(spb_chess_engine* e, int32_t learner_rank, spb_chess_position* buf, size_t capacity,
                                       size_t* written, uint64_t* game_ids /* nullable */);
+int32_t spb_chess_gather_trajectories_device(spb_chess_engine* e, int32_t learner_rank, spb_chess_position* buf_dev,
+                                             size_t capacity, size_t* written, uint64_t* game_ids_dev /* nullable */);
 /*
  * ref: learner_concurrent.rs:126-146, learner.rs:162-182 — the tensors the learners train on, from n compact records
  * (host only, no GPU needed): encodings[n][3][R][C] (get_encoding of the recorded root state, connect_four.rs:242-259),
@@ -478,6 +505,19 @@ int32_t spb_chess_gather_trajectories(spb_chess_engine* e, int32_t learner_rank,
  */
 int32_t spb_positions_to_training(int32_t game, const spb_position* positions, size_t n, float* encodings, float* policies,
                                   float* values);
+/*
+ * The same tensors built on the device for the engine's game, per minibatch, from records held in device memory.  Output
+ * row i comes from positions_dev[indices_dev ? indices_dev[i] : i]; without indices n <= n_positions.  Every pointer is
+ * device (or managed) memory of e's GPU, the records and indices 8-byte aligned and the outputs 4-byte aligned (else
+ * SPB_ERR_ARG naming the argument, nothing written), each output nullable: encodings_dev[n][3][R][C], policies_dev[n][A],
+ * values_dev[n].  The results are bit-identical to spb_positions_to_training(game, ...) of the same records, which reads
+ * current_player & 1 (a record whose counts sum to 0 gives NaN policies on both sides, with the NaN bit pattern of each
+ * processor).  An index >= n_positions gives SPB_ERR_ARG, nothing is written, and spb_last_error names the first bad row.
+ * Enqueued on the engine's stream; returns once the outputs are written.
+ */
+int32_t spb_positions_to_training_device(spb_engine* e, const spb_position* positions_dev, size_t n_positions,
+                                         const uint64_t* indices_dev /* nullable */, size_t n,
+                                         float* encodings_dev, float* policies_dev, float* values_dev);
 
 /* ---- counters / timing -------------------------------------------------- */
 int32_t spb_get_counters(spb_engine* e, spb_counters* out);

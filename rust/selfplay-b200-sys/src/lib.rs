@@ -155,6 +155,7 @@ extern "C" {
     pub fn spb_game_encode(e: *mut spb_engine, states: *const spb_state, n: u32, out: *mut f32) -> i32;
     pub fn spb_selfplay_step(e: *mut spb_engine, rule: i32, temperature: f32, seed: u64, restart_roots: *const spb_state, n_finished: *mut u32) -> i32;
     pub fn spb_drain_trajectories(e: *mut spb_engine, buf: *mut spb_position, capacity: usize, written: *mut usize, game_ids: *mut u64) -> i32;
+    pub fn spb_drain_trajectories_device(e: *mut spb_engine, buf_dev: *mut spb_position, capacity: usize, written: *mut usize, game_ids_dev: *mut u64) -> i32;
     pub fn spb_chess_create(cfg: *const spb_config, out: *mut *mut spb_chess_engine) -> i32;
     pub fn spb_chess_destroy(e: *mut spb_chess_engine) -> i32;
     pub fn spb_chess_last_error(e: *const spb_chess_engine) -> *const c_char;
@@ -187,16 +188,20 @@ extern "C" {
     pub fn spb_chess_reset_counters(e: *mut spb_chess_engine) -> i32;
     pub fn spb_chess_selfplay_step(e: *mut spb_chess_engine, rule: i32, temperature: f32, seed: u64, restart_roots: *const spb_chess_state, restart_history: *const u64, n_finished: *mut u32) -> i32;
     pub fn spb_chess_drain_trajectories(e: *mut spb_chess_engine, buf: *mut spb_chess_position, capacity: usize, written: *mut usize, game_ids: *mut u64) -> i32;
+    pub fn spb_chess_drain_trajectories_device(e: *mut spb_chess_engine, buf_dev: *mut spb_chess_position, capacity: usize, written: *mut usize, game_ids_dev: *mut u64) -> i32;
     pub fn spb_chess_positions_to_training(positions: *const spb_chess_position, n: usize, encodings: *mut f32, policies: *mut f32, values: *mut f32) -> i32;
     pub fn spb_chess_positions_to_training_device(e: *mut spb_chess_engine, positions: *const spb_chess_position, n_positions: usize, indices: *const u64, n: usize, encodings: *mut f32, policies: *mut f32, values: *mut f32) -> i32;
     pub fn spb_comm_unique_id(id: *mut u8) -> i32;
     pub fn spb_comm_init(e: *mut spb_engine, id: *const u8, rank: i32, world_size: i32) -> i32;
     pub fn spb_comm_destroy(e: *mut spb_engine) -> i32;
     pub fn spb_gather_trajectories(e: *mut spb_engine, learner_rank: i32, buf: *mut spb_position, capacity: usize, written: *mut usize, game_ids: *mut u64) -> i32;
+    pub fn spb_gather_trajectories_device(e: *mut spb_engine, learner_rank: i32, buf_dev: *mut spb_position, capacity: usize, written: *mut usize, game_ids_dev: *mut u64) -> i32;
     pub fn spb_chess_comm_init(e: *mut spb_chess_engine, id: *const u8, rank: i32, world_size: i32) -> i32;
     pub fn spb_chess_comm_destroy(e: *mut spb_chess_engine) -> i32;
     pub fn spb_chess_gather_trajectories(e: *mut spb_chess_engine, learner_rank: i32, buf: *mut spb_chess_position, capacity: usize, written: *mut usize, game_ids: *mut u64) -> i32;
+    pub fn spb_chess_gather_trajectories_device(e: *mut spb_chess_engine, learner_rank: i32, buf_dev: *mut spb_chess_position, capacity: usize, written: *mut usize, game_ids_dev: *mut u64) -> i32;
     pub fn spb_positions_to_training(game: i32, positions: *const spb_position, n: usize, encodings: *mut f32, policies: *mut f32, values: *mut f32) -> i32;
+    pub fn spb_positions_to_training_device(e: *mut spb_engine, positions_dev: *const spb_position, n_positions: usize, indices_dev: *const u64, n: usize, encodings_dev: *mut f32, policies_dev: *mut f32, values_dev: *mut f32) -> i32;
     pub fn spb_get_counters(e: *mut spb_engine, out: *mut spb_counters) -> i32;
     pub fn spb_reset_counters(e: *mut spb_engine) -> i32;
     pub fn spb_last_search_timing(e: *mut spb_engine, search_ms: *mut f32, evaluator_ms: *mut f32, evaluator_launches: *mut u32) -> i32;

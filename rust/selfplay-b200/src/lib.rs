@@ -189,6 +189,38 @@ impl<S: AbiState> Mcts<S> {
         }
         Ok((pos, ids))
     }
+    /// The records of `drain_trajectories`, ordered on the device into `buf_dev[..capacity]` and `game_ids_dev` (nullable),
+    /// e.g. a slice of a replay buffer on the GPU; a null `buf_dev` is the size query.  Returns the number of records.
+    ///
+    /// # Safety
+    /// Every non-null pointer is 8-byte aligned device (or managed) memory of this engine's GPU holding `capacity` elements;
+    /// no other work uses it during the call.
+    pub unsafe fn drain_trajectories_device(&mut self, buf_dev: *mut Position, capacity: usize, game_ids_dev: *mut u64) -> Result<usize> {
+        let mut n = 0usize;
+        self.check(sys::spb_drain_trajectories_device(self.raw, buf_dev, capacity, &mut n, game_ids_dev))?;
+        Ok(n)
+    }
+    /// COLLECTIVE: `gather_trajectories` into device memory of the learner rank (0 records elsewhere); a null or short
+    /// buffer keeps the records staged on the device for the next call.  A result of 0 stages nothing: the next call is a
+    /// new collective, so make the delivering call only when the size query returned more than 0.
+    ///
+    /// # Safety
+    /// As for `drain_trajectories_device`.
+    pub unsafe fn gather_trajectories_device(&mut self, learner_rank: i32, buf_dev: *mut Position, capacity: usize, game_ids_dev: *mut u64) -> Result<usize> {
+        let mut n = 0usize;
+        self.check(sys::spb_gather_trajectories_device(self.raw, learner_rank, buf_dev, capacity, &mut n, game_ids_dev))?;
+        Ok(n)
+    }
+    /// The training tensors of `positions_to_training` for this engine's game, built on its GPU from records in its device
+    /// memory: row i from `positions[indices[i]]`, or `positions[i]` when `indices` is null (then `n <= n_positions`).
+    /// Outputs (each nullable) are bit-identical to the host builder; an index out of range is `SPB_ERR_ARG`, nothing written.
+    ///
+    /// # Safety
+    /// As for `ChessMcts::positions_to_training_device`.
+    pub unsafe fn positions_to_training_device(&mut self, positions: *const Position, n_positions: usize, indices: *const u64, n: usize,
+                                               encodings: *mut f32, policies: *mut f32, values: *mut f32) -> Result<()> {
+        self.check(sys::spb_positions_to_training_device(self.raw, positions, n_positions, indices, n, encodings, policies, values))
+    }
     pub fn counters(&mut self) -> Result<sys::spb_counters> {
         let mut c = sys::spb_counters::default();
         self.check(unsafe { sys::spb_get_counters(self.raw, &mut c) })?;
@@ -410,6 +442,25 @@ impl ChessMcts {
             self.check(unsafe { sys::spb_chess_gather_trajectories(self.raw, learner_rank, pos.as_mut_ptr(), n, &mut n, ids.as_mut_ptr()) })?;
         }
         Ok((pos, ids))
+    }
+    /// The device form of `drain_trajectories` (see `Mcts::drain_trajectories_device`).
+    ///
+    /// # Safety
+    /// As for `Mcts::drain_trajectories_device`.
+    pub unsafe fn drain_trajectories_device(&mut self, buf_dev: *mut ChessPosition, capacity: usize, game_ids_dev: *mut u64) -> Result<usize> {
+        let mut n = 0usize;
+        self.check(sys::spb_chess_drain_trajectories_device(self.raw, buf_dev, capacity, &mut n, game_ids_dev))?;
+        Ok(n)
+    }
+    /// COLLECTIVE: the device form of `gather_trajectories` (see `Mcts::gather_trajectories_device`).
+    ///
+    /// # Safety
+    /// As for `Mcts::drain_trajectories_device`.
+    pub unsafe fn gather_trajectories_device(&mut self, learner_rank: i32, buf_dev: *mut ChessPosition, capacity: usize,
+                                             game_ids_dev: *mut u64) -> Result<usize> {
+        let mut n = 0usize;
+        self.check(sys::spb_chess_gather_trajectories_device(self.raw, learner_rank, buf_dev, capacity, &mut n, game_ids_dev))?;
+        Ok(n)
     }
     /// The training tensors of `chess_positions_to_training`, built on this engine's GPU from records in its device memory
     /// (a replay buffer of `n_positions` records; ref: learner_concurrent.rs:87-165, :126-146).  Row i comes from

@@ -244,6 +244,13 @@ class ChessEngine:
             self._chk(self._L.spb_chess_drain_trajectories(self._h, pos.ctypes.data, n.value, C.byref(n), ids.ctypes.data))
         return pos[:n.value], ids[:n.value]
 
+    def drain_trajectories_device(self, out=None, ids_out=None):
+        """The records of drain_trajectories, ordered on the device -> (CUDA uint8 [n, 1624], CUDA int64 [n]); out / ids_out as
+        for Engine.drain_trajectories_device."""
+        return E._records_to_device(
+            lambda b, cap, n, i: self._chk(self._L.spb_chess_drain_trajectories_device(self._h, b, cap, n, i)),
+            self.device, CHESS_POSITION_DTYPE.itemsize, out, ids_out)
+
     # ---- multi-GPU: trajectories to the learner rank (the contract of Engine's methods) -------------------------------
     def comm_init(self, comm_id: bytes, rank: int, world_size: int):
         buf = (C.c_uint8 * E.COMM_ID_BYTES).from_buffer_copy(comm_id)
@@ -262,6 +269,13 @@ class ChessEngine:
         if n.value:
             self._chk(self._L.spb_chess_gather_trajectories(self._h, learner_rank, pos.ctypes.data, n.value, C.byref(n), ids.ctypes.data))
         return pos[:n.value], ids[:n.value]
+
+    def gather_trajectories_device(self, learner_rank: int = 0, out=None, ids_out=None):
+        """COLLECTIVE: gather_trajectories into device memory of the learner rank -> (CUDA uint8 [n, 1624], CUDA int64 [n]),
+        empty elsewhere."""
+        return E._records_to_device(
+            lambda b, cap, n, i: self._chk(self._L.spb_chess_gather_trajectories_device(self._h, learner_rank, b, cap, n, i)),
+            self.device, CHESS_POSITION_DTYPE.itemsize, out, ids_out)
 
     def get_state(self, slot: int, node_id: int) -> np.ndarray:
         out = np.zeros(1, CHESS_STATE_DTYPE)

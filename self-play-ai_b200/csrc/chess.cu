@@ -295,16 +295,9 @@ int32_t spb_chess_positions_to_training_device(spb_chess_engine* e, const spb_ch
   SPB_ARG(e, indices || n <= n_positions, "n > n_positions without indices");
   if (n == 0) return SPB_OK;
   SPB_ARG(e, positions, "null positions");
-  const void* ptrs[5] = {positions, indices, encodings, policies, values};
-  const char* names[5] = {"positions", "indices", "encodings", "policies", "values"};
-  for (int k = 0; k < 5; ++k) {
-    if (!ptrs[k]) continue;
-    cudaPointerAttributes a{};
-    const cudaError_t ce = cudaPointerGetAttributes(&a, ptrs[k]);
-    if (ce != cudaSuccess) cudaGetLastError();
-    const bool ok = ce == cudaSuccess && (a.type == cudaMemoryTypeManaged || (a.type == cudaMemoryTypeDevice && a.device == e->cfg.device));
-    SPB_ARG(e, ok, std::string(names[k]) + " is not device memory of the engine's GPU");
-  }
+  if (int32_t rc = e->check_device_pointers({{positions, "positions", 8}, {indices, "indices", 8}, {encodings, "encodings", 4},
+                                              {policies, "policies", 4}, {values, "values", 4}}))
+    return rc;
   const unsigned long long none = ~0ull;
   unsigned long long* d_bad = e->d_misc;                               // the engine's scratch word; every call ends synchronised
   const auto* idx = reinterpret_cast<const unsigned long long*>(indices);

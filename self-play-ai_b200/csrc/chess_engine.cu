@@ -983,6 +983,12 @@ int32_t spb_chess_drain_trajectories(spb_chess_engine* e, spb_chess_position* bu
   return e->drain_trajectories(buf, capacity, written, game_ids);
 }
 
+int32_t spb_chess_drain_trajectories_device(spb_chess_engine* e, spb_chess_position* buf_dev, size_t capacity, size_t* written,
+                                            uint64_t* game_ids_dev) {
+  SPB_GUARD(e);
+  return e->drain_trajectories_device(buf_dev, capacity, written, game_ids_dev);
+}
+
 int32_t spb_chess_get_counters(spb_chess_engine* e, spb_counters* out) {
   SPB_GUARD(e);
   return e->get_counters(out, true, [e] { ch::k_chess_nodes_live<<<(e->T.G + 127) / 128, 128, 0, e->stream>>>(e->T, e->d_misc); });

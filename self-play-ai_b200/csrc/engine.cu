@@ -732,6 +732,11 @@ int32_t spb_drain_trajectories(spb_engine* e, spb_position* buf, size_t capacity
   return e->drain_trajectories(buf, capacity, written, game_ids);
 }
 
+int32_t spb_drain_trajectories_device(spb_engine* e, spb_position* buf_dev, size_t capacity, size_t* written, uint64_t* game_ids_dev) {
+  SPB_GUARD(e);
+  return e->drain_trajectories_device(buf_dev, capacity, written, game_ids_dev);
+}
+
 // ---- counters -----------------------------------------------------------------------------------
 int32_t spb_get_counters(spb_engine* e, spb_counters* out) {
   SPB_GUARD(e);

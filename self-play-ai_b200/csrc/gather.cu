@@ -119,81 +119,119 @@ int32_t comm_destroy(HostEngine<Trees, Rec, Move>* e) {
   return SPB_OK;
 }
 
-// spb_gather_trajectories / spb_chess_gather_trajectories over the engine's trajectory buffers P (record type Rec).  Everything
-// runs on e->stream: the self-play steps that filled P ran there, and the chess search's second stream rejoins it before
-// spb_chess_search returns.  Buffers not allocated yet (a chess engine that never played, P.out == NULL) take part with 0
-// records and stay unallocated.
+// The checks both gather forms make before the collective.
 template <class Trees, class Rec, class Move>
-int32_t gather_trajectories(HostEngine<Trees, Rec, Move>* e, int32_t learner_rank, Rec* buf, size_t capacity, size_t* written,
-                            uint64_t* game_ids) {
-  if (!written) return SPB_ERR_ARG;
-  SPB_GUARD(e);
+int32_t gather_ready(HostEngine<Trees, Rec, Move>* e, int32_t learner_rank) {
   if (!e->nccl_comm) { e->set_error(std::string("no communicator: call ") + e->api + "comm_init first"); return SPB_ERR_STATE; }
   SPB_ARG(e, learner_rank >= 0 && learner_rank < e->comm_world, "learner rank out of range");
+  return SPB_OK;
+}
+
+// The collective of spb_gather_trajectories and its device form, over the engine's trajectory buffers P (record type Rec):
+// all-gather of the per-rank record counts, then grouped send/recv of every rank's records into one device buffer of the
+// learner rank, rank by rank (*d_pos / *d_ids, allocated here and freed by the caller; NULL when *total is 0).  The local
+// output buffer is handed over and emptied.  *total = records on the learner rank, 0 on the others.  Everything runs on
+// e->stream: the self-play steps that filled P ran there, and the chess search's second stream rejoins it before
+// spb_chess_search returns.  Buffers not allocated yet (a chess engine that never played, P.out == NULL) take part with 0
+// records and stay unallocated.  Returns with the stream synchronised.
+template <class Trees, class Rec, class Move>
+int32_t exchange(HostEngine<Trees, Rec, Move>* e, int32_t learner_rank, Rec** d_pos_out, unsigned long long** d_ids_out, size_t* total_out) {
   NcclApi* N = nccl_api();
   ncclComm_t comm = static_cast<ncclComm_t>(e->nccl_comm);
   const int rank = e->comm_rank, world = e->comm_world;
   const bool learner = rank == learner_rank;
   const auto& P = e->P;
+  *d_pos_out = nullptr;
+  *d_ids_out = nullptr;
+  *total_out = 0;
+  unsigned long long n_local = 0;
+  if (P.out) {
+    SPB_CUDA(e, cudaMemcpyAsync(&n_local, P.out_cursor, 8, cudaMemcpyDeviceToHost, e->stream));
+    SPB_CUDA(e, cudaStreamSynchronize(e->stream));
+    n_local = std::min<unsigned long long>(n_local, P.out_cap);
+  }
+  unsigned long long* d_counts = nullptr;
+  SPB_CUDA(e, cudaMalloc((void**)&d_counts, (size_t)world * 8));
+  std::vector<unsigned long long> counts((size_t)world, 0);
+  cudaError_t ce = cudaMemcpyAsync(d_counts + rank, &n_local, 8, cudaMemcpyHostToDevice, e->stream);
+  ncclResult_t nr = ce == cudaSuccess ? N->AllGather(d_counts + rank, d_counts, 1, ncclUint64, comm, e->stream) : ncclSuccess;
+  if (ce == cudaSuccess && nr == ncclSuccess) ce = cudaMemcpyAsync(counts.data(), d_counts, (size_t)world * 8, cudaMemcpyDeviceToHost, e->stream);
+  if (ce == cudaSuccess && nr == ncclSuccess) ce = cudaStreamSynchronize(e->stream);
+  cudaFree(d_counts);
+  if (nr != ncclSuccess) { e->set_error(std::string("ncclAllGather: ") + N->GetErrorString(nr)); return SPB_ERR_CUDA; }
+  if (ce != cudaSuccess) { e->set_error(std::string("gather counts: ") + cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
+  size_t total = 0;
+  std::vector<size_t> off((size_t)world, 0);
+  for (int r = 0; r < world; ++r) { off[r] = total; total += (size_t)counts[r]; }
+
+  Rec* d_pos = nullptr;
+  unsigned long long* d_ids = nullptr;
+  if (learner && total) {
+    ce = cudaMalloc((void**)&d_pos, total * sizeof(Rec));
+    if (ce == cudaSuccess) ce = cudaMalloc((void**)&d_ids, total * 8);
+    if (ce != cudaSuccess) { if (d_pos) cudaFree(d_pos); e->set_error("gather: out of device memory"); return SPB_ERR_NOMEM; }
+  }
+  nr = N->GroupStart();
+  if (learner) {
+    for (int r = 0; r < world && nr == ncclSuccess; ++r) {
+      if (r == rank || counts[r] == 0) continue;
+      nr = N->Recv(d_pos + off[r], (size_t)counts[r] * sizeof(Rec), ncclUint8, r, comm, e->stream);
+      if (nr == ncclSuccess) nr = N->Recv(d_ids + off[r], (size_t)counts[r] * 8, ncclUint8, r, comm, e->stream);
+    }
+  } else if (n_local) {
+    nr = N->Send(P.out, (size_t)n_local * sizeof(Rec), ncclUint8, learner_rank, comm, e->stream);
+    if (nr == ncclSuccess) nr = N->Send(P.out_game, (size_t)n_local * 8, ncclUint8, learner_rank, comm, e->stream);
+  }
+  ncclResult_t nr2 = N->GroupEnd();
+  if (nr == ncclSuccess) nr = nr2;
+  ce = cudaSuccess;
+  if (learner && n_local) {
+    ce = cudaMemcpyAsync(d_pos + off[rank], P.out, (size_t)n_local * sizeof(Rec), cudaMemcpyDeviceToDevice, e->stream);
+    if (ce == cudaSuccess) ce = cudaMemcpyAsync(d_ids + off[rank], P.out_game, (size_t)n_local * 8, cudaMemcpyDeviceToDevice, e->stream);
+  }
+  if (ce == cudaSuccess && P.out) ce = cudaMemsetAsync(P.out_cursor, 0, 8, e->stream);   // the local buffer has been handed over
+  if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
+  if (nr != ncclSuccess || ce != cudaSuccess) {
+    if (d_pos) cudaFree(d_pos);
+    if (d_ids) cudaFree(d_ids);
+    e->set_error(nr != ncclSuccess ? std::string("gather send/recv: ") + N->GetErrorString(nr) : std::string("gather: ") + cudaGetErrorString(ce));
+    return SPB_ERR_CUDA;
+  }
+  *d_pos_out = d_pos;
+  *d_ids_out = d_ids;
+  *total_out = learner ? total : 0;
+  return SPB_OK;
+}
+
+// spb_gather_trajectories / spb_chess_gather_trajectories: the gathered records are ordered on the host and staged there
+// until a call delivers them.
+template <class Trees, class Rec, class Move>
+int32_t gather_trajectories(HostEngine<Trees, Rec, Move>* e, int32_t learner_rank, Rec* buf, size_t capacity, size_t* written,
+                            uint64_t* game_ids) {
+  if (!written) return SPB_ERR_ARG;
+  SPB_GUARD(e);
+  if (int32_t rc = gather_ready(e, learner_rank)) return rc;
+  if (e->gather_dpos) {
+    e->set_error(std::string("the gathered records are staged in device memory: call ") + e->api + "gather_trajectories_device");
+    return SPB_ERR_STATE;
+  }
+  const bool learner = e->comm_rank == learner_rank;
 
   if (!e->gather_pending) {
-    // ---- the collective: counts, then the records -----------------------------------------------------------------
-    unsigned long long n_local = 0;
-    if (P.out) {
-      SPB_CUDA(e, cudaMemcpyAsync(&n_local, P.out_cursor, 8, cudaMemcpyDeviceToHost, e->stream));
-      SPB_CUDA(e, cudaStreamSynchronize(e->stream));
-      n_local = std::min<unsigned long long>(n_local, P.out_cap);
-    }
-    unsigned long long* d_counts = nullptr;
-    SPB_CUDA(e, cudaMalloc((void**)&d_counts, (size_t)world * 8));
-    std::vector<unsigned long long> counts((size_t)world, 0);
-    cudaError_t ce = cudaMemcpyAsync(d_counts + rank, &n_local, 8, cudaMemcpyHostToDevice, e->stream);
-    ncclResult_t nr = ce == cudaSuccess ? N->AllGather(d_counts + rank, d_counts, 1, ncclUint64, comm, e->stream) : ncclSuccess;
-    if (ce == cudaSuccess && nr == ncclSuccess) ce = cudaMemcpyAsync(counts.data(), d_counts, (size_t)world * 8, cudaMemcpyDeviceToHost, e->stream);
-    if (ce == cudaSuccess && nr == ncclSuccess) ce = cudaStreamSynchronize(e->stream);
-    cudaFree(d_counts);
-    if (nr != ncclSuccess) { e->set_error(std::string("ncclAllGather: ") + N->GetErrorString(nr)); return SPB_ERR_CUDA; }
-    if (ce != cudaSuccess) { e->set_error(std::string("gather counts: ") + cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
-    size_t total = 0;
-    std::vector<size_t> off((size_t)world, 0);
-    for (int r = 0; r < world; ++r) { off[r] = total; total += (size_t)counts[r]; }
-
     Rec* d_pos = nullptr;
     unsigned long long* d_ids = nullptr;
-    if (learner && total) {
-      ce = cudaMalloc((void**)&d_pos, total * sizeof(Rec));
-      if (ce == cudaSuccess) ce = cudaMalloc((void**)&d_ids, total * 8);
-      if (ce != cudaSuccess) { if (d_pos) cudaFree(d_pos); e->set_error("gather: out of device memory"); return SPB_ERR_NOMEM; }
-    }
-    nr = N->GroupStart();
-    if (learner) {
-      for (int r = 0; r < world && nr == ncclSuccess; ++r) {
-        if (r == rank || counts[r] == 0) continue;
-        nr = N->Recv(d_pos + off[r], (size_t)counts[r] * sizeof(Rec), ncclUint8, r, comm, e->stream);
-        if (nr == ncclSuccess) nr = N->Recv(d_ids + off[r], (size_t)counts[r] * 8, ncclUint8, r, comm, e->stream);
-      }
-    } else if (n_local) {
-      nr = N->Send(P.out, (size_t)n_local * sizeof(Rec), ncclUint8, learner_rank, comm, e->stream);
-      if (nr == ncclSuccess) nr = N->Send(P.out_game, (size_t)n_local * 8, ncclUint8, learner_rank, comm, e->stream);
-    }
-    ncclResult_t nr2 = N->GroupEnd();
-    if (nr == ncclSuccess) nr = nr2;
-    ce = cudaSuccess;
-    if (learner && n_local) {
-      ce = cudaMemcpyAsync(d_pos + off[rank], P.out, (size_t)n_local * sizeof(Rec), cudaMemcpyDeviceToDevice, e->stream);
-      if (ce == cudaSuccess) ce = cudaMemcpyAsync(d_ids + off[rank], P.out_game, (size_t)n_local * 8, cudaMemcpyDeviceToDevice, e->stream);
-    }
-    if (ce == cudaSuccess && P.out) ce = cudaMemsetAsync(P.out_cursor, 0, 8, e->stream);   // the local buffer has been handed over
-    e->gather_pos.assign(learner ? total : 0, Rec{});
-    e->gather_ids.assign(learner ? total : 0, 0ull);
-    if (ce == cudaSuccess && learner && total) {
+    size_t total = 0;
+    if (int32_t rc = exchange(e, learner_rank, &d_pos, &d_ids, &total)) return rc;
+    e->gather_pos.assign(total, Rec{});
+    e->gather_ids.assign(total, 0ull);
+    cudaError_t ce = cudaSuccess;
+    if (total) {
       ce = cudaMemcpyAsync(e->gather_pos.data(), d_pos, total * sizeof(Rec), cudaMemcpyDeviceToHost, e->stream);
       if (ce == cudaSuccess) ce = cudaMemcpyAsync(e->gather_ids.data(), d_ids, total * 8, cudaMemcpyDeviceToHost, e->stream);
     }
     if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
     if (d_pos) cudaFree(d_pos);
     if (d_ids) cudaFree(d_ids);
-    if (nr != ncclSuccess) { e->set_error(std::string("gather send/recv: ") + N->GetErrorString(nr)); return SPB_ERR_CUDA; }
     if (ce != cudaSuccess) { e->set_error(std::string("gather: ") + cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
     if (learner) sort_records(e->gather_pos, e->gather_ids);
     e->gather_pending = true;
@@ -209,6 +247,36 @@ int32_t gather_trajectories(HostEngine<Trees, Rec, Move>* e, int32_t learner_ran
   e->gather_pos.clear();
   e->gather_ids.clear();
   e->gather_pending = false;
+  return SPB_OK;
+}
+
+// spb_gather_trajectories_device / spb_chess_gather_trajectories_device: the gathered records stay in device memory, in
+// arrival order, until a call orders them into the caller's device buffers (order_records, records.cu).
+template <class Trees, class Rec, class Move>
+int32_t gather_trajectories_device(HostEngine<Trees, Rec, Move>* e, int32_t learner_rank, Rec* buf_dev, size_t capacity, size_t* written,
+                                   uint64_t* game_ids_dev) {
+  if (!written) return SPB_ERR_ARG;
+  SPB_GUARD(e);
+  if (int32_t rc = gather_ready(e, learner_rank)) return rc;
+  if (e->gather_pending) {
+    e->set_error(std::string("the gathered records are staged in host memory: call ") + e->api + "gather_trajectories");
+    return SPB_ERR_STATE;
+  }
+  if (!e->gather_dpos) {
+    if (int32_t rc = exchange(e, learner_rank, &e->gather_dpos, &e->gather_dids, &e->gather_dn)) return rc;
+  }
+  const size_t n = e->gather_dn;
+  *written = n;
+  if (n && (!buf_dev || capacity < n)) return SPB_OK;             // size query: the records stay staged for the next call
+  // the caller's pointers are checked by order_into, after the collective: a bad one leaves the records staged and has
+  // not kept the other ranks waiting
+  if (n)
+    if (int32_t rc = e->order_into(e->gather_dpos, e->gather_dids, n, buf_dev, game_ids_dev)) return rc;
+  if (e->gather_dpos) cudaFree(e->gather_dpos);
+  if (e->gather_dids) cudaFree(e->gather_dids);
+  e->gather_dpos = nullptr;
+  e->gather_dids = nullptr;
+  e->gather_dn = 0;
   return SPB_OK;
 }
 
@@ -233,12 +301,20 @@ int32_t spb_gather_trajectories(spb_engine* e, int32_t learner_rank, spb_positio
                                 uint64_t* game_ids) {
   return gather_trajectories(e, learner_rank, buf, capacity, written, game_ids);
 }
+int32_t spb_gather_trajectories_device(spb_engine* e, int32_t learner_rank, spb_position* buf_dev, size_t capacity, size_t* written,
+                                       uint64_t* game_ids_dev) {
+  return gather_trajectories_device(e, learner_rank, buf_dev, capacity, written, game_ids_dev);
+}
 
 int32_t spb_chess_comm_init(spb_chess_engine* e, const uint8_t* id, int32_t rank, int32_t world_size) { return comm_init(e, id, rank, world_size); }
 int32_t spb_chess_comm_destroy(spb_chess_engine* e) { return comm_destroy(e); }
 int32_t spb_chess_gather_trajectories(spb_chess_engine* e, int32_t learner_rank, spb_chess_position* buf, size_t capacity, size_t* written,
                                       uint64_t* game_ids) {
   return gather_trajectories(e, learner_rank, buf, capacity, written, game_ids);
+}
+int32_t spb_chess_gather_trajectories_device(spb_chess_engine* e, int32_t learner_rank, spb_chess_position* buf_dev, size_t capacity,
+                                             size_t* written, uint64_t* game_ids_dev) {
+  return gather_trajectories_device(e, learner_rank, buf_dev, capacity, written, game_ids_dev);
 }
 
 // ref: learner_concurrent.rs:126-146 / learner.rs:162-182 — the (N,3,R,C) / (N,A) / (N,1) training tensors.
@@ -273,6 +349,37 @@ int32_t spb_positions_to_training(int32_t game, const spb_position* positions, s
     }
     if (values) values[i] = (float)p.outcome;
   }
+  return SPB_OK;
+}
+
+// The same tensors built on the device from records in device memory (launch_training_tensors, records.cu), for the
+// engine's game; row i from positions[indices ? indices[i] : i].
+int32_t spb_positions_to_training_device(spb_engine* e, const spb_position* positions, size_t n_positions, const uint64_t* indices, size_t n,
+                                         float* encodings, float* policies, float* values) {
+  SPB_GUARD(e);
+  SPB_ARG(e, indices || n <= n_positions, "n > n_positions without indices");
+  if (n == 0) return SPB_OK;
+  SPB_ARG(e, positions, "null positions");
+  if (int32_t rc = e->check_device_pointers({{positions, "positions", 8}, {indices, "indices", 8}, {encodings, "encodings", 4},
+                                              {policies, "policies", 4}, {values, "values", 4}}))
+    return rc;
+  const auto* idx = reinterpret_cast<const unsigned long long*>(indices);
+  int sms = 0;
+  SPB_CUDA(e, cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, e->cfg.device));
+  if (idx) {
+    const unsigned long long none = ~0ull;
+    unsigned long long bad = none;
+    unsigned long long* d_bad = e->d_misc;                             // the engine's scratch word; every call ends synchronised
+    SPB_CUDA(e, cudaMemsetAsync(d_bad, 0xFF, 8, e->stream));
+    SPB_CUDA(e, launch_index_check(idx, n, n_positions, d_bad, sms, e->stream));
+    ++e->launches;
+    SPB_CUDA(e, cudaMemcpyAsync(&bad, d_bad, 8, cudaMemcpyDeviceToHost, e->stream));
+    SPB_CUDA(e, cudaStreamSynchronize(e->stream));
+    if (bad != none) { e->set_error("training row " + std::to_string(bad) + ": index out of range"); return SPB_ERR_ARG; }
+  }
+  SPB_CUDA(e, launch_training_tensors(e->cfg.game, positions, idx, n, encodings, policies, values, sms, e->stream));
+  ++e->launches;
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
   return SPB_OK;
 }
 

@@ -6,12 +6,14 @@
 #include <algorithm>
 #include <cfloat>
 #include <cstring>
+#include <initializer_list>
 #include <new>
 #include <string>
 #include <vector>
 
 #include <cuda_runtime.h>
 
+#include "records.cuh"
 #include "trajectory.cuh"
 #include "tree.cuh"
 
@@ -68,6 +70,11 @@ struct HostEngine {
   bool gather_pending = false;
   std::vector<Rec> gather_pos;
   std::vector<unsigned long long> gather_ids;
+  // a gather staged by the device form (gather_trajectories_device): the learner's records in arrival order, not yet
+  // ordered, until a call delivers them; freed by that call or by release()
+  Rec* gather_dpos = nullptr;
+  unsigned long long* gather_dids = nullptr;
+  size_t gather_dn = 0;
   // EXTENSION: Dirichlet noise at the root (set_root_noise).  The buffers are allocated by the first call that turns the
   // noise on (an engine that never enables it keeps its footprint); T.root_noise points at them while it is on.
   float* d_noise_eta = nullptr;
@@ -162,6 +169,8 @@ struct HostEngine {
     allocs.clear();
     if (d_stage) cudaFree(d_stage);
     if (h_stage) cudaFreeHost(h_stage);
+    if (gather_dpos) cudaFree(gather_dpos);
+    if (gather_dids) cudaFree(gather_dids);
     if (ev0) cudaEventDestroy(ev0);
     if (ev1) cudaEventDestroy(ev1);
     if (stream) cudaStreamDestroy(stream);
@@ -219,6 +228,37 @@ struct HostEngine {
     if (bits & ERRBIT_BOUNDS) { set_error("device check failed at site " + std::to_string((bits >> 8) & 0xFFu) + " (see ERRBIT_BOUNDS in csrc/)"); return SPB_ERR_STATE; }
     set_error("NaN PUCT score (the reference panics here, mcts.rs:109)");   // ERRBIT_NAN: Connect4 / tic-tac-toe
     return SPB_ERR_STATE;
+  }
+
+  // A pointer argument of a device entry point: the kernels read or write it with accesses of `align` bytes.
+  struct DevicePointer { const void* p; const char* name; size_t align; };
+
+  // Every non-null pointer must be device memory of the engine's GPU, or managed memory, aligned for the kernels' accesses
+  // (a misaligned one would fault on the device): SPB_ERR_ARG naming the first that is not.
+  int32_t check_device_pointers(std::initializer_list<DevicePointer> ptrs) {
+    for (const DevicePointer& d : ptrs) {
+      if (!d.p) continue;
+      cudaPointerAttributes a{};
+      const cudaError_t ce = cudaPointerGetAttributes(&a, d.p);
+      if (ce != cudaSuccess) cudaGetLastError();
+      const bool ok = ce == cudaSuccess && (a.type == cudaMemoryTypeManaged || (a.type == cudaMemoryTypeDevice && a.device == cfg.device));
+      SPB_ARG(this, ok, std::string(d.name) + " is not device memory of the engine's GPU");
+      SPB_ARG(this, reinterpret_cast<uintptr_t>(d.p) % d.align == 0, std::string(d.name) + " is not " + std::to_string(d.align) + "-byte aligned");
+    }
+    return SPB_OK;
+  }
+
+  // Orders n records of src / src_ids into the caller's dst / dst_ids (order_records, records.cu) with scratch from the
+  // stage, then waits for the stream.  The caller's pointers are checked here, where they are first needed: a failed
+  // check leaves the records where they were.
+  int32_t order_into(const Rec* src, const unsigned long long* src_ids, size_t n, Rec* dst, uint64_t* dst_ids) {
+    SPB_ARG(this, n < ((size_t)1 << 31), "more than 2^31 - 1 records to order");
+    if (int32_t rc = check_device_pointers({{dst, "buf_dev", 8}, {dst_ids, "game_ids_dev", 8}})) return rc;
+    if (int32_t rc = ensure_stage(order_scratch_bytes<Rec>(n), 0)) return rc;
+    SPB_CUDA(this, order_records(src, src_ids, n, dst, reinterpret_cast<unsigned long long*>(dst_ids), d_stage, stream));
+    ++launches;
+    SPB_CUDA(this, cudaStreamSynchronize(stream));
+    return SPB_OK;
   }
 
   // ---- bodies of the entry points both ABIs have (spb_X / spb_chess_X) ---------------------------------------------
@@ -326,6 +366,26 @@ struct HostEngine {
       buf[i] = pos[order[i]];
       if (game_ids) game_ids[i] = ids[order[i]];
     }
+    return SPB_OK;
+  }
+
+  // The device form of drain_trajectories: the same records in the same order, written to the caller's device buffers.
+  // capacity < n is SPB_ERR_ARG with nothing drained.
+  int32_t drain_trajectories_device(Rec* buf_dev, size_t capacity, size_t* written, uint64_t* game_ids_dev) {
+    SPB_ARG(this, written, "null written");
+    unsigned long long cur = 0;
+    if (P.out) {
+      SPB_CUDA(this, cudaMemcpyAsync(&cur, P.out_cursor, 8, cudaMemcpyDeviceToHost, stream));
+      SPB_CUDA(this, cudaStreamSynchronize(stream));
+    }
+    const size_t n = (size_t)std::min<unsigned long long>(cur, P.out_cap);
+    *written = n;
+    if (!buf_dev) return SPB_OK;                    // size query
+    SPB_ARG(this, capacity >= n, "trajectory buffer too small");
+    if (n == 0) return SPB_OK;
+    if (int32_t rc = order_into(P.out, P.out_game, n, buf_dev, game_ids_dev)) return rc;
+    SPB_CUDA(this, cudaMemsetAsync(P.out_cursor, 0, 8, stream));
+    SPB_CUDA(this, cudaStreamSynchronize(stream));
     return SPB_OK;
   }
 };

@@ -96,11 +96,14 @@ ABI = {
     "spb_game_encode": (C.c_int32, [_vp, _vp, C.c_uint32, _vp]),
     "spb_selfplay_step": (C.c_int32, [_vp, C.c_int32, C.c_float, C.c_uint64, _vp, _u32p]),
     "spb_drain_trajectories": (C.c_int32, [_vp, _vp, C.c_size_t, C.POINTER(C.c_size_t), _vp]),
+    "spb_drain_trajectories_device": (C.c_int32, [_vp, _vp, C.c_size_t, C.POINTER(C.c_size_t), _vp]),
     "spb_comm_unique_id": (C.c_int32, [_vp]),
     "spb_comm_init": (C.c_int32, [_vp, _vp, C.c_int32, C.c_int32]),
     "spb_comm_destroy": (C.c_int32, [_vp]),
     "spb_gather_trajectories": (C.c_int32, [_vp, C.c_int32, _vp, C.c_size_t, C.POINTER(C.c_size_t), _vp]),
+    "spb_gather_trajectories_device": (C.c_int32, [_vp, C.c_int32, _vp, C.c_size_t, C.POINTER(C.c_size_t), _vp]),
     "spb_positions_to_training": (C.c_int32, [C.c_int32, _vp, C.c_size_t, _vp, _vp, _vp]),
+    "spb_positions_to_training_device": (C.c_int32, [_vp, _vp, C.c_size_t, _vp, C.c_size_t, _vp, _vp, _vp]),
     # chess (ref: src/game/chess.rs, src/model/chess.rs); typed wrappers in chess.py
     "spb_chess_create": (C.c_int32, [C.POINTER(Config), C.POINTER(_vp)]),
     "spb_chess_destroy": (C.c_int32, [_vp]),
@@ -133,11 +136,13 @@ ABI = {
     "spb_chess_reset_counters": (C.c_int32, [_vp]),
     "spb_chess_selfplay_step": (C.c_int32, [_vp, C.c_int32, C.c_float, C.c_uint64, _vp, _vp, _u32p]),
     "spb_chess_drain_trajectories": (C.c_int32, [_vp, _vp, C.c_size_t, C.POINTER(C.c_size_t), _vp]),
+    "spb_chess_drain_trajectories_device": (C.c_int32, [_vp, _vp, C.c_size_t, C.POINTER(C.c_size_t), _vp]),
     "spb_chess_positions_to_training": (C.c_int32, [_vp, C.c_size_t, _vp, _vp, _vp]),
     "spb_chess_positions_to_training_device": (C.c_int32, [_vp, _vp, C.c_size_t, _vp, C.c_size_t, _vp, _vp, _vp]),
     "spb_chess_comm_init": (C.c_int32, [_vp, _vp, C.c_int32, C.c_int32]),
     "spb_chess_comm_destroy": (C.c_int32, [_vp]),
     "spb_chess_gather_trajectories": (C.c_int32, [_vp, C.c_int32, _vp, C.c_size_t, C.POINTER(C.c_size_t), _vp]),
+    "spb_chess_gather_trajectories_device": (C.c_int32, [_vp, C.c_int32, _vp, C.c_size_t, C.POINTER(C.c_size_t), _vp]),
     "spb_get_counters": (C.c_int32, [_vp, C.POINTER(Counters)]),
     "spb_reset_counters": (C.c_int32, [_vp]),
     "spb_last_search_timing": (C.c_int32, [_vp, _f32p, _f32p, _u32p]),
@@ -227,6 +232,83 @@ def positions_to_training(game: int, positions: np.ndarray):
     return enc, pol, val
 
 
+def _check_cuda_tensor(t, dtype, width, name):
+    """Raises unless t is a contiguous CUDA tensor of `dtype`, [n, width] (width None: [n])."""
+    import torch
+    if not isinstance(t, torch.Tensor):
+        raise TypeError("%s must be a CUDA tensor, not %s" % (name, type(t).__name__))
+    if t.dtype not in ((dtype,) if not isinstance(dtype, tuple) else dtype):
+        raise TypeError("%s must be %s, not %s" % (name, dtype, t.dtype))
+    if (width is None and t.dim() != 1) or (width is not None and (t.dim() != 2 or t.shape[1] != width)):
+        raise ValueError("%s must be [n%s], not %s" % (name, "" if width is None else ", %d" % width, tuple(t.shape)))
+    if not t.is_cuda:
+        raise TypeError("%s must be a CUDA tensor, not on %s" % (name, t.device))
+    if not t.is_contiguous():
+        raise ValueError("%s must be contiguous" % name)
+
+
+def _records_to_device(call, device, width, out, ids_out):
+    """The device forms of drain / gather: `call(buf, capacity, n_ref, ids)` is the entry point with the engine's
+    arguments bound.  Size query, then the records into `out` / `ids_out` (allocated when None) -> their [:n] views."""
+    import torch
+    if out is not None:
+        _check_cuda_tensor(out, torch.uint8, width, "out")
+    if ids_out is not None:
+        _check_cuda_tensor(ids_out, torch.int64, None, "ids_out")
+    dev = torch.device("cuda", device)
+    n = C.c_size_t()
+    call(None, 0, C.byref(n), None)
+    k = n.value
+    if out is None:
+        out = torch.empty((k, width), dtype=torch.uint8, device=dev)
+    if ids_out is None:
+        ids_out = torch.empty(k, dtype=torch.int64, device=dev)
+    if len(out) < k or len(ids_out) < k:
+        raise ValueError("out / ids_out hold %d / %d records, %d are ready" % (len(out), len(ids_out), k))
+    if k:
+        torch.cuda.current_stream(dev).synchronize()                   # the caller's work on out / ids_out comes first
+        call(out.data_ptr(), len(out), C.byref(n), ids_out.data_ptr())
+    return out[:n.value], ids_out[:n.value]
+
+
+def positions_to_training_device(engine: "Engine", positions, indices=None):
+    """spb_positions_to_training_device: the tensors of positions_to_training(engine.game, ...), built on the engine's GPU
+    -> torch CUDA tensors (encodings[n,3,R,C], policies[n,A], values[n,1]) f32, bit-identical to the host builder.
+    positions: POSITION_DTYPE numpy array (copied to the device) or a CUDA uint8 tensor [n_positions, 56], e.g. a replay
+    buffer kept in device memory.  indices (numpy or CUDA int64 / uint64 tensor): row i is built from
+    positions[indices[i]]; without it every record is built.  An index out of range raises EngineError(-1) and nothing is
+    written."""
+    import torch
+    if isinstance(positions, torch.Tensor):
+        _check_cuda_tensor(positions, torch.uint8, POSITION_DTYPE.itemsize, "positions")
+        pos = positions
+    if indices is not None and isinstance(indices, torch.Tensor):
+        _check_cuda_tensor(indices, (torch.int64, torch.uint64), None, "indices")
+    dev = torch.device("cuda", engine.device)
+    if not isinstance(positions, torch.Tensor):
+        a = np.ascontiguousarray(positions, dtype=POSITION_DTYPE).reshape(-1)
+        pos = torch.from_numpy(a.view(np.uint8).reshape(len(a), POSITION_DTYPE.itemsize)).to(dev)
+    idx = None
+    if indices is not None:
+        if isinstance(indices, torch.Tensor):
+            idx = indices
+        else:
+            i = np.ascontiguousarray(indices).reshape(-1)
+            if i.dtype.kind not in "iu":
+                raise TypeError("indices must be integers, not %s" % i.dtype)
+            idx = torch.from_numpy(i.astype(np.int64)).to(dev)
+    n = len(pos) if idx is None else len(idx)
+    R, Cc = BOARD[engine.game]
+    enc = torch.empty((n, 3, R, Cc), dtype=torch.float32, device=dev)
+    pol = torch.empty((n, NUM_ACTIONS[engine.game]), dtype=torch.float32, device=dev)
+    val = torch.empty((n, 1), dtype=torch.float32, device=dev)
+    torch.cuda.current_stream(dev).synchronize()                       # the engine's stream reads the inputs
+    engine._chk(engine._L.spb_positions_to_training_device(
+        engine._h, pos.data_ptr() if len(pos) else None, len(pos), None if idx is None else idx.data_ptr(), n,
+        enc.data_ptr(), pol.data_ptr(), val.data_ptr()))
+    return enc, pol, val
+
+
 class Engine:
     """One engine = `Mcts` + its `Vec<Tree>` on one GPU (ref: mcts.rs:41-44, learner_concurrent.rs:174)."""
 
@@ -244,7 +326,7 @@ class Engine:
         if rc != 0:
             raise EngineError(rc, L.spb_last_error(None).decode())
         self._h, self._L = h, L
-        self.game, self.G, self.A = game, num_games, NUM_ACTIONS[game]
+        self.game, self.G, self.A, self.device = game, num_games, NUM_ACTIONS[game], device
 
     def close(self):
         if getattr(self, "_h", None):
@@ -398,6 +480,12 @@ class Engine:
             self._chk(self._L.spb_drain_trajectories(self._h, pos.ctypes.data, n.value, C.byref(n), ids.ctypes.data))
         return pos[:n.value], ids[:n.value]
 
+    def drain_trajectories_device(self, out=None, ids_out=None):
+        """The records of drain_trajectories, ordered on the device -> (CUDA uint8 [n, 56], CUDA int64 [n]).  out / ids_out:
+        caller tensors to write into (e.g. replay[head:]); the [:n] views of them are returned."""
+        return _records_to_device(lambda b, cap, n, i: self._chk(self._L.spb_drain_trajectories_device(self._h, b, cap, n, i)),
+                                  self.device, POSITION_DTYPE.itemsize, out, ids_out)
+
     # ---- multi-GPU: trajectories to the learner rank --------------------------------------------
     def comm_init(self, comm_id: bytes, rank: int, world_size: int):
         buf = (C.c_uint8 * COMM_ID_BYTES).from_buffer_copy(comm_id)
@@ -415,6 +503,13 @@ class Engine:
         if n.value:
             self._chk(self._L.spb_gather_trajectories(self._h, learner_rank, pos.ctypes.data, n.value, C.byref(n), ids.ctypes.data))
         return pos, ids
+
+    def gather_trajectories_device(self, learner_rank: int = 0, out=None, ids_out=None):
+        """COLLECTIVE: gather_trajectories into device memory of the learner rank -> (CUDA uint8 [n, 56], CUDA int64 [n]),
+        empty elsewhere; out / ids_out as for drain_trajectories_device."""
+        return _records_to_device(
+            lambda b, cap, n, i: self._chk(self._L.spb_gather_trajectories_device(self._h, learner_rank, b, cap, n, i)),
+            self.device, POSITION_DTYPE.itemsize, out, ids_out)
 
     # ---- counters ----------------------------------------------------------------------------
     def counters(self) -> dict:

@@ -133,6 +133,27 @@ class Mcts {
   }
   spb_engine* raw() { return e_; }
 
+  // The learner hand-off in device memory.  Pointers ending in _dev are device memory of this engine's GPU (e.g. a slice
+  // of a replay buffer); a null buf_dev is the size query.  Each returns the number of records held / written.
+  // Finished games' positions ordered by (game id, ply), with their global game ids (game_ids_dev nullable).
+  size_t drain_trajectories_device(spb_position* buf_dev, size_t capacity, uint64_t* game_ids_dev = nullptr) {
+    size_t n = 0;
+    check(spb_drain_trajectories_device(e_, buf_dev, capacity, &n, game_ids_dev));
+    return n;
+  }
+  // COLLECTIVE: every rank's records to learner_rank (0 elsewhere); a null or short buffer keeps them staged on the device.
+  size_t gather_trajectories_device(int32_t learner_rank, spb_position* buf_dev, size_t capacity, uint64_t* game_ids_dev = nullptr) {
+    size_t n = 0;
+    check(spb_gather_trajectories_device(e_, learner_rank, buf_dev, capacity, &n, game_ids_dev));
+    return n;
+  }
+  // The training tensors of spb_positions_to_training for this engine's game, built on the device; row i from
+  // positions_dev[indices_dev ? indices_dev[i] : i], each output nullable.
+  void positions_to_training_device(const spb_position* positions_dev, size_t n_positions, const uint64_t* indices_dev, size_t n,
+                                    float* encodings_dev, float* policies_dev, float* values_dev) {
+    check(spb_positions_to_training_device(e_, positions_dev, n_positions, indices_dev, n, encodings_dev, policies_dev, values_dev));
+  }
+
  private:
   void check(int rc) { if (rc != SPB_OK) throw Error(rc, spb_last_error(e_)); }
   spb_engine* e_ = nullptr;
@@ -263,6 +284,17 @@ class ChessMcts {
     pos.resize(n);
     ids.resize(n);
     return {std::move(pos), std::move(ids)};
+  }
+  // The device forms (as Mcts::drain_trajectories_device / gather_trajectories_device), chess records.
+  size_t drain_trajectories_device(spb_chess_position* buf_dev, size_t capacity, uint64_t* game_ids_dev = nullptr) {
+    size_t n = 0;
+    check(spb_chess_drain_trajectories_device(e_, buf_dev, capacity, &n, game_ids_dev));
+    return n;
+  }
+  size_t gather_trajectories_device(int32_t learner_rank, spb_chess_position* buf_dev, size_t capacity, uint64_t* game_ids_dev = nullptr) {
+    size_t n = 0;
+    check(spb_chess_gather_trajectories_device(e_, learner_rank, buf_dev, capacity, &n, game_ids_dev));
+    return n;
   }
   // The training tensors of chess records (host only): encodings [n][19][8][8], policies [n][4672], values [n].
   struct TrainingBatch { std::vector<float> encodings, policies, values; };
