@@ -216,10 +216,24 @@ class ChessNet(nn.Module):
         return pairs
 
 
-def make_chess_net(seed=0, randomize_bn=True, blocks=10):
+def make_chess_net(seed=0, randomize_bn=True, blocks=10, calibrated=False):
+    """calibrated: the counterpart of make_net(trained_like=True), calibrated on chess_calibration_encodings().  BatchNorm
+    as after training: gammas 0.5..2, shifted betas, and running statistics that are those of the conv outputs they normalise
+    (random statistics would make the torso blow small differences up, which a trained torso does not).  Heads: the value
+    conv's pre-activation is standardised, fc2's pre-tanh scaled to mean 0 and standard deviation 0.8 (values spread over
+    (-1, 1), some near saturation), and policy_conv2 scaled so that the position-dependent part of the logits (each logit
+    minus its mean over the positions) has standard deviation 1.  A fresh net's value is nearly constant and its logits
+    barely depend on the position, so a comparison against it cannot see the heads."""
     g = torch.Generator().manual_seed(seed)
     torch.manual_seed(seed)
     net = ChessNet(blocks=blocks).eval()
+    if calibrated:
+        with torch.no_grad():
+            for _, bn in net.conv_bn_pairs():
+                bn.weight.copy_(torch.rand(bn.num_features, generator=g) * 1.5 + 0.5)
+                bn.bias.copy_(torch.randn(bn.num_features, generator=g) * 0.3)
+            _calibrate_chess_net(net, chess_calibration_encodings())
+        return net
     if randomize_bn:
         with torch.no_grad():
             for _, bn in net.conv_bn_pairs():
@@ -228,6 +242,51 @@ def make_chess_net(seed=0, randomize_bn=True, blocks=10):
                 bn.weight.copy_(torch.rand(bn.num_features, generator=g) * 0.5 + 0.75)
                 bn.bias.copy_(torch.randn(bn.num_features, generator=g) * 0.1)
     return net
+
+
+def chess_calibration_encodings(n=64, seed=97):
+    """Encodings of n fixed positions: the position after a random playout of 0..99 plies (oracle rules, seeded)."""
+    from . import pychess
+    rng = np.random.default_rng(seed)
+    out = []
+    while len(out) < n:
+        g = pychess.Game()
+        for _ in range(int(rng.integers(0, 100))):
+            lm = g.legal_moves()
+            if g.status() != 0 or not lm:
+                break
+            g.make_move(int(lm[rng.integers(len(lm))]))
+        if g.status() == 0:
+            out.append(g.encode())
+    return np.stack(out)
+
+
+def _calibrate_chess_net(net, enc):
+    def bn_from(conv, bn, x):
+        u = conv(x)
+        bn.running_mean.copy_(u.mean((0, 2, 3)))
+        bn.running_var.copy_(u.var((0, 2, 3)))
+        return bn(u)
+    x = torch.from_numpy(np.ascontiguousarray(enc, dtype=np.float32))
+    x = torch.relu(bn_from(net.stem, net.stem_bn, x))
+    for b in net.blocks:
+        x = torch.relu(x + bn_from(b.conv2, b.bn2, torch.relu(bn_from(b.conv1, b.bn1, x))))
+    u = net.vconv(x)
+    m, s = u.mean(), u.std()
+    net.vconv.weight.div_(s)
+    net.vconv.bias.sub_(m).div_(s)
+    z = net.fc2(torch.relu(net.fc1(torch.relu(net.vconv(x)).flatten(1))))
+    m, s = z.mean(), z.std() / 0.8
+    net.fc2.weight.div_(s)
+    net.fc2.bias.sub_(m).div_(s)
+    lg = net.p2(torch.relu(net.p1(x))).flatten(1)
+    net.p2.weight.div_((lg - lg.mean(0)).std())
+
+
+def chess_logit_deviation(logits):
+    """Standard deviation of the position-dependent part of the logits: each logit minus its mean over the positions."""
+    lg = np.asarray(logits, np.float64)
+    return float((lg - lg.mean(0)).std())
 
 
 def chess_to_safetensors_explicit(net) -> bytes:

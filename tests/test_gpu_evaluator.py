@@ -51,9 +51,27 @@ def test_simt_evaluator_matches_torch(game):
 
 
 @pytest.mark.parametrize("game", [S.GAME_C4, S.GAME_TTT], ids=["c4", "ttt"])
-@pytest.mark.parametrize("n", [1, 9, 10, 300, 2000])
+@pytest.mark.parametrize("n", [1, 9, 10, 300, 2000, 19000])
 def test_tcgen05_evaluator_matches_torch(game, n):
+    """19,000 positions: about 128 per CTA, so every CTA runs its static batch loop well past the first batch (15 batches of
+    9 boards for Connect4, 5 of 32 for tic-tac-toe)."""
     _check(game, 0, n, 2, torch_net.to_safetensors_tch)
+
+
+@pytest.mark.parametrize("trained_like", [False, True], ids=["fresh", "trained-like"])
+@pytest.mark.parametrize("game", [S.GAME_C4, S.GAME_TTT], ids=["c4", "ttt"])
+def test_tcgen05_evaluator_is_roll_invariant_bit_for_bit(game, trained_like):
+    """A position's outputs do not depend on where it sits in the batch: rolled by 7, every position lands in another slot
+    of another static batch of another CTA, and its logits and value must not change by a bit."""
+    n = 19000
+    net = torch_net.make_net(game, seed=5, trained_like=trained_like)
+    states = random_states(game, n, seed=6, include_terminal=False)
+    with S.Engine(game=game, num_games=4, evaluator=S.EVAL_NET) as e:
+        e.load_weights(torch_net.to_safetensors_tch(net))
+        pol, v, lg = e.predict(states, want_logits=True)
+        pol_r, v_r, lg_r = e.predict(states[-7:] + states[:-7], want_logits=True)
+    assert np.array_equal(np.roll(lg, 7, axis=0), lg_r) and np.array_equal(np.roll(v, 7), v_r)
+    assert np.array_equal(np.roll(pol, 7, axis=0), pol_r)
 
 
 @pytest.mark.parametrize("game", [S.GAME_C4, S.GAME_TTT], ids=["c4", "ttt"])

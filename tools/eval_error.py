@@ -1,8 +1,13 @@
-"""Error of the evaluator kernels against the torch fp32 network over several nets: fresh (random init, randomised BatchNorm)
-and trained-like (BatchNorm gammas 0.5..2, shifted statistics, larger heads).  Reported per net: max |dlogit| / max |logit|
-(the bound of tests/test_gpu_evaluator.py), the worst per-position relative L2 error of the logit vector, the largest change of
-a softmax probability, max |dvalue|.  Also the chess 10x256 network.  Needs a B200."""
+"""Error of the evaluator kernels over several nets.  Connect4 / tic-tac-toe against the torch fp32 network: fresh (random
+init, randomised BatchNorm) and trained-like (BatchNorm gammas 0.5..2, shifted statistics, larger heads); reported per net:
+max |dlogit| / max |logit| (the bound of tests/test_gpu_evaluator.py), the worst per-position relative L2 error of the logit
+vector, the largest change of a softmax probability, max |dvalue|.  The chess 10x256 network, fresh (seed 0) and calibrated
+(make_chess_net(calibrated=True)), on the 4,096 distinct positions of tests/test_net_numerics.py at every batch size of
+its tile-loop regimes, against the bf16-faithful reference (tests/chess_net_ref.py; |dlogit| over the logit's
+position-dependent spread, the bound of that test) and against torch fp32.  Needs a B200; prints the card and its power
+limit first."""
 import os
+import subprocess
 import sys
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -12,6 +17,9 @@ import numpy as np  # noqa: E402
 import selfplay_b200 as S  # noqa: E402
 from helpers import random_states  # noqa: E402
 from oracle import pyoracle as O, torch_net  # noqa: E402
+
+print(subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True, text=True).stdout.strip(),
+      flush=True)
 
 
 def report(tag, lg, v, logit_ref, v_ref):
@@ -35,16 +43,34 @@ for game, tag in ((S.GAME_C4, "c4"), (S.GAME_TTT, "ttt")):
                     _, v, lg = e.predict(states, want_logits=True)
                 report("%s %s seed %d %s" % (tag, "trained-like" if trained else "fresh", seed, name), lg, v, logit_ref, v_ref)
 
-sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests"))
-from test_chess import export_all, random_games  # noqa: E402
+import torch  # noqa: E402
 
-games = [g for g in random_games(6, seed=41, max_plies=100) if g.status() == 0][::5][:64]
-st, hist = export_all(games)
-enc = np.stack([g.encode() for g in games])
-for seed in range(2):
-    net = torch_net.make_chess_net(seed=seed)
-    _, v_ref, logit_ref = torch_net.chess_forward(net, enc)
-    with S.ChessEngine(num_games=64, evaluator=S.EVAL_NET) as e:
-        e.load_weights(torch_net.chess_to_safetensors_tch(net))
-        _, v, lg = e.predict(st, hist, want_logits=True)
-    report("chess 10x256 seed %d tcgen05" % seed, lg, v, logit_ref, v_ref)
+import chess_net_ref as R  # noqa: E402
+import test_net_numerics as T  # noqa: E402
+
+torch.backends.cuda.matmul.allow_tf32 = False
+torch.backends.cudnn.allow_tf32 = False
+with S.ChessEngine(num_games=T.G, evaluator=S.EVAL_NET) as e:
+    st, hist = T.distinct_positions(e, T.G)
+    enc = e.encode(st, hist)
+    pairs = T.conv_pairs(T.G, torch.cuda.get_device_properties(0).multi_processor_count)
+    for name, kw in T.NETS.items():
+        net = torch_net.make_chess_net(**kw)
+        ref_lg, ref_v = R.ChessNetRef(net, device="cuda").forward(enc)
+        spread = ref_lg.std(0)
+        with torch.no_grad():
+            out = [net.cuda()(torch.from_numpy(enc[i:i + 512]).cuda()) for i in range(0, T.G, 512)]
+        lg32 = torch.cat([o[0] for o in out]).cpu().numpy()
+        v32 = torch.cat([o[1] for o in out]).reshape(-1).cpu().numpy()
+        e.load_weights(torch_net.chess_to_safetensors_explicit(net.cpu()))
+        print("chess 10x256 %s: value std %.3f, logit scale %.1f, position-dependent logit spread %.3g (median per logit %.3g)" % (
+            name, ref_v.std(), np.abs(ref_lg).max(), torch_net.chess_logit_deviation(ref_lg), np.median(spread)), flush=True)
+        for n in T.batch_sizes(pairs):
+            _, v, lg = e.predict(st[:n], hist[:n], want_logits=True)
+            r = np.abs(lg - ref_lg[:n]) / spread
+            dv = np.abs(v - ref_v[:n])
+            print("  n %4d it<=%2d | vs bf16 reference: |dlogit|/spread max %.2e p99.99 %.2e median %.2e; |dv| max %.2e p99 %.2e "
+                  "| vs fp32: max|dlogit|/scale %.2e |dlogit|/spread max %.2e |dv| max %.2e" % (
+                      n, T.max_pass(n, pairs), r.max(), np.quantile(r, 0.9999), np.median(r), dv.max(), np.quantile(dv, 0.99),
+                      np.abs(lg - lg32[:n]).max() / np.abs(lg32[:n]).max(), (np.abs(lg - lg32[:n]) / spread).max(),
+                      np.abs(v - v32[:n]).max()), flush=True)
