@@ -149,6 +149,35 @@ int32_t spb_load_weights(spb_engine* e, const void* safetensors_blob, size_t num
  */
 int32_t spb_check_weights(int32_t game, const void* safetensors_blob, size_t num_bytes, char* err, size_t err_cap);
 
+/*
+ * Weights straight from a learner's device tensors, with no file in between.  One table entry per tensor, named by either
+ * scheme spb_load_weights accepts (explicit names, or the tch VarStore names that VarStore::variables() returns, e.g.
+ * "weight__12"); tensors no role needs are ignored, as in a blob.  data is device memory of the engine's GPU (or managed
+ * memory), contiguous, row-major, aligned to its element size.  The accepted dtypes are those of the blob: F32, BF16, F64
+ * (SPB_DTYPE_F16 is rejected with the blob's message).
+ */
+#define SPB_DTYPE_F32  0
+#define SPB_DTYPE_BF16 1
+#define SPB_DTYPE_F64  2
+#define SPB_DTYPE_F16  3
+typedef struct spb_tensor {
+  const char* name;
+  const void* data;
+  int32_t dtype;                 /* SPB_DTYPE_* */
+  int32_t ndim;                  /* 0..4 */
+  int64_t shape[4];
+} spb_tensor;                    /* 56 bytes */
+/*
+ * BatchNorm is folded and the image packed on the device, byte for byte the image spb_load_weights writes for the same
+ * tensors.  Ordering: the caller has finished writing the tensors before the call (e.g. a stream synchronisation); the call
+ * synchronises the engine's stream before it returns, after which it no longer reads them (the next optimizer step may
+ * update them in place).  Names, shapes, dtypes and pointers are checked before anything is written: a bad table returns
+ * SPB_ERR_WEIGHTS (as the blob would) or SPB_ERR_ARG (NULL table or name, ndim outside 0..4, a pointer that is not device
+ * memory of the engine's GPU or is misaligned) and leaves the loaded net as it was.  The image is rewritten in place (no
+ * device allocation after the engine's first load); a CUDA error while writing it leaves the engine without weights.
+ */
+int32_t spb_load_weights_device(spb_engine* e, const spb_tensor* tensors, uint32_t n);
+
 /* ---- trees (ref: Tree::default mcts.rs:67, Tree::with_root_state mcts.rs:86) ---- */
 
 /*
@@ -321,6 +350,8 @@ const char* spb_chess_last_error(const spb_chess_engine* e);
 /* VarStore::load (main.rs:61) for model/chess.rs:50-73: safetensors bytes, BatchNorm folded, bf16 packed for tcgen05. */
 int32_t spb_chess_load_weights(spb_chess_engine* e, const void* blob, size_t n);
 int32_t spb_chess_check_weights(const void* blob, size_t n, char* err, size_t err_cap);   /* host only */
+/* spb_load_weights_device for the chess net (the names of spb_chess_load_weights); the network is created on first use. */
+int32_t spb_chess_load_weights_device(spb_chess_engine* e, const spb_tensor* tensors, uint32_t n);
 
 /* State::default(), chess.rs:94-102 (host only). */
 int32_t spb_chess_start_position(spb_chess_state* out);
@@ -486,6 +517,15 @@ int32_t spb_gather_trajectories(spb_engine* e, int32_t learner_rank, spb_positio
 int32_t spb_gather_trajectories_device(spb_engine* e, int32_t learner_rank, spb_position* buf_dev, size_t capacity,
                                        size_t* written, uint64_t* game_ids_dev /* nullable */);
 /*
+ * COLLECTIVE over the communicator: the weight image of root_rank, as it stands, replaces every other rank's (a rank needs
+ * no weights beforehand).  First every rank learns what every rank holds (all-gather of a small descriptor): if the root
+ * has no weights (SPB_ERR_STATE), a rank cannot hold the image (SPB_ERR_NOMEM) or the ranks' games differ (SPB_ERR_ARG),
+ * every rank returns that error, no second collective is issued and every net stays as it was.  Then the image is
+ * broadcast on the engine's stream; a non-root rank whose image did not arrive is left without weights.  No communicator:
+ * SPB_ERR_STATE; root_rank out of range: SPB_ERR_ARG.  Trajectory staging is not touched.
+ */
+int32_t spb_broadcast_weights(spb_engine* e, int32_t root_rank);
+/*
  * The same for chess engines (ref: learner_concurrent.rs:281-288), with the contract of spb_comm_init, spb_comm_destroy and
  * spb_gather_trajectories; the id comes from spb_comm_unique_id.  The gather hands over what spb_chess_drain_trajectories
  * would return; an engine that never played (no trajectory buffers yet) takes part with 0 records.  spb_chess_destroy
@@ -497,6 +537,7 @@ int32_t spb_chess_gather_trajectories(spb_chess_engine* e, int32_t learner_rank,
                                       size_t* written, uint64_t* game_ids /* nullable */);
 int32_t spb_chess_gather_trajectories_device(spb_chess_engine* e, int32_t learner_rank, spb_chess_position* buf_dev,
                                              size_t capacity, size_t* written, uint64_t* game_ids_dev /* nullable */);
+int32_t spb_chess_broadcast_weights(spb_chess_engine* e, int32_t root_rank);   /* spb_broadcast_weights for chess */
 /*
  * ref: learner_concurrent.rs:126-146, learner.rs:162-182 — the tensors the learners train on, from n compact records
  * (host only, no GPU needed): encodings[n][3][R][C] (get_encoding of the recorded root state, connect_four.rs:242-259),

@@ -36,6 +36,10 @@ pub const SPB_FLAG_LOCKSTEP: u32 = 32;
 pub const SPB_FLAG_FIXED_POOL: u32 = 16;
 pub const SPB_MOVE_GREEDY_LAST_MAX: i32 = 0;
 pub const SPB_MOVE_TEMPERATURE: i32 = 1;
+pub const SPB_DTYPE_F32: i32 = 0;
+pub const SPB_DTYPE_BF16: i32 = 1;
+pub const SPB_DTYPE_F64: i32 = 2;
+pub const SPB_DTYPE_F16: i32 = 3;
 
 #[repr(C)]
 #[derive(Clone, Copy, Debug, Default, PartialEq, Eq)]
@@ -119,6 +123,16 @@ pub struct spb_chess_position {
 }
 
 #[repr(C)]
+#[derive(Clone, Copy, Debug)]
+pub struct spb_tensor {
+    pub name: *const c_char,
+    pub data: *const c_void,
+    pub dtype: i32,
+    pub ndim: i32,
+    pub shape: [i64; 4],
+}
+
+#[repr(C)]
 pub struct spb_engine {
     _private: [u8; 0],
 }
@@ -136,6 +150,7 @@ extern "C" {
     pub fn spb_last_error(e: *const spb_engine) -> *const c_char;
     pub fn spb_load_weights(e: *mut spb_engine, blob: *const c_void, num_bytes: usize) -> i32;
     pub fn spb_check_weights(game: i32, blob: *const c_void, num_bytes: usize, err: *mut c_char, err_cap: usize) -> i32;
+    pub fn spb_load_weights_device(e: *mut spb_engine, tensors: *const spb_tensor, n: u32) -> i32;
     pub fn spb_reset_games(e: *mut spb_engine, slots: *const u32, n: u32, roots: *const spb_state) -> i32;
     pub fn spb_search(e: *mut spb_engine, num_searches: u32) -> i32;
     pub fn spb_root_children(e: *mut spb_engine, slot: u32, actions: *mut u8, visit_counts: *mut u32, child_ids: *mut u32, n_children: *mut u32) -> i32;
@@ -160,6 +175,7 @@ extern "C" {
     pub fn spb_chess_destroy(e: *mut spb_chess_engine) -> i32;
     pub fn spb_chess_last_error(e: *const spb_chess_engine) -> *const c_char;
     pub fn spb_chess_load_weights(e: *mut spb_chess_engine, blob: *const c_void, num_bytes: usize) -> i32;
+    pub fn spb_chess_load_weights_device(e: *mut spb_chess_engine, tensors: *const spb_tensor, n: u32) -> i32;
     pub fn spb_chess_check_weights(blob: *const c_void, num_bytes: usize, err: *mut c_char, err_cap: usize) -> i32;
     pub fn spb_chess_start_position(out: *mut spb_chess_state) -> i32;
     pub fn spb_chess_legal_moves(e: *mut spb_chess_engine, states: *const spb_chess_state, history: *const u64, n: u32, moves: *mut u16, counts: *mut u32, policy_index: *mut u16, status: *mut u8, repetitions: *mut u32) -> i32;
@@ -196,10 +212,12 @@ extern "C" {
     pub fn spb_comm_destroy(e: *mut spb_engine) -> i32;
     pub fn spb_gather_trajectories(e: *mut spb_engine, learner_rank: i32, buf: *mut spb_position, capacity: usize, written: *mut usize, game_ids: *mut u64) -> i32;
     pub fn spb_gather_trajectories_device(e: *mut spb_engine, learner_rank: i32, buf_dev: *mut spb_position, capacity: usize, written: *mut usize, game_ids_dev: *mut u64) -> i32;
+    pub fn spb_broadcast_weights(e: *mut spb_engine, root_rank: i32) -> i32;
     pub fn spb_chess_comm_init(e: *mut spb_chess_engine, id: *const u8, rank: i32, world_size: i32) -> i32;
     pub fn spb_chess_comm_destroy(e: *mut spb_chess_engine) -> i32;
     pub fn spb_chess_gather_trajectories(e: *mut spb_chess_engine, learner_rank: i32, buf: *mut spb_chess_position, capacity: usize, written: *mut usize, game_ids: *mut u64) -> i32;
     pub fn spb_chess_gather_trajectories_device(e: *mut spb_chess_engine, learner_rank: i32, buf_dev: *mut spb_chess_position, capacity: usize, written: *mut usize, game_ids_dev: *mut u64) -> i32;
+    pub fn spb_chess_broadcast_weights(e: *mut spb_chess_engine, root_rank: i32) -> i32;
     pub fn spb_positions_to_training(game: i32, positions: *const spb_position, n: usize, encodings: *mut f32, policies: *mut f32, values: *mut f32) -> i32;
     pub fn spb_positions_to_training_device(e: *mut spb_engine, positions_dev: *const spb_position, n_positions: usize, indices_dev: *const u64, n: usize, encodings_dev: *mut f32, policies_dev: *mut f32, values_dev: *mut f32) -> i32;
     pub fn spb_get_counters(e: *mut spb_engine, out: *mut spb_counters) -> i32;

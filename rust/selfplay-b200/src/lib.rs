@@ -22,6 +22,24 @@ pub trait AbiState: Sized {
     fn from_abi(s: &sys::spb_state) -> Self;
 }
 
+/// The `spb_tensor` table of a device load; owns the NUL-terminated names for the call.
+struct TensorTable { _names: Vec<std::ffi::CString>, raw: Vec<sys::spb_tensor> }
+impl TensorTable {
+    fn new(tensors: &[(&str, *const std::os::raw::c_void, i32, &[i64])]) -> Result<Self> {
+        let mut names = Vec::with_capacity(tensors.len());
+        let mut raw = Vec::with_capacity(tensors.len());
+        for (name, data, dtype, shape) in tensors {
+            if shape.len() > 4 { return Err(Error { code: sys::SPB_ERR_ARG, message: format!("{}: more than 4 dimensions", name) }); }
+            let c = std::ffi::CString::new(*name).map_err(|_| Error { code: sys::SPB_ERR_ARG, message: format!("{}: NUL in the name", name) })?;
+            let mut s = [0i64; 4];
+            s[..shape.len()].copy_from_slice(shape);
+            raw.push(sys::spb_tensor { name: c.as_ptr(), data: *data, dtype: *dtype, ndim: shape.len() as i32, shape: s });
+            names.push(c);
+        }
+        Ok(TensorTable { _names: names, raw })
+    }
+}
+
 /// ref: `Args` mcts.rs:8-18 — only `c` and `num_searches` are read on the search path.
 #[derive(Clone, Copy)]
 pub struct Args { pub c: f32, pub num_searches: u32, pub num_parallel_self_play_games: usize }
@@ -69,6 +87,19 @@ impl<S: AbiState> Mcts<S> {
     /// May be called again on a live engine (hot swap between generations, learner_concurrent.rs:158-159).
     pub fn load_weights(&mut self, safetensors: &[u8]) -> Result<()> {
         self.check(unsafe { sys::spb_load_weights(self.raw, safetensors.as_ptr() as *const _, safetensors.len()) })
+    }
+    /// The learner's live parameters, with no file in between: `(name, device pointer, dtype, shape)` per tensor, named as
+    /// `VarStore::variables()` names them (e.g. `tensor.data_ptr()`, `SPB_DTYPE_F32`, `tensor.size()`).  The caller has
+    /// finished writing the tensors (e.g. synchronised its stream); once this returns they may change.
+    /// # Safety
+    /// Each pointer must be a contiguous tensor of that dtype and shape in device memory of this engine's GPU.
+    pub unsafe fn load_weights_device(&mut self, tensors: &[(&str, *const std::os::raw::c_void, i32, &[i64])]) -> Result<()> {
+        let table = TensorTable::new(tensors)?;
+        self.check(sys::spb_load_weights_device(self.raw, table.raw.as_ptr(), table.raw.len() as u32))
+    }
+    /// COLLECTIVE over the communicator: every rank takes `root_rank`'s weights.
+    pub fn broadcast_weights(&mut self, root_rank: i32) -> Result<()> {
+        self.check(unsafe { sys::spb_broadcast_weights(self.raw, root_rank) })
     }
     /// EXTENSION (not in the reference, mcts.rs:204-207 is a TODO; DESIGN.md §4.6): Dirichlet noise on the root priors of
     /// every search, P' = (1 - epsilon) P + epsilon eta with eta ~ Dir(alpha).  epsilon = 0 turns it off (the default).
@@ -286,6 +317,15 @@ impl ChessMcts {
     }
     pub fn load_weights(&mut self, safetensors: &[u8]) -> Result<()> {
         self.check(unsafe { sys::spb_chess_load_weights(self.raw, safetensors.as_ptr() as *const _, safetensors.len()) })
+    }
+    /// # Safety
+    /// As `Mcts::load_weights_device`.
+    pub unsafe fn load_weights_device(&mut self, tensors: &[(&str, *const std::os::raw::c_void, i32, &[i64])]) -> Result<()> {
+        let table = TensorTable::new(tensors)?;
+        self.check(sys::spb_chess_load_weights_device(self.raw, table.raw.as_ptr(), table.raw.len() as u32))
+    }
+    pub fn broadcast_weights(&mut self, root_rank: i32) -> Result<()> {
+        self.check(unsafe { sys::spb_chess_broadcast_weights(self.raw, root_rank) })
     }
     fn padded_history(history: &[u64]) -> Vec<u64> {
         let mut h = vec![0u64; sys::SPB_CHESS_MAX_HISTORY];

@@ -145,6 +145,15 @@ class ChessEngine:
         buf = (C.c_char * len(blob)).from_buffer_copy(blob)
         self._chk(self._L.spb_chess_load_weights(self._h, C.cast(buf, C.c_void_p), len(blob)))
 
+    def load_weights_device(self, named):
+        """spb_chess_load_weights_device: the net from (name, CUDA tensor) pairs on the engine's GPU (the names of
+        load_weights); the same image as load_weights of a checkpoint of these tensors."""
+        E._load_weights_device(lambda t, n: self._chk(self._L.spb_chess_load_weights_device(self._h, t, n)), named, self.device)
+
+    def broadcast_weights(self, root: int = 0):
+        """COLLECTIVE: every rank takes root's weight image (spb_chess_broadcast_weights)."""
+        self._chk(self._L.spb_chess_broadcast_weights(self._h, root))
+
     def predict(self, states, history=None, want_logits=False):
         st = _states(states)
         n = len(st)

@@ -34,6 +34,7 @@
 
 #include <cstring>
 
+#include "bf16.cuh"
 #include "chess_engine.hpp"
 #include "chess_net.cuh"
 #include "umma_ptx.cuh"
@@ -464,14 +465,6 @@ struct Net {
   bool attrs_set = false;
 };
 
-static inline uint16_t f2bf(float f) {
-  uint32_t u;
-  std::memcpy(&u, &f, 4);
-  if ((u & 0x7F800000u) == 0x7F800000u) return (uint16_t)(u >> 16);
-  u += 0x7FFFu + ((u >> 16) & 1u);
-  return (uint16_t)(u >> 16);
-}
-
 // weight stages of one conv: [kc32][tap][4 chunks][N][8] bf16; input channels padded to kc32*32, outputs to N
 // cta_group::2 convolutions: a stage is two halves [rank][4 chunks][N/2][8], rank r = output channels r N/2 .. (r+1) N/2 - 1
 static void pack_conv(const HostNet::Conv& cv, int kc32, int N, uint16_t* dst) {
@@ -539,6 +532,19 @@ void net_destroy(Net* net) {
 }
 
 bool net_loaded(const Net* net) { return net && net->loaded; }
+void net_set_loaded(Net* net, bool ok) { net->loaded = ok; }
+
+NetImage net_image(Net* net) {
+  NetImage m;
+  m.d_w = net->d_w; m.w_bytes = net->w_bytes;
+  m.d_f = net->d_f; m.f_count = net->off_f2b + 8;
+  for (int i = 0; i < NET_CONV3; ++i) { m.off_conv[i] = net->off_conv[i]; m.off_bias[i] = net->off_bias[i]; }
+  m.off_p1 = net->off_p1; m.off_p2 = net->off_p2;
+  m.off_bp1 = net->off_bp1; m.off_bp2 = net->off_bp2; m.off_vw = net->off_vw; m.off_vb = net->off_vb;
+  m.off_f1w = net->off_f1w; m.off_f1b = net->off_f1b; m.off_f2w = net->off_f2w; m.off_f2b = net->off_f2b;
+  m.res_halves = conv_cta2(8, 9, 256);
+  return m;
+}
 
 double net_flops_per_position() {
   double f = 2.0 * 64 * NET_IN * 9 * 256;                               // stem

@@ -40,7 +40,25 @@ Net* net_create(uint32_t max_positions, std::string* err);
 void net_destroy(Net* net);
 bool net_upload(Net* net, const HostNet& host, std::string* err);
 bool net_loaded(const Net* net);
+void net_set_loaded(Net* net, bool ok);
 double net_flops_per_position();
+
+// The weight image net_upload writes, for the device packer (weights_device.cu) and the broadcast (gather.cu).
+//   d_w: per 3x3 conv (i < 21; KC32 = 1 for the stem, 8 after) and per policy 1x1 conv (p1: N = 256, p2: N = 80) the
+//        stages [kc32][tap][4 chunks][N][8] bf16 of pack_conv, output channels >= OC and input channels >= IC zero; a
+//        residual conv run by CTA pairs (res_halves) splits every stage into two halves [rank][4 chunks][N/2][8]
+//   d_f: f32 at the offsets below (in floats): folded biases, p1 / p2 biases, the value conv's weights and bias, fc1
+//        transposed to [64][256], fc1 bias, fc2 weights and bias; every other float zero
+struct NetImage {
+  uint8_t* d_w = nullptr;
+  size_t w_bytes = 0;
+  float* d_f = nullptr;
+  size_t f_count = 0;
+  size_t off_conv[NET_CONV3] = {}, off_p1 = 0, off_p2 = 0;
+  size_t off_bias[NET_CONV3] = {}, off_bp1 = 0, off_bp2 = 0, off_vw = 0, off_vb = 0, off_f1w = 0, off_f1b = 0, off_f2w = 0, off_f2b = 0;
+  bool res_halves = false;
+};
+NetImage net_image(Net* net);
 
 // Evaluates pos[list[i]] (repetition count reps[list[i]] for plane 16) for i < *count_dev (read on the device, at most the
 // capacity of activation set `set`: 0 = max_positions, 1 = half of it) and writes logits[list[i]][4672] (raw, f32) and values[list[i]] (tanh).  list == nullptr: identity.

@@ -18,6 +18,7 @@
 #include <cstring>
 #include <vector>
 
+#include "bf16.cuh"
 #include "evaluator.cuh"
 #include "evaluator_umma.cuh"
 
@@ -27,14 +28,6 @@ namespace {
 
 __device__ __forceinline__ float bf16_bits_to_float(uint16_t b) { return __uint_as_float((uint32_t)b << 16); }
 __device__ __forceinline__ float round_bf16(float x) { return __bfloat162float(__float2bfloat16_rn(x)); }
-
-inline uint16_t host_f2bf(float f) {   // round-to-nearest-even, NaN-safe enough for finite weights
-  uint32_t u;
-  std::memcpy(&u, &f, 4);
-  if ((u & 0x7F800000u) == 0x7F800000u) return (uint16_t)(u >> 16);
-  u += 0x7FFFu + ((u >> 16) & 1u);
-  return (uint16_t)(u >> 16);
-}
 
 // 3x3 conv, pad 1, over one board held in shared memory: in[IC][P] -> f(oc, p, acc + bias).
 template <class G, class F>
@@ -137,31 +130,60 @@ double Evaluator::flops_per_position() const {
   return 2.0 * macs;
 }
 
+Evaluator::Layout Evaluator::layout(int game) {
+  const bool c4 = game == SPB_GAME_CONNECT4;
+  const size_t P = c4 ? 42 : 9, A = c4 ? 7 : 9;
+  Layout L;
+  // all sections 256-byte aligned; the gaps are zero
+  auto reserve = [&](size_t bytes) { const size_t off = (L.bytes + 255) & ~(size_t)255; L.bytes = off + bytes; return off; };
+  for (int i = 0; i < NET_CONVS; ++i) {
+    const size_t oc = i <= 8 ? NET_HIDDEN : (i == 9 ? NET_POLICY_CH : NET_VALUE_CH), ic = i == 0 ? 3 : NET_HIDDEN;
+    L.wsimt[i] = reserve(oc * ic * 9 * 2);
+    L.bias[i] = reserve(oc * 4);
+  }
+  L.pw = reserve(A * NET_POLICY_CH * P * 4);
+  L.pb = reserve(A * 4);
+  L.vw = reserve(NET_VALUE_CH * P * 4);
+  L.vb = reserve(4);
+  L.umma = reserve(umma::image_layout(game).bytes);
+  return L;
+}
+
+void Evaluator::point_at(int game) {
+  const Layout L = layout(game);
+  const uint8_t* d = static_cast<const uint8_t*>(d_blob_);
+  for (int i = 0; i < NET_CONVS; ++i) {
+    dev_.w_simt[i] = reinterpret_cast<const uint16_t*>(d + L.wsimt[i]);
+    dev_.bias[i] = reinterpret_cast<const float*>(d + L.bias[i]);
+  }
+  dev_.pfc_w = reinterpret_cast<const float*>(d + L.pw);
+  dev_.pfc_b = reinterpret_cast<const float*>(d + L.pb);
+  dev_.vfc_w = reinterpret_cast<const float*>(d + L.vw);
+  dev_.vfc_b = reinterpret_cast<const float*>(d + L.vb);
+  dev_.w_umma = reinterpret_cast<const uint16_t*>(d + L.umma);
+  game_ = game;
+  rows_ = dev_.rows = game == SPB_GAME_CONNECT4 ? 6 : 3;
+  cols_ = dev_.cols = game == SPB_GAME_CONNECT4 ? 7 : 3;
+  actions_ = dev_.actions = game == SPB_GAME_CONNECT4 ? 7 : 9;
+}
+
 bool Evaluator::upload(const HostNet& net, std::string* err) {
-  const int P = net.rows * net.cols, A = net.actions;
-  // blob layout (all sections 256-byte aligned)
-  std::vector<uint8_t> blob;
-  auto reserve = [&](size_t bytes) { size_t off = (blob.size() + 255) & ~(size_t)255; blob.resize(off + bytes, 0); return off; };
-  size_t off_wsimt[NET_CONVS], off_bias[NET_CONVS];
+  const Layout L = layout(net.game);
+  std::vector<uint8_t> blob(L.bytes, 0);
   for (int i = 0; i < NET_CONVS; ++i) {
     const auto& c = net.conv[i];
-    off_wsimt[i] = reserve((size_t)c.oc * c.ic * 9 * 2);
-    uint16_t* w = reinterpret_cast<uint16_t*>(blob.data() + off_wsimt[i]);
-    for (size_t k = 0; k < c.w.size(); ++k) w[k] = host_f2bf(c.w[k]);
-    off_bias[i] = reserve((size_t)c.oc * 4);
-    std::memcpy(blob.data() + off_bias[i], c.b.data(), (size_t)c.oc * 4);
+    uint16_t* w = reinterpret_cast<uint16_t*>(blob.data() + L.wsimt[i]);
+    for (size_t k = 0; k < c.w.size(); ++k) w[k] = f2bf(c.w[k]);
+    std::memcpy(blob.data() + L.bias[i], c.b.data(), (size_t)c.oc * 4);
   }
-  const size_t off_pw = reserve(net.pfc_w.size() * 4), off_pb = reserve(net.pfc_b.size() * 4);
-  const size_t off_vw = reserve(net.vfc_w.size() * 4), off_vb = reserve(net.vfc_b.size() * 4);
-  std::memcpy(blob.data() + off_pw, net.pfc_w.data(), net.pfc_w.size() * 4);
-  std::memcpy(blob.data() + off_pb, net.pfc_b.data(), net.pfc_b.size() * 4);
-  std::memcpy(blob.data() + off_vw, net.vfc_w.data(), net.vfc_w.size() * 4);
-  std::memcpy(blob.data() + off_vb, net.vfc_b.data(), net.vfc_b.size() * 4);
+  std::memcpy(blob.data() + L.pw, net.pfc_w.data(), net.pfc_w.size() * 4);
+  std::memcpy(blob.data() + L.pb, net.pfc_b.data(), net.pfc_b.size() * 4);
+  std::memcpy(blob.data() + L.vw, net.vfc_w.data(), net.vfc_w.size() * 4);
+  std::memcpy(blob.data() + L.vb, net.vfc_b.data(), net.vfc_b.size() * 4);
   // tcgen05 operand images + epilogue tables
   std::vector<uint8_t> umma_img;
   umma::pack_weights(net, &umma_img);
-  const size_t off_umma = reserve(umma_img.size());
-  std::memcpy(blob.data() + off_umma, umma_img.data(), umma_img.size());
+  std::memcpy(blob.data() + L.umma, umma_img.data(), umma_img.size());
 
   // new image first, then swap: a failed upload keeps the previous checkpoint usable
   void* nblob = nullptr;
@@ -176,21 +198,28 @@ bool Evaluator::upload(const HostNet& net, std::string* err) {
   if (d_blob_) cudaFree(d_blob_);
   d_blob_ = nblob;
   blob_bytes_ = blob.size();
-  const uint8_t* d = static_cast<const uint8_t*>(d_blob_);
-  for (int i = 0; i < NET_CONVS; ++i) {
-    dev_.w_simt[i] = reinterpret_cast<const uint16_t*>(d + off_wsimt[i]);
-    dev_.bias[i] = reinterpret_cast<const float*>(d + off_bias[i]);
-  }
-  dev_.pfc_w = reinterpret_cast<const float*>(d + off_pw);
-  dev_.pfc_b = reinterpret_cast<const float*>(d + off_pb);
-  dev_.vfc_w = reinterpret_cast<const float*>(d + off_vw);
-  dev_.vfc_b = reinterpret_cast<const float*>(d + off_vb);
-  dev_.w_umma = reinterpret_cast<const uint16_t*>(d + off_umma);
-  dev_.rows = net.rows; dev_.cols = net.cols; dev_.actions = A;
-  game_ = net.game; rows_ = net.rows; cols_ = net.cols; actions_ = A;
-  (void)P;
+  point_at(net.game);
   loaded_ = true;
   return true;
+}
+
+uint8_t* Evaluator::image_for(int game, std::string* err) {
+  const size_t bytes = layout(game).bytes;
+  if (!d_blob_ || blob_bytes_ != bytes) {
+    void* nblob = nullptr;
+    const cudaError_t e = cudaMalloc(&nblob, bytes);
+    if (e != cudaSuccess) {
+      cudaGetLastError();
+      *err = std::string("weight image: ") + cudaGetErrorString(e);
+      return nullptr;
+    }
+    if (d_blob_) cudaFree(d_blob_);
+    d_blob_ = nblob;
+    blob_bytes_ = bytes;
+    loaded_ = false;
+    point_at(game);
+  }
+  return static_cast<uint8_t*>(d_blob_);
 }
 
 cudaError_t Evaluator::launch(const PState* states, const uint32_t* list, const uint32_t* count_dev, uint32_t max_n, float* out,

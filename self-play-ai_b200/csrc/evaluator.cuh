@@ -43,10 +43,23 @@ class Evaluator {
   Evaluator(const Evaluator&) = delete;
   Evaluator& operator=(const Evaluator&) = delete;
 
+  // Byte offsets of the sections of the weight image of `game` (upload writes them, weights_device.cu packs them on the
+  // device): per conv the bf16 weights of the SIMT kernel [OC][IC*9] and the f32 biases, the f32 Linear layers, and the
+  // tcgen05 image (umma::image_layout).  Every section starts 256-byte aligned; the gaps are zero.
+  struct Layout { size_t wsimt[NET_CONVS], bias[NET_CONVS], pw, pb, vw, vb, umma, bytes = 0; };
+  static Layout layout(int game);
+
   // Uploads the folded net: bf16 conv weights in the tcgen05 shared-memory layout + f32 biases / FCs.
   bool upload(const HostNet& net, std::string* err);
+  // The image of `game` to be rewritten in place (the device load, the broadcast of a non-root rank): allocated, and the
+  // net marked unloaded, only when there is none of that size yet; nullptr (err set) when out of memory.  The caller marks
+  // the net unloaded before it writes and loaded once the image is whole.
+  uint8_t* image_for(int game, std::string* err);
+  void set_loaded(bool ok) { loaded_ = ok; }
   bool loaded() const { return loaded_; }
   int game() const { return game_; }
+  uint8_t* image() const { return static_cast<uint8_t*>(d_blob_); }
+  size_t image_bytes() const { return blob_bytes_; }
 
   // Evaluates states[list[i]] for i < *count_dev (count read on the device; at most max_n) and writes
   // out[list[i]*stride + 0..A) = softmax(logits) (NOT masked), out[list[i]*stride + A] = tanh value.
@@ -63,6 +76,7 @@ class Evaluator {
   double flops_per_position() const;
 
  private:
+  void point_at(int game);      // dev_ and the geometry for the image of `game` in d_blob_
   bool loaded_ = false;
   int game_ = -1, rows_ = 0, cols_ = 0, actions_ = 0;
   void* d_blob_ = nullptr;      // one allocation holding everything below

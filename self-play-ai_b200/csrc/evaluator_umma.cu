@@ -33,6 +33,7 @@
 #include <cstring>
 #include <mutex>
 
+#include "bf16.cuh"
 #include "evaluator_umma.cuh"
 #include "umma_ptx.cuh"
 
@@ -75,13 +76,19 @@ template <class G> __host__ __device__ constexpr size_t image_bytes() { return o
 // ---------------------------------------------------------------------------------------------------
 // host: weight image
 // ---------------------------------------------------------------------------------------------------
-static inline uint16_t f2bf(float f) {
-  uint32_t u;
-  std::memcpy(&u, &f, 4);
-  if ((u & 0x7F800000u) == 0x7F800000u) return (uint16_t)(u >> 16);
-  u += 0x7FFFu + ((u >> 16) & 1u);
-  return (uint16_t)(u >> 16);
+template <class G>
+static ImageLayout image_layout_t() {
+  ImageLayout L;
+  for (int l = 0; l < N_LAYERS; ++l) {
+    L.layer_offset[l] = layer_offset(l);
+    L.layer_n[l] = layer_n(l);
+    L.layer_kchunks[l] = layer_kchunks(l);
+  }
+  L.off_bias = OFF_BIAS; L.off_wp = OFF_WP; L.off_wv = off_wv<G>(); L.off_fcb = off_fcb<G>(); L.bytes = image_bytes<G>();
+  return L;
 }
+
+ImageLayout image_layout(int game) { return game == SPB_GAME_CONNECT4 ? image_layout_t<Connect4>() : image_layout_t<TicTacToe>(); }
 
 template <class G>
 static void pack_t(const HostNet& net, std::vector<uint8_t>* out) {

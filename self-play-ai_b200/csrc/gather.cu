@@ -18,6 +18,7 @@
 #include <mutex>
 
 #include "chess_engine.hpp"
+#include "chess_net.cuh"
 #include "engine.hpp"
 
 using namespace spb;
@@ -30,6 +31,7 @@ struct NcclApi {
   ncclResult_t (*CommInitRank)(ncclComm_t*, int, ncclUniqueId, int) = nullptr;
   ncclResult_t (*CommDestroy)(ncclComm_t) = nullptr;
   ncclResult_t (*AllGather)(const void*, void*, size_t, ncclDataType_t, ncclComm_t, cudaStream_t) = nullptr;
+  ncclResult_t (*Broadcast)(const void*, void*, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
   ncclResult_t (*GroupStart)() = nullptr;
   ncclResult_t (*GroupEnd)() = nullptr;
   ncclResult_t (*Send)(const void*, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
@@ -54,6 +56,7 @@ NcclApi* nccl_api() {
     api.CommInitRank = reinterpret_cast<decltype(api.CommInitRank)>(sym("ncclCommInitRank"));
     api.CommDestroy = reinterpret_cast<decltype(api.CommDestroy)>(sym("ncclCommDestroy"));
     api.AllGather = reinterpret_cast<decltype(api.AllGather)>(sym("ncclAllGather"));
+    api.Broadcast = reinterpret_cast<decltype(api.Broadcast)>(sym("ncclBroadcast"));
     api.GroupStart = reinterpret_cast<decltype(api.GroupStart)>(sym("ncclGroupStart"));
     api.GroupEnd = reinterpret_cast<decltype(api.GroupEnd)>(sym("ncclGroupEnd"));
     api.Send = reinterpret_cast<decltype(api.Send)>(sym("ncclSend"));
@@ -280,6 +283,97 @@ int32_t gather_trajectories_device(HostEngine<Trees, Rec, Move>* e, int32_t lear
   return SPB_OK;
 }
 
+// ---- weight broadcast -------------------------------------------------------------------------------------------------
+// The weight image of one rank: up to two device ranges (Connect4 / tic-tac-toe: the evaluator's blob; chess: d_w, d_f).
+struct WeightImage {
+  bool ready = false;              // a range to send from or receive into exists
+  bool loaded = false;
+  int game = -1;
+  uint8_t* p[2] = {nullptr, nullptr};
+  size_t bytes[2] = {0, 0};
+};
+
+// The root sends what it holds; another rank makes room for its game's image (allocated on first use only).
+WeightImage weight_image(spb_engine* e, bool root) {
+  WeightImage w;
+  w.game = e->cfg.game;
+  std::string err;
+  w.p[0] = root ? e->evaluator.image() : e->evaluator.image_for(e->cfg.game, &err);
+  w.bytes[0] = w.p[0] ? e->evaluator.image_bytes() : 0;
+  w.ready = w.p[0] != nullptr;
+  w.loaded = e->evaluator.loaded();
+  return w;
+}
+WeightImage weight_image(spb_chess_engine* e, bool root) {
+  WeightImage w;
+  w.game = SPB_GAME_CHESS;
+  std::string err;
+  if (!e->net && !root && cudaStreamSynchronize(e->stream) == cudaSuccess) e->net = chess::net_create(e->T.G, &err);
+  if (!e->net) return w;
+  const chess::NetImage m = chess::net_image(e->net);
+  w.p[0] = m.d_w; w.bytes[0] = m.w_bytes;
+  w.p[1] = reinterpret_cast<uint8_t*>(m.d_f); w.bytes[1] = m.f_count * 4;
+  w.ready = true;
+  w.loaded = chess::net_loaded(e->net);
+  return w;
+}
+void set_weights_loaded(spb_engine* e, bool ok) {
+  e->evaluator.set_loaded(ok);
+  e->drop_step_graph();                                                // as spb_load_weights
+  e->last_eval_parity = -1;
+}
+void set_weights_loaded(spb_chess_engine* e, bool ok) { chess::net_set_loaded(e->net, ok); }
+
+// spb_broadcast_weights / spb_chess_broadcast_weights.  Phase 1: all-gather of every rank's descriptor (ready, loaded, game,
+// sizes), so that every rank reaches the same verdict and a bad root never leaves the others waiting in phase 2.  Phase 2:
+// ncclBroadcast of the image range by range on e->stream.
+template <class Eng>
+int32_t broadcast_weights(Eng* e, int32_t root) {
+  SPB_GUARD(e);
+  if (!e->nccl_comm) { e->set_error(std::string("no communicator: call ") + e->api + "comm_init first"); return SPB_ERR_STATE; }
+  SPB_ARG(e, root >= 0 && root < e->comm_world, "root rank out of range");
+  NcclApi* N = nccl_api();
+  ncclComm_t comm = static_cast<ncclComm_t>(e->nccl_comm);
+  const int rank = e->comm_rank, world = e->comm_world;
+  const bool is_root = rank == root;
+  const WeightImage w = weight_image(e, is_root);
+  constexpr int D = 4;
+  const unsigned long long mine[D] = {(w.ready ? 1ull : 0ull) | (w.loaded ? 2ull : 0ull), (unsigned long long)w.game, w.bytes[0], w.bytes[1]};
+  std::vector<unsigned long long> all((size_t)world * D);
+  if (int32_t rc = e->ensure_stage(all.size() * 8, 0)) return rc;
+  auto* d_desc = e->template d_at<unsigned long long>(0);
+  SPB_CUDA(e, cudaMemcpyAsync(d_desc + (size_t)rank * D, mine, sizeof mine, cudaMemcpyHostToDevice, e->stream));
+  SPB_NCCL(e, N->AllGather(d_desc + (size_t)rank * D, d_desc, D, ncclUint64, comm, e->stream));
+  SPB_CUDA(e, cudaMemcpyAsync(all.data(), d_desc, all.size() * 8, cudaMemcpyDeviceToHost, e->stream));
+  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
+  const unsigned long long* r0 = &all[(size_t)root * D];
+  if (!(r0[0] & 2)) {
+    e->set_error("broadcast_weights: root rank " + std::to_string(root) + " has no weights loaded");
+    return SPB_ERR_STATE;
+  }
+  for (int r = 0; r < world; ++r) {
+    const unsigned long long* d = &all[(size_t)r * D];
+    if (!(d[0] & 1)) {
+      e->set_error("broadcast_weights: rank " + std::to_string(r) + " cannot hold the weight image (out of device memory)");
+      return SPB_ERR_NOMEM;
+    }
+    if (d[1] != r0[1] || d[2] != r0[2] || d[3] != r0[3]) {
+      e->set_error("broadcast_weights: rank " + std::to_string(r) + " plays game " + std::to_string(d[1]) + ", the root game " + std::to_string(r0[1]) +
+                   " (image of " + std::to_string(d[2] + d[3]) + " bytes, the root's " + std::to_string(r0[2] + r0[3]) + ")");
+      return SPB_ERR_ARG;
+    }
+  }
+  if (!is_root) set_weights_loaded(e, false);
+  ncclResult_t nr = ncclSuccess;
+  for (int k = 0; k < 2 && nr == ncclSuccess; ++k)
+    if (w.bytes[k]) nr = N->Broadcast(w.p[k], w.p[k], w.bytes[k], ncclUint8, root, comm, e->stream);
+  const cudaError_t ce = cudaStreamSynchronize(e->stream);
+  if (nr != ncclSuccess) { e->set_error(std::string("ncclBroadcast: ") + N->GetErrorString(nr)); return SPB_ERR_CUDA; }
+  if (ce != cudaSuccess) { e->set_error(std::string("broadcast_weights: ") + cudaGetErrorString(ce)); return SPB_ERR_CUDA; }
+  if (!is_root) set_weights_loaded(e, true);
+  return SPB_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -305,6 +399,9 @@ int32_t spb_gather_trajectories_device(spb_engine* e, int32_t learner_rank, spb_
                                        uint64_t* game_ids_dev) {
   return gather_trajectories_device(e, learner_rank, buf_dev, capacity, written, game_ids_dev);
 }
+
+int32_t spb_broadcast_weights(spb_engine* e, int32_t root_rank) { return broadcast_weights(e, root_rank); }
+int32_t spb_chess_broadcast_weights(spb_chess_engine* e, int32_t root_rank) { return broadcast_weights(e, root_rank); }
 
 int32_t spb_chess_comm_init(spb_chess_engine* e, const uint8_t* id, int32_t rank, int32_t world_size) { return comm_init(e, id, rank, world_size); }
 int32_t spb_chess_comm_destroy(spb_chess_engine* e) { return comm_destroy(e); }

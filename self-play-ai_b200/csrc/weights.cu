@@ -15,22 +15,17 @@
 #include <algorithm>
 #include <cmath>
 #include <cstring>
+#include <functional>
 #include <map>
 #include <string>
 #include <vector>
 
 #include "chess_net.cuh"
 #include "evaluator.cuh"
+#include "weights.cuh"
 
 namespace spb {
 namespace {
-
-struct TensorInfo {
-  std::string name;
-  std::string dtype;
-  std::vector<int64_t> shape;
-  size_t begin = 0, end = 0;
-};
 
 // Minimal JSON reader for the safetensors header: {"name": {"dtype": "..", "shape": [..], "data_offsets": [b, e]}, ...}
 struct JsonCursor {
@@ -81,7 +76,7 @@ struct JsonCursor {
   }
 };
 
-bool parse_header(const uint8_t* blob, size_t n, std::vector<TensorInfo>* out, size_t* data_off, std::string* err) {
+bool parse_header(const uint8_t* blob, size_t n, std::vector<WeightEntry>* out, size_t* data_off, std::string* err) {
   if (n < 8) { *err = "blob shorter than the 8-byte header length"; return false; }
   uint64_t hlen = 0;
   std::memcpy(&hlen, blob, 8);
@@ -94,7 +89,7 @@ bool parse_header(const uint8_t* blob, size_t n, std::vector<TensorInfo>* out, s
     std::string name = c.str();
     if (c.fail || !c.eat(':')) { *err = "malformed header near key"; return false; }
     if (name == "__metadata__") { c.skip_value(); if (c.fail) { *err = "malformed __metadata__"; return false; } continue; }
-    TensorInfo t;
+    WeightEntry t;
     t.name = name;
     if (!c.eat('{')) { *err = "tensor entry is not an object: " + name; return false; }
     do {
@@ -120,27 +115,20 @@ bool parse_header(const uint8_t* blob, size_t n, std::vector<TensorInfo>* out, s
   return true;
 }
 
-struct Loaded {
-  std::vector<int64_t> shape;
-  std::vector<float> data;
-};
-
-bool load_f32(const uint8_t* blob, size_t n, size_t data_off, const TensorInfo& t, Loaded* out, std::string* err) {
-  size_t count = 1;
-  for (int64_t d : t.shape) { if (d < 0) { *err = "negative dim: " + t.name; return false; } count *= (size_t)d; }
-  size_t esz = t.dtype == "F32" ? 4 : (t.dtype == "F64" ? 8 : (t.dtype == "BF16" || t.dtype == "F16" ? 2 : 0));
-  if (esz == 0 || t.dtype == "F16") { *err = "unsupported dtype " + t.dtype + " for " + t.name + " (expected F32)"; return false; }
+bool load_f32(const uint8_t* blob, size_t n, size_t data_off, const WeightEntry& t, std::vector<float>* out, std::string* err) {
+  size_t count = 0;
+  const size_t esz = element_size(t, &count, err);
+  if (esz == 0) return false;
   if (t.end < t.begin || t.end - t.begin != count * esz || data_off + t.end > n) { *err = "data_offsets do not match shape: " + t.name; return false; }
   const uint8_t* src = blob + data_off + t.begin;
-  out->shape = t.shape;
-  out->data.resize(count);
-  if (t.dtype == "F32") std::memcpy(out->data.data(), src, count * 4);
-  else if (t.dtype == "F64") { for (size_t i = 0; i < count; ++i) { double d; std::memcpy(&d, src + i * 8, 8); out->data[i] = (float)d; } }
-  else { for (size_t i = 0; i < count; ++i) { uint16_t h; std::memcpy(&h, src + i * 2, 2); uint32_t u = (uint32_t)h << 16; std::memcpy(&out->data[i], &u, 4); } }
+  out->resize(count);
+  if (t.dtype == "F32") std::memcpy(out->data(), src, count * 4);
+  else if (t.dtype == "F64") { for (size_t i = 0; i < count; ++i) { double d; std::memcpy(&d, src + i * 8, 8); (*out)[i] = (float)d; } }
+  else { for (size_t i = 0; i < count; ++i) { uint16_t h; std::memcpy(&h, src + i * 2, 2); uint32_t u = (uint32_t)h << 16; std::memcpy(&(*out)[i], &u, 4); } }
   return true;
 }
 
-bool shape_is(const Loaded& l, std::initializer_list<int64_t> s) { return l.shape == std::vector<int64_t>(s); }
+bool shape_is(const WeightEntry& t, std::initializer_list<int64_t> s) { return t.shape == std::vector<int64_t>(s); }
 
 // splits "weight__12" into ("weight", 12); no suffix -> index -1 (the first variable of that name).
 void split_suffix(const std::string& name, std::string* base, long* idx) {
@@ -157,100 +145,151 @@ void split_suffix(const std::string& name, std::string* base, long* idx) {
   if (dot != std::string::npos) *base = base->substr(dot + 1);
 }
 
-}  // namespace
-
-bool parse_safetensors_net(const void* blob_v, size_t n, int game, HostNet* out, std::string* err) {
-  const uint8_t* blob = static_cast<const uint8_t*>(blob_v);
-  std::vector<TensorInfo> infos;
-  size_t data_off = 0;
-  if (!parse_header(blob, n, &infos, &data_off, err)) return false;
-  const int R = game == SPB_GAME_CONNECT4 ? 6 : 3, C = game == SPB_GAME_CONNECT4 ? 7 : 3, A = game == SPB_GAME_CONNECT4 ? 7 : 9;
-  const int P = R * C;
-  out->game = game; out->rows = R; out->cols = C; out->actions = A;
-
-  std::map<std::string, const TensorInfo*> by_name;
-  for (const auto& t : infos) by_name[t.name] = &t;
-
-  struct Raw { Loaded w, b, g, beta, mean, var; } conv[NET_CONVS];
-  Loaded pfc_w, pfc_b, vfc_w, vfc_b;
-
-  auto get = [&](const std::string& name, Loaded* dst) -> bool {
-    auto it = by_name.find(name);
-    if (it == by_name.end()) { *err = "missing tensor " + name; return false; }
-    return load_f32(blob, n, data_off, *it->second, dst, err);
-  };
-
-  if (by_name.count("conv0.weight")) {
-    for (int i = 0; i < NET_CONVS; ++i) {
-      std::string c = "conv" + std::to_string(i), b = "bn" + std::to_string(i);
-      if (!get(c + ".weight", &conv[i].w) || !get(c + ".bias", &conv[i].b) || !get(b + ".weight", &conv[i].g) ||
-          !get(b + ".bias", &conv[i].beta) || !get(b + ".running_mean", &conv[i].mean) || !get(b + ".running_var", &conv[i].var))
-        return false;
-    }
-    if (!get("policy_fc.weight", &pfc_w) || !get("policy_fc.bias", &pfc_b) || !get("value_fc.weight", &vfc_w) || !get("value_fc.bias", &vfc_b))
-      return false;
-  } else {
-    // tch creation-order scheme
-    struct Item { long idx; const TensorInfo* t; };
-    std::vector<Item> w4, w1, w2, bias, rmean, rvar;
-    for (const auto& t : infos) {
+// The tch creation-order classes: weights by rank (4: conv, 1: BatchNorm, 2: Linear), biases, running statistics, each
+// sorted by the numeric suffix.
+struct Census {
+  std::vector<size_t> w4, w1, w2, bias, rmean, rvar;
+  explicit Census(const std::vector<WeightEntry>& entries) {
+    struct Item { long idx; size_t e; };
+    std::vector<Item> c[6];
+    for (size_t e = 0; e < entries.size(); ++e) {
+      const WeightEntry& t = entries[e];
       std::string base; long idx;
       split_suffix(t.name, &base, &idx);
       if (base == "weight") {
-        if (t.shape.size() == 4) w4.push_back({idx, &t});
-        else if (t.shape.size() == 1) w1.push_back({idx, &t});
-        else if (t.shape.size() == 2) w2.push_back({idx, &t});
-      } else if (base == "bias") bias.push_back({idx, &t});
-      else if (base == "running_mean") rmean.push_back({idx, &t});
-      else if (base == "running_var") rvar.push_back({idx, &t});
+        if (t.shape.size() == 4) c[0].push_back({idx, e});
+        else if (t.shape.size() == 1) c[1].push_back({idx, e});
+        else if (t.shape.size() == 2) c[2].push_back({idx, e});
+      } else if (base == "bias") c[3].push_back({idx, e});
+      else if (base == "running_mean") c[4].push_back({idx, e});
+      else if (base == "running_var") c[5].push_back({idx, e});
     }
-    auto by_idx = [](const Item& a, const Item& b) { return a.idx < b.idx; };
-    for (auto* v : {&w4, &w1, &w2, &bias, &rmean, &rvar}) std::stable_sort(v->begin(), v->end(), by_idx);
-    if (w4.size() != NET_CONVS || w1.size() != NET_CONVS || rmean.size() != NET_CONVS || rvar.size() != NET_CONVS ||
-        w2.size() != 2 || bias.size() != 2 * NET_CONVS + 2) {
-      *err = "unexpected tensor census for the 4x64 ResNet: conv weights " + std::to_string(w4.size()) + ", bn weights " +
-             std::to_string(w1.size()) + ", linear weights " + std::to_string(w2.size()) + ", biases " + std::to_string(bias.size()) +
-             ", running_mean " + std::to_string(rmean.size()) + ", running_var " + std::to_string(rvar.size());
+    std::vector<size_t>* out[6] = {&w4, &w1, &w2, &bias, &rmean, &rvar};
+    for (int k = 0; k < 6; ++k) {
+      std::stable_sort(c[k].begin(), c[k].end(), [](const Item& a, const Item& b) { return a.idx < b.idx; });
+      for (const Item& it : c[k]) out[k]->push_back(it.e);
+    }
+  }
+};
+
+// Assigns roles and calls take in order; `set(role, entry)` records and takes one role.
+struct Assign {
+  size_t* role_entry;
+  const TakeRole& take;
+  std::string* err;
+  bool operator()(int role, size_t e) const { role_entry[role] = e; return take(role, e, err); }
+};
+
+// The explicit names of conv i: conv{i}.{weight,bias}, bn{i}.{weight,bias,running_mean,running_var}, taken in that order.
+bool take_explicit_conv(const std::map<std::string, size_t>& by_name, int i, const Assign& set, std::string* err) {
+  const std::string c = "conv" + std::to_string(i), b = "bn" + std::to_string(i);
+  const std::string names[6] = {c + ".weight", c + ".bias", b + ".weight", b + ".bias", b + ".running_mean", b + ".running_var"};
+  for (int k = 0; k < 6; ++k) {
+    auto it = by_name.find(names[k]);
+    if (it == by_name.end()) { *err = "missing tensor " + names[k]; return false; }
+    if (!set(6 * i + k, it->second)) return false;
+  }
+  return true;
+}
+
+bool take_named(const std::map<std::string, size_t>& by_name, const char* name, int role, const Assign& set, std::string* err) {
+  auto it = by_name.find(name);
+  if (it == by_name.end()) { *err = std::string("missing tensor ") + name; return false; }
+  return set(role, it->second);
+}
+
+// The shapes of conv i's six roles: weight [oc][ic][3][3], the rest [oc].
+bool conv_shapes_are(const std::vector<WeightEntry>& t, const size_t* re, int i, int oc, int ic) {
+  if (!shape_is(t[re[6 * i + ROLE_W]], {oc, ic, 3, 3})) return false;
+  for (int k = ROLE_B; k <= ROLE_VAR; ++k)
+    if (!shape_is(t[re[6 * i + k]], {oc})) return false;
+  return true;
+}
+
+// BatchNorm (eval mode) folded into conv i: y = (conv(x)+b - mean) * g / sqrt(var + eps) + beta
+template <class Conv>
+void fold_conv(const std::vector<float>* raw, int i, int oc, int ic, float eps, Conv* h) {
+  const std::vector<float> &w = raw[6 * i + ROLE_W], &b = raw[6 * i + ROLE_B], &g = raw[6 * i + ROLE_G], &beta = raw[6 * i + ROLE_BETA],
+                           &mean = raw[6 * i + ROLE_MEAN], &var = raw[6 * i + ROLE_VAR];
+  h->oc = oc; h->ic = ic;
+  h->w.resize((size_t)oc * ic * 9);
+  h->b.resize(oc);
+  for (int o = 0; o < oc; ++o) {
+    const double s = (double)g[o] / std::sqrt((double)var[o] + (double)eps);
+    for (int k = 0; k < ic * 9; ++k) h->w[(size_t)o * ic * 9 + k] = (float)((double)w[(size_t)o * ic * 9 + k] * s);
+    h->b[o] = (float)(((double)b[o] - (double)mean[o]) * s + (double)beta[o]);
+  }
+}
+
+}  // namespace
+
+size_t element_size(const WeightEntry& t, size_t* count, std::string* err) {
+  *count = 1;
+  for (int64_t d : t.shape) { if (d < 0) { *err = "negative dim: " + t.name; return 0; } *count *= (size_t)d; }
+  size_t esz = t.dtype == "F32" ? 4 : (t.dtype == "F64" ? 8 : (t.dtype == "BF16" || t.dtype == "F16" ? 2 : 0));
+  if (esz == 0 || t.dtype == "F16") { *err = "unsupported dtype " + t.dtype + " for " + t.name + " (expected F32)"; return 0; }
+  return esz;
+}
+
+bool resolve_net(const std::vector<WeightEntry>& entries, int game, size_t* re, const TakeRole& take, std::string* err) {
+  const int P = game == SPB_GAME_CONNECT4 ? 42 : 9, A = game == SPB_GAME_CONNECT4 ? 7 : 9;
+  std::map<std::string, size_t> by_name;
+  for (size_t e = 0; e < entries.size(); ++e) by_name[entries[e].name] = e;
+  const Assign set{re, take, err};
+  if (by_name.count("conv0.weight")) {
+    for (int i = 0; i < NET_CONVS; ++i)
+      if (!take_explicit_conv(by_name, i, set, err)) return false;
+    if (!take_named(by_name, "policy_fc.weight", NET_ROLE_PFC_W, set, err) || !take_named(by_name, "policy_fc.bias", NET_ROLE_PFC_B, set, err) ||
+        !take_named(by_name, "value_fc.weight", NET_ROLE_VFC_W, set, err) || !take_named(by_name, "value_fc.bias", NET_ROLE_VFC_B, set, err))
+      return false;
+  } else {
+    // tch creation-order scheme
+    const Census c(entries);
+    if (c.w4.size() != NET_CONVS || c.w1.size() != NET_CONVS || c.rmean.size() != NET_CONVS || c.rvar.size() != NET_CONVS ||
+        c.w2.size() != 2 || c.bias.size() != 2 * NET_CONVS + 2) {
+      *err = "unexpected tensor census for the 4x64 ResNet: conv weights " + std::to_string(c.w4.size()) + ", bn weights " +
+             std::to_string(c.w1.size()) + ", linear weights " + std::to_string(c.w2.size()) + ", biases " + std::to_string(c.bias.size()) +
+             ", running_mean " + std::to_string(c.rmean.size()) + ", running_var " + std::to_string(c.rvar.size());
       return false;
     }
     // bias order: conv0, bn0, ..., conv8, bn8, conv9, bn9, policy_fc, conv10, bn10, value_fc
     int bi = 0;
     for (int i = 0; i < NET_CONVS; ++i) {
-      if (!load_f32(blob, n, data_off, *w4[i].t, &conv[i].w, err) || !load_f32(blob, n, data_off, *w1[i].t, &conv[i].g, err) ||
-          !load_f32(blob, n, data_off, *rmean[i].t, &conv[i].mean, err) || !load_f32(blob, n, data_off, *rvar[i].t, &conv[i].var, err))
+      if (!set(6 * i + ROLE_W, c.w4[i]) || !set(6 * i + ROLE_G, c.w1[i]) || !set(6 * i + ROLE_MEAN, c.rmean[i]) || !set(6 * i + ROLE_VAR, c.rvar[i]))
         return false;
-      if (!load_f32(blob, n, data_off, *bias[bi++].t, &conv[i].b, err) || !load_f32(blob, n, data_off, *bias[bi++].t, &conv[i].beta, err))
-        return false;
-      if (i == 9) { if (!load_f32(blob, n, data_off, *bias[bi++].t, &pfc_b, err)) return false; }
-      if (i == 10) { if (!load_f32(blob, n, data_off, *bias[bi++].t, &vfc_b, err)) return false; }
+      if (!set(6 * i + ROLE_B, c.bias[bi++]) || !set(6 * i + ROLE_BETA, c.bias[bi++])) return false;
+      if (i == 9 && !set(NET_ROLE_PFC_B, c.bias[bi++])) return false;
+      if (i == 10 && !set(NET_ROLE_VFC_B, c.bias[bi++])) return false;
     }
-    if (!load_f32(blob, n, data_off, *w2[0].t, &pfc_w, err) || !load_f32(blob, n, data_off, *w2[1].t, &vfc_w, err)) return false;
+    if (!set(NET_ROLE_PFC_W, c.w2[0]) || !set(NET_ROLE_VFC_W, c.w2[1])) return false;
   }
-
-  // shape checks + BN folding (eval mode): y = (conv(x)+b - mean) * g / sqrt(var + eps) + beta
   for (int i = 0; i < NET_CONVS; ++i) {
     const int ic = i == 0 ? 3 : NET_HIDDEN;
     const int oc = i <= 8 ? NET_HIDDEN : (i == 9 ? NET_POLICY_CH : NET_VALUE_CH);
-    if (!shape_is(conv[i].w, {oc, ic, 3, 3}) || !shape_is(conv[i].b, {oc}) || !shape_is(conv[i].g, {oc}) || !shape_is(conv[i].beta, {oc}) ||
-        !shape_is(conv[i].mean, {oc}) || !shape_is(conv[i].var, {oc})) {
-      *err = "shape mismatch in conv/bn layer " + std::to_string(i);
-      return false;
-    }
-    HostNet::Conv& h = out->conv[i];
-    h.oc = oc; h.ic = ic;
-    h.w.resize((size_t)oc * ic * 9);
-    h.b.resize(oc);
-    for (int o = 0; o < oc; ++o) {
-      double s = (double)conv[i].g.data[o] / std::sqrt((double)conv[i].var.data[o] + (double)BN_EPS);
-      for (int k = 0; k < ic * 9; ++k) h.w[(size_t)o * ic * 9 + k] = (float)((double)conv[i].w.data[(size_t)o * ic * 9 + k] * s);
-      h.b[o] = (float)(((double)conv[i].b.data[o] - (double)conv[i].mean.data[o]) * s + (double)conv[i].beta.data[o]);
-    }
+    if (!conv_shapes_are(entries, re, i, oc, ic)) { *err = "shape mismatch in conv/bn layer " + std::to_string(i); return false; }
   }
-  if (!shape_is(pfc_w, {A, NET_POLICY_CH * P}) || !shape_is(pfc_b, {A}) || !shape_is(vfc_w, {1, NET_VALUE_CH * P}) || !shape_is(vfc_b, {1})) {
+  if (!shape_is(entries[re[NET_ROLE_PFC_W]], {A, NET_POLICY_CH * P}) || !shape_is(entries[re[NET_ROLE_PFC_B]], {A}) ||
+      !shape_is(entries[re[NET_ROLE_VFC_W]], {1, NET_VALUE_CH * P}) || !shape_is(entries[re[NET_ROLE_VFC_B]], {1})) {
     *err = "shape mismatch in the policy/value linear layers";
     return false;
   }
-  out->pfc_w = pfc_w.data; out->pfc_b = pfc_b.data; out->vfc_w = vfc_w.data; out->vfc_b = vfc_b.data;
+  return true;
+}
+
+bool parse_safetensors_net(const void* blob_v, size_t n, int game, HostNet* out, std::string* err) {
+  const uint8_t* blob = static_cast<const uint8_t*>(blob_v);
+  std::vector<WeightEntry> infos;
+  size_t data_off = 0;
+  if (!parse_header(blob, n, &infos, &data_off, err)) return false;
+  out->game = game; out->rows = game == SPB_GAME_CONNECT4 ? 6 : 3; out->cols = game == SPB_GAME_CONNECT4 ? 7 : 3;
+  out->actions = game == SPB_GAME_CONNECT4 ? 7 : 9;
+  std::vector<float> raw[NET_ROLES];
+  size_t re[NET_ROLES];
+  const TakeRole load = [&](int role, size_t e, std::string* er) { return load_f32(blob, n, data_off, infos[e], &raw[role], er); };
+  if (!resolve_net(infos, game, re, load, err)) return false;
+  for (int i = 0; i < NET_CONVS; ++i)
+    fold_conv(raw, i, i <= 8 ? NET_HIDDEN : (i == 9 ? NET_POLICY_CH : NET_VALUE_CH), i == 0 ? 3 : NET_HIDDEN, BN_EPS, &out->conv[i]);
+  out->pfc_w = raw[NET_ROLE_PFC_W]; out->pfc_b = raw[NET_ROLE_PFC_B]; out->vfc_w = raw[NET_ROLE_VFC_W]; out->vfc_b = raw[NET_ROLE_VFC_B];
   return true;
 }
 
@@ -259,97 +298,72 @@ bool parse_safetensors_net(const void* blob_v, size_t n, int game, HostNet* out,
 // Explicit names: conv{i}.{weight,bias} + bn{i}.{weight,bias,running_mean,running_var} for i = 0 (stem), 1..20 (residual
 // convs); policy_conv1 / policy_conv2 / value_conv / value_fc1 / value_fc2 .{weight,bias}.  tch VarStore names: creation
 // order as for the small nets — torso (conv, bn) x 21, policy convs, value conv, the two Linear layers.
+bool resolve_chess(const std::vector<WeightEntry>& entries, size_t* re, const TakeRole& take, std::string* err) {
+  using chess::NET_CONV3; using chess::NET_IN; using chess::NET_MOVE_PLANES;
+  constexpr int NET_HIDDEN = chess::NET_HIDDEN;
+  std::map<std::string, size_t> by_name;
+  for (size_t e = 0; e < entries.size(); ++e) by_name[entries[e].name] = e;
+  const Assign set{re, take, err};
+  if (by_name.count("conv0.weight")) {
+    for (int i = 0; i < NET_CONV3; ++i)
+      if (!take_explicit_conv(by_name, i, set, err)) return false;
+    static const char* const heads[10] = {"policy_conv1.weight", "policy_conv1.bias", "policy_conv2.weight", "policy_conv2.bias", "value_conv.weight",
+                                          "value_conv.bias",     "value_fc1.weight",  "value_fc1.bias",      "value_fc2.weight",  "value_fc2.bias"};
+    for (int k = 0; k < 10; ++k)
+      if (!take_named(by_name, heads[k], CH_ROLE_P1_W + k, set, err)) return false;
+  } else {
+    const Census c(entries);
+    if (c.w4.size() != NET_CONV3 + 3 || c.w1.size() != NET_CONV3 || c.rmean.size() != NET_CONV3 || c.rvar.size() != NET_CONV3 || c.w2.size() != 2 ||
+        c.bias.size() != 2 * NET_CONV3 + 5) {
+      *err = "unexpected tensor census for the chess 10x256 ResNet: conv weights " + std::to_string(c.w4.size()) + ", bn weights " +
+             std::to_string(c.w1.size()) + ", linear weights " + std::to_string(c.w2.size()) + ", biases " + std::to_string(c.bias.size());
+      return false;
+    }
+    int bi = 0;
+    for (int i = 0; i < NET_CONV3; ++i)
+      if (!set(6 * i + ROLE_W, c.w4[i]) || !set(6 * i + ROLE_G, c.w1[i]) || !set(6 * i + ROLE_MEAN, c.rmean[i]) || !set(6 * i + ROLE_VAR, c.rvar[i]) ||
+          !set(6 * i + ROLE_B, c.bias[bi++]) || !set(6 * i + ROLE_BETA, c.bias[bi++]))
+        return false;
+    if (!set(CH_ROLE_P1_W, c.w4[NET_CONV3]) || !set(CH_ROLE_P1_B, c.bias[bi++]) || !set(CH_ROLE_P2_W, c.w4[NET_CONV3 + 1]) ||
+        !set(CH_ROLE_P2_B, c.bias[bi++]) || !set(CH_ROLE_V_W, c.w4[NET_CONV3 + 2]) || !set(CH_ROLE_V_B, c.bias[bi++]) ||
+        !set(CH_ROLE_F1_W, c.w2[0]) || !set(CH_ROLE_F1_B, c.bias[bi++]) || !set(CH_ROLE_F2_W, c.w2[1]) || !set(CH_ROLE_F2_B, c.bias[bi++]))
+      return false;
+  }
+  for (int i = 0; i < NET_CONV3; ++i)
+    if (!conv_shapes_are(entries, re, i, NET_HIDDEN, i == 0 ? NET_IN : NET_HIDDEN)) {
+      *err = "shape mismatch in conv/bn layer " + std::to_string(i) + " of the chess net";
+      return false;
+    }
+  auto is = [&](int role, std::initializer_list<int64_t> s) { return shape_is(entries[re[role]], s); };
+  if (!is(CH_ROLE_P1_W, {NET_HIDDEN, NET_HIDDEN, 1, 1}) || !is(CH_ROLE_P1_B, {NET_HIDDEN}) || !is(CH_ROLE_P2_W, {NET_MOVE_PLANES, NET_HIDDEN, 1, 1}) ||
+      !is(CH_ROLE_P2_B, {NET_MOVE_PLANES}) || !is(CH_ROLE_V_W, {1, NET_HIDDEN, 1, 1}) || !is(CH_ROLE_V_B, {1}) || !is(CH_ROLE_F1_W, {256, 64}) ||
+      !is(CH_ROLE_F1_B, {256}) || !is(CH_ROLE_F2_W, {1, 256}) || !is(CH_ROLE_F2_B, {1})) {
+    *err = "shape mismatch in the heads of the chess net";
+    return false;
+  }
+  return true;
+}
+
 namespace chess {
 
 bool parse_safetensors_chess(const void* blob_v, size_t n, HostNet* out, std::string* err) {
   const uint8_t* blob = static_cast<const uint8_t*>(blob_v);
-  std::vector<TensorInfo> infos;
+  std::vector<WeightEntry> infos;
   size_t data_off = 0;
   if (!parse_header(blob, n, &infos, &data_off, err)) return false;
-  std::map<std::string, const TensorInfo*> by_name;
-  for (const auto& t : infos) by_name[t.name] = &t;
-  struct Raw { Loaded w, b, g, beta, mean, var; } conv[NET_CONV3];
-  Loaded p1w, p1b, p2w, p2b, vw, vb, f1w, f1b, f2w, f2b;
-  auto get = [&](const std::string& name, Loaded* dst) -> bool {
-    auto it = by_name.find(name);
-    if (it == by_name.end()) { *err = "missing tensor " + name; return false; }
-    return load_f32(blob, n, data_off, *it->second, dst, err);
-  };
-  if (by_name.count("conv0.weight")) {
-    for (int i = 0; i < NET_CONV3; ++i) {
-      const std::string c = "conv" + std::to_string(i), b = "bn" + std::to_string(i);
-      if (!get(c + ".weight", &conv[i].w) || !get(c + ".bias", &conv[i].b) || !get(b + ".weight", &conv[i].g) ||
-          !get(b + ".bias", &conv[i].beta) || !get(b + ".running_mean", &conv[i].mean) || !get(b + ".running_var", &conv[i].var))
-        return false;
-    }
-    if (!get("policy_conv1.weight", &p1w) || !get("policy_conv1.bias", &p1b) || !get("policy_conv2.weight", &p2w) ||
-        !get("policy_conv2.bias", &p2b) || !get("value_conv.weight", &vw) || !get("value_conv.bias", &vb) ||
-        !get("value_fc1.weight", &f1w) || !get("value_fc1.bias", &f1b) || !get("value_fc2.weight", &f2w) || !get("value_fc2.bias", &f2b))
-      return false;
-  } else {
-    struct Item { long idx; const TensorInfo* t; };
-    std::vector<Item> w4, w1, w2, bias, rmean, rvar;
-    for (const auto& t : infos) {
-      std::string base; long idx;
-      split_suffix(t.name, &base, &idx);
-      if (base == "weight") {
-        if (t.shape.size() == 4) w4.push_back({idx, &t});
-        else if (t.shape.size() == 1) w1.push_back({idx, &t});
-        else if (t.shape.size() == 2) w2.push_back({idx, &t});
-      } else if (base == "bias") bias.push_back({idx, &t});
-      else if (base == "running_mean") rmean.push_back({idx, &t});
-      else if (base == "running_var") rvar.push_back({idx, &t});
-    }
-    auto by_idx = [](const Item& a, const Item& b) { return a.idx < b.idx; };
-    for (auto* v : {&w4, &w1, &w2, &bias, &rmean, &rvar}) std::stable_sort(v->begin(), v->end(), by_idx);
-    if (w4.size() != NET_CONV3 + 3 || w1.size() != NET_CONV3 || rmean.size() != NET_CONV3 || rvar.size() != NET_CONV3 || w2.size() != 2 ||
-        bias.size() != 2 * NET_CONV3 + 5) {
-      *err = "unexpected tensor census for the chess 10x256 ResNet: conv weights " + std::to_string(w4.size()) + ", bn weights " +
-             std::to_string(w1.size()) + ", linear weights " + std::to_string(w2.size()) + ", biases " + std::to_string(bias.size());
-      return false;
-    }
-    int bi = 0;
-    for (int i = 0; i < NET_CONV3; ++i) {
-      if (!load_f32(blob, n, data_off, *w4[i].t, &conv[i].w, err) || !load_f32(blob, n, data_off, *w1[i].t, &conv[i].g, err) ||
-          !load_f32(blob, n, data_off, *rmean[i].t, &conv[i].mean, err) || !load_f32(blob, n, data_off, *rvar[i].t, &conv[i].var, err) ||
-          !load_f32(blob, n, data_off, *bias[bi++].t, &conv[i].b, err) || !load_f32(blob, n, data_off, *bias[bi++].t, &conv[i].beta, err))
-        return false;
-    }
-    if (!load_f32(blob, n, data_off, *w4[NET_CONV3].t, &p1w, err) || !load_f32(blob, n, data_off, *bias[bi++].t, &p1b, err) ||
-        !load_f32(blob, n, data_off, *w4[NET_CONV3 + 1].t, &p2w, err) || !load_f32(blob, n, data_off, *bias[bi++].t, &p2b, err) ||
-        !load_f32(blob, n, data_off, *w4[NET_CONV3 + 2].t, &vw, err) || !load_f32(blob, n, data_off, *bias[bi++].t, &vb, err) ||
-        !load_f32(blob, n, data_off, *w2[0].t, &f1w, err) || !load_f32(blob, n, data_off, *bias[bi++].t, &f1b, err) ||
-        !load_f32(blob, n, data_off, *w2[1].t, &f2w, err) || !load_f32(blob, n, data_off, *bias[bi++].t, &f2b, err))
-      return false;
-  }
+  std::vector<float> raw[CH_ROLES];
+  size_t re[CH_ROLES];
+  const TakeRole load = [&](int role, size_t e, std::string* er) { return load_f32(blob, n, data_off, infos[e], &raw[role], er); };
+  if (!resolve_chess(infos, re, load, err)) return false;
   for (int i = 0; i < NET_CONV3; ++i) {
-    const int ic = i == 0 ? NET_IN : NET_HIDDEN, oc = NET_HIDDEN;
-    if (!shape_is(conv[i].w, {oc, ic, 3, 3}) || !shape_is(conv[i].b, {oc}) || !shape_is(conv[i].g, {oc}) || !shape_is(conv[i].beta, {oc}) ||
-        !shape_is(conv[i].mean, {oc}) || !shape_is(conv[i].var, {oc})) {
-      *err = "shape mismatch in conv/bn layer " + std::to_string(i) + " of the chess net";
-      return false;
-    }
-    HostNet::Conv& h = out->conv3[i];
-    h.oc = oc; h.ic = ic; h.k = 3;
-    h.w.resize((size_t)oc * ic * 9);
-    h.b.resize(oc);
-    for (int o = 0; o < oc; ++o) {
-      const double s = (double)conv[i].g.data[o] / std::sqrt((double)conv[i].var.data[o] + (double)NET_BN_EPS);
-      for (int k = 0; k < ic * 9; ++k) h.w[(size_t)o * ic * 9 + k] = (float)((double)conv[i].w.data[(size_t)o * ic * 9 + k] * s);
-      h.b[o] = (float)(((double)conv[i].b.data[o] - (double)conv[i].mean.data[o]) * s + (double)conv[i].beta.data[o]);
-    }
+    fold_conv(raw, i, NET_HIDDEN, i == 0 ? NET_IN : NET_HIDDEN, NET_BN_EPS, &out->conv3[i]);
+    out->conv3[i].k = 3;
   }
-  if (!shape_is(p1w, {NET_HIDDEN, NET_HIDDEN, 1, 1}) || !shape_is(p1b, {NET_HIDDEN}) || !shape_is(p2w, {NET_MOVE_PLANES, NET_HIDDEN, 1, 1}) ||
-      !shape_is(p2b, {NET_MOVE_PLANES}) || !shape_is(vw, {1, NET_HIDDEN, 1, 1}) || !shape_is(vb, {1}) || !shape_is(f1w, {256, 64}) ||
-      !shape_is(f1b, {256}) || !shape_is(f2w, {1, 256}) || !shape_is(f2b, {1})) {
-    *err = "shape mismatch in the heads of the chess net";
-    return false;
-  }
-  auto set1x1 = [](HostNet::Conv& h, const Loaded& w, const Loaded& b, int oc) { h.oc = oc; h.ic = NET_HIDDEN; h.k = 1; h.w = w.data; h.b = b.data; };
-  set1x1(out->p1, p1w, p1b, NET_HIDDEN);
-  set1x1(out->p2, p2w, p2b, NET_MOVE_PLANES);
-  set1x1(out->vconv, vw, vb, 1);
-  out->fc1_w = f1w.data; out->fc1_b = f1b.data; out->fc2_w = f2w.data; out->fc2_b = f2b.data;
+  auto set1x1 = [&](HostNet::Conv& h, int role_w, int oc) { h.oc = oc; h.ic = NET_HIDDEN; h.k = 1; h.w = raw[role_w]; h.b = raw[role_w + 1]; };
+  set1x1(out->p1, CH_ROLE_P1_W, NET_HIDDEN);
+  set1x1(out->p2, CH_ROLE_P2_W, NET_MOVE_PLANES);
+  set1x1(out->vconv, CH_ROLE_V_W, 1);
+  out->fc1_w = raw[CH_ROLE_F1_W]; out->fc1_b = raw[CH_ROLE_F1_B]; out->fc2_w = raw[CH_ROLE_F2_W]; out->fc2_b = raw[CH_ROLE_F2_B];
   return true;
 }
 

@@ -68,6 +68,16 @@ POSITION_DTYPE = np.dtype([("stones", "<u8", (2,)), ("visit_counts", "<u4", (MAX
 assert STATE_DTYPE.itemsize == C.sizeof(State) == 24
 assert POSITION_DTYPE.itemsize == C.sizeof(Position) == 56
 
+DTYPE_F32, DTYPE_BF16, DTYPE_F64, DTYPE_F16 = 0, 1, 2, 3
+
+
+class Tensor(C.Structure):
+    """spb_tensor: one entry of the table spb_load_weights_device reads (a device tensor and its checkpoint name)."""
+    _fields_ = [("name", C.c_char_p), ("data", C.c_void_p), ("dtype", C.c_int32), ("ndim", C.c_int32), ("shape", C.c_int64 * 4)]
+
+
+assert C.sizeof(Tensor) == 56
+
 # Every symbol include/selfplay_b200.h declares: name -> (restype, argtypes)
 _u32p, _u8p, _f32p, _i32p = C.POINTER(C.c_uint32), C.POINTER(C.c_uint8), C.POINTER(C.c_float), C.POINTER(C.c_int32)
 _vp = C.c_void_p
@@ -79,6 +89,8 @@ ABI = {
     "spb_last_error": (C.c_char_p, [_vp]),
     "spb_load_weights": (C.c_int32, [_vp, _vp, C.c_size_t]),
     "spb_check_weights": (C.c_int32, [C.c_int32, _vp, C.c_size_t, C.c_char_p, C.c_size_t]),
+    "spb_load_weights_device": (C.c_int32, [_vp, C.POINTER(Tensor), C.c_uint32]),
+    "spb_broadcast_weights": (C.c_int32, [_vp, C.c_int32]),
     "spb_reset_games": (C.c_int32, [_vp, _vp, C.c_uint32, _vp]),
     "spb_search": (C.c_int32, [_vp, C.c_uint32]),
     "spb_root_children": (C.c_int32, [_vp, C.c_uint32, _u8p, _u32p, _u32p, _u32p]),
@@ -110,6 +122,8 @@ ABI = {
     "spb_chess_last_error": (C.c_char_p, [_vp]),
     "spb_chess_load_weights": (C.c_int32, [_vp, _vp, C.c_size_t]),
     "spb_chess_check_weights": (C.c_int32, [_vp, C.c_size_t, C.c_char_p, C.c_size_t]),
+    "spb_chess_load_weights_device": (C.c_int32, [_vp, C.POINTER(Tensor), C.c_uint32]),
+    "spb_chess_broadcast_weights": (C.c_int32, [_vp, C.c_int32]),
     "spb_chess_start_position": (C.c_int32, [_vp]),
     "spb_chess_legal_moves": (C.c_int32, [_vp, _vp, _vp, C.c_uint32, _vp, _vp, _vp, _vp, _vp]),
     "spb_chess_next_states": (C.c_int32, [_vp, _vp, _vp, _vp, C.c_uint32, _vp, _vp]),
@@ -230,6 +244,48 @@ def positions_to_training(game: int, positions: np.ndarray):
     if rc != 0:
         raise EngineError(rc, "spb_positions_to_training: bad argument")
     return enc, pol, val
+
+
+def _dtype_codes():
+    import torch
+    return {torch.float32: DTYPE_F32, torch.bfloat16: DTYPE_BF16, torch.float64: DTYPE_F64, torch.float16: DTYPE_F16}
+
+
+def tensor_table(named, device):
+    """(name, tensor) pairs (a mapping or an iterable, e.g. a module's state_dict() or tch's VarStore::variables()) ->
+    (ctypes array of spb_tensor, n, the encoded names to keep alive for the call).  Every tensor must be a contiguous CUDA
+    tensor on `device` of at most 4 dimensions, in f32, bf16 or f64 (f16 is passed on and refused by the library, as in a
+    checkpoint)."""
+    import torch
+    items = list(named.items()) if hasattr(named, "items") else list(named)
+    codes = _dtype_codes()
+    table = (Tensor * max(len(items), 1))()
+    names = []
+    for i, (name, t) in enumerate(items):
+        if not isinstance(t, torch.Tensor) or not t.is_cuda:
+            raise TypeError("%s must be a CUDA tensor" % name)
+        if t.device.index != device:
+            raise ValueError("%s is on %s, the engine on cuda:%d" % (name, t.device, device))
+        if not t.is_contiguous():
+            raise ValueError("%s must be contiguous" % name)
+        if t.dim() > 4 or t.dtype not in codes:
+            raise ValueError("%s: %d dimensions of %s (at most 4 of float32, bfloat16, float64)" % (name, t.dim(), t.dtype))
+        names.append(name.encode())
+        table[i].name, table[i].data = names[-1], t.data_ptr()
+        table[i].dtype, table[i].ndim = codes[t.dtype], t.dim()
+        for k, d in enumerate(t.shape):
+            table[i].shape[k] = d
+    return table, len(items), names
+
+
+def _load_weights_device(call, named, device):
+    """The device loads: the caller's writes to the tensors finish before the engine reads them; `items` and `names` keep
+    the tensors and the table's names alive until the call has returned, after which the engine no longer reads them."""
+    import torch
+    items = list(named.items()) if hasattr(named, "items") else list(named)
+    table, n, names = tensor_table(items, device)
+    torch.cuda.current_stream(torch.device("cuda", device)).synchronize()
+    call(table, n)
 
 
 def _check_cuda_tensor(t, dtype, width, name):
@@ -353,6 +409,15 @@ class Engine:
     def load_weights(self, blob: bytes):
         buf = (C.c_char * len(blob)).from_buffer_copy(blob)
         self._chk(self._L.spb_load_weights(self._h, C.cast(buf, _vp), len(blob)))
+
+    def load_weights_device(self, named):
+        """spb_load_weights_device: the net from (name, CUDA tensor) pairs on the engine's GPU, named as in a checkpoint
+        (explicit names or tch VarStore names); the same image as load_weights of a checkpoint of these tensors."""
+        _load_weights_device(lambda t, n: self._chk(self._L.spb_load_weights_device(self._h, t, n)), named, self.device)
+
+    def broadcast_weights(self, root: int = 0):
+        """COLLECTIVE: every rank takes root's weight image (spb_broadcast_weights)."""
+        self._chk(self._L.spb_broadcast_weights(self._h, root))
 
     # ---- trees -------------------------------------------------------------------------------
     def reset_games(self, roots=None, slots=None):

@@ -85,6 +85,10 @@ class Mcts {
 
   // ref: VarStore::load, main.rs:61 — the bytes of the safetensors file VarStore::save wrote (learner.rs:192).
   void load_weights(const std::vector<uint8_t>& safetensors) { check(spb_load_weights(e_, safetensors.data(), safetensors.size())); }
+  // The learner's device tensors, named as in the checkpoint (spb_load_weights_device); they may change once this returns.
+  void load_weights_device(const std::vector<spb_tensor>& tensors) { check(spb_load_weights_device(e_, tensors.data(), (uint32_t)tensors.size())); }
+  // COLLECTIVE: every rank takes root_rank's weights.
+  void broadcast_weights(int32_t root_rank) { check(spb_broadcast_weights(e_, root_rank)); }
 
   // ref: Tree::default (mcts.rs:67) / Tree::with_root_state (mcts.rs:86)
   Tree make_tree(uint32_t slot) { check(spb_reset_games(e_, &slot, 1, nullptr)); return Tree(slot); }
@@ -195,6 +199,8 @@ class ChessMcts {
   ChessMcts& operator=(const ChessMcts&) = delete;
 
   void load_weights(const std::vector<uint8_t>& safetensors) { check(spb_chess_load_weights(e_, safetensors.data(), safetensors.size())); }
+  void load_weights_device(const std::vector<spb_tensor>& tensors) { check(spb_chess_load_weights_device(e_, tensors.data(), (uint32_t)tensors.size())); }
+  void broadcast_weights(int32_t root_rank) { check(spb_chess_broadcast_weights(e_, root_rank)); }
   // ref: Tree::with_root_state, mcts.rs:86
   ChessTree with_root_state(uint32_t slot, const ChessState& s) {
     std::vector<uint64_t> h(SPB_CHESS_MAX_HISTORY, 0);
