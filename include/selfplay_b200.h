@@ -190,6 +190,11 @@ int32_t spb_reset_games(spb_engine* e, const uint32_t* slots, uint32_t n, const 
  * ref: Mcts::search mcts.rs:196-332.  Runs `num_searches` lock-step simulations
  * (mcts.rs:214) for every slot.  Statistics accumulate on top of whatever the tree
  * already holds (subtree reuse, mcts.rs:161-192).
+ * The asynchronous pipeline (Connect4 / tic-tac-toe, K = 1, without SPB_FLAG_LOCKSTEP) keeps per tree an evaluation cache
+ * of the current search: a leaf whose position the tree has already sent to the evaluator in this search is expanded with
+ * that record, bit-identical to evaluating it again.  Its table is allocated by the first search that needs a larger
+ * one and kept: per tree the next power of two >= 2 * num_searches slots (32..4096) of 16 + 4 + 4 * EVAL_STRIDE bytes,
+ * 0.45 GB for 4,096 Connect4 trees at 800 simulations.  When it cannot be allocated the search runs without it.
  */
 int32_t spb_search(spb_engine* e, uint32_t num_searches);
 
@@ -575,6 +580,8 @@ int32_t spb_synchronize(spb_engine* e);
  * Statistics of the most recent search through the asynchronous pipeline (zeros for the other pipelines), out[0..n):
  * [0] evaluator batches, [1] boards in them, [2] ns the evaluator CTAs waited for leaves (sum over CTAs), [3] ns the tree
  * warps spent on trees (sum over warps), [4] tree visits, [5] tree warps, [6] evaluator CTAs.
+ * [1] counts the positions the evaluator really received, also with the built-in evaluators; spb_counters.evaluations
+ * minus [1] is the number of leaves the evaluation cache served (see spb_search).
  */
 int32_t spb_last_async_stats(spb_engine* e, uint64_t* out, uint32_t n);
 /*

@@ -36,6 +36,8 @@ struct AsyncCtl {
   uint32_t* abort;             // watchdog: set when the pipeline made no progress for stall_ns (a bug, never expected)
   unsigned long long* stats;   // [ASTAT_COUNT] pipeline statistics of the search (summed over CTAs / warps at kernel exit)
   unsigned long long stall_ns;
+  EvalCache cache;             // per-tree evaluation cache (tree.cuh); cache.key == nullptr: none
+  uint32_t epoch;              // this search's epoch: cache entries of other epochs are empty slots
 };
 enum AsyncStat { ASTAT_BATCHES = 0, ASTAT_BOARDS, ASTAT_CLAIM_WAIT_NS, ASTAT_TREE_BUSY_NS, ASTAT_TREE_PHASES, ASTAT_TREE_WARPS,
                  ASTAT_EVAL_CTAS, ASTAT_CLAIM_EMPTY, ASTAT_TICKET_WAIT_NS, ASTAT_AVAIL_SUM, ASTAT_READY_BACKLOG, ASTAT_READY_STARVED, ASTAT_COUNT };
@@ -203,69 +205,124 @@ __device__ __forceinline__ void flush_counters(const Trees& T, const unsigned lo
   }
 }
 
+// ---- evaluation cache (tree.cuh: EvalCache) ------------------------------------------------------------------------
+// The evaluator is a pure function of the 16-byte position, so a leaf whose position tree g has already sent to the
+// evaluator in this search gets that record back from the cache, with the same bits the evaluator would produce again.
+// Only the warp that owns tree g touches its table.  Reads go to L2 (ld.cg): the previous owner of the tree was another
+// SM, and a line of this SM's L1 left from an earlier visit could pair a fresh key with a stale record.  Writes reach the
+// next owner through the __threadfence + release of the ring push, as the node records do.
+constexpr uint32_t CACHE_NONE = 0xFFFFFFFFu;
+
+// One warp-wide probe: lane i examines slot (hash + i) mod slots.  Returns the first slot of the window that holds `st`
+// (hit = true) or is empty (hit = false: where its record goes once evaluated); CACHE_NONE = no table or a full window.
+// A hit needs all 128 bits of the key to be equal.
+__device__ __forceinline__ uint32_t cache_probe(const EvalCache& E, uint32_t epoch, uint32_t g, const PState& st, int lane, bool& hit) {
+  hit = false;
+  if (E.key == nullptr) return CACHE_NONE;
+  const uint32_t s = ((uint32_t)splitmix64(st.x ^ splitmix64(st.o)) + (uint32_t)lane) & (E.slots - 1u);
+  const size_t e = (size_t)g * E.slots + s;
+  const uint32_t ep = __ldcg(E.epoch + e);
+  const ulonglong2 k = __ldcg(E.key + e);
+  const bool empty = ep != epoch;
+  const uint32_t stop = __ballot_sync(0xffffffffu, empty || (k.x == st.x && k.y == st.o));
+  if (stop == 0u) return CACHE_NONE;
+  const int first = __ffs((int)stop) - 1;
+  hit = !__shfl_sync(0xffffffffu, empty, first);
+  return __shfl_sync(0xffffffffu, s, first);
+}
+
+// Entry `s` of tree g := (st, record, epoch).  Lane a writes word a of the record (words past the value are padding).
+template <class G>
+__device__ __forceinline__ void cache_insert(const EvalCache& E, uint32_t epoch, uint32_t g, uint32_t s, const PState& st,
+                                             const float* probs, float v, int lane) {
+  const size_t e = (size_t)g * E.slots + s;
+  float w = 0.0f;
+#pragma unroll
+  for (int a = 0; a < G::A; ++a) if (lane == a) w = probs[a];
+  if (lane == G::A) w = v;
+  if (lane < G::EVAL_STRIDE) E.rec[e * G::EVAL_STRIDE + lane] = w;
+  if (lane == 0) {
+    E.key[e] = make_ulonglong2(st.x, st.o);
+    E.epoch[e] = epoch;
+  }
+}
+
+// expand of an evaluated leaf with its record's probabilities (mcts.rs:278-281), then the backup of its value along the
+// path (mcts.rs:282-284).  false = the node pool is full (reported in the error word).
+template <class G>
+__device__ __forceinline__ bool expand_backup(const Trees& T, uint32_t g, NodeRec* rec, uint32_t* par, uint32_t& n_nodes, uint32_t leaf,
+                                              const PState& st, const float* probs, float v, const WarpPath& path, int depth, int lane,
+                                              unsigned long long* ctr) {
+  const uint32_t before = n_nodes;
+  if (!expand<G>(rec, par, T.cap, n_nodes, leaf, st, probs, lane)) {
+    if (lane == 0) atomicOr(T.error, ERRBIT_POOL);
+    return false;
+  }
+  ctr[CTR_CHILDREN] += n_nodes - before;
+  if (lane == 0) T.n_nodes[g] = n_nodes;
+  backup_regs(rec, path, depth, v, lane);                           // backprop, mcts.rs:145-159: N += 1, W += +-v
+  return true;
+}
+
 // One visit of tree g to a tree warp: expand + backup of the evaluated leaf (mcts.rs:278-284), then selects
 // (mcts.rs:236-252) until a leaf needs the evaluator or the tree has started all its simulations.  Terminal leaves are
 // backed up at once and the tree carries on: in the reference they take part in the iteration without an evaluation.
+// So are leaves whose position the evaluation cache holds: expand + backup with the cached record, then the next select.
 template <class G>
 __device__ __forceinline__ void tree_phase(const Trees& T, const AsyncCtl& C, uint32_t g, int lane, unsigned long long* ctr) {
   const uint32_t slot = g;                                          // one leaf in flight per tree
   uint32_t* pathm = T.path + (size_t)slot * G::MAX_DEPTH;
   const uint32_t b = T.buf[g];                                      // constant during a search
   const PState root = T.root_state[g];                              // constant during a search
-  const uint32_t li = __ldcg(&T.leaf_info[slot]);
+  uint32_t li = __ldcg(&T.leaf_info[slot]);
   uint32_t n_nodes = __ldcg(&T.n_nodes[g]);
   uint32_t remaining = __ldcg(&C.sims_left[g]);
   NodeRec* rec = T.rec[b] + (size_t)g * T.cap;
   uint32_t* par = T.par[b] + (size_t)g * T.cap;
-  bool ok = true;
+  WarpPath path;
+  uint32_t leaf = 0;
+  int depth = 0;
+  PState st{};
+  const float* src = nullptr;                                       // record of the leaf to expand: eval_out or the cache
 
-  if (li & LEAF_PENDING) {
-    const int depth = (int)(li & 0xFFu);
-    PState st;
+  if (li & LEAF_PENDING) {                                          // the evaluator's record has arrived
+    depth = (int)(li & 0xFFu);
     {
       const ulonglong2 raw = __ldcg(reinterpret_cast<const ulonglong2*>(&T.leaf_state[slot]));
       st.x = raw.x; st.o = raw.y;
     }
-    const float* eo = T.eval_out + (size_t)slot * G::EVAL_STRIDE;
-    float probs[G::A];
-#pragma unroll
-    for (int a = 0; a < G::A; ++a) probs[a] = __ldcg(eo + a);
-    const float v = __ldcg(eo + G::A);
     const uint32_t pn0 = (lane < G::MAX_DEPTH) ? __ldcg(pathm + lane) : 0u;
     const uint32_t pn1 = (lane + 32 < G::MAX_DEPTH) ? __ldcg(pathm + lane + 32) : 0u;
-    const uint32_t leaf = __shfl_sync(0xffffffffu, depth < 32 ? pn0 : pn1, depth & 31);
+    leaf = __shfl_sync(0xffffffffu, depth < 32 ? pn0 : pn1, depth & 31);
     SPB_ASSERT(T.error, depth < G::MAX_DEPTH && (lane > depth || pn0 < n_nodes) && (lane + 32 > depth || pn1 < n_nodes), 2);
-    uint2 nw0 = make_uint2(0, 0), nw1 = make_uint2(0, 0);
+    uint2 nw0 = make_uint2(0, 0), nw1 = make_uint2(0, 0);           // the path in registers, as the descent left it
     if (lane <= depth) nw0 = __ldcg(reinterpret_cast<const uint2*>(&rec[pn0]));
     if (lane + 32 <= depth) nw1 = __ldcg(reinterpret_cast<const uint2*>(&rec[pn1]));
-    const uint32_t before = n_nodes;
-    if (!expand<G>(rec, par, T.cap, n_nodes, leaf, st, probs, lane)) {
-      if (lane == 0) atomicOr(T.error, ERRBIT_POOL);
-      ok = false;
-    } else {
-      ctr[CTR_CHILDREN] += n_nodes - before;
-      if (lane == 0) T.n_nodes[g] = n_nodes;
-      if (lane <= depth) {                                          // backprop, mcts.rs:145-159: N += 1, W += +-v
-        nw0.x += 1u;
-        nw0.y = __float_as_uint(__fadd_rn(__uint_as_float(nw0.y), ((depth - lane) & 1) ? -v : v));
-        *reinterpret_cast<uint2*>(&rec[pn0]) = nw0;
-      }
-      if (lane + 32 <= depth) {
-        nw1.x += 1u;
-        nw1.y = __float_as_uint(__fadd_rn(__uint_as_float(nw1.y), ((depth - lane - 32) & 1) ? -v : v));
-        *reinterpret_cast<uint2*>(&rec[pn1]) = nw1;
-      }
-    }
-    if (lane == 0) T.leaf_info[slot] = 0;
-    __syncwarp();
+    path.node[0] = pn0; path.N[0] = nw0.x; path.W[0] = __uint_as_float(nw0.y);
+    path.node[1] = pn1; path.N[1] = nw1.x; path.W[1] = __uint_as_float(nw1.y);
+    src = T.eval_out + (size_t)slot * G::EVAL_STRIDE;
   }
 
-  while (ok && remaining > 0) {
+  for (;;) {
+    if (src != nullptr) {
+      float probs[G::A];
+#pragma unroll
+      for (int a = 0; a < G::A; ++a) probs[a] = __ldcg(src + a);
+      const float v = __ldcg(src + G::A);
+      if (li & LEAF_PENDING) {                                      // the network's record: into the cache, for the next visits
+        const uint32_t ins = li >> LEAF_INSERT_SHIFT;
+        if (ins != 0u) cache_insert<G>(C.cache, C.epoch, g, ins - 1u, st, probs, v, lane);
+        if (lane == 0) T.leaf_info[slot] = 0;
+        li = 0;
+      }
+      src = nullptr;
+      const bool ok = expand_backup<G>(T, g, rec, par, n_nodes, leaf, st, probs, v, path, depth, lane, ctr);
+      __syncwarp();
+      if (!ok) break;
+    }
+    if (remaining == 0) break;
     --remaining;
-    WarpPath path;
-    uint32_t leaf, linfo;
-    int depth;
-    PState st;
+    uint32_t linfo;
     descend<G, true>(rec, root, T.c, root_noise_of(T, g), lane, path, leaf, depth, st, linfo, T.error, n_nodes);
     SPB_ASSERT(T.error, leaf < n_nodes && depth < G::MAX_DEPTH, 3);
     ctr[CTR_SIMS] += 1;
@@ -277,7 +334,13 @@ __device__ __forceinline__ void tree_phase(const Trees& T, const AsyncCtl& C, ui
       __syncwarp();
       continue;
     }
-    ctr[CTR_EVALS] += 1;                                            // mcts.rs:249-250: queue the leaf
+    ctr[CTR_EVALS] += 1;                                            // mcts.rs:249-250: the leaf goes to the evaluator
+    bool hit;
+    const uint32_t cs = cache_probe(C.cache, C.epoch, g, st, lane, hit);
+    if (hit) {                                                      // ... which gave its record earlier in this search
+      src = C.cache.rec + ((size_t)g * C.cache.slots + cs) * G::EVAL_STRIDE;
+      continue;
+    }
 #pragma unroll
     for (int s = 0; s < 2; ++s) {
       const int d = lane + 32 * s;
@@ -285,7 +348,7 @@ __device__ __forceinline__ void tree_phase(const Trees& T, const AsyncCtl& C, ui
     }
     if (lane == 0) {
       T.leaf_state[slot] = st;
-      T.leaf_info[slot] = (uint32_t)depth | LEAF_PENDING;
+      T.leaf_info[slot] = (uint32_t)depth | LEAF_PENDING | ((cs + 1u) << LEAF_INSERT_SHIFT);   // CACHE_NONE + 1 = 0: no insert
       C.sims_left[g] = remaining;
     }
     __threadfence();                                                // every lane's stores are at L2 before the hand-off
@@ -336,10 +399,15 @@ __device__ __forceinline__ void builtin_eval_worker(const Trees& T, const AsyncC
   Spin sp;
   sp.init(C, *C.n_active);
   LeafClaimer lc;
+  unsigned long long boards = 0;
   for (;;) {
     uint32_t slot = RING_NONE;
     const uint32_t k = claim_batch(C, lc, n_workers, 32u, 2000u, sp, lane, &slot);
-    if (k == 0) break;
+    if (k == 0) {
+      if (lane == 0) atomicAdd(&C.stats[ASTAT_BOARDS], boards);   // positions evaluated, as the network's stager counts them
+      break;
+    }
+    boards += k;
     SPB_ASSERT(T.error, (uint32_t)lane >= k || slot < T.G * T.K, 5);
     if ((uint32_t)lane < k) {
       PState st;

@@ -278,10 +278,47 @@ int32_t spb_engine::launch_root_noise() {
   return SPB_OK;
 }
 
+// The evaluation cache of the asynchronous pipeline: per tree the next power of two >= 2 x num_searches slots (at least
+// one probe window, at most EVAL_CACHE_MAX_SLOTS), so that the <= num_searches records of one search fill at most half of
+// it.  Grow-only like the node pools; zeroed once when allocated (epoch 0 = empty).  No result depends on the cache, so
+// when the allocation fails the searches run without one.
+int32_t spb_engine::ensure_eval_cache(uint32_t num_searches) {
+  uint32_t want = EVAL_CACHE_WINDOW;
+  while (want < 2ull * num_searches && want < EVAL_CACHE_MAX_SLOTS) want <<= 1;
+  if (want <= ctl.cache.slots || want <= cache_tried) return SPB_OK;
+  cache_tried = want;
+  const size_t n = (size_t)T.G * want;
+  EvalCache nc{nullptr, nullptr, nullptr, want};
+  cudaError_t ce = cudaMalloc((void**)&nc.key, n * sizeof(ulonglong2));
+  if (ce == cudaSuccess) ce = cudaMalloc((void**)&nc.epoch, n * sizeof(uint32_t));
+  if (ce == cudaSuccess) ce = cudaMalloc((void**)&nc.rec, n * (size_t)eval_stride * sizeof(float));
+  if (ce == cudaSuccess) ce = cudaMemsetAsync(nc.epoch, 0, n * sizeof(uint32_t), stream);
+  if (ce != cudaSuccess) {
+    for (void* p : {(void*)nc.key, (void*)nc.epoch, (void*)nc.rec}) if (p) cudaFree(p);
+    cudaGetLastError();                                              // an allocation failure is not sticky: clear it
+    return SPB_OK;                                                   // keep the smaller table (or none)
+  }
+  SPB_CUDA(this, cudaStreamSynchronize(stream));                     // no search of the old table is in flight
+  for (void* old : {(void*)ctl.cache.key, (void*)ctl.cache.epoch, (void*)ctl.cache.rec}) {
+    if (!old) continue;
+    allocs.erase(std::find(allocs.begin(), allocs.end(), old));
+    cudaFree(old);
+  }
+  for (void* p : {(void*)nc.key, (void*)nc.epoch, (void*)nc.rec}) allocs.push_back(p);
+  ctl.cache = nc;
+  return SPB_OK;
+}
+
 // One search through the asynchronous pipeline: rings reset, every live tree queued, ONE resident kernel until all trees
 // have completed their simulations (network: evaluator CTAs + tree warps; built-in evaluators: evaluator warps + tree warps).
 template <class G>
 int32_t spb_engine::search_async(uint32_t num_searches) {
+  { int32_t rc = ensure_eval_cache(num_searches); if (rc != SPB_OK) return rc; }
+  if (++cache_epoch == 0u) {   // the epoch wrapped: entries of epoch 1 could look live again
+    if (ctl.cache.epoch) SPB_CUDA(this, cudaMemsetAsync(ctl.cache.epoch, 0, (size_t)T.G * ctl.cache.slots * 4, stream));
+    cache_epoch = 1u;
+  }
+  ctl.epoch = cache_epoch;
   SPB_CUDA(this, cudaMemsetAsync(d_ctl_words, 0, (size_t)CTL_WORDS * 4, stream));
   SPB_CUDA(this, cudaMemsetAsync(d_ring_slots, 0, 2 * (size_t)ring_size * 8, stream));
   k_async_init<<<(T.G + 127) / 128, 128, 0, stream>>>(T, ctl, num_searches);

@@ -40,9 +40,14 @@ struct spb_engine : spb::HostEngine<spb::Trees, spb_position, uint8_t> {
   unsigned long long* d_ring_slots = nullptr;   // [2][ring_size]
   uint32_t ring_size = 0;
   uint64_t last_async_stats[16] = {};
+  // evaluation cache of the asynchronous pipeline (ctl.cache, tree.cuh: EvalCache): grow-only, never cleared between
+  // searches; every asynchronous search takes the next epoch
+  uint32_t cache_epoch = 0;
+  uint32_t cache_tried = 0;    // largest table (slots per tree) an allocation was attempted for
   int A = 0, max_depth = 0, eval_stride = 0, max_ply = 0;
 
   int32_t ensure_capacity(uint32_t num_searches);
+  int32_t ensure_eval_cache(uint32_t num_searches);
   void drop_step_graph() {
     if (step_graph) { cudaGraphExecDestroy(step_graph); step_graph = nullptr; }
   }

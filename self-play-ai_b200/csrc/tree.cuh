@@ -51,8 +51,23 @@ enum ErrorBits : uint32_t { ERRBIT_POOL = 1u, ERRBIT_NAN = 2u, ERRBIT_TRAJ_FULL 
 #define SPB_ASSERT(err, cond, code) ((void)0)
 #endif
 
-// leaf_info[slot]: depth[0,8) | pending-eval flag (bit 8)
+// leaf_info[slot]: depth[0,8) | pending-eval flag (bit 8) | asynchronous pipeline: evaluation-cache insert position + 1
+// [9,32) (0 = no insert)
 constexpr uint32_t LEAF_PENDING = 1u << 8;
+constexpr int LEAF_INSERT_SHIFT = 9;
+
+// Evaluation cache of the asynchronous pipeline (async.cuh, DESIGN.md §4.2a): per tree an open-addressed table of the
+// records the evaluator produced during the current search, keyed by the full 16-byte position.  An entry is live only
+// while its epoch equals the search's epoch, so the table is never cleared between searches.  key = nullptr: no table
+// (every lookup misses).
+constexpr uint32_t EVAL_CACHE_MAX_SLOTS = 4096;   // per tree; the table holds num_searches records at load <= 0.5 up to here
+constexpr int EVAL_CACHE_WINDOW = 32;             // consecutive slots one probe examines (one per lane)
+struct EvalCache {
+  ulonglong2* key;       // [G][slots]  PState {x, o} of the entry
+  uint32_t* epoch;       // [G][slots]  search epoch that wrote the entry (0 = never written)
+  float* rec;            // [G][slots][EVAL_STRIDE]  the evaluator's record: unmasked softmax + value
+  uint32_t slots;        // per tree, a power of two
+};
 
 struct Trees {
   NodeRec* rec[2];
