@@ -60,15 +60,28 @@ class Net(nn.Module):
         return pairs
 
 
-def make_net(game, seed=0, randomize_bn=True, trained_like=False):
+def make_net(game, seed=0, randomize_bn=True, trained_like=False, calibrated=False):
     """game: 0 tic-tac-toe, 1 connect4.  Default torch init under manual_seed; BN running stats and affine
     parameters are randomised (when asked) so that BN folding is actually exercised.  trained_like: statistics of a net
     that has been trained for a while instead of a fresh one — BatchNorm gammas spread over 0.5..2, shifted and scaled
-    running statistics, larger head weights (logits of several units, tanh driven towards saturation)."""
+    running statistics, larger head weights (logits of several units, tanh driven towards saturation).
+    calibrated: the counterpart of make_chess_net(calibrated=True), calibrated on calibration_encodings(game).  BatchNorm
+    gammas 0.5..2 and shifted betas, running statistics that are those of the conv outputs they normalise (head convs
+    included); value_fc scaled so that the value before tanh has mean 0 and standard deviation 0.8, and every row of
+    policy_fc so that its logit's position-dependent part (the logit minus its mean over the positions) has standard
+    deviation 1.  A fresh or trained-like net's value hardly depends on the position (standard deviation 0.02 over
+    random positions), so a comparison against it cannot see the value head."""
     rows, cols, actions = (6, 7, 7) if game == 1 else (3, 3, 9)
     g = torch.Generator().manual_seed(seed)
     torch.manual_seed(seed)
     net = Net(rows, cols, actions).eval()
+    if calibrated:
+        with torch.no_grad():
+            for _, bn in net.conv_bn_pairs():
+                bn.weight.copy_(torch.rand(bn.num_features, generator=g) * 1.5 + 0.5)
+                bn.bias.copy_(torch.randn(bn.num_features, generator=g) * 0.3)
+            _calibrate_net(net, calibration_encodings(game))
+        return net
     if trained_like:
         with torch.no_grad():
             for _, bn in net.conv_bn_pairs():
@@ -87,6 +100,46 @@ def make_net(game, seed=0, randomize_bn=True, trained_like=False):
                 bn.weight.copy_(torch.rand(bn.num_features, generator=g) * 0.5 + 0.75)
                 bn.bias.copy_(torch.randn(bn.num_features, generator=g) * 0.1)
     return net
+
+
+def calibration_states(game, n=256, seed=97):
+    """n fixed ongoing positions: the position after a uniform random playout of a random length (oracle rules, seeded)."""
+    from . import pyoracle as O
+    rng = np.random.default_rng(seed)
+    max_len = 42 if game == O.GAME_C4 else 9
+    out = []
+    while len(out) < n:
+        s = O.State()
+        for _ in range(int(rng.integers(0, max_len))):
+            s = O.next_state(game, s, int(rng.choice(O.valid_actions(game, s))))
+            if s.status != O.ONGOING:
+                break
+        if s.status == O.ONGOING:
+            out.append(s)
+    return out
+
+
+def calibration_encodings(game, n=256, seed=97):
+    from . import pyoracle as O
+    return np.stack([O.encode(game, s) for s in calibration_states(game, n, seed)])
+
+
+def _calibrate_net(net, enc):
+    def bn_from(conv, bn, x):
+        u = conv(x)
+        bn.running_mean.copy_(u.mean((0, 2, 3)))
+        bn.running_var.copy_(u.var((0, 2, 3)))
+        return bn(u)
+    x = torch.from_numpy(np.ascontiguousarray(enc, dtype=np.float32)).view(-1, 3, net.rows, net.cols)
+    x = torch.relu(bn_from(net.stem, net.stem_bn, x))
+    for b in net.blocks:
+        x = torch.relu(x + bn_from(b.conv2, b.bn2, torch.relu(bn_from(b.conv1, b.bn1, x))))
+    z = net.vfc(torch.relu(bn_from(net.vconv, net.vbn, x)).flatten(1))
+    m, s = z.mean(), z.std() / 0.8
+    net.vfc.weight.div_(s)
+    net.vfc.bias.sub_(m).div_(s)
+    lg = net.pfc(torch.relu(bn_from(net.pconv, net.pbn, x)).flatten(1))
+    net.pfc.weight.div_(lg.std(0)[:, None])
 
 
 def _write_safetensors(tensors):

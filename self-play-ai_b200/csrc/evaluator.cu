@@ -5,8 +5,9 @@
 //   encode (3 planes) -> stem conv3x3+BN+ReLU -> 4 x [conv-BN-ReLU-conv-BN, +skip, ReLU]
 //   -> policy head conv3x3(64->32)+BN+ReLU -> Linear -> softmax
 //   -> value  head conv3x3(64->3)+BN+ReLU  -> Linear -> tanh
-// BatchNorm (eval) is folded into the convs on the host; weights are bf16, accumulation f32,
-// activations are rounded to bf16 between layers (both kernels do the same roundings).
+// BatchNorm (eval) is folded into the convs on the host; conv weights are bf16, accumulation f32,
+// activations are rounded to bf16 between layers and after the head convs; the Linear heads' weights
+// and every bias are f32.  Both kernels do the same roundings; tests/small_net_ref.py restates them.
 //
 // Two kernels:
 //   k_eval_umma  — the product path: implicit-GEMM 3x3 convs on tcgen05 tensor cores, accumulators
@@ -84,10 +85,11 @@ __global__ void __launch_bounds__(256) k_eval_simt(Evaluator::DevNet net, const 
                       [&](int oc, int p, float v) { xa[oc * P + p] = round_bf16(fmaxf(v + xa[oc * P + p], 0.0f)); });   // (x + f(x)).relu()
       __syncthreads();
     }
+    // the head convs' activations are stored as bf16, as k_eval_umma's head epilogue stores them
     conv3x3_simt<G>(xa, NET_HIDDEN, net.w_simt[9], net.bias[9], NET_POLICY_CH,
-                    [&](int oc, int p, float v) { head[oc * P + p] = fmaxf(v, 0.0f); });
+                    [&](int oc, int p, float v) { head[oc * P + p] = round_bf16(fmaxf(v, 0.0f)); });
     conv3x3_simt<G>(xa, NET_HIDDEN, net.w_simt[10], net.bias[10], NET_VALUE_CH,
-                    [&](int oc, int p, float v) { head[(NET_POLICY_CH + oc) * P + p] = fmaxf(v, 0.0f); });
+                    [&](int oc, int p, float v) { head[(NET_POLICY_CH + oc) * P + p] = round_bf16(fmaxf(v, 0.0f)); });
     __syncthreads();
     // Linear layers: one warp per output (flat_view index = channel*P + row*C + col).
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;

@@ -17,14 +17,20 @@ RTOL = 1e-2
 
 
 def _check(game, flags, n, seed, blob_fn, trained_like=False):
-    RTOL = 1.5e-2 if trained_like else 1e-2
     net = torch_net.make_net(game, seed=seed, trained_like=trained_like)
     states = random_states(game, n, seed=seed + 1, include_terminal=False)
-    enc = np.stack([O.encode(game, s) for s in states])
-    probs_ref, v_ref, logit_ref = torch_net.forward_probs(net, enc)
     with S.Engine(game=game, num_games=4, evaluator=S.EVAL_NET, flags=flags) as e:
         e.load_weights(blob_fn(net))
         pol, v, lg = e.predict(states, want_logits=True)
+    check_against_fp32(game, net, states, pol, v, lg, trained_like)
+    return lg, v
+
+
+def check_against_fp32(game, net, states, pol, v, lg, trained_like=False):
+    """The comparison of _check: an evaluator's masked policies, values and logits against the torch fp32 net."""
+    RTOL = 1.5e-2 if trained_like else 1e-2
+    enc = np.stack([O.encode(game, s) for s in states])
+    probs_ref, v_ref, logit_ref = torch_net.forward_probs(net, enc)
     scale = float(np.abs(logit_ref).max())
     assert np.allclose(lg, logit_ref, rtol=RTOL, atol=RTOL * scale), float(np.abs(lg - logit_ref).max())
     assert np.allclose(v, v_ref, rtol=RTOL, atol=RTOL), float(np.abs(v - v_ref).max())
@@ -42,7 +48,6 @@ def _check(game, flags, n, seed, blob_fn, trained_like=False):
         legal = set(O.valid_actions(game, s))
         assert all((p[a] > 0) == (a in legal) or p[a] == 0 for a in range(len(p)))
         assert all(p[a] == 0 for a in range(len(p)) if a not in legal)
-    return lg, v
 
 
 @pytest.mark.parametrize("game", [S.GAME_C4, S.GAME_TTT], ids=["c4", "ttt"])

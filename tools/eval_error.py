@@ -4,7 +4,9 @@ max |dlogit| / max |logit| (the bound of tests/test_gpu_evaluator.py), the worst
 vector, the largest change of a softmax probability, max |dvalue|.  The chess 10x256 network, fresh (seed 0) and calibrated
 (make_chess_net(calibrated=True)), on the 4,096 distinct positions of tests/test_net_numerics.py at every batch size of
 its tile-loop regimes, against the bf16-faithful reference (tests/chess_net_ref.py; |dlogit| over the logit's
-position-dependent spread, the bound of that test) and against torch fp32.  Needs a B200; prints the card and its power
+position-dependent spread, the bound of that test) and against torch fp32.  Connect4 / tic-tac-toe again, on the nets,
+positions and batch sizes of tests/test_eval_numerics.py, per kernel: against the bf16-faithful reference
+(tests/small_net_ref.py; the metrics of that test) next to torch fp32.  Needs a B200; prints the card and its power
 limit first."""
 import os
 import subprocess
@@ -74,3 +76,26 @@ with S.ChessEngine(num_games=T.G, evaluator=S.EVAL_NET) as e:
                       n, T.max_pass(n, pairs), r.max(), np.quantile(r, 0.9999), np.median(r), dv.max(), np.quantile(dv, 0.99),
                       np.abs(lg - lg32[:n]).max() / np.abs(lg32[:n]).max(), (np.abs(lg - lg32[:n]) / spread).max(),
                       np.abs(v - v32[:n]).max()), flush=True)
+
+# ---- Connect4 / tic-tac-toe against the bf16-faithful reference (tests/small_net_ref.py) --------------------------------
+import small_net_ref as SR  # noqa: E402
+import test_eval_numerics as EN  # noqa: E402
+
+sms = torch.cuda.get_device_properties(0).multi_processor_count
+for tag in EN.GAMES:
+    for name in EN.NETS:
+        c = EN.case(tag, name)
+        _, v32, lg32 = torch_net.forward_probs(c["net"], c["enc"])
+        print("%s %s: %d positions, value std %.3f, logit scale %.2f, position-dependent logit spread %.3g (median per logit %.3g)" % (
+            tag, name, len(c["enc"]), c["ref_v"].std(), np.abs(c["ref_lg"]).max(), torch_net.chess_logit_deviation(c["ref_lg"]),
+            np.median(c["spread"])), flush=True)
+        for kernel, flags in EN.KERNELS.items():
+            with S.Engine(game=EN.GAMES[tag], num_games=4, evaluator=S.EVAL_NET, flags=flags) as e:
+                e.load_weights(c["blob"])
+                for n in [len(c["enc"])] + EN.batch_sizes(EN.GAMES[tag], sms):
+                    idx = np.arange(n) % len(c["enc"])
+                    pol, v, lg = e.predict(c["states"][idx], want_logits=True)
+                    m = EN.metrics(c, lg, v, pol, idx=idx)
+                    print("  %-7s n %5d | vs bf16 reference: |dlogit|/spread max %.2e, position RMS max %.2e median %.2e, |dv| max %.2e, |dp| max %.2e "
+                          "| vs fp32: max|dlogit|/scale %.2e |dv| max %.2e" % (
+                              (kernel, n) + m + (np.abs(lg - lg32[idx]).max() / np.abs(lg32[idx]).max(), np.abs(v - v32[idx]).max())), flush=True)
