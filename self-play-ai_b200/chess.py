@@ -62,44 +62,17 @@ def _history(history, n):
     return h
 
 
-class ChessEngine:
+class ChessEngine(E.EngineBase):
     """The chess engine: `Mcts<chess Net>` + its trees on one GPU (ref: src/mcts.rs:41-44 over src/game/chess.rs and
     src/model/chess.rs) — batched `State` methods, search, re-rooting, `Model::predict`."""
+    _PREFIX, _RECORD, _STATE, _ROOT_WIDTH, _MOVE = "spb_chess_", CHESS_POSITION_DTYPE, CHESS_STATE_DTYPE, MAX_MOVES, np.uint16
+    A = POLICY_SIZE
 
     def __init__(self, num_games=64, evaluator=E.EVAL_NET, c=2.0, device=0, max_nodes_per_tree=0, flags=0, trajectory_capacity=0,
                  game_id_base=0, game_id_stride=0):
-        L = E.load_library()
-        cfg = E.Config()
-        L.spb_default_config(C.byref(cfg))
-        cfg.game, cfg.num_games, cfg.evaluator, cfg.c, cfg.device = E.GAME_CHESS, num_games, evaluator, c, device
-        cfg.max_nodes_per_tree, cfg.flags, cfg.leaves_per_tree = max_nodes_per_tree, flags, 1
-        cfg.trajectory_capacity, cfg.game_id_base, cfg.game_id_stride = trajectory_capacity, game_id_base, game_id_stride
-        h = C.c_void_p()
-        rc = L.spb_chess_create(C.byref(cfg), C.byref(h))
-        if rc != 0:
-            raise E.EngineError(rc, L.spb_chess_last_error(None).decode())
-        self._h, self._L, self.G, self.device = h, L, num_games, device
-
-    def close(self):
-        if getattr(self, "_h", None):
-            self._L.spb_chess_destroy(self._h)
-            self._h = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
-
-    def __enter__(self):
-        return self
-
-    def __exit__(self, *a):
-        self.close()
-
-    def _chk(self, rc):
-        if rc != 0:
-            raise E.EngineError(rc, self._L.spb_chess_last_error(self._h).decode())
+        super().__init__(game=E.GAME_CHESS, num_games=num_games, evaluator=evaluator, c=c, device=device,
+                         max_nodes_per_tree=max_nodes_per_tree, flags=flags, leaves_per_tree=1,
+                         trajectory_capacity=trajectory_capacity, game_id_base=game_id_base, game_id_stride=game_id_stride)
 
     # ---- State trait, batched ----------------------------------------------------------------------------------------
     def legal_moves(self, states, history=None):
@@ -140,20 +113,7 @@ class ChessEngine:
         self._chk(self._L.spb_chess_perft(self._h, st.ctypes.data, depth, C.byref(nodes)))
         return int(nodes.value)
 
-    # ---- weights / Model::predict ------------------------------------------------------------------------------------
-    def load_weights(self, blob: bytes):
-        buf = (C.c_char * len(blob)).from_buffer_copy(blob)
-        self._chk(self._L.spb_chess_load_weights(self._h, C.cast(buf, C.c_void_p), len(blob)))
-
-    def load_weights_device(self, named):
-        """spb_chess_load_weights_device: the net from (name, CUDA tensor) pairs on the engine's GPU (the names of
-        load_weights); the same image as load_weights of a checkpoint of these tensors."""
-        E._load_weights_device(lambda t, n: self._chk(self._L.spb_chess_load_weights_device(self._h, t, n)), named, self.device)
-
-    def broadcast_weights(self, root: int = 0):
-        """COLLECTIVE: every rank takes root's weight image (spb_chess_broadcast_weights)."""
-        self._chk(self._L.spb_chess_broadcast_weights(self._h, root))
-
+    # ---- Model::predict ----------------------------------------------------------------------------------------------
     def predict(self, states, history=None, want_logits=False):
         st = _states(states)
         n = len(st)
@@ -176,58 +136,10 @@ class ChessEngine:
         self._chk(self._L.spb_chess_reset_games(self._h, None if sl is None else sl.ctypes.data, n, None if st is None else st.ctypes.data,
                                                 None if h is None else h.ctypes.data))
 
-    def search(self, num_searches: int):
-        self._chk(self._L.spb_chess_search(self._h, num_searches))
-
     def last_search_ms(self) -> float:
         ms = C.c_float()
         self._chk(self._L.spb_chess_last_search_ms(self._h, C.byref(ms)))
         return ms.value
-
-    def root_children(self, slot: int):
-        mv, cnt, ids = np.zeros(MAX_MOVES, np.uint16), np.zeros(MAX_MOVES, np.uint32), np.zeros(MAX_MOVES, np.uint32)
-        n = C.c_uint32()
-        self._chk(self._L.spb_chess_root_children(self._h, slot, mv.ctypes.data, cnt.ctypes.data, ids.ctypes.data, C.byref(n)))
-        k = n.value
-        return mv[:k].tolist(), cnt[:k].tolist(), ids[:k].tolist()
-
-    def root_children_all(self, out=None):
-        """`out`: the four arrays of an earlier call (e.g. in pinned host memory), written in place."""
-        if out is not None:
-            mv, cnt, ids, n = out
-            assert mv.shape == (self.G, MAX_MOVES) and mv.dtype == np.uint16 and cnt.dtype == np.uint32 and ids.dtype == np.uint32 and n.shape == (self.G,)
-            assert all(x.flags.c_contiguous for x in out)
-        else:
-            mv = np.zeros((self.G, MAX_MOVES), np.uint16)
-            cnt = np.zeros((self.G, MAX_MOVES), np.uint32)
-            ids = np.zeros((self.G, MAX_MOVES), np.uint32)
-            n = np.zeros(self.G, np.uint32)
-        self._chk(self._L.spb_chess_root_children_all(self._h, mv.ctypes.data, cnt.ctypes.data, ids.ctypes.data, n.ctypes.data))
-        return mv, cnt, ids, n
-
-    def root_policy(self, slot: int) -> np.ndarray:
-        p = np.zeros(POLICY_SIZE, np.float32)
-        self._chk(self._L.spb_chess_root_policy(self._h, slot, p.ctypes.data))
-        return p
-
-    # ---- EXTENSION: Dirichlet noise at the root (DESIGN.md §4.6) ------------------------------
-    def set_root_noise(self, alpha: float, epsilon: float, seed: int = 0):
-        """P' = (1 - epsilon) P + epsilon eta, eta ~ Dir(alpha), at the root of every search; epsilon = 0 turns it off."""
-        self._chk(self._L.spb_chess_set_root_noise(self._h, alpha, epsilon, seed))
-
-    def root_noise(self, slot: int) -> np.ndarray:
-        """The eta the next search of `slot`'s root uses, one entry per legal move of the root (child order)."""
-        eta = np.zeros(MAX_MOVES, np.float32)
-        n = C.c_uint32()
-        self._chk(self._L.spb_chess_root_noise(self._h, slot, eta.ctypes.data_as(C.POINTER(C.c_float)), C.byref(n)))
-        return eta[:n.value].copy()
-
-    def advance(self, child_ids, slots=None) -> np.ndarray:
-        ids = np.ascontiguousarray(child_ids, dtype=np.uint32)
-        sl = None if slots is None else np.ascontiguousarray(slots, dtype=np.uint32)
-        out = np.zeros(len(ids), CHESS_STATE_DTYPE)
-        self._chk(self._L.spb_chess_advance(self._h, None if sl is None else sl.ctypes.data, ids.ctypes.data, len(ids), out.ctypes.data))
-        return out
 
     # ---- self-play (ref: SelfPlayWorker::self_play, learner_concurrent.rs:169-242) --------------------------------------
     def selfplay_step(self, rule=E.MOVE_GREEDY_LAST_MAX, temperature=1.25, seed=0, restart_roots=None, restart_history=None) -> int:
@@ -243,58 +155,10 @@ class ChessEngine:
                                                   None if h is None else h.ctypes.data, C.byref(fin)))
         return fin.value
 
-    def drain_trajectories(self):
-        """-> (positions[CHESS_POSITION_DTYPE], game_ids[u64]) ordered by (game id, ply)."""
-        n = C.c_size_t()
-        self._chk(self._L.spb_chess_drain_trajectories(self._h, None, 0, C.byref(n), None))
-        pos = np.zeros(n.value, dtype=CHESS_POSITION_DTYPE)
-        ids = np.zeros(n.value, dtype=np.uint64)
-        if n.value:
-            self._chk(self._L.spb_chess_drain_trajectories(self._h, pos.ctypes.data, n.value, C.byref(n), ids.ctypes.data))
-        return pos[:n.value], ids[:n.value]
-
-    def drain_trajectories_device(self, out=None, ids_out=None):
-        """The records of drain_trajectories, ordered on the device -> (CUDA uint8 [n, 1624], CUDA int64 [n]); out / ids_out as
-        for Engine.drain_trajectories_device."""
-        return E._records_to_device(
-            lambda b, cap, n, i: self._chk(self._L.spb_chess_drain_trajectories_device(self._h, b, cap, n, i)),
-            self.device, CHESS_POSITION_DTYPE.itemsize, out, ids_out)
-
-    # ---- multi-GPU: trajectories to the learner rank (the contract of Engine's methods) -------------------------------
-    def comm_init(self, comm_id: bytes, rank: int, world_size: int):
-        buf = (C.c_uint8 * E.COMM_ID_BYTES).from_buffer_copy(comm_id)
-        self._chk(self._L.spb_chess_comm_init(self._h, C.cast(buf, C.c_void_p), rank, world_size))
-
-    def comm_destroy(self):
-        self._chk(self._L.spb_chess_comm_destroy(self._h))
-
-    def gather_trajectories(self, learner_rank: int = 0):
-        """COLLECTIVE: -> (positions[CHESS_POSITION_DTYPE], game_ids) ordered by (game id, ply) on the learner rank, empty
-        elsewhere."""
-        n = C.c_size_t()
-        self._chk(self._L.spb_chess_gather_trajectories(self._h, learner_rank, None, 0, C.byref(n), None))
-        pos = np.zeros(n.value, dtype=CHESS_POSITION_DTYPE)
-        ids = np.zeros(n.value, dtype=np.uint64)
-        if n.value:
-            self._chk(self._L.spb_chess_gather_trajectories(self._h, learner_rank, pos.ctypes.data, n.value, C.byref(n), ids.ctypes.data))
-        return pos[:n.value], ids[:n.value]
-
-    def gather_trajectories_device(self, learner_rank: int = 0, out=None, ids_out=None):
-        """COLLECTIVE: gather_trajectories into device memory of the learner rank -> (CUDA uint8 [n, 1624], CUDA int64 [n]),
-        empty elsewhere."""
-        return E._records_to_device(
-            lambda b, cap, n, i: self._chk(self._L.spb_chess_gather_trajectories_device(self._h, learner_rank, b, cap, n, i)),
-            self.device, CHESS_POSITION_DTYPE.itemsize, out, ids_out)
-
     def get_state(self, slot: int, node_id: int) -> np.ndarray:
         out = np.zeros(1, CHESS_STATE_DTYPE)
         self._chk(self._L.spb_chess_get_state(self._h, slot, node_id, out.ctypes.data))
         return out[0]
-
-    def arena_len(self, slot: int) -> int:
-        n = C.c_uint32()
-        self._chk(self._L.spb_chess_arena_len(self._h, slot, C.byref(n)))
-        return n.value
 
     def node_stats(self, slot: int, node_id: int) -> dict:
         n, fc, nc = C.c_uint32(), C.c_uint32(), C.c_uint32()
@@ -313,14 +177,9 @@ class ChessEngine:
         return ms.value, n.value, fl.value, fp.value
 
     def counters(self) -> dict:
-        c = E.Counters()
-        self._chk(self._L.spb_chess_get_counters(self._h, C.byref(c)))
-        d = c.as_dict()
-        d["largest_arena"] = int(c.reserved[0])
-        return d
-
-    def reset_counters(self):
-        self._chk(self._L.spb_chess_reset_counters(self._h))
+        """Engine.counters, plus largest_arena: the largest arena_len of any tree."""
+        c = self._read_counters()
+        return dict(c.as_dict(), largest_arena=int(c.reserved[0]))
 
 
 def positions_to_training(positions):
@@ -341,42 +200,12 @@ def positions_to_training(positions):
 def positions_to_training_device(engine: ChessEngine, positions, indices=None):
     """spb_chess_positions_to_training_device: the tensors of positions_to_training, built on the engine's GPU ->
     torch CUDA tensors (encodings[n,19,8,8], policies[n,4672], values[n,1]) f32, bit-identical to the host builder.
-    positions: CHESS_POSITION_DTYPE numpy array (copied to the device) or a CUDA uint8 tensor [n_positions, 1624], e.g. a
-    replay buffer kept in device memory.  indices (numpy or CUDA int64 / uint64 tensor): row i is built from
+    positions: CHESS_POSITION_DTYPE numpy array (copied to the device) or a contiguous CUDA uint8 tensor [n_positions, 1624],
+    e.g. a replay buffer kept in device memory.  indices (numpy or CUDA int64 / uint64 tensor): row i is built from
     positions[indices[i]]; without it every record is built.  A malformed row raises EngineError(-1) and nothing is written."""
-    import torch
-    dev = torch.device("cuda", engine.device)
-    if isinstance(positions, torch.Tensor):
-        assert positions.is_cuda and positions.dtype == torch.uint8 and positions.dim() == 2 and positions.shape[1] == CHESS_POSITION_DTYPE.itemsize, \
-            (positions.device, positions.dtype, tuple(positions.shape))
-        pos = positions.contiguous()
-    else:
-        a = np.ascontiguousarray(positions, dtype=CHESS_POSITION_DTYPE).reshape(-1)
-        pos = torch.from_numpy(a.view(np.uint8).reshape(len(a), CHESS_POSITION_DTYPE.itemsize)).to(dev)
-    idx = None
-    if indices is not None:
-        if isinstance(indices, torch.Tensor):
-            assert indices.is_cuda and indices.dtype in (torch.int64, torch.uint64) and indices.dim() == 1, (indices.device, indices.dtype)
-            idx = indices.contiguous()
-        else:
-            i = np.ascontiguousarray(indices).reshape(-1)
-            assert i.dtype.kind in "iu", i.dtype
-            idx = torch.from_numpy(i.astype(np.int64)).to(dev)
-    n = len(pos) if idx is None else len(idx)
-    enc = torch.empty((n, PLANES, 8, 8), dtype=torch.float32, device=dev)
-    pol = torch.empty((n, POLICY_SIZE), dtype=torch.float32, device=dev)
-    val = torch.empty((n, 1), dtype=torch.float32, device=dev)
-    torch.cuda.current_stream(dev).synchronize()                       # the engine's stream reads the inputs
-    engine._chk(engine._L.spb_chess_positions_to_training_device(
-        engine._h, pos.data_ptr() if len(pos) else None, len(pos), None if idx is None else idx.data_ptr(), n,
-        enc.data_ptr(), pol.data_ptr(), val.data_ptr()))
-    return enc, pol, val
+    return E._positions_to_training_device(engine, positions, indices, (PLANES, 8, 8))
 
 
 def check_weights(blob: bytes):
     """Host-only validation of a chess checkpoint -> (code, message)."""
-    L = E.load_library()
-    buf = (C.c_char * len(blob)).from_buffer_copy(blob)
-    err = C.create_string_buffer(512)
-    rc = L.spb_chess_check_weights(C.cast(buf, C.c_void_p), len(blob), err, 512)
-    return rc, err.value.decode()
+    return E._check_weights(E.load_library().spb_chess_check_weights, blob)

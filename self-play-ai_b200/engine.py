@@ -2,6 +2,7 @@
 from __future__ import annotations
 
 import ctypes as C
+import functools
 import os
 import subprocess
 
@@ -210,10 +211,14 @@ def states_array(states) -> np.ndarray:
 
 def check_weights(game: int, blob: bytes):
     """Host-only checkpoint validation -> (code, message)."""
-    L = load_library()
+    return _check_weights(functools.partial(load_library().spb_check_weights, game), blob)
+
+
+def _check_weights(call, blob: bytes):
+    """check_weights and chess.check_weights: `call(blob, size, err, err_cap)` is the entry point, its game bound."""
     buf = (C.c_char * len(blob)).from_buffer_copy(blob)
     err = C.create_string_buffer(512)
-    rc = L.spb_check_weights(game, C.cast(buf, _vp), len(blob), err, 512)
+    rc = call(C.cast(buf, _vp), len(blob), err, 512)
     return rc, err.value.decode()
 
 
@@ -278,16 +283,6 @@ def tensor_table(named, device):
     return table, len(items), names
 
 
-def _load_weights_device(call, named, device):
-    """The device loads: the caller's writes to the tensors finish before the engine reads them; `items` and `names` keep
-    the tensors and the table's names alive until the call has returned, after which the engine no longer reads them."""
-    import torch
-    items = list(named.items()) if hasattr(named, "items") else list(named)
-    table, n, names = tensor_table(items, device)
-    torch.cuda.current_stream(torch.device("cuda", device)).synchronize()
-    call(table, n)
-
-
 def _check_cuda_tensor(t, dtype, width, name):
     """Raises unless t is a contiguous CUDA tensor of `dtype`, [n, width] (width None: [n])."""
     import torch
@@ -303,30 +298,6 @@ def _check_cuda_tensor(t, dtype, width, name):
         raise ValueError("%s must be contiguous" % name)
 
 
-def _records_to_device(call, device, width, out, ids_out):
-    """The device forms of drain / gather: `call(buf, capacity, n_ref, ids)` is the entry point with the engine's
-    arguments bound.  Size query, then the records into `out` / `ids_out` (allocated when None) -> their [:n] views."""
-    import torch
-    if out is not None:
-        _check_cuda_tensor(out, torch.uint8, width, "out")
-    if ids_out is not None:
-        _check_cuda_tensor(ids_out, torch.int64, None, "ids_out")
-    dev = torch.device("cuda", device)
-    n = C.c_size_t()
-    call(None, 0, C.byref(n), None)
-    k = n.value
-    if out is None:
-        out = torch.empty((k, width), dtype=torch.uint8, device=dev)
-    if ids_out is None:
-        ids_out = torch.empty(k, dtype=torch.int64, device=dev)
-    if len(out) < k or len(ids_out) < k:
-        raise ValueError("out / ids_out hold %d / %d records, %d are ready" % (len(out), len(ids_out), k))
-    if k:
-        torch.cuda.current_stream(dev).synchronize()                   # the caller's work on out / ids_out comes first
-        call(out.data_ptr(), len(out), C.byref(n), ids_out.data_ptr())
-    return out[:n.value], ids_out[:n.value]
-
-
 def positions_to_training_device(engine: "Engine", positions, indices=None):
     """spb_positions_to_training_device: the tensors of positions_to_training(engine.game, ...), built on the engine's GPU
     -> torch CUDA tensors (encodings[n,3,R,C], policies[n,A], values[n,1]) f32, bit-identical to the host builder.
@@ -334,16 +305,23 @@ def positions_to_training_device(engine: "Engine", positions, indices=None):
     buffer kept in device memory.  indices (numpy or CUDA int64 / uint64 tensor): row i is built from
     positions[indices[i]]; without it every record is built.  An index out of range raises EngineError(-1) and nothing is
     written."""
+    return _positions_to_training_device(engine, positions, indices, (3,) + BOARD[engine.game])
+
+
+def _positions_to_training_device(engine, positions, indices, encoding_shape):
+    """positions_to_training_device and chess.positions_to_training_device: records of the engine's record dtype, an
+    encoding of `encoding_shape` and a policy of engine.A entries per row."""
     import torch
+    width = engine._RECORD.itemsize
     if isinstance(positions, torch.Tensor):
-        _check_cuda_tensor(positions, torch.uint8, POSITION_DTYPE.itemsize, "positions")
+        _check_cuda_tensor(positions, torch.uint8, width, "positions")
         pos = positions
     if indices is not None and isinstance(indices, torch.Tensor):
         _check_cuda_tensor(indices, (torch.int64, torch.uint64), None, "indices")
     dev = torch.device("cuda", engine.device)
     if not isinstance(positions, torch.Tensor):
-        a = np.ascontiguousarray(positions, dtype=POSITION_DTYPE).reshape(-1)
-        pos = torch.from_numpy(a.view(np.uint8).reshape(len(a), POSITION_DTYPE.itemsize)).to(dev)
+        a = np.ascontiguousarray(positions, dtype=engine._RECORD).reshape(-1)
+        pos = torch.from_numpy(a.view(np.uint8).reshape(len(a), width)).to(dev)
     idx = None
     if indices is not None:
         if isinstance(indices, torch.Tensor):
@@ -354,39 +332,46 @@ def positions_to_training_device(engine: "Engine", positions, indices=None):
                 raise TypeError("indices must be integers, not %s" % i.dtype)
             idx = torch.from_numpy(i.astype(np.int64)).to(dev)
     n = len(pos) if idx is None else len(idx)
-    R, Cc = BOARD[engine.game]
-    enc = torch.empty((n, 3, R, Cc), dtype=torch.float32, device=dev)
-    pol = torch.empty((n, NUM_ACTIONS[engine.game]), dtype=torch.float32, device=dev)
+    enc = torch.empty((n,) + encoding_shape, dtype=torch.float32, device=dev)
+    pol = torch.empty((n, engine.A), dtype=torch.float32, device=dev)
     val = torch.empty((n, 1), dtype=torch.float32, device=dev)
     torch.cuda.current_stream(dev).synchronize()                       # the engine's stream reads the inputs
-    engine._chk(engine._L.spb_positions_to_training_device(
+    engine._chk(engine._fn("positions_to_training_device")(
         engine._h, pos.data_ptr() if len(pos) else None, len(pos), None if idx is None else idx.data_ptr(), n,
         enc.data_ptr(), pol.data_ptr(), val.data_ptr()))
     return enc, pol, val
 
 
-class Engine:
-    """One engine = `Mcts` + its `Vec<Tree>` on one GPU (ref: mcts.rs:41-44, learner_concurrent.rs:174)."""
+class EngineBase:
+    """The entry points Engine and ChessEngine share, each stated once.  What differs between the two is a class attribute
+    of each:
+      _PREFIX       the entry points' prefix, "spb_" or "spb_chess_";
+      _RECORD       the numpy dtype of a trajectory record;
+      _STATE        the numpy dtype of a state, as advance returns it;
+      _ROOT_WIDTH   the children a root row holds, and _MOVE the numpy type of their moves;
+      A             the width of a root_policy row."""
 
-    def __init__(self, game=GAME_C4, num_games=100, evaluator=EVAL_NET, c=2.0, device=0, max_nodes_per_tree=0,
-                 flags=0, leaves_per_tree=1, game_id_base=0, game_id_stride=0, trajectory_capacity=0):
+    def __init__(self, **config):
+        """Creates the engine from `config`, fields of Config; the others keep spb_default_config's values."""
         L = load_library()
         cfg = Config()
         L.spb_default_config(C.byref(cfg))
-        cfg.game, cfg.num_games, cfg.evaluator, cfg.c, cfg.device = game, num_games, evaluator, c, device
-        cfg.max_nodes_per_tree, cfg.flags, cfg.leaves_per_tree = max_nodes_per_tree, flags, leaves_per_tree
-        cfg.game_id_base, cfg.game_id_stride = game_id_base, game_id_stride
-        cfg.trajectory_capacity = trajectory_capacity
+        for k, v in config.items():
+            setattr(cfg, k, v)
         h = _vp()
-        rc = L.spb_create(C.byref(cfg), C.byref(h))
+        rc = getattr(L, self._PREFIX + "create")(C.byref(cfg), C.byref(h))
         if rc != 0:
-            raise EngineError(rc, L.spb_last_error(None).decode())
+            raise EngineError(rc, getattr(L, self._PREFIX + "last_error")(None).decode())
         self._h, self._L = h, L
-        self.game, self.G, self.A, self.device = game, num_games, NUM_ACTIONS[game], device
+        self.G, self.device = config["num_games"], config["device"]
+
+    def _fn(self, name):
+        """The entry point of this engine's prefix: "search" -> spb_search or spb_chess_search."""
+        return getattr(self._L, self._PREFIX + name)
 
     def close(self):
         if getattr(self, "_h", None):
-            self._L.spb_destroy(self._h)
+            self._fn("destroy")(self._h)
             self._h = None
 
     def __del__(self):
@@ -403,21 +388,174 @@ class Engine:
 
     def _chk(self, rc):
         if rc != 0:
-            raise EngineError(rc, self._L.spb_last_error(self._h).decode())
+            raise EngineError(rc, self._fn("last_error")(self._h).decode())
 
     # ---- weights -----------------------------------------------------------------------------
     def load_weights(self, blob: bytes):
         buf = (C.c_char * len(blob)).from_buffer_copy(blob)
-        self._chk(self._L.spb_load_weights(self._h, C.cast(buf, _vp), len(blob)))
+        self._chk(self._fn("load_weights")(self._h, C.cast(buf, _vp), len(blob)))
 
     def load_weights_device(self, named):
         """spb_load_weights_device: the net from (name, CUDA tensor) pairs on the engine's GPU, named as in a checkpoint
-        (explicit names or tch VarStore names); the same image as load_weights of a checkpoint of these tensors."""
-        _load_weights_device(lambda t, n: self._chk(self._L.spb_load_weights_device(self._h, t, n)), named, self.device)
+        (the names load_weights accepts); the same image as load_weights of a checkpoint of these tensors."""
+        import torch
+        # the caller's writes to the tensors finish before the engine reads them; `items` and `names` keep the tensors and
+        # the table's names alive until the call has returned, after which the engine no longer reads them
+        items = list(named.items()) if hasattr(named, "items") else list(named)
+        table, n, names = tensor_table(items, self.device)
+        torch.cuda.current_stream(torch.device("cuda", self.device)).synchronize()
+        self._chk(self._fn("load_weights_device")(self._h, table, n))
 
     def broadcast_weights(self, root: int = 0):
         """COLLECTIVE: every rank takes root's weight image (spb_broadcast_weights)."""
-        self._chk(self._L.spb_broadcast_weights(self._h, root))
+        self._chk(self._fn("broadcast_weights")(self._h, root))
+
+    # ---- trees -------------------------------------------------------------------------------
+    def search(self, num_searches: int):
+        self._chk(self._fn("search")(self._h, num_searches))
+
+    def root_children(self, slot: int):
+        """-> (moves, visit_counts, child_ids) of `slot`'s root as lists, child order."""
+        mv = np.zeros(self._ROOT_WIDTH, self._MOVE)
+        cnt, ids = np.zeros(self._ROOT_WIDTH, np.uint32), np.zeros(self._ROOT_WIDTH, np.uint32)
+        n = C.c_uint32()
+        self._chk(self._fn("root_children")(self._h, slot, *map(np.ctypeslib.as_ctypes, (mv, cnt, ids)), C.byref(n)))
+        k = n.value
+        return mv[:k].tolist(), cnt[:k].tolist(), ids[:k].tolist()
+
+    def root_children_all(self, out=None):
+        """-> (moves[G,W], visit_counts[G,W] u32, child_ids[G,W] u32, n_children[G] u32), child order; W and the move type
+        are _ROOT_WIDTH and _MOVE (9 u8 actions, or 256 u16 chess moves).  `out`: the four arrays of an earlier call (e.g.
+        in pinned host memory), written in place."""
+        W = self._ROOT_WIDTH
+        if out is not None:
+            mv, cnt, ids, n = out
+            assert mv.shape == (self.G, W) and mv.dtype == self._MOVE and cnt.dtype == np.uint32 and ids.dtype == np.uint32 and n.shape == (self.G,)
+            assert all(x.flags.c_contiguous for x in out)
+        else:
+            mv = np.zeros((self.G, W), self._MOVE)
+            cnt = np.zeros((self.G, W), np.uint32)
+            ids = np.zeros((self.G, W), np.uint32)
+            n = np.zeros(self.G, np.uint32)
+        self._chk(self._fn("root_children_all")(self._h, mv.ctypes.data, cnt.ctypes.data, ids.ctypes.data, n.ctypes.data))
+        return mv, cnt, ids, n
+
+    def root_policy(self, slot: int) -> np.ndarray:
+        p = np.zeros(self.A, np.float32)
+        self._chk(self._fn("root_policy")(self._h, slot, p.ctypes.data_as(_f32p)))
+        return p
+
+    def advance(self, node_ids, slots=None) -> np.ndarray:
+        ids = np.ascontiguousarray(node_ids, dtype=np.uint32)
+        sl = None if slots is None else np.ascontiguousarray(slots, dtype=np.uint32)
+        out = np.zeros(len(ids), dtype=self._STATE)
+        self._chk(self._fn("advance")(self._h, None if sl is None else sl.ctypes.data, ids.ctypes.data, len(ids), out.ctypes.data))
+        return out
+
+    def arena_len(self, slot: int) -> int:
+        n = C.c_uint32()
+        self._chk(self._fn("arena_len")(self._h, slot, C.byref(n)))
+        return n.value
+
+    # ---- EXTENSION: Dirichlet noise at the root (DESIGN.md §4.6) ------------------------------
+    def set_root_noise(self, alpha: float, epsilon: float, seed: int = 0):
+        """P' = (1 - epsilon) P + epsilon eta, eta ~ Dir(alpha), at the root of every search; epsilon = 0 turns it off."""
+        self._chk(self._fn("set_root_noise")(self._h, alpha, epsilon, seed))
+
+    def root_noise(self, slot: int) -> np.ndarray:
+        """The eta the next search of `slot`'s root uses, one entry per root child (child order)."""
+        eta = np.zeros(self._ROOT_WIDTH, np.float32)
+        n = C.c_uint32()
+        self._chk(self._fn("root_noise")(self._h, slot, eta.ctypes.data_as(_f32p), C.byref(n)))
+        return eta[:n.value].copy()
+
+    # ---- trajectories ------------------------------------------------------------------------
+    def drain_trajectories(self):
+        """-> (positions[_RECORD], game_ids[u64]) ordered by (game id, ply)."""
+        return self._records(functools.partial(self._fn("drain_trajectories"), self._h))
+
+    def drain_trajectories_device(self, out=None, ids_out=None):
+        """The records of drain_trajectories, ordered on the device -> (CUDA uint8 [n, record bytes], CUDA int64 [n]).
+        out / ids_out: caller tensors to write into (e.g. replay[head:]); the [:n] views of them are returned."""
+        return self._records_to_device(functools.partial(self._fn("drain_trajectories_device"), self._h), out, ids_out)
+
+    def gather_trajectories(self, learner_rank: int = 0):
+        """COLLECTIVE: -> (positions, game_ids) ordered by (game id, ply) on the learner rank, empty elsewhere."""
+        return self._records(functools.partial(self._fn("gather_trajectories"), self._h, learner_rank))
+
+    def gather_trajectories_device(self, learner_rank: int = 0, out=None, ids_out=None):
+        """COLLECTIVE: gather_trajectories into device memory of the learner rank -> (CUDA uint8 [n, record bytes], CUDA
+        int64 [n]), empty elsewhere; out / ids_out as for drain_trajectories_device."""
+        return self._records_to_device(functools.partial(self._fn("gather_trajectories_device"), self._h, learner_rank),
+                                       out, ids_out)
+
+    def _records(self, call):
+        """The host forms of drain / gather: `call(buf, capacity, n_ref, ids)` is the entry point with the engine's
+        arguments bound.  Size query, then the records -> the [:n] the second call wrote."""
+        n = C.c_size_t()
+        self._chk(call(None, 0, C.byref(n), None))
+        pos = np.zeros(n.value, dtype=self._RECORD)
+        ids = np.zeros(n.value, dtype=np.uint64)
+        if n.value:
+            self._chk(call(pos.ctypes.data, n.value, C.byref(n), ids.ctypes.data))
+        return pos[:n.value], ids[:n.value]
+
+    def _records_to_device(self, call, out, ids_out):
+        """The device forms of drain / gather, `call` as for _records: the records into `out` / `ids_out` (allocated when
+        None) -> their [:n] views."""
+        import torch
+        width = self._RECORD.itemsize
+        if out is not None:
+            _check_cuda_tensor(out, torch.uint8, width, "out")
+        if ids_out is not None:
+            _check_cuda_tensor(ids_out, torch.int64, None, "ids_out")
+        dev = torch.device("cuda", self.device)
+        n = C.c_size_t()
+        self._chk(call(None, 0, C.byref(n), None))
+        k = n.value
+        if out is None:
+            out = torch.empty((k, width), dtype=torch.uint8, device=dev)
+        if ids_out is None:
+            ids_out = torch.empty(k, dtype=torch.int64, device=dev)
+        if len(out) < k or len(ids_out) < k:
+            raise ValueError("out / ids_out hold %d / %d records, %d are ready" % (len(out), len(ids_out), k))
+        if k:
+            torch.cuda.current_stream(dev).synchronize()                   # the caller's work on out / ids_out comes first
+            self._chk(call(out.data_ptr(), len(out), C.byref(n), ids_out.data_ptr()))
+        return out[:n.value], ids_out[:n.value]
+
+    # ---- multi-GPU: trajectories to the learner rank --------------------------------------------
+    def comm_init(self, comm_id: bytes, rank: int, world_size: int):
+        buf = (C.c_uint8 * COMM_ID_BYTES).from_buffer_copy(comm_id)
+        self._chk(self._fn("comm_init")(self._h, C.cast(buf, _vp), rank, world_size))
+
+    def comm_destroy(self):
+        self._chk(self._fn("comm_destroy")(self._h))
+
+    # ---- counters ----------------------------------------------------------------------------
+    def counters(self) -> dict:
+        return self._read_counters().as_dict()
+
+    def _read_counters(self) -> Counters:
+        c = Counters()
+        self._chk(self._fn("get_counters")(self._h, C.byref(c)))
+        return c
+
+    def reset_counters(self):
+        self._chk(self._fn("reset_counters")(self._h))
+
+
+class Engine(EngineBase):
+    """One engine = `Mcts` + its `Vec<Tree>` on one GPU (ref: mcts.rs:41-44, learner_concurrent.rs:174)."""
+    _PREFIX, _RECORD, _STATE, _ROOT_WIDTH, _MOVE = "spb_", POSITION_DTYPE, STATE_DTYPE, MAX_ACTIONS, np.uint8
+    A = property(lambda self: NUM_ACTIONS[self.game], doc="The game's actions: the width of a policy row.")
+
+    def __init__(self, game=GAME_C4, num_games=100, evaluator=EVAL_NET, c=2.0, device=0, max_nodes_per_tree=0,
+                 flags=0, leaves_per_tree=1, game_id_base=0, game_id_stride=0, trajectory_capacity=0):
+        super().__init__(game=game, num_games=num_games, evaluator=evaluator, c=c, device=device,
+                         max_nodes_per_tree=max_nodes_per_tree, flags=flags, leaves_per_tree=leaves_per_tree,
+                         game_id_base=game_id_base, game_id_stride=game_id_stride, trajectory_capacity=trajectory_capacity)
+        self.game = game
 
     # ---- trees -------------------------------------------------------------------------------
     def reset_games(self, roots=None, slots=None):
@@ -429,70 +567,16 @@ class Engine:
         self._chk(self._L.spb_reset_games(self._h, None if sl is None else sl.ctypes.data, n,
                                           None if arr is None else arr.ctypes.data))
 
-    def search(self, num_searches: int):
-        self._chk(self._L.spb_search(self._h, num_searches))
-
-    def root_children(self, slot: int):
-        a, c, i = (C.c_uint8 * MAX_ACTIONS)(), (C.c_uint32 * MAX_ACTIONS)(), (C.c_uint32 * MAX_ACTIONS)()
-        n = C.c_uint32()
-        self._chk(self._L.spb_root_children(self._h, slot, a, c, i, C.byref(n)))
-        k = n.value
-        return list(a[:k]), list(c[:k]), list(i[:k])
-
-    def root_children_all(self, out=None):
-        """-> (actions[G,9] u8, visit_counts[G,9] u32, child_ids[G,9] u32, n_children[G] u32), child order.
-        `out`: the four arrays of an earlier call (e.g. in pinned host memory), written in place."""
-        if out is not None:
-            a, c, i, n = out
-            assert a.shape == (self.G, MAX_ACTIONS) and a.dtype == np.uint8 and c.dtype == np.uint32 and i.dtype == np.uint32 and n.shape == (self.G,)
-            assert all(x.flags.c_contiguous for x in out)
-        else:
-            a = np.zeros((self.G, MAX_ACTIONS), np.uint8)
-            c = np.zeros((self.G, MAX_ACTIONS), np.uint32)
-            i = np.zeros((self.G, MAX_ACTIONS), np.uint32)
-            n = np.zeros(self.G, np.uint32)
-        self._chk(self._L.spb_root_children_all(self._h, a.ctypes.data, c.ctypes.data, i.ctypes.data, n.ctypes.data))
-        return a, c, i, n
-
-    def root_policy(self, slot: int) -> np.ndarray:
-        p = np.zeros(self.A, np.float32)
-        self._chk(self._L.spb_root_policy(self._h, slot, p.ctypes.data_as(_f32p)))
-        return p
-
-    def advance(self, node_ids, slots=None) -> np.ndarray:
-        ids = np.ascontiguousarray(node_ids, dtype=np.uint32)
-        sl = None if slots is None else np.ascontiguousarray(slots, dtype=np.uint32)
-        out = np.zeros(len(ids), dtype=STATE_DTYPE)
-        self._chk(self._L.spb_advance(self._h, None if sl is None else sl.ctypes.data, ids.ctypes.data, len(ids), out.ctypes.data))
-        return out
-
     def get_state(self, slot: int, node_id: int) -> State:
         s = State()
         self._chk(self._L.spb_get_state(self._h, slot, node_id, C.byref(s)))
         return s
-
-    def arena_len(self, slot: int) -> int:
-        n = C.c_uint32()
-        self._chk(self._L.spb_arena_len(self._h, slot, C.byref(n)))
-        return n.value
 
     def node_stats(self, slot: int, node_id: int) -> dict:
         n, fc, nc = C.c_uint32(), C.c_uint32(), C.c_uint32()
         w, p = C.c_float(), C.c_float()
         self._chk(self._L.spb_node_stats(self._h, slot, node_id, C.byref(n), C.byref(w), C.byref(p), C.byref(fc), C.byref(nc)))
         return dict(visit_count=n.value, value_sum=w.value, prior=p.value, first_child=fc.value, n_children=nc.value)
-
-    # ---- EXTENSION: Dirichlet noise at the root (DESIGN.md §4.6) ------------------------------
-    def set_root_noise(self, alpha: float, epsilon: float, seed: int = 0):
-        """P' = (1 - epsilon) P + epsilon eta, eta ~ Dir(alpha), at the root of every search; epsilon = 0 turns it off."""
-        self._chk(self._L.spb_set_root_noise(self._h, alpha, epsilon, seed))
-
-    def root_noise(self, slot: int) -> np.ndarray:
-        """The eta the next search of `slot`'s root uses, one entry per root child (child order)."""
-        eta = np.zeros(MAX_ACTIONS, np.float32)
-        n = C.c_uint32()
-        self._chk(self._L.spb_root_noise(self._h, slot, eta.ctypes.data_as(_f32p), C.byref(n)))
-        return eta[:n.value].copy()
 
     # ---- evaluator / game rules --------------------------------------------------------------
     def predict(self, states, want_logits=False):
@@ -535,56 +619,7 @@ class Engine:
         self._chk(self._L.spb_selfplay_step(self._h, rule, temperature, seed, None if arr is None else arr.ctypes.data, C.byref(fin)))
         return fin.value
 
-    def drain_trajectories(self):
-        """-> (positions[POSITION_DTYPE], game_ids[u64]) ordered by (game id, ply)."""
-        n = C.c_size_t()
-        self._chk(self._L.spb_drain_trajectories(self._h, None, 0, C.byref(n), None))
-        pos = np.zeros(n.value, dtype=POSITION_DTYPE)
-        ids = np.zeros(n.value, dtype=np.uint64)
-        if n.value:
-            self._chk(self._L.spb_drain_trajectories(self._h, pos.ctypes.data, n.value, C.byref(n), ids.ctypes.data))
-        return pos[:n.value], ids[:n.value]
-
-    def drain_trajectories_device(self, out=None, ids_out=None):
-        """The records of drain_trajectories, ordered on the device -> (CUDA uint8 [n, 56], CUDA int64 [n]).  out / ids_out:
-        caller tensors to write into (e.g. replay[head:]); the [:n] views of them are returned."""
-        return _records_to_device(lambda b, cap, n, i: self._chk(self._L.spb_drain_trajectories_device(self._h, b, cap, n, i)),
-                                  self.device, POSITION_DTYPE.itemsize, out, ids_out)
-
-    # ---- multi-GPU: trajectories to the learner rank --------------------------------------------
-    def comm_init(self, comm_id: bytes, rank: int, world_size: int):
-        buf = (C.c_uint8 * COMM_ID_BYTES).from_buffer_copy(comm_id)
-        self._chk(self._L.spb_comm_init(self._h, C.cast(buf, _vp), rank, world_size))
-
-    def comm_destroy(self):
-        self._chk(self._L.spb_comm_destroy(self._h))
-
-    def gather_trajectories(self, learner_rank: int = 0):
-        """COLLECTIVE: -> (positions, game_ids) ordered by (game id, ply) on the learner rank, empty elsewhere."""
-        n = C.c_size_t()
-        self._chk(self._L.spb_gather_trajectories(self._h, learner_rank, None, 0, C.byref(n), None))
-        pos = np.zeros(n.value, dtype=POSITION_DTYPE)
-        ids = np.zeros(n.value, dtype=np.uint64)
-        if n.value:
-            self._chk(self._L.spb_gather_trajectories(self._h, learner_rank, pos.ctypes.data, n.value, C.byref(n), ids.ctypes.data))
-        return pos, ids
-
-    def gather_trajectories_device(self, learner_rank: int = 0, out=None, ids_out=None):
-        """COLLECTIVE: gather_trajectories into device memory of the learner rank -> (CUDA uint8 [n, 56], CUDA int64 [n]),
-        empty elsewhere; out / ids_out as for drain_trajectories_device."""
-        return _records_to_device(
-            lambda b, cap, n, i: self._chk(self._L.spb_gather_trajectories_device(self._h, learner_rank, b, cap, n, i)),
-            self.device, POSITION_DTYPE.itemsize, out, ids_out)
-
-    # ---- counters ----------------------------------------------------------------------------
-    def counters(self) -> dict:
-        c = Counters()
-        self._chk(self._L.spb_get_counters(self._h, C.byref(c)))
-        return c.as_dict()
-
-    def reset_counters(self):
-        self._chk(self._L.spb_reset_counters(self._h))
-
+    # ---- timing ------------------------------------------------------------------------------
     def last_search_timing(self):
         s, ev, n = C.c_float(), C.c_float(), C.c_uint32()
         self._chk(self._L.spb_last_search_timing(self._h, C.byref(s), C.byref(ev), C.byref(n)))

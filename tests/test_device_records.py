@@ -1,7 +1,8 @@
 """The learner hand-off in device memory: spb_drain_trajectories_device / spb_chess_drain_trajectories_device,
 spb_gather_trajectories_device / spb_chess_gather_trajectories_device and spb_positions_to_training_device.
 
-CPU: the Python wrappers reject CPU tensors, wrong dtypes and wrong widths before they reach the library.
+CPU: the Python wrappers reject CPU tensors, wrong dtypes and wrong widths before they reach the library, and the
+methods both engines share ask for entry points the library declares.
 GPU: every device form equals its host form byte for byte (records, ids, training tensors) for Connect4, tic-tac-toe and
 chess; size queries, short and host buffers, offset slices, parking, staging across calls and the form rules of a pending
 gather; with two GPUs, a two-rank device gather equals one rank playing all the games.
@@ -51,14 +52,61 @@ def test_wrappers_reject_cpu_tensors_wrong_dtypes_and_widths():
             drain(ids_out=torch.zeros(4, dtype=torch.float64))
         with pytest.raises(TypeError, match="CUDA"):
             drain(ids_out=torch.zeros(4, dtype=torch.int64))
-    with pytest.raises(TypeError, match="CUDA"):
-        S.positions_to_training_device(c4, torch.zeros((4, W_C4), dtype=torch.uint8))
-    with pytest.raises(ValueError, match="n, 56"):
-        S.positions_to_training_device(c4, torch.zeros((4, W_CHESS), dtype=torch.uint8))
-    with pytest.raises(TypeError, match="torch.uint8"):
-        S.positions_to_training_device(c4, torch.zeros((4, W_C4), dtype=torch.float32))
-    with pytest.raises(TypeError, match="indices"):
-        S.positions_to_training_device(c4, np.zeros(4, S.POSITION_DTYPE), torch.zeros(4, dtype=torch.float32))
+    for build, e, width, other, dtype in ((S.positions_to_training_device, c4, W_C4, W_CHESS, S.POSITION_DTYPE),
+                                          (CH.positions_to_training_device, chess, W_CHESS, W_C4, CH.CHESS_POSITION_DTYPE)):
+        with pytest.raises(TypeError, match="CUDA"):
+            build(e, torch.zeros((4, width), dtype=torch.uint8))
+        with pytest.raises(ValueError, match="n, %d" % width):
+            build(e, torch.zeros((4, other), dtype=torch.uint8))
+        with pytest.raises(TypeError, match="torch.uint8"):
+            build(e, torch.zeros((4, width), dtype=torch.float32))
+        with pytest.raises(TypeError, match="indices"):
+            build(e, np.zeros(4, dtype), torch.zeros(4, dtype=torch.float32))
+
+
+class RecordingLibrary:
+    """A stand-in for the library: records the name of every entry point asked for, and each returns 0."""
+
+    def __init__(self):
+        self.names = []
+
+    def __getattr__(self, name):
+        self.names.append(name)
+        return lambda *args: 0
+
+
+def test_shared_methods_call_entry_points_of_their_prefix(monkeypatch):
+    """EngineBase looks its entry points up by name at run time: each name either class asks for is declared, with the
+    class's prefix, and both ask for the same entry points."""
+    stems = {}
+    for cls, prefix, attrs in ((S.Engine, "spb_", dict(game=S.GAME_C4)), (CH.ChessEngine, "spb_chess_", {})):
+        lib = RecordingLibrary()
+        monkeypatch.setattr(S.engine, "load_library", lambda: lib)
+        cls()                                                          # its handle stays NULL: nothing to destroy
+        e = fake(cls, _L=lib, _h=C.c_void_p(1), G=2, **attrs)
+        e.load_weights(b"\0" * 8)
+        e.broadcast_weights(0)
+        e.search(1)
+        e.root_children(0)
+        e.root_children_all()
+        e.root_policy(0)
+        e.advance([1])
+        e.arena_len(0)
+        e.set_root_noise(0.3, 0.25, 1)
+        e.root_noise(0)
+        e.drain_trajectories()
+        e.gather_trajectories(0)
+        e.comm_init(bytes(S.COMM_ID_BYTES), 0, 1)
+        e.comm_destroy()
+        e.counters()
+        e.reset_counters()
+        e.close()
+        names = [n for n in lib.names if n != "spb_default_config"]
+        assert all(n in S.engine.ABI and n.startswith(prefix) for n in names), names
+        stems[cls] = [n[len(prefix):] for n in names]
+        with pytest.raises(S.EngineError):                             # _chk reads the message through the library
+            fake(cls)._chk(-1)
+    assert stems[S.Engine] == stems[CH.ChessEngine] and len(stems[S.Engine]) == 18   # one per call above, and create
 
 
 # ---- GPU: helpers ----------------------------------------------------------------------------------------------------
