@@ -183,6 +183,8 @@ int32_t spb_load_weights_device(spb_engine* e, const spb_tensor* tensors, uint32
 /*
  * (Re)start the trees in `slots[0..n)` from `roots[i]`; roots == NULL means the
  * default state (empty board, X to move).  slots == NULL means slots 0..n-1.
+ * SPB_ERR_ARG, with no tree touched, if n > num_games or a slot is out of range or
+ * listed twice.
  */
 int32_t spb_reset_games(spb_engine* e, const uint32_t* slots, uint32_t n, const spb_state* roots);
 
@@ -201,15 +203,19 @@ int32_t spb_search(spb_engine* e, uint32_t num_searches);
 /*
  * ref: mcts.rs:310-331 — the second element of search()'s result for one tree:
  * for each root child in child (= legal action) order: action taken, visit count,
- * arena id.  Any output pointer may be NULL.  Arrays need SPB_MAX_ACTIONS entries.
+ * arena id.  Any output pointer may be NULL, n_children too.  Arrays need
+ * SPB_MAX_ACTIONS entries and are written whole: entries past n_children hold
+ * action 0xFF, count 0 and id 0.
  */
 int32_t spb_root_children(spb_engine* e, uint32_t slot, uint8_t* actions,
                           uint32_t* visit_counts, uint32_t* child_ids, uint32_t* n_children);
 
 /*
- * Batched form for all G slots in one device->host copy.  Row i belongs to slot i;
- * visit_counts / child_ids are [G][SPB_MAX_ACTIONS] indexed by CHILD ORDER,
- * actions likewise; n_children is [G].
+ * Batched form for all G slots: one device->host copy per non-NULL array, straight
+ * into it, and one synchronise.  Row i belongs to slot i, written whole as by
+ * spb_root_children; visit_counts / child_ids are [G][SPB_MAX_ACTIONS] indexed by
+ * CHILD ORDER, actions likewise; n_children is [G].  Any pointer may be NULL.
+ * Page-locked arrays make the copies direct.
  */
 int32_t spb_root_children_all(spb_engine* e, uint8_t* actions, uint32_t* visit_counts,
                               uint32_t* child_ids, uint32_t* n_children);
@@ -225,6 +231,9 @@ int32_t spb_root_policy(spb_engine* e, uint32_t slot, float* policy);
  * ref: Tree::use_subtree mcts.rs:161-192.  Re-roots slot[i] at arena node
  * node_ids[i] (BFS compaction that keeps visit_count / value_sum / prior and child
  * order).  out_states (nullable) receives the new root state of each slot.
+ * slots == NULL means slots 0..n-1.  Every entry is checked before any tree moves:
+ * n > num_games, a slot out of range or listed twice, or a node id outside its
+ * slot's arena is SPB_ERR_ARG with no tree touched.
  */
 int32_t spb_advance(spb_engine* e, const uint32_t* slots, const uint32_t* node_ids,
                     uint32_t n, spb_state* out_states);
@@ -386,20 +395,25 @@ int32_t spb_chess_policy_index(int32_t side, uint16_t move);
 uint16_t spb_chess_action(int32_t side, int32_t channel, int32_t row, int32_t col);
 
 /* Tree::with_root_state (mcts.rs:86-89) for n slots (slots NULL = 0..n-1; roots NULL = the start position; history
- * [n][SPB_CHESS_MAX_HISTORY], NULL = games that start at their root). */
+ * [n][SPB_CHESS_MAX_HISTORY], NULL = games that start at their root).  SPB_ERR_ARG, with no tree touched, if n > num_games,
+ * a slot is out of range or listed twice, or a root is malformed. */
 int32_t spb_chess_reset_games(spb_chess_engine* e, const uint32_t* slots, uint32_t n, const spb_chess_state* roots, const uint64_t* history);
 /* Mcts::search (mcts.rs:196-332): num_searches simulations for every live tree.  SPB_EVAL_NET runs the reference's loop
  * literally — per simulation one select over all trees, one network batch, one expand + backup. */
 int32_t spb_chess_search(spb_chess_engine* e, uint32_t num_searches);
 int32_t spb_chess_last_search_ms(spb_chess_engine* e, float* ms);   /* device time of the last spb_chess_search */
 /* Result of search for one tree / all trees (mcts.rs:315-328), child order: moves, visit counts, arena ids; arrays of
- * SPB_CHESS_MAX_MOVES entries per tree. */
+ * SPB_CHESS_MAX_MOVES entries per tree, written whole (entries past n_children: move 0xFFFF, count 0, id 0).  Any pointer may
+ * be NULL, n_children too.  The batched form makes one device->host copy per non-NULL array, straight into it, and one
+ * synchronise. */
 int32_t spb_chess_root_children(spb_chess_engine* e, uint32_t slot, uint16_t* moves, uint32_t* visit_counts, uint32_t* child_ids, uint32_t* n_children);
 int32_t spb_chess_root_children_all(spb_chess_engine* e, uint16_t* moves, uint32_t* visit_counts, uint32_t* child_ids, uint32_t* n_children);
 /* The Policy half of the result: visit counts scattered by set_prob and normalised, out[SPB_CHESS_POLICY_SIZE]. */
 int32_t spb_chess_root_policy(spb_chess_engine* e, uint32_t slot, float* out);
-/* Tree::use_subtree(child id) (mcts.rs:161-192) for n trees; the root position advances, the game history grows by one
- * ply.  out_states (nullable) receives the new root states.  SPB_ERR_ARG if an id is not a child of its root. */
+/* Tree::use_subtree(child id) (mcts.rs:161-192) for n trees (slots NULL = 0..n-1); the root position advances, the game
+ * history grows by one ply.  out_states (nullable) receives the new root states.  Every entry is checked before any tree
+ * moves: n > num_games, a slot out of range or listed twice, or an id that is not a child of its root is SPB_ERR_ARG, a
+ * full history SPB_ERR_STATE, and then no tree moves (out_states receive the unchanged roots). */
 int32_t spb_chess_advance(spb_chess_engine* e, const uint32_t* slots, const uint32_t* child_ids, uint32_t n, spb_chess_state* out_states);
 /* arena[node_id].state (mcts.rs:22). */
 int32_t spb_chess_get_state(spb_chess_engine* e, uint32_t slot, uint32_t node_id, spb_chess_state* out);

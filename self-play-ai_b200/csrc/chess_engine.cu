@@ -322,7 +322,8 @@ __global__ void k_chess_root_children(CTrees T, uint16_t* moves, uint32_t* count
 // copies the children of the 32 nodes one node after the other (lanes stride over up to 218 children).  A copied node
 // keeps its OLD first_child in rec.w until its own turn in the window.  The root position advances by the child's move
 // and the hash of the old root's move list joins the game history (chess.rs:121-122).  The caller has checked that `id`
-// is a child of the root and that the history has room; lane 0 writes the new root to *out_state when it is not null.
+// is a child of the root and that the history has room (k_chess_advance_check); lane 0 writes the new root to *out_state
+// when it is not null.
 __device__ __forceinline__ void reroot(const CTrees& T, uint32_t g, uint32_t id, int lane, Pos* out_state) {
   const uint32_t b = T.buf[g], nb = b ^ 1u;
   const uint4* orec = T.rec[b] + (size_t)g * T.cap;
@@ -380,10 +381,11 @@ __device__ __forceinline__ void reroot(const CTrees& T, uint32_t g, uint32_t id,
   }
 }
 
-__global__ void __launch_bounds__(THREADS) k_chess_advance(CTrees T, const uint32_t* slots, const uint32_t* node_ids, uint32_t n, Pos* out_states,
-                                                           int32_t* out_err) {
-  const int lane = threadIdx.x & 31;
-  const uint32_t i = blockIdx.x * WARPS + (threadIdx.x >> 5);
+// The checks of spb_chess_advance, one thread per entry, before any tree moves: out_err[i], and a flag in *bad when an
+// entry failed.
+__global__ void k_chess_advance_check(CTrees T, const uint32_t* slots, const uint32_t* node_ids, uint32_t n, int32_t* out_err,
+                                      unsigned long long* bad) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   const uint32_t g = slots ? slots[i] : i;
   const uint2* ometa = T.meta[T.buf[g]] + (size_t)g * T.cap;
@@ -391,12 +393,23 @@ __global__ void __launch_bounds__(THREADS) k_chess_advance(CTrees T, const uint3
   int32_t err = SPB_OK;
   if (!T.live[g] || id == 0 || id >= T.n_nodes[g] || ometa[id].x != 0u) err = SPB_ERR_ARG;        // must be a child of the root
   else if (T.root[g].hist_len >= SPB_CHESS_MAX_HISTORY) err = SPB_ERR_STATE;
-  if (err != SPB_OK) {
-    if (lane == 0) { out_err[i] = err; if (out_states) out_states[i] = T.root[g]; }
+  out_err[i] = err;
+  if (err != SPB_OK) atomicOr(bad, 1ull);
+}
+
+// Re-roots every entry when k_chess_advance_check found no fault (*bad == 0); otherwise no tree moves and out_states
+// receive the unchanged roots.
+__global__ void __launch_bounds__(THREADS) k_chess_advance(CTrees T, const uint32_t* slots, const uint32_t* node_ids, uint32_t n, Pos* out_states,
+                                                           const unsigned long long* bad) {
+  const int lane = threadIdx.x & 31;
+  const uint32_t i = blockIdx.x * WARPS + (threadIdx.x >> 5);
+  if (i >= n) return;
+  const uint32_t g = slots ? slots[i] : i;
+  if (*bad) {
+    if (lane == 0 && out_states) out_states[i] = T.root[g];
     return;
   }
-  if (lane == 0) out_err[i] = SPB_OK;
-  reroot(T, g, id, lane, out_states ? out_states + i : nullptr);
+  reroot(T, g, node_ids[i], lane, out_states ? out_states + i : nullptr);
 }
 
 // ---- self-play ply (ref: learner_concurrent.rs:179-238) ------------------------------------------------------------
@@ -713,10 +726,9 @@ static int32_t stage_roots(spb_chess_engine* e, const uint32_t* slots, const spb
 
 int32_t spb_chess_reset_games(spb_chess_engine* e, const uint32_t* slots, uint32_t n, const spb_chess_state* roots, const uint64_t* history) {
   SPB_GUARD(e);
-  SPB_ARG(e, n <= e->T.G, "more slots than games");
+  if (int32_t rc = e->check_slots(slots, n)) return rc;
   SPB_ARG(e, !(history && !roots), "history without roots");
   if (n == 0) return SPB_OK;
-  if (slots) for (uint32_t i = 0; i < n; ++i) SPB_ARG(e, slots[i] < e->T.G, "slot out of range");
   uint32_t* d_slots = nullptr; ch::Pos* d_roots = nullptr; unsigned long long* d_hist = nullptr;
   if (int32_t rc = stage_roots(e, slots, roots, history, n, &d_slots, &d_roots, &d_hist)) return rc;
   ch::k_chess_reset<<<n, 64, 0, e->stream>>>(e->T, e->P, d_slots, d_roots, d_hist, n);
@@ -737,12 +749,12 @@ static int32_t launch_chess_root_noise(spb_chess_engine* e) {
 
 int32_t spb_chess_set_root_noise(spb_chess_engine* e, float alpha, float epsilon, uint64_t seed) {
   SPB_GUARD(e);
-  return e->set_root_noise(alpha, epsilon, seed, SPB_CHESS_MAX_MOVES);
+  return e->set_root_noise(alpha, epsilon, seed);
 }
 
 int32_t spb_chess_root_noise(spb_chess_engine* e, uint32_t slot, float* eta, uint32_t* n) {
   SPB_GUARD(e);
-  return e->root_noise(slot, eta, n, SPB_CHESS_MAX_MOVES, [e] { return launch_chess_root_noise(e); });
+  return e->root_noise(slot, eta, n, [e] { return launch_chess_root_noise(e); });
 }
 
 int32_t spb_chess_search(spb_chess_engine* e, uint32_t num_searches) {
@@ -797,15 +809,13 @@ int32_t spb_chess_search(spb_chess_engine* e, uint32_t num_searches) {
     for (uint32_t s = 0; s < num_searches; ++s) {
       SPB_CUDA(e, cudaMemsetAsync(e->T.eval_count, 0, 4, e->stream));
       ch::k_chess_select<<<blocks, ch::THREADS, 0, e->stream>>>(e->T, all);
-      if (e->cfg.evaluator == SPB_EVAL_DET) ch::k_chess_builtin_eval<SPB_EVAL_DET><<<blocks, ch::THREADS, 0, e->stream>>>(e->T, all);
-      else ch::k_chess_builtin_eval<SPB_EVAL_UNIFORM><<<blocks, ch::THREADS, 0, e->stream>>>(e->T, all);
+      with_builtin_eval(e->cfg.evaluator, [&](auto ev) { ch::k_chess_builtin_eval<decltype(ev)::value><<<blocks, ch::THREADS, 0, e->stream>>>(e->T, all); });
       ch::k_chess_finish<true><<<blocks, ch::THREADS, 0, e->stream>>>(e->T, all);
       SPB_CUDA(e, cudaGetLastError());
       e->launches += 3;
     }
   } else {
-    if (e->cfg.evaluator == SPB_EVAL_DET) ch::k_chess_search_fused<SPB_EVAL_DET><<<blocks, ch::THREADS, 0, e->stream>>>(e->T, num_searches);
-    else ch::k_chess_search_fused<SPB_EVAL_UNIFORM><<<blocks, ch::THREADS, 0, e->stream>>>(e->T, num_searches);
+    with_builtin_eval(e->cfg.evaluator, [&](auto ev) { ch::k_chess_search_fused<decltype(ev)::value><<<blocks, ch::THREADS, 0, e->stream>>>(e->T, num_searches); });
     SPB_CUDA(e, cudaGetLastError());
     ++e->launches;
   }
@@ -832,30 +842,12 @@ static int32_t fetch_root_children(spb_chess_engine* e) {
 
 int32_t spb_chess_root_children_all(spb_chess_engine* e, uint16_t* moves, uint32_t* visit_counts, uint32_t* child_ids, uint32_t* n_children) {
   SPB_GUARD(e);
-  int32_t rc = fetch_root_children(e);
-  if (rc) return rc;
-  const size_t G = e->T.G, M = ch::MAX_MOVES;
-  if (moves) SPB_CUDA(e, cudaMemcpyAsync(moves, e->d_rc_moves, G * M * 2, cudaMemcpyDeviceToHost, e->stream));
-  if (visit_counts) SPB_CUDA(e, cudaMemcpyAsync(visit_counts, e->d_rc_counts, G * M * 4, cudaMemcpyDeviceToHost, e->stream));
-  if (child_ids) SPB_CUDA(e, cudaMemcpyAsync(child_ids, e->d_rc_ids, G * M * 4, cudaMemcpyDeviceToHost, e->stream));
-  if (n_children) SPB_CUDA(e, cudaMemcpyAsync(n_children, e->d_rc_n, G * 4, cudaMemcpyDeviceToHost, e->stream));
-  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
-  return SPB_OK;
+  return e->root_children(0, e->T.G, moves, visit_counts, child_ids, n_children, [e] { return fetch_root_children(e); });
 }
 
 int32_t spb_chess_root_children(spb_chess_engine* e, uint32_t slot, uint16_t* moves, uint32_t* visit_counts, uint32_t* child_ids, uint32_t* n_children) {
   SPB_GUARD(e);
-  SPB_ARG(e, slot < e->T.G, "slot out of range");
-  SPB_ARG(e, n_children, "null argument");
-  int32_t rc = fetch_root_children(e);
-  if (rc) return rc;
-  const size_t M = ch::MAX_MOVES;
-  if (moves) SPB_CUDA(e, cudaMemcpyAsync(moves, e->d_rc_moves + slot * M, M * 2, cudaMemcpyDeviceToHost, e->stream));
-  if (visit_counts) SPB_CUDA(e, cudaMemcpyAsync(visit_counts, e->d_rc_counts + slot * M, M * 4, cudaMemcpyDeviceToHost, e->stream));
-  if (child_ids) SPB_CUDA(e, cudaMemcpyAsync(child_ids, e->d_rc_ids + slot * M, M * 4, cudaMemcpyDeviceToHost, e->stream));
-  SPB_CUDA(e, cudaMemcpyAsync(n_children, e->d_rc_n + slot, 4, cudaMemcpyDeviceToHost, e->stream));
-  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
-  return SPB_OK;
+  return e->root_children(slot, 1, moves, visit_counts, child_ids, n_children, [e] { return fetch_root_children(e); });
 }
 
 // Policy of Mcts::search's result (mcts.rs:315-328): the root children's visit counts scattered into the 73x8x8 table by
@@ -879,9 +871,9 @@ int32_t spb_chess_root_policy(spb_chess_engine* e, uint32_t slot, float* out) {
 
 int32_t spb_chess_advance(spb_chess_engine* e, const uint32_t* slots, const uint32_t* child_ids, uint32_t n, spb_chess_state* out_states) {
   SPB_GUARD(e);
-  SPB_ARG(e, child_ids && n <= e->T.G, "bad argument");
+  SPB_ARG(e, child_ids, "null child_ids");
+  if (int32_t rc = e->check_slots(slots, n)) return rc;
   if (n == 0) return SPB_OK;
-  if (slots) for (uint32_t i = 0; i < n; ++i) SPB_ARG(e, slots[i] < e->T.G, "slot out of range");
   StageLayout L;
   const size_t o_slots = L.take(slots ? (size_t)n * 4 : 0), o_ids = L.take((size_t)n * 4), o_out = L.take((size_t)n * sizeof(ch::Pos)), o_err = L.take((size_t)n * 4);
   if (int32_t rc = e->ensure_stage(L.bytes, 0)) return rc;
@@ -891,9 +883,11 @@ int32_t spb_chess_advance(spb_chess_engine* e, const uint32_t* slots, const uint
   int32_t* d_err = e->d_at<int32_t>(o_err);
   if (slots) SPB_CUDA(e, cudaMemcpyAsync(d_slots, slots, (size_t)n * 4, cudaMemcpyHostToDevice, e->stream));
   SPB_CUDA(e, cudaMemcpyAsync(d_ids, child_ids, (size_t)n * 4, cudaMemcpyHostToDevice, e->stream));
-  ch::k_chess_advance<<<(n + ch::WARPS - 1) / ch::WARPS, ch::THREADS, 0, e->stream>>>(e->T, d_slots, d_ids, n, d_out, d_err);
+  SPB_CUDA(e, cudaMemsetAsync(e->d_misc, 0, 8, e->stream));
+  ch::k_chess_advance_check<<<(n + 127) / 128, 128, 0, e->stream>>>(e->T, d_slots, d_ids, n, d_err, e->d_misc);
+  ch::k_chess_advance<<<(n + ch::WARPS - 1) / ch::WARPS, ch::THREADS, 0, e->stream>>>(e->T, d_slots, d_ids, n, d_out, e->d_misc);
   SPB_CUDA(e, cudaGetLastError());
-  ++e->launches;
+  e->launches += 2;
   std::vector<int32_t> err(n);
   SPB_CUDA(e, cudaMemcpyAsync(err.data(), d_err, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
   if (out_states) SPB_CUDA(e, cudaMemcpyAsync(out_states, d_out, (size_t)n * sizeof(ch::Pos), cudaMemcpyDeviceToHost, e->stream));
@@ -957,7 +951,6 @@ int32_t spb_chess_node_stats(spb_chess_engine* e, uint32_t slot, uint32_t node_i
 int32_t spb_chess_selfplay_step(spb_chess_engine* e, int32_t rule, float temperature, uint64_t seed, const spb_chess_state* restart_roots,
                                 const uint64_t* restart_history, uint32_t* n_finished) {
   SPB_GUARD(e);
-  SPB_ARG(e, rule == SPB_MOVE_GREEDY_LAST_MAX || rule == SPB_MOVE_TEMPERATURE, "unknown move rule");
   SPB_ARG(e, !(restart_history && !restart_roots), "history without roots");
   const uint32_t G = e->T.G;
   ch::Pos* d_roots = nullptr; unsigned long long* d_hist = nullptr;
@@ -967,15 +960,9 @@ int32_t spb_chess_selfplay_step(spb_chess_engine* e, int32_t rule, float tempera
     rc = e->alloc_trajectories(SPB_CHESS_MAX_HISTORY);
     if (rc) return rc;
   }
-  SPB_CUDA(e, cudaMemsetAsync(e->P.finished, 0, 4, e->stream));
-  ch::k_chess_selfplay_step<<<(G + ch::WARPS - 1) / ch::WARPS, ch::THREADS, 0, e->stream>>>(e->T, e->P, rule, temperature, seed, d_roots, d_hist);
-  SPB_CUDA(e, cudaGetLastError());
-  ++e->launches;
-  uint32_t fin = 0;
-  SPB_CUDA(e, cudaMemcpyAsync(&fin, e->P.finished, 4, cudaMemcpyDeviceToHost, e->stream));
-  rc = e->check_device_errors();                                       // synchronises the stream
-  if (n_finished) *n_finished = fin;
-  return rc;
+  return e->selfplay_step(rule, n_finished, [&] {
+    ch::k_chess_selfplay_step<<<(G + ch::WARPS - 1) / ch::WARPS, ch::THREADS, 0, e->stream>>>(e->T, e->P, rule, temperature, seed, d_roots, d_hist);
+  });
 }
 
 int32_t spb_chess_drain_trajectories(spb_chess_engine* e, spb_chess_position* buf, size_t capacity, size_t* written, uint64_t* game_ids) {

@@ -22,7 +22,7 @@ struct Net;   // chess_net.cu
 // The self-play trajectories P are allocated by the first spb_chess_selfplay_step (an engine that never plays does not
 // pay for them); P.parked[g] = 1 | won << 1 | terminal side to move << 2 | adjudicated << 3.
 struct spb_chess_engine : spb::HostEngine<spb::chess::CTrees, spb_chess_position, uint16_t> {
-  spb_chess_engine() : HostEngine("spb_chess_") {}
+  spb_chess_engine() : HostEngine("spb_chess_", SPB_CHESS_MAX_MOVES) {}
   cudaStream_t stream2 = nullptr;   // the second half of the trees in the network pipeline
   cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
   spb::chess::Net* net = nullptr;

@@ -11,6 +11,11 @@ using namespace spb;
 
 thread_local std::string g_create_error;
 
+template <class G_> struct GameType { using type = G_; };
+// f(GameType<Connect4>) or f(GameType<TicTacToe>) for `game`; in f: using G = typename decltype(g)::type.
+template <class F> static auto with_game(int32_t game, F&& f) {
+  return game == SPB_GAME_CONNECT4 ? f(GameType<Connect4>{}) : f(GameType<TicTacToe>{});
+}
 
 int32_t spb_engine::init() {
   int32_t rc = open_device();
@@ -137,10 +142,10 @@ int32_t spb_engine::launch_eval_step(uint32_t parity) {
   if (cfg.evaluator == SPB_EVAL_NET) {
     SPB_CUDA(this, evaluator.launch(T.leaf_state, T.eval_list, &T.eval_count[parity & 1], slots, T.eval_out, G::EVAL_STRIDE, nullptr,
                                     (cfg.flags & SPB_FLAG_EVAL_SIMT) != 0, stream));
-  } else if (cfg.evaluator == SPB_EVAL_DET) {
-    k_eval_builtin<G, SPB_EVAL_DET><<<(slots + 255) / 256, 256, 0, stream>>>(T.leaf_state, T.eval_list, &T.eval_count[parity & 1], T.eval_out);
   } else {
-    k_eval_builtin<G, SPB_EVAL_UNIFORM><<<(slots + 255) / 256, 256, 0, stream>>>(T.leaf_state, T.eval_list, &T.eval_count[parity & 1], T.eval_out);
+    with_builtin_eval(cfg.evaluator, [&](auto ev) {
+      k_eval_builtin<G, decltype(ev)::value><<<(slots + 255) / 256, 256, 0, stream>>>(T.leaf_state, T.eval_list, &T.eval_count[parity & 1], T.eval_out);
+    });
   }
   ++launches;
   return SPB_OK;
@@ -180,8 +185,7 @@ int32_t spb_engine::search_t(uint32_t num_searches) {
     int32_t rc = search_async<G>(num_searches);
     if (rc != SPB_OK) return rc;
   } else if (!split) {
-    if (cfg.evaluator == SPB_EVAL_DET) k_search_fused<G, SPB_EVAL_DET><<<blocks, THREADS, 0, stream>>>(T, num_searches);
-    else k_search_fused<G, SPB_EVAL_UNIFORM><<<blocks, THREADS, 0, stream>>>(T, num_searches);
+    with_builtin_eval(cfg.evaluator, [&](auto ev) { k_search_fused<G, decltype(ev)::value><<<blocks, THREADS, 0, stream>>>(T, num_searches); });
     SPB_CUDA(this, cudaGetLastError());
     ++launches;
   } else if (T.K > 1) {
@@ -271,8 +275,9 @@ int32_t spb_engine::search_t(uint32_t num_searches) {
 // EXTENSION (DESIGN.md §4.6): eta of every live root into T.root_noise (k_root_noise).
 int32_t spb_engine::launch_root_noise() {
   const uint32_t blocks = (T.G + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK;
-  if (cfg.game == SPB_GAME_CONNECT4) k_root_noise<Connect4><<<blocks, THREADS, 0, stream>>>(T, P.game_id, noise_alpha, noise_seed);
-  else k_root_noise<TicTacToe><<<blocks, THREADS, 0, stream>>>(T, P.game_id, noise_alpha, noise_seed);
+  with_game(cfg.game, [&](auto g) {
+    k_root_noise<typename decltype(g)::type><<<blocks, THREADS, 0, stream>>>(T, P.game_id, noise_alpha, noise_seed);
+  });
   SPB_CUDA(this, cudaGetLastError());
   ++launches;
   return SPB_OK;
@@ -329,8 +334,7 @@ int32_t spb_engine::search_async(uint32_t num_searches) {
     ++last_eval_launches;
   } else {
     const uint32_t grid = std::max(1u, std::min(592u, (T.G + 3u) / 4u));
-    if (cfg.evaluator == SPB_EVAL_DET) k_async_builtin<G, SPB_EVAL_DET><<<grid, THREADS, 0, stream>>>(T, ctl);
-    else k_async_builtin<G, SPB_EVAL_UNIFORM><<<grid, THREADS, 0, stream>>>(T, ctl);
+    with_builtin_eval(cfg.evaluator, [&](auto ev) { k_async_builtin<G, decltype(ev)::value><<<grid, THREADS, 0, stream>>>(T, ctl); });
     SPB_CUDA(this, cudaGetLastError());
   }
   ++launches;
@@ -341,8 +345,6 @@ int32_t spb_engine::search_async(uint32_t num_searches) {
 // ------------------------------------------------------------------------------------------------
 // C ABI
 // ------------------------------------------------------------------------------------------------
-#define DISPATCH_GAME(e, CALL_C4, CALL_TTT) ((e)->cfg.game == SPB_GAME_CONNECT4 ? (CALL_C4) : (CALL_TTT))
-
 extern "C" {
 
 int32_t spb_abi_version(void) { return SPB_ABI_VERSION; }
@@ -420,9 +422,8 @@ int32_t spb_check_weights(int32_t game, const void* blob, size_t n, char* err, s
 
 int32_t spb_reset_games(spb_engine* e, const uint32_t* slots, uint32_t n, const spb_state* roots) {
   SPB_GUARD(e);
-  SPB_ARG(e, n <= e->T.G, "more slots than games");
+  if (int32_t rc = e->check_slots(slots, n)) return rc;
   if (n == 0) return SPB_OK;
-  if (slots) for (uint32_t i = 0; i < n; ++i) SPB_ARG(e, slots[i] < e->T.G, "slot out of range");
   StageLayout L;
   const size_t o_slots = L.take(slots ? (size_t)n * 4 : 0), o_roots = L.take(roots ? (size_t)n * sizeof(PState) : 0);
   if (int32_t rc = e->ensure_stage(L.bytes, L.bytes)) return rc;
@@ -442,7 +443,7 @@ int32_t spb_reset_games(spb_engine* e, const uint32_t* slots, uint32_t n, const 
 
 int32_t spb_search(spb_engine* e, uint32_t num_searches) {
   SPB_GUARD(e);
-  return DISPATCH_GAME(e, e->search_t<Connect4>(num_searches), e->search_t<TicTacToe>(num_searches));
+  return with_game(e->cfg.game, [&](auto g) { return e->search_t<typename decltype(g)::type>(num_searches); });
 }
 
 static int32_t fetch_root_children(spb_engine* e) {
@@ -454,45 +455,12 @@ static int32_t fetch_root_children(spb_engine* e) {
 
 int32_t spb_root_children_all(spb_engine* e, uint8_t* actions, uint32_t* visit_counts, uint32_t* child_ids, uint32_t* n_children) {
   SPB_GUARD(e);
-  int32_t rc = fetch_root_children(e);
-  if (rc) return rc;
-  const size_t G = e->T.G;
-  // one pinned staging area, one sync
-  StageLayout L;
-  const size_t o_counts = L.take(G * SPB_MAX_ACTIONS * 4), o_ids = L.take(G * SPB_MAX_ACTIONS * 4), o_n = L.take(G * 4), o_act = L.take(G * SPB_MAX_ACTIONS);
-  rc = e->ensure_stage(0, L.bytes);
-  if (rc) return rc;
-  auto* hs = e->h_at<uint8_t>(0);
-  if (visit_counts) SPB_CUDA(e, cudaMemcpyAsync(hs + o_counts, e->d_rc_counts, G * SPB_MAX_ACTIONS * 4, cudaMemcpyDeviceToHost, e->stream));
-  if (child_ids) SPB_CUDA(e, cudaMemcpyAsync(hs + o_ids, e->d_rc_ids, G * SPB_MAX_ACTIONS * 4, cudaMemcpyDeviceToHost, e->stream));
-  if (n_children) SPB_CUDA(e, cudaMemcpyAsync(hs + o_n, e->d_rc_n, G * 4, cudaMemcpyDeviceToHost, e->stream));
-  if (actions) SPB_CUDA(e, cudaMemcpyAsync(hs + o_act, e->d_rc_moves, G * SPB_MAX_ACTIONS, cudaMemcpyDeviceToHost, e->stream));
-  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
-  if (visit_counts) std::memcpy(visit_counts, hs + o_counts, G * SPB_MAX_ACTIONS * 4);
-  if (child_ids) std::memcpy(child_ids, hs + o_ids, G * SPB_MAX_ACTIONS * 4);
-  if (n_children) std::memcpy(n_children, hs + o_n, G * 4);
-  if (actions) std::memcpy(actions, hs + o_act, G * SPB_MAX_ACTIONS);
-  return SPB_OK;
+  return e->root_children(0, e->T.G, actions, visit_counts, child_ids, n_children, [e] { return fetch_root_children(e); });
 }
 
 int32_t spb_root_children(spb_engine* e, uint32_t slot, uint8_t* actions, uint32_t* visit_counts, uint32_t* child_ids, uint32_t* n_children) {
   SPB_GUARD(e);
-  SPB_ARG(e, slot < e->T.G, "slot out of range");
-  int32_t rc = fetch_root_children(e);
-  if (rc) return rc;
-  uint8_t a[SPB_MAX_ACTIONS]; uint32_t c[SPB_MAX_ACTIONS], ids[SPB_MAX_ACTIONS], n = 0;
-  SPB_CUDA(e, cudaMemcpyAsync(a, e->d_rc_moves + (size_t)slot * SPB_MAX_ACTIONS, SPB_MAX_ACTIONS, cudaMemcpyDeviceToHost, e->stream));
-  SPB_CUDA(e, cudaMemcpyAsync(c, e->d_rc_counts + (size_t)slot * SPB_MAX_ACTIONS, SPB_MAX_ACTIONS * 4, cudaMemcpyDeviceToHost, e->stream));
-  SPB_CUDA(e, cudaMemcpyAsync(ids, e->d_rc_ids + (size_t)slot * SPB_MAX_ACTIONS, SPB_MAX_ACTIONS * 4, cudaMemcpyDeviceToHost, e->stream));
-  SPB_CUDA(e, cudaMemcpyAsync(&n, e->d_rc_n + slot, 4, cudaMemcpyDeviceToHost, e->stream));
-  SPB_CUDA(e, cudaStreamSynchronize(e->stream));
-  for (uint32_t i = 0; i < n; ++i) {
-    if (actions) actions[i] = a[i];
-    if (visit_counts) visit_counts[i] = c[i];
-    if (child_ids) child_ids[i] = ids[i];
-  }
-  if (n_children) *n_children = n;
-  return SPB_OK;
+  return e->root_children(slot, 1, actions, visit_counts, child_ids, n_children, [e] { return fetch_root_children(e); });
 }
 
 int32_t spb_root_policy(spb_engine* e, uint32_t slot, float* policy) {
@@ -514,20 +482,13 @@ int32_t spb_root_policy(spb_engine* e, uint32_t slot, float* policy) {
 int32_t spb_advance(spb_engine* e, const uint32_t* slots, const uint32_t* node_ids, uint32_t n, spb_state* out_states) {
   SPB_GUARD(e);
   SPB_ARG(e, node_ids, "null node_ids");
-  SPB_ARG(e, n <= e->T.G, "more slots than games");
+  if (int32_t rc = e->check_slots(slots, n)) return rc;
   if (n == 0) return SPB_OK;
   // validate against arena lengths (one D2H of n_nodes)
   std::vector<uint32_t> nn(e->T.G);
   SPB_CUDA(e, cudaMemcpyAsync(nn.data(), e->T.n_nodes, (size_t)e->T.G * 4, cudaMemcpyDeviceToHost, e->stream));
   SPB_CUDA(e, cudaStreamSynchronize(e->stream));
-  std::vector<uint8_t> seen(e->T.G, 0);
-  for (uint32_t i = 0; i < n; ++i) {
-    uint32_t g = slots ? slots[i] : i;
-    SPB_ARG(e, g < e->T.G, "slot out of range");
-    SPB_ARG(e, !seen[g], "slot listed twice");
-    seen[g] = 1;
-    SPB_ARG(e, node_ids[i] < nn[g], "node id out of range");
-  }
+  for (uint32_t i = 0; i < n; ++i) SPB_ARG(e, node_ids[i] < nn[slots ? slots[i] : i], "node id out of range");
   StageLayout L;
   const size_t o_slots = L.take(slots ? (size_t)n * 4 : 0), o_ids = L.take((size_t)n * 4), o_out = L.take((size_t)n * sizeof(PState));
   if (int32_t rc = e->ensure_stage(L.bytes, L.bytes)) return rc;
@@ -538,8 +499,7 @@ int32_t spb_advance(spb_engine* e, const uint32_t* slots, const uint32_t* node_i
   const uint32_t* dsl = slots ? e->d_at<uint32_t>(o_slots) : nullptr;
   const uint32_t* dn = e->d_at<uint32_t>(o_ids);
   PState* dout = e->d_at<PState>(o_out);
-  if (e->cfg.game == SPB_GAME_CONNECT4) k_advance<Connect4><<<blocks, THREADS, 0, e->stream>>>(e->T, dsl, dn, n, dout);
-  else k_advance<TicTacToe><<<blocks, THREADS, 0, e->stream>>>(e->T, dsl, dn, n, dout);
+  with_game(e->cfg.game, [&](auto g) { k_advance<typename decltype(g)::type><<<blocks, THREADS, 0, e->stream>>>(e->T, dsl, dn, n, dout); });
   ++e->launches;
   SPB_CUDA(e, cudaGetLastError());
   SPB_CUDA(e, cudaMemcpyAsync(e->h_at<PState>(o_out), dout, (size_t)n * sizeof(PState), cudaMemcpyDeviceToHost, e->stream));
@@ -565,8 +525,7 @@ int32_t spb_get_state(spb_engine* e, uint32_t slot, uint32_t node_id, spb_state*
   SPB_ARG(e, node_id < len, "node id out of range");
   rc = e->ensure_stage(sizeof(PState), 0);
   if (rc) return rc;
-  if (e->cfg.game == SPB_GAME_CONNECT4) k_get_state<Connect4><<<1, 1, 0, e->stream>>>(e->T, slot, node_id, e->d_at<PState>(0));
-  else k_get_state<TicTacToe><<<1, 1, 0, e->stream>>>(e->T, slot, node_id, e->d_at<PState>(0));
+  with_game(e->cfg.game, [&](auto g) { k_get_state<typename decltype(g)::type><<<1, 1, 0, e->stream>>>(e->T, slot, node_id, e->d_at<PState>(0)); });
   ++e->launches;
   PState ps;
   SPB_CUDA(e, cudaGetLastError());
@@ -578,7 +537,7 @@ int32_t spb_get_state(spb_engine* e, uint32_t slot, uint32_t node_id, spb_state*
 
 int32_t spb_set_root_noise(spb_engine* e, float alpha, float epsilon, uint64_t seed) {
   SPB_GUARD(e);
-  const int32_t rc = e->set_root_noise(alpha, epsilon, seed, SPB_MAX_ACTIONS);
+  const int32_t rc = e->set_root_noise(alpha, epsilon, seed);
   // the captured step graph holds the previous Trees (and with it the noise settings): the next search captures anew
   if (rc == SPB_OK) e->drop_step_graph();
   return rc;
@@ -586,7 +545,7 @@ int32_t spb_set_root_noise(spb_engine* e, float alpha, float epsilon, uint64_t s
 
 int32_t spb_root_noise(spb_engine* e, uint32_t slot, float* eta, uint32_t* n) {
   SPB_GUARD(e);
-  return e->root_noise(slot, eta, n, SPB_MAX_ACTIONS, [e] { return e->launch_root_noise(); });
+  return e->root_noise(slot, eta, n, [e] { return e->launch_root_noise(); });
 }
 
 int32_t spb_node_stats(spb_engine* e, uint32_t slot, uint32_t node_id, uint32_t* visit_count, float* value_sum, float* prior,
@@ -642,10 +601,9 @@ static int32_t predict_t(spb_engine* e, const spb_state* states, uint32_t n, flo
     for (uint32_t i = 0; i < n; ++i) idl[i] = i;
     SPB_CUDA(e, cudaMemcpyAsync(dlog, idl.data(), (size_t)n * 4, cudaMemcpyHostToDevice, e->stream));
     SPB_CUDA(e, cudaStreamSynchronize(e->stream));
-    if (e->cfg.evaluator == SPB_EVAL_DET)
-      k_eval_builtin<G, SPB_EVAL_DET><<<(n + 255) / 256, 256, 0, e->stream>>>(dstates, reinterpret_cast<uint32_t*>(dlog), dcnt, dout);
-    else
-      k_eval_builtin<G, SPB_EVAL_UNIFORM><<<(n + 255) / 256, 256, 0, e->stream>>>(dstates, reinterpret_cast<uint32_t*>(dlog), dcnt, dout);
+    with_builtin_eval(e->cfg.evaluator, [&](auto ev) {
+      k_eval_builtin<G, decltype(ev)::value><<<(n + 255) / 256, 256, 0, e->stream>>>(dstates, reinterpret_cast<uint32_t*>(dlog), dcnt, dout);
+    });
     SPB_CUDA(e, cudaGetLastError());
   }
   ++e->launches;
@@ -666,8 +624,7 @@ int32_t spb_predict(spb_engine* e, const spb_state* states, uint32_t n, float* p
   SPB_GUARD(e);
   SPB_ARG(e, states || n == 0, "null states");
   if (n == 0) return SPB_OK;
-  return DISPATCH_GAME(e, predict_t<Connect4>(e, states, n, policies, values, raw_logits),
-                       predict_t<TicTacToe>(e, states, n, policies, values, raw_logits));
+  return with_game(e->cfg.game, [&](auto g) { return predict_t<typename decltype(g)::type>(e, states, n, policies, values, raw_logits); });
 }
 
 // ---- game rules ---------------------------------------------------------------------------------
@@ -689,10 +646,10 @@ int32_t spb_game_next_states(spb_engine* e, const spb_state* states, const uint8
   if (int32_t rc = upload_states(e, states, n, L.bytes, L.bytes)) return rc;
   std::memcpy(e->h_at<uint8_t>(o_act), actions, n);
   SPB_CUDA(e, cudaMemcpyAsync(e->d_stage, e->h_stage, o_out, cudaMemcpyHostToDevice, e->stream));   // the inputs: everything before o_out
-  if (e->cfg.game == SPB_GAME_CONNECT4)
-    k_game_next<Connect4><<<(n + 127) / 128, 128, 0, e->stream>>>(e->d_at<PState>(o_states), e->d_at<uint8_t>(o_act), n, e->d_at<PState>(o_out), e->d_at<int32_t>(o_err));
-  else
-    k_game_next<TicTacToe><<<(n + 127) / 128, 128, 0, e->stream>>>(e->d_at<PState>(o_states), e->d_at<uint8_t>(o_act), n, e->d_at<PState>(o_out), e->d_at<int32_t>(o_err));
+  with_game(e->cfg.game, [&](auto g) {
+    k_game_next<typename decltype(g)::type><<<(n + 127) / 128, 128, 0, e->stream>>>(e->d_at<PState>(o_states), e->d_at<uint8_t>(o_act), n, e->d_at<PState>(o_out),
+                                                                                   e->d_at<int32_t>(o_err));
+  });
   ++e->launches;
   SPB_CUDA(e, cudaGetLastError());
   SPB_CUDA(e, cudaMemcpyAsync(e->h_at<uint8_t>(o_out), e->d_at<uint8_t>(o_out), L.bytes - o_out, cudaMemcpyDeviceToHost, e->stream));   // states, errors
@@ -711,8 +668,9 @@ int32_t spb_game_valid_actions(spb_engine* e, const spb_state* states, uint32_t 
   const size_t o_states = L.take((size_t)n * sizeof(PState)), o_out = L.take((size_t)n * 4);
   if (int32_t rc = upload_states(e, states, n, L.bytes, o_out)) return rc;
   SPB_CUDA(e, cudaMemcpyAsync(e->d_stage, e->h_stage, o_out, cudaMemcpyHostToDevice, e->stream));
-  if (e->cfg.game == SPB_GAME_CONNECT4) k_game_valid<Connect4><<<(n + 127) / 128, 128, 0, e->stream>>>(e->d_at<PState>(o_states), n, e->d_at<uint32_t>(o_out));
-  else k_game_valid<TicTacToe><<<(n + 127) / 128, 128, 0, e->stream>>>(e->d_at<PState>(o_states), n, e->d_at<uint32_t>(o_out));
+  with_game(e->cfg.game, [&](auto g) {
+    k_game_valid<typename decltype(g)::type><<<(n + 127) / 128, 128, 0, e->stream>>>(e->d_at<PState>(o_states), n, e->d_at<uint32_t>(o_out));
+  });
   ++e->launches;
   SPB_CUDA(e, cudaGetLastError());
   SPB_CUDA(e, cudaMemcpyAsync(masks, e->d_at<uint32_t>(o_out), (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
@@ -724,14 +682,14 @@ int32_t spb_game_encode(spb_engine* e, const spb_state* states, uint32_t n, floa
   SPB_GUARD(e);
   SPB_ARG(e, states && out, "null argument");
   if (n == 0) return SPB_OK;
-  const bool c4 = e->cfg.game == SPB_GAME_CONNECT4;
-  const size_t total = (size_t)n * (c4 ? 3 * 6 * 7 : 27);
+  const size_t total = (size_t)n * (e->cfg.game == SPB_GAME_CONNECT4 ? 3 * 6 * 7 : 27);
   StageLayout L;
   const size_t o_states = L.take((size_t)n * sizeof(PState)), o_out = L.take(total * 4);
   if (int32_t rc = upload_states(e, states, n, L.bytes, o_out)) return rc;
   SPB_CUDA(e, cudaMemcpyAsync(e->d_stage, e->h_stage, o_out, cudaMemcpyHostToDevice, e->stream));
-  if (c4) k_game_encode<Connect4><<<(unsigned)((total + 255) / 256), 256, 0, e->stream>>>(e->d_at<PState>(o_states), n, e->d_at<float>(o_out));
-  else k_game_encode<TicTacToe><<<(unsigned)((total + 255) / 256), 256, 0, e->stream>>>(e->d_at<PState>(o_states), n, e->d_at<float>(o_out));
+  with_game(e->cfg.game, [&](auto g) {
+    k_game_encode<typename decltype(g)::type><<<(unsigned)((total + 255) / 256), 256, 0, e->stream>>>(e->d_at<PState>(o_states), n, e->d_at<float>(o_out));
+  });
   ++e->launches;
   SPB_CUDA(e, cudaGetLastError());
   SPB_CUDA(e, cudaMemcpyAsync(out, e->d_at<float>(o_out), total * 4, cudaMemcpyDeviceToHost, e->stream));
@@ -742,7 +700,6 @@ int32_t spb_game_encode(spb_engine* e, const spb_state* states, uint32_t n, floa
 // ---- self-play ----------------------------------------------------------------------------------
 int32_t spb_selfplay_step(spb_engine* e, int32_t rule, float temperature, uint64_t seed, const spb_state* restart_roots, uint32_t* n_finished) {
   SPB_GUARD(e);
-  SPB_ARG(e, rule == SPB_MOVE_GREEDY_LAST_MAX || rule == SPB_MOVE_TEMPERATURE, "unknown move rule");
   const uint32_t G = e->T.G;
   PState* droots = nullptr;
   if (restart_roots) {
@@ -751,17 +708,12 @@ int32_t spb_selfplay_step(spb_engine* e, int32_t rule, float temperature, uint64
     SPB_CUDA(e, cudaMemcpyAsync(e->d_stage, e->h_stage, bytes, cudaMemcpyHostToDevice, e->stream));
     droots = e->d_at<PState>(0);
   }
-  SPB_CUDA(e, cudaMemsetAsync(e->P.finished, 0, 4, e->stream));
   const uint32_t blocks = (G + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK;
-  if (e->cfg.game == SPB_GAME_CONNECT4) k_selfplay_step<Connect4><<<blocks, THREADS, 0, e->stream>>>(e->T, e->P, rule, temperature, seed, droots);
-  else k_selfplay_step<TicTacToe><<<blocks, THREADS, 0, e->stream>>>(e->T, e->P, rule, temperature, seed, droots);
-  ++e->launches;
-  uint32_t fin = 0;
-  SPB_CUDA(e, cudaGetLastError());
-  SPB_CUDA(e, cudaMemcpyAsync(&fin, e->P.finished, 4, cudaMemcpyDeviceToHost, e->stream));
-  int32_t rc = e->check_device_errors();
-  if (n_finished) *n_finished = fin;
-  return rc;
+  return e->selfplay_step(rule, n_finished, [&] {
+    with_game(e->cfg.game, [&](auto g) {
+      k_selfplay_step<typename decltype(g)::type><<<blocks, THREADS, 0, e->stream>>>(e->T, e->P, rule, temperature, seed, droots);
+    });
+  });
 }
 
 int32_t spb_drain_trajectories(spb_engine* e, spb_position* buf, size_t capacity, size_t* written, uint64_t* game_ids) {

@@ -27,7 +27,7 @@ using SelfPlay = Trajectories<spb_position>;
 // Members shared with the chess engine are in HostEngine (host_engine.hpp).
 struct spb_engine : spb::HostEngine<spb::Trees, spb_position, uint8_t> {
   using Evaluator = spb::Evaluator; using AsyncCtl = spb::AsyncCtl;
-  spb_engine() : HostEngine("spb_") {}
+  spb_engine() : HostEngine("spb_", SPB_MAX_ACTIONS) {}
   Evaluator evaluator;
   float last_eval_ms = 0.f;
   uint32_t last_eval_launches = 0;

@@ -9,6 +9,7 @@
 #include <initializer_list>
 #include <new>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include <cuda_runtime.h>
@@ -37,6 +38,12 @@ extern thread_local std::string g_create_error;   // text of the last failure th
 
 namespace spb {
 
+// f(std::integral_constant<int, SPB_EVAL_DET>) or f(…, SPB_EVAL_UNIFORM): a built-in evaluator as a compile-time constant
+// for the kernels templated on it.
+template <class F> auto with_builtin_eval(int32_t evaluator, F&& f) {
+  return evaluator == SPB_EVAL_DET ? f(std::integral_constant<int, SPB_EVAL_DET>{}) : f(std::integral_constant<int, SPB_EVAL_UNIFORM>{});
+}
+
 // Byte offsets of an entry point's arrays in the engine's stage: take(n) reserves the next n bytes, 16-byte aligned, and
 // returns their offset; `bytes` is what the stage must hold.
 struct StageLayout {
@@ -48,9 +55,10 @@ struct StageLayout {
 // whole-batch root query reports it (action index / chess move).
 template <class Trees, class Rec, class Move>
 struct HostEngine {
-  explicit HostEngine(const char* api_) : api(api_) {}
+  HostEngine(const char* api_, uint32_t row_) : api(api_), row(row_) {}
 
   const char* api;   // "spb_" / "spb_chess_": the prefix of this engine's entry points, for messages
+  uint32_t row;      // the width of a root's row of moves: SPB_MAX_ACTIONS / SPB_CHESS_MAX_MOVES
   spb_config cfg{};
   std::string err;
   Trees T{};
@@ -261,12 +269,25 @@ struct HostEngine {
     return SPB_OK;
   }
 
+  // The slot list of reset_games / advance (NULL: 0..n-1): SPB_ERR_ARG if it names more than G slots, a slot out of range
+  // or one slot twice (the kernel would rebuild that tree twice at once).
+  int32_t check_slots(const uint32_t* slots, uint32_t n) {
+    SPB_ARG(this, n <= T.G, "more slots than games");
+    if (!slots) return SPB_OK;
+    std::vector<uint8_t> seen(T.G, 0);
+    for (uint32_t i = 0; i < n; ++i) {
+      SPB_ARG(this, slots[i] < T.G, "slot out of range");
+      SPB_ARG(this, !seen[slots[i]], "slot listed twice");
+      seen[slots[i]] = 1;
+    }
+    return SPB_OK;
+  }
+
   // ---- bodies of the entry points both ABIs have (spb_X / spb_chess_X) ---------------------------------------------
-  // `row`: the width of a root's row of moves (SPB_MAX_ACTIONS / SPB_CHESS_MAX_MOVES).
 
   static const char* last_error(const HostEngine* e) { return e ? e->err.c_str() : g_create_error.c_str(); }
 
-  int32_t set_root_noise(float alpha, float epsilon, uint64_t seed, uint32_t row) {
+  int32_t set_root_noise(float alpha, float epsilon, uint64_t seed) {
     SPB_ARG(this, epsilon >= 0.0f && epsilon <= 1.0f, "root noise: epsilon must be in [0, 1]");
     SPB_ARG(this, epsilon == 0.0f || (alpha > 0.0f && alpha <= FLT_MAX), "root noise: alpha must be finite and > 0");
     if (epsilon > 0.0f && !d_noise_eta) {
@@ -286,7 +307,7 @@ struct HostEngine {
 
   // launch(): the engine's noise kernel, which draws eta of every live root into T.root_noise
   template <class Launch>
-  int32_t root_noise(uint32_t slot, float* eta, uint32_t* n, uint32_t row, Launch launch) {
+  int32_t root_noise(uint32_t slot, float* eta, uint32_t* n, Launch launch) {
     SPB_ARG(this, slot < T.G && eta && n, "bad argument");
     if (!T.root_noise) { set_error(std::string("root noise is off (") + api + "set_root_noise)"); return SPB_ERR_STATE; }
     int32_t rc = launch();
@@ -298,6 +319,22 @@ struct HostEngine {
     if (rc) return rc;
     for (uint32_t i = hn; i < row; ++i) eta[i] = 0.0f;
     *n = hn;
+    return SPB_OK;
+  }
+
+  // launch(): the engine's kernel that writes the root children of every slot, whole rows in child order, to d_rc_*.
+  // The rows of slots [first, first + rows) go straight into the caller's arrays (each may be NULL), then the stream is
+  // synchronised.
+  template <class Launch>
+  int32_t root_children(uint32_t first, uint32_t rows, Move* moves, uint32_t* counts, uint32_t* ids, uint32_t* n, Launch launch) {
+    SPB_ARG(this, first < T.G && rows <= T.G - first, "slot out of range");
+    if (int32_t rc = launch()) return rc;
+    const size_t off = (size_t)first * row, cells = (size_t)rows * row;
+    if (moves) SPB_CUDA(this, cudaMemcpyAsync(moves, d_rc_moves + off, cells * sizeof(Move), cudaMemcpyDeviceToHost, stream));
+    if (counts) SPB_CUDA(this, cudaMemcpyAsync(counts, d_rc_counts + off, cells * 4, cudaMemcpyDeviceToHost, stream));
+    if (ids) SPB_CUDA(this, cudaMemcpyAsync(ids, d_rc_ids + off, cells * 4, cudaMemcpyDeviceToHost, stream));
+    if (n) SPB_CUDA(this, cudaMemcpyAsync(n, d_rc_n + first, (size_t)rows * 4, cudaMemcpyDeviceToHost, stream));
+    SPB_CUDA(this, cudaStreamSynchronize(stream));
     return SPB_OK;
   }
 
@@ -339,6 +376,22 @@ struct HostEngine {
     SPB_CUDA(this, cudaStreamSynchronize(stream));
     launches = 0;
     return SPB_OK;
+  }
+
+  // A self-play step once the engine has staged its restart roots and has trajectory buffers: launch() enqueues the
+  // engine's self-play kernel; n_finished (nullable) receives the games it emitted.  Synchronises the stream.
+  template <class Launch>
+  int32_t selfplay_step(int32_t rule, uint32_t* n_finished, Launch launch) {
+    SPB_ARG(this, rule == SPB_MOVE_GREEDY_LAST_MAX || rule == SPB_MOVE_TEMPERATURE, "unknown move rule");
+    SPB_CUDA(this, cudaMemsetAsync(P.finished, 0, 4, stream));
+    launch();
+    SPB_CUDA(this, cudaGetLastError());
+    ++launches;
+    uint32_t fin = 0;
+    SPB_CUDA(this, cudaMemcpyAsync(&fin, P.finished, 4, cudaMemcpyDeviceToHost, stream));
+    const int32_t rc = check_device_errors();
+    if (n_finished) *n_finished = fin;
+    return rc;
   }
 
   // Copies the finished records out (buf == NULL: size query) and empties the output buffer.  Buffers not allocated yet

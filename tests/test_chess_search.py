@@ -263,8 +263,18 @@ def test_device_use_subtree_and_greedy_play_match_oracle():
                 want, _ = f.state(i, deep).export()
                 want.hist_len = ws.hist_len
                 assert got.tobytes() == bytes(want), (ply, i)
-        with pytest.raises(S.EngineError):
-            e.advance([0, 1, 1])                                   # node 0 is not a child of the root
+        # a call with one bad entry, or a slot listed twice, moves no tree
+        def snapshot():
+            return [(e.arena_len(i), tree_table_device(e, i), e.get_state(i, 0).tobytes()) for i in range(len(games))]
+        before = snapshot()
+        child = e.root_children(1)[2][0]
+        for call in (lambda: e.advance([0, 1, 1]),              # node 0 is not a child of the root
+                     lambda: e.advance([child, child], slots=[1, 1]),
+                     lambda: e.reset_games(st[:2], hist[:2], slots=[2, 2])):
+            with pytest.raises(S.EngineError) as ei:
+                call()
+            assert ei.value.code == -1
+            assert snapshot() == before
 
 
 @pytest.mark.gpu

@@ -112,6 +112,19 @@ def test_use_subtree_and_greedy_games_match_oracle(game):
                 f.reset([roots[s] for s in done], slots=done)
             if move > 12 and not nxt:
                 break
+        # a slot listed twice is refused before any tree is touched
+        e.search(sims)
+
+        def snapshot(s):
+            n = e.arena_len(s)
+            return n, [e.node_stats(s, i) for i in range(n)], [e.get_state(s, i).key() for i in range(n)]
+        before = snapshot(0)
+        child = e.root_children(0)[2][0]
+        for call in (lambda: e.advance([child, child], slots=[0, 0]), lambda: e.reset_games([roots[1], roots[2]], slots=[0, 0])):
+            with pytest.raises(S.EngineError) as ei:
+                call()
+            assert ei.value.code == -1
+            assert snapshot(0) == before
 
 
 def test_survey_greedy_game_800():
@@ -343,13 +356,35 @@ def test_gather_over_the_c_abi_with_one_rank_equals_drain():
 
 @pytest.mark.gpu
 def test_root_children_all_writes_into_caller_buffers():
-    """bench.py's end-to-end steps hand page-locked arrays to root_children_all(out=...): same numbers as a fresh call."""
-    with S.Engine(game=S.GAME_C4, num_games=16, evaluator=S.EVAL_DET) as e:
-        e.reset_games()
-        e.search(50)
-        fresh = e.root_children_all()
-        bufs = tuple(np.full_like(x, 0xFF) for x in fresh)
-        got = e.root_children_all(bufs)
-        assert all(g is b for g, b in zip(got, bufs))
-        for g, f in zip(got, fresh):
-            assert (g == f).all()
+    """bench.py's end-to-end steps hand page-locked arrays to root_children_all(out=...): same numbers as a fresh call,
+    into pageable and page-locked arrays.  Each row equals the per-slot call's, which writes whole rows (no move, count 0
+    and id 0 past n) and takes a NULL n_children.  For both engines; the odd slots hold no tree."""
+    import torch
+    keep = []
+
+    def pinned(x):
+        t = torch.empty(max(1, x.nbytes), dtype=torch.uint8, pin_memory=True)
+        keep.append(t)
+        out = t.numpy()[:x.nbytes].view(x.dtype).reshape(x.shape)
+        out[...] = 0xFF
+        return out
+    for make in (lambda: S.Engine(game=S.GAME_C4, num_games=16, evaluator=S.EVAL_DET),
+                 lambda: S.Engine(game=S.GAME_TTT, num_games=16, evaluator=S.EVAL_DET),
+                 lambda: S.ChessEngine(num_games=16, evaluator=S.EVAL_DET)):
+        with make() as e:
+            e.reset_games(slots=list(range(0, 16, 2)))
+            e.search(50)
+            fresh = e.root_children_all()
+            for bufs in (tuple(np.full_like(x, 0xFF) for x in fresh), tuple(pinned(x) for x in fresh)):
+                got = e.root_children_all(bufs)
+                assert all(g is b for g, b in zip(got, bufs))
+                for g, f in zip(got, fresh):
+                    assert (g == f).all()
+            mv, cnt, ids, n = fresh
+            assert n[0] > 0 and n[1] == 0
+            for slot in range(16):
+                row = [np.full_like(x[slot], 0xAB) for x in (mv, cnt, ids)]
+                e._chk(e._fn("root_children")(e._h, slot, *map(np.ctypeslib.as_ctypes, row), None))
+                assert all((r == x[slot]).all() for r, x in zip(row, (mv, cnt, ids)))
+                k = int(n[slot])
+                assert (row[0][k:] == np.iinfo(mv.dtype).max).all() and not row[1][k:].any() and not row[2][k:].any()
